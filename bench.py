@@ -21,8 +21,11 @@ one CUDA graph (plus the batch-wise test pass of mr_gan.py:219-223).  Folds shar
               cores busy -- the way a CPU user would run the sweep.  Keras 2.0.9 / Theano 0.9 cannot be installed here
               (SURVEY.md 8c).
   --workload table1 : the whole table-1 sweep (294 fold-trainings, 7 widths) through the drop-in's scheduler, wall clock.
+  --dump-outputs DIR : after the timed steps, what the last of them computed (see dump_outputs), so that two builds can be
+              compared output for output; the inputs depend only on the arguments.
 """
 import argparse
+import atexit
 import json
 import multiprocessing as mp
 import os
@@ -33,6 +36,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the source tree, which may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -62,7 +66,7 @@ def peaks():
 
 
 class ClockSampler:
-    """nvidia-smi clocks / throttle reasons during the timed region (B200_PROFILING.md recipe)."""
+    """nvidia-smi clocks / throttle reasons during the timed region (read-only queries, sampled every period_ms)."""
     Q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
          "clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,clocks_event_reasons.sw_power_cap")
 
@@ -70,23 +74,33 @@ class ClockSampler:
         self.gpu, self.period = gpu_index, period_ms
         self.rows = []
         self.proc = None
+        self.reader = None
 
     def start(self):
         try:
             self.proc = subprocess.Popen(["nvidia-smi", "--query-gpu=" + self.Q, "--format=csv,noheader,nounits",
                                           "-lms", str(self.period), "-i", str(self.gpu)], stdout=subprocess.PIPE, text=True)
-            threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
+            return
+        atexit.register(self._end)      # `nvidia-smi -lms` loops until killed: it must not outlive a run that fails
+        self.reader = threading.Thread(target=self._read, daemon=True)
+        self.reader.start()
 
     def _read(self):
         for line in self.proc.stdout:
             self.rows.append([c.strip() for c in line.split(",")])
 
+    def _end(self):
+        if self.proc.poll() is None:
+            self.proc.terminate()
+        self.proc.wait()
+        self.reader.join(timeout=5)
+
     def stop(self):
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"], "samples": 0}
-        self.proc.terminate()
+        self._end()
         sm, mx, reasons = [], [], set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         for r in self.rows:
@@ -118,6 +132,22 @@ def make_jobs(D_modality, n_folds, seed):
                 folds.append((foldprep.prepare_fold_indices(y, tr, te, percents[k % len(percents)], None, rng), rng))
         k += 1
     return X, y.astype(np.int32), folds
+
+
+DUMP_PARAM_VALUES = 1 << 23     # trained parameter values --dump-outputs writes (32 MB of float32), over all folds and both nets
+
+
+def dump_outputs(path, fg, stats):
+    """What a train_epoch caller receives from the last timed step, as float32 .npy files: epoch_stats [folds, 5] (loss_lab,
+    loss_unl, train_err, loss_gen, test_err, as returned), and disc_params / gen_params [folds, k]: every fold's trained
+    weights at k flat positions (reference weight order) drawn once from a fixed seed -- one fold's weights alone are 11 MB at D=1200."""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "epoch_stats.npy"), np.asarray(stats, dtype=np.float32))
+    for net, name in ((0, "disc_params"), (1, "gen_params")):
+        n = fg.num_params(0, net)                   # every fold of the group has the same width
+        pick = np.sort(np.random.default_rng(net).choice(n, min(n, DUMP_PARAM_VALUES // (2 * fg.n_folds)), replace=False))
+        rows = [np.concatenate([p.ravel() for p in fg.get_params(i, net)])[pick] for i in range(fg.n_folds)]
+        np.save(os.path.join(path, name + ".npy"), np.stack(rows).astype(np.float32))
 
 
 # ------------------------------------------------------------------ CPU arm (the oracle's torch twin; test infrastructure
@@ -379,7 +409,13 @@ def main():
     ap.add_argument("--dp-width", type=int, default=12032, help="input width of the dp workload (1 s contact mic, table 5)")
     ap.add_argument("--epochs", type=int, default=100, help="table1 workload: epochs per fold")
     ap.add_argument("--group", type=int, default=84, help="table1 workload: largest number of folds per handle")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="sweep workload: write what the last timed step computed to DIR/*.npy "
+                                                          "(rank 0's folds; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "sweep"):
+        ap.error("--dump-outputs applies to the sweep workload of the b200 arm")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -452,6 +488,8 @@ def main():
     barrier()
     wall1 = time.perf_counter() - t0
     launches = fg.kernel_launches - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fg, st)
     # ---- region 2: end to end through the host API -----------------------------------------
     barrier()
     t0 = time.perf_counter()
