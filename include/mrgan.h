@@ -5,7 +5,8 @@
  *   the three opaque callables that Keras builds with K.function at
  *   mr_gan.py:169-171 (train_batch_disc / train_batch_gen / test_batch), the
  *   inner epoch loop that drives them (mr_gan.py:183-230) and mr_nn's
- *   model.fit / model.evaluate pair (mr_nn.py:114-118).  SURVEY.md section 8(b).
+ *   model.fit / model.evaluate pair (mr_nn.py:114-118).  SURVEY.md section 8(b).  mr_svm.py's
+ *   SVC(kernel='rbf', C).fit / .predict (mr_svm.py:106) on the same resident fold data.
  *
  * Conventions
  *   - plain C types only; every matrix is row-major float32, labels/indices int32;
@@ -46,7 +47,8 @@ typedef enum {
 
 enum { MRGAN_NET_D = 0, MRGAN_NET_G = 1 };
 enum { MRGAN_MODEL_GAN = 0,   /* mr_gan.py: G + D, feature matching          */
-       MRGAN_MODEL_NN = 1 };  /* mr_nn.py: D as a plain classifier, MSE loss */
+       MRGAN_MODEL_NN = 1,    /* mr_nn.py: D as a plain classifier, MSE loss */
+       MRGAN_MODEL_SVM = 2 }; /* mr_svm.py: RBF C-SVC, one-vs-one (fold data + SVM workspace only: no nets) */
 enum { MRGAN_PREC_FP32 = 0,   /* FFMA kernels, fp32 operands (parity mode)                  */
        MRGAN_PREC_TF32 = 1,   /* tcgen05 kind::tf32 tensor-core kernels, fp32 accumulate    */
        MRGAN_PREC_F16 = 2 };  /* tcgen05 kind::f16 on 16-bit operand COPIES: fp16 weights and activations (the same
@@ -180,6 +182,15 @@ int  mrnn_train_epoch(mrgan_handle* h, const int32_t* idx, int n_idx, float* los
 /* model.evaluate(X_test, y_test) -> {mse loss, accuracy} */
 int  mrnn_evaluate(mrgan_handle* h, int fold, float out[2]);
 
+/* mr_svm.py:106 SVC(kernel='rbf', C).fit(x_labeled, y_labeled) for ALL folds of the handle (created with MRGAN_MODEL_SVM),
+ * libsvm's solver (sklearn/svm/src/libsvm/svm.cpp) without shrinking; then the prediction of every fold's full resident X_test.
+ *   lab_rows [n_folds][n_lab]: rows of the resident X_train, class-major (labels non-decreasing); gamma [n_folds];
+ *   tol: libsvm eps.  A class pair has at most 8192 rows.
+ *   n_iter [n_folds][K(K-1)/2] or NULL; returns MRGAN_ERR_STATE if a pair hit the iteration cap max(1e7, 100 n). */
+int  mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, const float* gamma, float tol, int32_t* n_iter);
+int  mrgan_svm_eval(mrgan_handle* h, int fold, float* err);                 /* full resident X_test, ovo vote */
+int  mrgan_svm_decision(mrgan_handle* h, int fold, float* dst);             /* test hook: [n_test][K(K-1)/2] */
+
 /* Utilities used by tests and bench */
 int  mrgan_fill_normal(mrgan_handle* h, int fold, int step, int tensor_id, int rows, int cols,
                        int row0, float* dst /* host [rows, cols] */);
@@ -190,12 +201,17 @@ int  mrgan_adam_flat(mrgan_handle* h, float* p, float* m, float* v, const float*
  * Mutates the training state (run it after the measured region). */
 enum { MRGAN_TIME_ADAM_D = 0, MRGAN_TIME_ADAM_G = 1, MRGAN_TIME_DW1 = 2, MRGAN_TIME_FWD1 = 3,
        MRGAN_TIME_DISC_STEP = 4, MRGAN_TIME_GEN_STEP = 5,
-       MRGAN_TIME_DX1 = 6 };   /* dFake = dZ1 W1^T of the generator step: the dX pass over the widest layer */
+       MRGAN_TIME_DX1 = 6,     /* dFake = dZ1 W1^T of the generator step: the dX pass over the widest layer */
+       /* SVM handles, after mrgan_svm_fit (re-running a phase reproduces its results bitwise): */
+       MRGAN_TIME_SVM_KMAT = 7,     /* both kernel matrices of all folds (operand split + tcgen05 GEMM + RBF) */
+       MRGAN_TIME_SVM_SMO = 8,      /* the SMO solver of every (fold, class pair) */
+       MRGAN_TIME_SVM_PREDICT = 9 };/* decision values, vote and error count of every test row */
 int  mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg);
 /* Debug/test hook: copy an intermediate buffer of the last step of one fold to the host
  * (dst is [rows, cols] dense).  which: 0..5 = noisy layer inputs a[l], 10+l = post-ReLU h[l],
  * 20+l = dZ[l], 30 = logits, 31 = dlogits, 32 = dFake, 40 = z, 41 = G h1, 42 = G BN out,
- * 43 = G h2, 44 = G dZ2, 45 = G dU, 46 = G dZ1, 50 = resident X_train, 51 = resident X_test. */
+ * 43 = G h2, 44 = G dZ2, 45 = G dU, 46 = G dZ1, 50 = resident X_train, 51 = resident X_test;
+ * SVM handles after mrgan_svm_fit: 60 = labeled x labeled kernel matrix [n_lab][n_lab], 61 = test x labeled [n_test][n_lab]. */
 int  mrgan_debug_buffer(mrgan_handle* h, int fold, int which, float* dst, int rows, int cols);
 /* Test hook: one stand-alone GEMM through the step's kernels (use_tc = 1: tcgen05 path, 0: fp32 path).
  * mode 0: C[M,N] = A[M,K] B[K,N]   mode 1: C[M,N] = A[M,K] B[N,K]^T   mode 2: C[M,N] = A[K,M]^T B[K,N]

@@ -8,6 +8,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
 #include <map>
 #include <string>
 #include <vector>
@@ -16,6 +17,7 @@
 #include "kernels_simt.cuh"
 #ifdef MRGAN_WITH_TC
 #include "kernels_tc.cuh"
+#include "kernels_svm.cuh"
 #endif
 #include "kernels_dp.cuh"
 
@@ -153,6 +155,18 @@ struct mrgan_handle {
                                       // 8 = HEAD_BN_BWD (no k_bn_bwd); 2 and 8 together also retire the generator's k_adam
   TcAdamOp* d_tcadam = nullptr;       // [NUM_OPS][nf]
   AdamRange* d_ranges_tc[2] = {nullptr, nullptr};   // what is left for k_adam: BN gamma/beta (G), nothing (D)
+  // MRGAN_MODEL_SVM: workspace of mrgan_svm_fit (one allocation, reused while it is large enough)
+  struct Svm {
+    char* mem = nullptr; size_t bytes = 0;
+    int n_lab = 0, npairs = 0, npmax = 0, max_rows = 0, max_nte = 0;
+    double C = 1.0, eps = 1e-3;
+    bool fitted = false;
+    std::vector<float*> Klab, Kte, dec;
+    std::vector<int*> wrong;
+    int *d_iters = nullptr, *d_capped = nullptr, *d_count = nullptr, *d_nte = nullptr;
+    SvmSplitOp* d_split = nullptr; SvmGemmOp* d_gemm = nullptr; SvmPairJob* d_jobs = nullptr;
+    float** d_Kt = nullptr; float** d_dec = nullptr; int** d_yte = nullptr; int** d_wrong = nullptr;
+  } svm;
 #endif
 };
 
@@ -240,6 +254,18 @@ void layout_buffers(mrgan_handle* h, Arena& ar) {
   const mrgan_config& c = h->cfg;
   const int B = c.batch, R = h->R, NE = h->NE, K = c.n_classes, nd = c.noise_dim, nf = h->nf;
   const bool gan = c.model == MRGAN_MODEL_GAN;
+  if (c.model == MRGAN_MODEL_SVM) {     // fold data only (what mrgan_load_fold / mrgan_prepare_fold write)
+    for (int f = 0; f < nf; ++f) {
+      FoldBuffers& b = h->fb[f];
+      const int D = h->shapes[f].D;
+      b.lda[0] = pitch8(D + 1);
+      b.xte = ar.take<float>((size_t)h->shapes[f].n_test * b.lda[0]);
+      b.xtr = ar.take<float>((size_t)h->shapes[f].n_train * pitch8(D));
+      b.ytr = ar.take<int>(h->shapes[f].n_train);
+      b.yte = ar.take<int>(h->shapes[f].n_test);
+    }
+    return;
+  }
   h->P = ar.take<float>(h->n_flat);
   h->Mo = ar.take<float>(h->n_flat);
   h->Vo = ar.take<float>(h->n_flat);
@@ -862,6 +888,13 @@ int check_fold(mrgan_handle* h, int fold) {
   return MRGAN_OK;
 }
 
+// GAN / NN entry points: an SVM handle has no nets
+int need_nets(mrgan_handle* h, const char* fn) {
+  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  if (h->cfg.model == MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, std::string(fn) + ": not available on an SVM handle");
+  return MRGAN_OK;
+}
+
 int finish_pending(mrgan_handle* h) {
   if (h->epoch_pending) {
     CK(cudaStreamSynchronize(h->stream));
@@ -1389,7 +1422,9 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
   *out = nullptr;
   if (cfg->n_folds < 1 || cfg->batch < 1 || cfg->n_classes < 2 || cfg->n_classes > 64 || cfg->noise_dim < 1)
     return fail(nullptr, MRGAN_ERR_ARG, "bad config (n_folds/batch/n_classes/noise_dim)");
-  if (cfg->model != MRGAN_MODEL_GAN && cfg->model != MRGAN_MODEL_NN) return fail(nullptr, MRGAN_ERR_ARG, "bad model");
+  if (cfg->model != MRGAN_MODEL_GAN && cfg->model != MRGAN_MODEL_NN && cfg->model != MRGAN_MODEL_SVM) return fail(nullptr, MRGAN_ERR_ARG, "bad model");
+  if (cfg->model == MRGAN_MODEL_SVM && cfg->precision != MRGAN_PREC_FP32)
+    return fail(nullptr, MRGAN_ERR_ARG, "bad config: the SVM has one arithmetic path (precision must be MRGAN_PREC_FP32)");
   if (cfg->batch > (1 << 16)) return fail(nullptr, MRGAN_ERR_ARG, "batch too large");
   if ((cfg->hidden_act != MRGAN_ACT_RELU && cfg->hidden_act != MRGAN_ACT_LEAKY_RELU) || !(cfg->dropout >= 0.0f && cfg->dropout < 1.0f))
     return fail(nullptr, MRGAN_ERR_ARG, "bad config (hidden_act / dropout)");
@@ -1426,7 +1461,7 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
   if (cudaSetDevice(cfg->device) != cudaSuccess) return cleanup(fail(nullptr, MRGAN_ERR_CUDA, "cudaSetDevice failed"));
   // flat parameter space: all D nets, then all G nets
   long long off = 0;
-  for (int n = 0; n < (cfg->model == MRGAN_MODEL_GAN ? 2 : 1); ++n) {
+  for (int n = 0; n < (cfg->model == MRGAN_MODEL_GAN ? 2 : (cfg->model == MRGAN_MODEL_NN ? 1 : 0)); ++n) {
     h->net[n].resize(h->nf);
     for (int f = 0; f < h->nf; ++f) {
       NetLayout L = n == 0 ? layout_disc(folds[f].D, cfg->n_classes) : layout_gen(folds[f].D, cfg->noise_dim);
@@ -1487,8 +1522,10 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
     ok = ok && cudaEventCreateWithFlags(&h->idx_free[s], cudaEventDisableTiming) == cudaSuccess;
   }
   if (!ok) return cleanup(fail(nullptr, MRGAN_ERR_CUDA, "stream/event/pinned allocation failed"));
-  { const int rc = build_descs(h); if (rc != MRGAN_OK) return cleanup(rc); }
-  init_ones(h);
+  if (cfg->model != MRGAN_MODEL_SVM) {
+    const int rc = build_descs(h); if (rc != MRGAN_OK) return cleanup(rc);
+    init_ones(h);
+  }
   if (cfg->model == MRGAN_MODEL_GAN && cfg->batch > 256) {   // large batch: row-parallel split BatchNorm / feature-matching kernels
     int rc = alloc_split_bufs(h);
     if (rc != MRGAN_OK) return cleanup(rc);
@@ -1524,6 +1561,7 @@ int mrgan_destroy(mrgan_handle* h) {
   if (h->d_dpbufs) cudaFree(h->d_dpbufs);
 #ifdef MRGAN_WITH_TC
   tc_teardown(h);
+  if (h->svm.mem) cudaFree(h->svm.mem);
 #endif
   if (h->arena) cudaFree(h->arena);
   if (h->harena) cudaFree(h->harena);
@@ -1558,7 +1596,7 @@ int64_t mrgan_num_params(const mrgan_handle* h, int fold, int net) {
 }
 
 int mrgan_set_params(mrgan_handle* h, int fold, int net, const float* src, int64_t n) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "set_params"); if (rc) return rc;
   if (net < 0 || net > 1 || h->net[net].empty()) return fail(h, MRGAN_ERR_ARG, "no such net in this model");
   const NetLayout& L = h->net[net][fold];
   if (!src || n != L.n_ref) return fail(h, MRGAN_ERR_ARG, "set_params: length does not match mrgan_num_params");
@@ -1589,7 +1627,7 @@ static int get_flat(mrgan_handle* h, int fold, int net, const float* dev, float*
 }
 
 int mrgan_get_params(mrgan_handle* h, int fold, int net, float* dst, int64_t n) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "get_params"); if (rc) return rc;
   if (net < 0 || net > 1 || h->net[net].empty()) return fail(h, MRGAN_ERR_ARG, "no such net in this model");
   CK(cudaSetDevice(h->cfg.device));
   rc = finish_pending(h); if (rc) return rc;
@@ -1597,7 +1635,7 @@ int mrgan_get_params(mrgan_handle* h, int fold, int net, float* dst, int64_t n) 
 }
 
 int mrgan_get_adam(mrgan_handle* h, int fold, int net, float* m, float* v, int64_t n) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "get_adam"); if (rc) return rc;
   if (net < 0 || net > 1 || h->net[net].empty()) return fail(h, MRGAN_ERR_ARG, "no such net in this model");
   CK(cudaSetDevice(h->cfg.device));
   rc = finish_pending(h); if (rc) return rc;
@@ -1606,7 +1644,7 @@ int mrgan_get_adam(mrgan_handle* h, int fold, int net, float* m, float* v, int64
 }
 
 int mrgan_get_counters(mrgan_handle* h, int fold, int* iterations, int* rng_step) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "get_counters"); if (rc) return rc;
   CK(cudaSetDevice(h->cfg.device));
   rc = finish_pending(h); if (rc) return rc;
   FoldState fs;
@@ -1751,7 +1789,7 @@ int mrgan_gen_step(mrgan_handle* h, int fold, const float* x_unl, const float* z
 }
 
 int mrgan_test_batch(mrgan_handle* h, int fold, const float* x, const int32_t* y, int n, float* err) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "test_batch"); if (rc) return rc;
   if (!x || !y || !err) return fail(h, MRGAN_ERR_ARG, "test_batch: null pointer");
   if (n < 1 || n > h->NE) return fail(h, MRGAN_ERR_ARG, "test_batch: n exceeds max(n_test, rows of a train step)");
   for (int i = 0; i < n; ++i)
@@ -1779,7 +1817,7 @@ int mrgan_test_batch(mrgan_handle* h, int fold, const float* x, const int32_t* y
 }
 
 int mrgan_eval(mrgan_handle* h, int fold, float* err) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "eval"); if (rc) return rc;
   if (!err) return fail(h, MRGAN_ERR_ARG, "eval: null pointer");
   if (!h->fb[fold].loaded) return fail(h, MRGAN_ERR_STATE, "eval before mrgan_load_fold");
   CK(cudaSetDevice(h->cfg.device));
@@ -1794,6 +1832,7 @@ int mrgan_eval(mrgan_handle* h, int fold, float* err) {
 
 int mrgan_epoch_result(mrgan_handle* h, mrgan_epoch_stats* stats) {
   if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  { const int rc0 = need_nets(h, "epoch_result"); if (rc0) return rc0; }
   CK(cudaSetDevice(h->cfg.device));
   int rc = finish_pending(h); if (rc) return rc;
   CKS();
@@ -1846,7 +1885,7 @@ int mrgan_train_epoch_seeded(mrgan_handle* h, uint32_t epoch, mrgan_epoch_stats*
 }
 
 int mrgan_debug_epoch_indices(mrgan_handle* h, int fold, int32_t* dst) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "debug_epoch_indices"); if (rc) return rc;
   if (!dst) return fail(h, MRGAN_ERR_ARG, "debug_epoch_indices: null pointer");
   CK(cudaSetDevice(h->cfg.device));
   rc = finish_pending(h); if (rc) return rc;
@@ -1952,7 +1991,7 @@ int mrnn_train_epoch(mrgan_handle* h, const int32_t* idx, int n_idx, float* loss
 }
 
 int mrnn_evaluate(mrgan_handle* h, int fold, float out[2]) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "evaluate"); if (rc) return rc;
   if (!out) return fail(h, MRGAN_ERR_ARG, "evaluate: null pointer");
   if (!h->fb[fold].loaded) return fail(h, MRGAN_ERR_STATE, "evaluate before mrgan_load_fold");
   CK(cudaSetDevice(h->cfg.device));
@@ -1966,7 +2005,7 @@ int mrnn_evaluate(mrgan_handle* h, int fold, float out[2]) {
 }
 
 int mrgan_fill_normal(mrgan_handle* h, int fold, int step, int tensor_id, int rows, int cols, int row0, float* dst) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "fill_normal"); if (rc) return rc;
   if (!dst || rows < 1 || cols < 1) return fail(h, MRGAN_ERR_ARG, "fill_normal: bad argument");
   CK(cudaSetDevice(h->cfg.device));
   rc = finish_pending(h); if (rc) return rc;
@@ -1984,6 +2023,7 @@ int mrgan_fill_normal(mrgan_handle* h, int fold, int step, int tensor_id, int ro
 
 int mrgan_adam_flat(mrgan_handle* h, float* p, float* m, float* v, const float* g, int64_t n, int t) {
   if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  { const int rc0 = need_nets(h, "adam_flat"); if (rc0) return rc0; }
   if (!p || !m || !v || !g || n < 1 || t < 1) return fail(h, MRGAN_ERR_ARG, "adam_flat: bad argument");
   CK(cudaSetDevice(h->cfg.device));
   int rc = finish_pending(h); if (rc) return rc;
@@ -2012,9 +2052,15 @@ int mrgan_adam_flat(mrgan_handle* h, float* p, float* m, float* v, const float* 
   return MRGAN_OK;
 }
 
+static int svm_time_op(mrgan_handle* h, int which, int reps, float* ms_avg);
+
 int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
   if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
   if (!ms_avg || reps < 1) return fail(h, MRGAN_ERR_ARG, "time_op: bad argument");
+  const bool svm = h->cfg.model == MRGAN_MODEL_SVM;
+  if (svm != (which >= MRGAN_TIME_SVM_KMAT && which <= MRGAN_TIME_SVM_PREDICT))
+    return fail(h, which < 0 || which > MRGAN_TIME_SVM_PREDICT ? MRGAN_ERR_ARG : MRGAN_ERR_STATE, "time_op: op does not exist for this model");
+  if (svm) return svm_time_op(h, which, reps, ms_avg);
   const bool gan = h->cfg.model == MRGAN_MODEL_GAN;
   if (!gan && (which == MRGAN_TIME_ADAM_G || which == MRGAN_TIME_GEN_STEP || which == MRGAN_TIME_DX1)) return fail(h, MRGAN_ERR_STATE, "time_op: no generator in this model");
   for (int f = 0; f < h->nf; ++f)
@@ -2166,6 +2212,16 @@ int mrgan_debug_buffer(mrgan_handle* h, int fold, int which, float* dst, int row
   const int K = h->cfg.n_classes, D = h->shapes[fold].D, nd = h->cfg.noise_dim;
   const bool gan = h->cfg.model == MRGAN_MODEL_GAN;
   const float* src = nullptr; int ld = 0;
+  if (h->cfg.model == MRGAN_MODEL_SVM) {
+    if (which != 50 && which != 51 && which != 60 && which != 61) return fail(h, MRGAN_ERR_STATE, "debug_buffer: an SVM handle has fold data and kernel matrices only");
+#ifdef MRGAN_WITH_TC
+    if (which >= 60) {
+      if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "debug_buffer: kernel matrices before mrgan_svm_fit");
+      if (rows > (which == 60 ? h->svm.n_lab : h->shapes[fold].n_test)) return fail(h, MRGAN_ERR_ARG, "debug_buffer: too many rows");
+      src = which == 60 ? h->svm.Klab[fold] : h->svm.Kte[fold]; ld = h->svm.n_lab;
+    }
+#endif
+  }
   if (which >= 0 && which <= 5) { src = b.a[which]; ld = b.lda[which]; }
   else if (which >= 11 && which <= 15) { src = b.hb[which - 10]; ld = b.lda[which - 10]; }
   else if (which >= 21 && which <= 25) { src = b.dz[which - 20]; ld = b.ldz[which - 20]; }
@@ -2208,6 +2264,7 @@ int mrgan_debug_buffer(mrgan_handle* h, int fold, int which, float* dst, int row
 
 int mrgan_debug_gemm(mrgan_handle* h, int mode, int M, int N, int K, const float* A, const float* B, float* C, int use_tc) {
   if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  { const int rc0 = need_nets(h, "debug_gemm"); if (rc0) return rc0; }
   if (mode < 0 || mode > 2 || M < 1 || N < 1 || K < 1 || !A || !B || !C) return fail(h, MRGAN_ERR_ARG, "debug_gemm: bad argument");
   CK(cudaSetDevice(h->cfg.device));
   int rc = finish_pending(h); if (rc) return rc;
@@ -2265,6 +2322,7 @@ int mrgan_debug_gemm(mrgan_handle* h, int mode, int M, int N, int K, const float
 
 int mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int groups, int reps, float* ms) {
   if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  { const int rc0 = need_nets(h, "debug_gemm_time"); if (rc0) return rc0; }
   if (mode < 0 || mode > 2 || M < 1 || N < 1 || K < 1 || groups < 1 || reps < 1 || !ms) return fail(h, MRGAN_ERR_ARG, "debug_gemm_time: bad argument");
 #ifndef MRGAN_WITH_TC
   return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
@@ -2310,6 +2368,221 @@ int mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int gr
   *ms = t_ms / reps;
   h->launches += reps + 1;
   cudaFree(buf); cudaFree(dops);
+  return MRGAN_OK;
+#endif
+}
+
+
+// ------------------------------------------------------------------ RBF C-SVC (MRGAN_MODEL_SVM, csrc/kernels_svm.cuh)
+#ifdef MRGAN_WITH_TC
+static void svm_launch(mrgan_handle* h, int phase) {
+  mrgan_handle::Svm& S = h->svm;
+  const int nf = h->nf;
+  if (phase == MRGAN_TIME_SVM_KMAT) {
+    k_svm_split<<<dim3((S.max_rows + 7) / 8, 2 * nf), 256, 0, h->stream>>>(S.d_split);
+    k_svm_kmat<<<dim3((S.n_lab + SVM_BM - 1) / SVM_BM, (S.max_rows + SVM_BN - 1) / SVM_BN, 2 * nf), SVM_KMAT_THREADS, SVM_KMAT_SMEM,
+                 h->stream>>>(S.d_gemm);
+    h->launches += 2;
+  } else if (phase == MRGAN_TIME_SVM_SMO) {
+    k_svm_smo<<<nf * S.npairs, SVM_SMO_THREADS, (size_t)20 * S.npmax, h->stream>>>(S.d_jobs, S.C, S.eps);
+    h->launches += 1;
+  } else {
+    k_svm_vote<<<dim3(S.max_nte, nf), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs, S.npairs, h->cfg.n_classes, S.d_Kt, S.d_yte, S.d_nte,
+                                                                         S.d_dec, S.d_wrong);
+    k_svm_count<<<nf, 256, 0, h->stream>>>(S.d_wrong, S.d_nte, S.d_count);
+    h->launches += 2;
+  }
+}
+#endif
+
+int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, const float* gamma, float tol, int32_t* n_iter) {
+  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_fit needs an SVM handle");
+#ifndef MRGAN_WITH_TC
+  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
+#else
+  if (!lab_rows || !gamma || n_lab < 2 || !(C > 0.0f) || !(tol > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_fit: bad argument");
+  const int nf = h->nf, K = h->cfg.n_classes, npairs = K * (K - 1) / 2;
+  for (int f = 0; f < nf; ++f)
+    if (!(gamma[f] > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_fit: gamma must be positive");
+  for (int f = 0; f < nf; ++f)
+    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "svm_fit before the fold data is loaded (mrgan_load_fold / mrgan_prepare_fold)");
+  CK(cudaSetDevice(h->cfg.device));
+  int rc = finish_pending(h); if (rc) return rc;
+  // class-major labeled rows: class c is the segment [start[f][c], start[f][c] + cnt[f][c])
+  std::vector<int> ytr(h->n_train), start((size_t)nf * K), cnt((size_t)nf * K, 0);
+  int npmax = 0;
+  for (int f = 0; f < nf; ++f) {
+    CK(cudaMemcpy(ytr.data(), h->fb[f].ytr, (size_t)h->n_train * sizeof(int), cudaMemcpyDeviceToHost));
+    const int32_t* lr = lab_rows + (size_t)f * n_lab;
+    int prev = -1;
+    for (int r = 0; r < n_lab; ++r) {
+      if (lr[r] < 0 || lr[r] >= h->n_train) return fail(h, MRGAN_ERR_ARG, "svm_fit: labeled row out of range");
+      const int c = ytr[lr[r]];
+      if (c < prev) return fail(h, MRGAN_ERR_ARG, "svm_fit: labeled rows must be class-major (labels non-decreasing)");
+      if (c != prev) start[(size_t)f * K + c] = r;
+      cnt[(size_t)f * K + c]++;
+      prev = c;
+    }
+    for (int c = 0; c < K; ++c)
+      if (cnt[(size_t)f * K + c] == 0) return fail(h, MRGAN_ERR_ARG, "svm_fit: every class needs a labeled row");
+    for (int a = 0; a < K; ++a)
+      for (int b = a + 1; b < K; ++b) {
+        const int np = cnt[(size_t)f * K + a] + cnt[(size_t)f * K + b];
+        if (np > SVM_MAX_PAIR) return fail(h, MRGAN_ERR_ARG, "svm_fit: a class pair has more than 8192 labeled rows (shared-memory limit of the solver)");
+        npmax = std::max(npmax, np);
+      }
+  }
+  // workspace
+  mrgan_handle::Svm& S = h->svm;
+  int max_nte = 0;
+  for (int f = 0; f < nf; ++f) max_nte = std::max(max_nte, h->shapes[f].n_test);
+  std::vector<float*> Hl(nf), Ll(nf), Ht(nf), Lt(nf), Klab(nf), Kte(nf), dec(nf);
+  std::vector<double*> nl(nf), nt(nf), coef(nf), rho(nf);
+  std::vector<int*> wrong(nf);
+  int* d_lab = nullptr;
+  auto layout = [&](Arena& ar) {
+    for (int f = 0; f < nf; ++f) {
+      const int Kp = round_up(h->shapes[f].D, 32), nte = h->shapes[f].n_test;
+      Hl[f] = ar.take<float>((size_t)n_lab * Kp); Ll[f] = ar.take<float>((size_t)n_lab * Kp);
+      Ht[f] = ar.take<float>((size_t)nte * Kp); Lt[f] = ar.take<float>((size_t)nte * Kp);
+      nl[f] = ar.take<double>(n_lab); nt[f] = ar.take<double>(nte);
+      Klab[f] = ar.take<float>((size_t)n_lab * n_lab); Kte[f] = ar.take<float>((size_t)nte * n_lab);
+      coef[f] = ar.take<double>((size_t)npairs * npmax); rho[f] = ar.take<double>(npairs);
+      dec[f] = ar.take<float>((size_t)nte * npairs); wrong[f] = ar.take<int>(nte);
+    }
+    d_lab = ar.take<int>((size_t)nf * n_lab);
+    S.d_iters = ar.take<int>((size_t)nf * npairs); S.d_capped = ar.take<int>((size_t)nf * npairs);
+    S.d_count = ar.take<int>(nf); S.d_nte = ar.take<int>(nf);
+    S.d_split = ar.take<SvmSplitOp>(2 * nf); S.d_gemm = ar.take<SvmGemmOp>(2 * nf); S.d_jobs = ar.take<SvmPairJob>((size_t)nf * npairs);
+    S.d_Kt = ar.take<float*>(nf); S.d_dec = ar.take<float*>(nf); S.d_yte = ar.take<int*>(nf); S.d_wrong = ar.take<int*>(nf);
+  };
+  Arena sizing;
+  layout(sizing);
+  S.fitted = false;
+  if (sizing.off + 256 > S.bytes) {
+    if (S.mem) { cudaFree(S.mem); S.mem = nullptr; S.bytes = 0; }
+    CK(cudaMalloc(&S.mem, sizing.off + 256));
+    S.bytes = sizing.off + 256;
+  }
+  Arena real; real.base = S.mem;
+  layout(real);
+  S.n_lab = n_lab; S.npairs = npairs; S.npmax = npmax; S.max_nte = max_nte; S.max_rows = std::max(n_lab, max_nte);
+  S.C = C; S.eps = tol;
+  S.Klab = Klab; S.Kte = Kte; S.dec = dec; S.wrong = wrong;
+  // descriptors
+  EncodeTiledFn fn = tc_encoder();
+  if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
+  std::vector<SvmSplitOp> sp(2 * nf);
+  std::vector<SvmGemmOp> gm(2 * nf);
+  std::vector<SvmPairJob> jobs((size_t)nf * npairs);
+  std::vector<int> nte_v(nf);
+  std::vector<int*> yte_v(nf);
+  memset(gm.data(), 0, sizeof(SvmGemmOp) * gm.size());
+  for (int f = 0; f < nf; ++f) {
+    const FoldBuffers& b = h->fb[f];
+    const int D = h->shapes[f].D, Kp = round_up(D, 32), nte = h->shapes[f].n_test;
+    sp[2 * f] = SvmSplitOp{b.xtr, pitch8(D), d_lab + (size_t)f * n_lab, n_lab, D, Kp, Hl[f], Ll[f], nl[f]};
+    sp[2 * f + 1] = SvmSplitOp{b.xte, b.lda[0], nullptr, nte, D, Kp, Ht[f], Lt[f], nt[f]};
+    for (int w = 0; w < 2; ++w) {
+      SvmGemmOp& g = gm[2 * f + w];
+      const int nA = w == 0 ? n_lab : nte;
+      bool ok = make_map(fn, &g.mapBh, Hl[f], Kp, n_lab, Kp, SVM_BM, false) && make_map(fn, &g.mapBl, Ll[f], Kp, n_lab, Kp, SVM_BM, false) &&
+                make_map(fn, &g.mapAh, w == 0 ? Hl[f] : Ht[f], Kp, nA, Kp, SVM_BN, false) &&
+                make_map(fn, &g.mapAl, w == 0 ? Ll[f] : Lt[f], Kp, nA, Kp, SVM_BN, false);
+      if (!ok) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
+      g.normA = w == 0 ? nl[f] : nt[f]; g.normB = nl[f];
+      g.C = w == 0 ? Klab[f] : Kte[f]; g.ldc = n_lab;
+      g.nA = nA; g.nB = n_lab; g.Kp = Kp; g.gamma = gamma[f]; g.same = w == 0;
+    }
+    int p = 0;
+    for (int a = 0; a < K; ++a)
+      for (int c = a + 1; c < K; ++c, ++p) {
+        SvmPairJob& jb = jobs[(size_t)f * npairs + p];
+        jb.K = Klab[f]; jb.ld = n_lab;
+        jb.a_off = start[(size_t)f * K + a]; jb.na = cnt[(size_t)f * K + a];
+        jb.b_off = start[(size_t)f * K + c]; jb.nb = cnt[(size_t)f * K + c];
+        jb.ca = a; jb.cb = c;
+        jb.coef = coef[f] + (size_t)p * npmax; jb.rho = rho[f] + p;
+        jb.n_iter = S.d_iters + (size_t)f * npairs + p; jb.capped = S.d_capped + (size_t)f * npairs + p;
+      }
+    nte_v[f] = nte; yte_v[f] = b.yte;
+  }
+  CK(cudaMemcpyAsync(d_lab, lab_rows, (size_t)nf * n_lab * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_split, sp.data(), sizeof(SvmSplitOp) * sp.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_gemm, gm.data(), sizeof(SvmGemmOp) * gm.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_jobs, jobs.data(), sizeof(SvmPairJob) * jobs.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_nte, nte_v.data(), sizeof(int) * nf, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_Kt, Kte.data(), sizeof(float*) * nf, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_dec, dec.data(), sizeof(float*) * nf, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_yte, yte_v.data(), sizeof(int*) * nf, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_wrong, wrong.data(), sizeof(int*) * nf, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaFuncSetAttribute(k_svm_kmat, cudaFuncAttributeMaxDynamicSharedMemorySize, SVM_KMAT_SMEM));
+  CK(cudaFuncSetAttribute(k_svm_smo, cudaFuncAttributeMaxDynamicSharedMemorySize, 20 * SVM_MAX_PAIR));
+  svm_launch(h, MRGAN_TIME_SVM_KMAT);
+  svm_launch(h, MRGAN_TIME_SVM_SMO);
+  svm_launch(h, MRGAN_TIME_SVM_PREDICT);
+  std::vector<int> it((size_t)nf * npairs), cap((size_t)nf * npairs);
+  CK(cudaMemcpyAsync(it.data(), S.d_iters, sizeof(int) * it.size(), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(cap.data(), S.d_capped, sizeof(int) * cap.size(), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  CK(cudaGetLastError());
+  if (n_iter) memcpy(n_iter, it.data(), sizeof(int) * it.size());
+  S.fitted = true;
+  for (size_t q = 0; q < cap.size(); ++q)
+    if (cap[q]) return fail(h, MRGAN_ERR_STATE, "svm_fit: fold " + std::to_string(q / npairs) + ", class pair " + std::to_string(q % npairs) +
+                                                    " hit the iteration cap max(1e7, 100 n)");
+  return MRGAN_OK;
+#endif
+}
+
+int mrgan_svm_eval(mrgan_handle* h, int fold, float* err) {
+  int rc = check_fold(h, fold); if (rc) return rc;
+  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_eval needs an SVM handle");
+  if (!err) return fail(h, MRGAN_ERR_ARG, "svm_eval: null pointer");
+#ifndef MRGAN_WITH_TC
+  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
+#else
+  if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "svm_eval before mrgan_svm_fit");
+  CK(cudaSetDevice(h->cfg.device));
+  int c = 0;
+  CK(cudaMemcpyAsync(&c, h->svm.d_count + fold, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  *err = (float)c / (float)h->shapes[fold].n_test;     // np.mean(predicted != y_test)
+  return MRGAN_OK;
+#endif
+}
+
+int mrgan_svm_decision(mrgan_handle* h, int fold, float* dst) {
+  int rc = check_fold(h, fold); if (rc) return rc;
+  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_decision needs an SVM handle");
+  if (!dst) return fail(h, MRGAN_ERR_ARG, "svm_decision: null pointer");
+#ifndef MRGAN_WITH_TC
+  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
+#else
+  if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "svm_decision before mrgan_svm_fit");
+  CK(cudaSetDevice(h->cfg.device));
+  CK(cudaMemcpyAsync(dst, h->svm.dec[fold], sizeof(float) * h->shapes[fold].n_test * h->svm.npairs, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return MRGAN_OK;
+#endif
+}
+
+static int svm_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
+#ifndef MRGAN_WITH_TC
+  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
+#else
+  if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "time_op: SVM phases before mrgan_svm_fit");
+  CK(cudaSetDevice(h->cfg.device));
+  svm_launch(h, which);                     // warm-up
+  CK(cudaEventRecord(h->ev0, h->stream));
+  for (int i = 0; i < reps; ++i) svm_launch(h, which);
+  CK(cudaEventRecord(h->ev1, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  CK(cudaGetLastError());
+  float ms = 0.f;
+  CK(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+  *ms_avg = ms / reps;
   return MRGAN_OK;
 #endif
 }

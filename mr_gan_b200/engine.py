@@ -14,7 +14,7 @@ import numpy as np
 from . import _lib
 from .model import disc_shapes, gen_shapes
 
-MODEL = {"gan": 0, "nn": 1}
+MODEL = {"gan": 0, "nn": 1, "svm": 2}
 PRECISION = {"fp32": 0, "tf32": 1, "f16": 2}      # f16: fp16 operand copies, fp32 master weights / accumulation (experimental)
 
 
@@ -291,6 +291,38 @@ class FoldGroup:
         self._chk(self.lib.mrnn_evaluate(self._h, fold, _lib.fptr(out)))
         return out[0], out[1]
 
+    # ------------------------------------------------------------------ mr_svm (model='svm')
+    @property
+    def n_pairs(self):
+        K = self.cfg.n_classes
+        return K * (K - 1) // 2
+
+    def svm_fit(self, lab_rows, C=1.0, gamma=None, tol=1e-3):
+        """mr_svm.py:106 ``SVC(kernel='rbf', C).fit`` for every fold, then the prediction of every fold's test set.
+        lab_rows: int32 [n_folds, n_lab] class-major rows of X_train; gamma: per-fold list / scalar (None: 1 / D).
+        Returns the SMO iterations, int32 [n_folds, n_pairs]."""
+        lab = _i32(lab_rows)
+        if lab.ndim != 2 or lab.shape[0] != self.n_folds:
+            raise ValueError("svm_fit: lab_rows must be [n_folds, n_lab]")
+        if gamma is None:
+            gamma = [1.0 / D for D, _, _, _ in self.shapes]
+        g = _f32(np.broadcast_to(np.asarray(gamma, dtype=np.float32), (self.n_folds,)))
+        it = np.zeros((self.n_folds, self.n_pairs), dtype=np.int32)
+        self._chk(self.lib.mrgan_svm_fit(self._h, _lib.iptr(lab), lab.shape[1], float(C), _lib.fptr(g), float(tol), _lib.iptr(it)))
+        return it
+
+    def svm_eval(self, fold):
+        """Error of the one-vs-one vote on the fold's full test set (np.mean(predicted != y_test))."""
+        out = np.zeros(1, dtype=np.float32)
+        self._chk(self.lib.mrgan_svm_eval(self._h, int(fold), _lib.fptr(out)))
+        return float(out[0])
+
+    def svm_decision(self, fold):
+        """Test hook: the one-vs-one decision values, float32 [n_test, n_pairs] (pairs (0,1), (0,2), ...)."""
+        out = np.zeros((self.shapes[fold][2], self.n_pairs), dtype=np.float32)
+        self._chk(self.lib.mrgan_svm_decision(self._h, int(fold), _lib.fptr(out)))
+        return out
+
     # ------------------------------------------------------------------ utilities
     def fill_normal(self, fold, step, tensor_id, rows, cols, row0=0):
         out = np.empty((rows, cols), dtype=np.float32)
@@ -326,7 +358,8 @@ class FoldGroup:
         self._chk(self.lib.mrgan_debug_gemm_time(self._h, mode, M, N, K, groups, reps, _lib.fptr(out)))
         return float(out[0])
 
-    TIME_OPS = {"adam_d": 0, "adam_g": 1, "dw1": 2, "fwd1": 3, "disc_step": 4, "gen_step": 5, "dx1": 6}
+    TIME_OPS = {"adam_d": 0, "adam_g": 1, "dw1": 2, "fwd1": 3, "disc_step": 4, "gen_step": 5, "dx1": 6,
+                "svm_kmat": 7, "svm_smo": 8, "svm_predict": 9}
 
     def time_op(self, which, reps=20):
         """Average device ms of one kernel (or one whole step) over all folds; mutates training state."""
