@@ -191,6 +191,22 @@ int  mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C,
 int  mrgan_svm_eval(mrgan_handle* h, int fold, float* err);                 /* full resident X_test, ovo vote */
 int  mrgan_svm_decision(mrgan_handle* h, int fold, float* dst);             /* test hook: [n_test][K(K-1)/2] */
 
+/* Predictions of a trained fold (GAN / NN: the current weights, the phase-0 forward of mrgan_eval; SVM: after mrgan_svm_fit).
+ * The predicted class is the first maximal logit (GAN / NN; the rule behind the error of mrgan_eval) or libsvm's one-vs-one
+ * vote, the first class with the most votes (SVM).  Scores are raw: logits, or decision values, not probabilities.
+ *   mrgan_predict: the fold's resident test set: pred [n_test]; scores [n_test][K] logits (GAN / NN)
+ *     or [n_test][K(K-1)/2] decision values (SVM, pairs (0,1),(0,2),...); scores may be NULL.
+ *   mrgan_predict_rows: rows x [n][D_fold] in the fold's SCALED input space (that of mrgan_test_batch and of the resident
+ *     X_test), 1 <= n <= n_test of the fold; same outputs.  Leaves every later result on the resident test set unchanged.
+ *   mrgan_confusion: every fold of the handle in one pass over its resident test set: out [n_folds][K][K] int32 counts,
+ *     rows = true class, columns = predicted class.
+ * MRGAN_ERR_ARG: null pred / x / out, fold or n out of range.  MRGAN_ERR_STATE: a GAN / NN fold not loaded, an SVM handle
+ * before mrgan_svm_fit, or a data-parallel handle (mrgan_dp_init / mrgan_dp_init_virtual).  Like mrgan_eval, each call first
+ * completes a pending asynchronous epoch, whose statistics it leaves unchanged. */
+int  mrgan_predict(mrgan_handle* h, int fold, int32_t* pred, float* scores);
+int  mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t* pred, float* scores);
+int  mrgan_confusion(mrgan_handle* h, int32_t* out);
+
 /* Utilities used by tests and bench */
 int  mrgan_fill_normal(mrgan_handle* h, int fold, int step, int tensor_id, int rows, int cols,
                        int row0, float* dst /* host [rows, cols] */);

@@ -70,6 +70,9 @@ SYMBOLS = {
     "mrgan_svm_fit": (C.c_int, [_H, _ip, C.c_int, C.c_float, _fp, C.c_float, _ip]),
     "mrgan_svm_eval": (C.c_int, [_H, C.c_int, _fp]),
     "mrgan_svm_decision": (C.c_int, [_H, C.c_int, _fp]),
+    "mrgan_predict": (C.c_int, [_H, C.c_int, _ip, _fp]),
+    "mrgan_predict_rows": (C.c_int, [_H, C.c_int, _fp, C.c_int, _ip, _fp]),
+    "mrgan_confusion": (C.c_int, [_H, _ip]),
     "mrgan_fill_normal": (C.c_int, [_H, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _fp]),
     "mrgan_adam_flat": (C.c_int, [_H, _fp, _fp, _fp, _fp, C.c_int64, C.c_int]),
     "mrgan_time_op": (C.c_int, [_H, C.c_int, C.c_int, _fp]),

@@ -718,13 +718,21 @@ k_fm_apply(const LossDesc* __restrict__ descs, const DpBufs* __restrict__ bufs, 
 }
 
 // ------------------------------------------------------------------ evaluation
-struct EvalDesc { const float* logits; int ld; const int* y; int n; int n_batched; float* out; };
+struct EvalDesc { const float* logits; int ld; const int* y; int n; int n_batched; float* out; int* pred; };
+
+// The predicted class of a row of logits: the FIRST maximal entry (strict > scan; a NaN never wins).  The one argmax rule
+// behind both the error of k_argmax_err and the per-row predictions.
+__device__ __forceinline__ int row_argmax(const float* l, int K) {
+  float mx = l[0]; int am = 0;
+  for (int k = 1; k < K; ++k) if (l[k] > mx) { mx = l[k]; am = k; }
+  return am;
+}
 
 // test_batch (mr_gan.py:162,171): mean(argmax != y); out[0] over the first n_batched rows
 // (= mean of the per-batch errors of mr_gan.py:221-223), out[1] over all rows (mr_gan.py:230),
-// out[2] = mse vs one-hot over all rows (mr_nn.py:118 evaluate()[0]).
+// out[2] = mse vs one-hot over all rows (mr_nn.py:118 evaluate()[0]).  with_pred: also store every row's class in d.pred.
 __global__ void __launch_bounds__(256)
-k_argmax_err(const EvalDesc* __restrict__ descs, int n_override, int K) {
+k_argmax_err(const EvalDesc* __restrict__ descs, int n_override, int K, int with_pred) {
   pdl_launch_dependents();
   pdl_wait();
   __shared__ float sh[32];
@@ -735,8 +743,8 @@ k_argmax_err(const EvalDesc* __restrict__ descs, int n_override, int K) {
   for (int r = threadIdx.x; r < n; r += blockDim.x) {
     const float* l = d.logits + (size_t)r * d.ld;
     const int y = d.y[r];
-    float mx = l[0]; int am = 0;
-    for (int k = 1; k < K; ++k) if (l[k] > mx) { mx = l[k]; am = k; }
+    const int am = row_argmax(l, K);
+    if (with_pred) d.pred[r] = am;
     for (int k = 0; k < K; ++k) { const float diff = l[k] - (k == y ? 1.f : 0.f); q = fmaf(diff, diff, q); }
     const float e = (am != y) ? 1.f : 0.f;
     e_all += e;
@@ -746,6 +754,22 @@ k_argmax_err(const EvalDesc* __restrict__ descs, int n_override, int K) {
   e_all = block_sum(e_all, sh);
   q = block_sum(q, sh);
   if (threadIdx.x == 0) { d.out[0] = nb > 0 ? e_b / nb : 0.f; d.out[1] = e_all / n; d.out[2] = q / ((float)n * K); }
+}
+
+// Confusion counts of every fold: out[f][y][pred] over the fold's d.n rows of (d.y, d.pred); out is zeroed beforehand.
+// grid (row chunks, folds); a block counts its chunk in shared memory, then adds its non-zero cells.  Integer atomics:
+// the counts are exact in any order.
+#define CONF_ROWS 1024
+__global__ void __launch_bounds__(256) k_confusion(const EvalDesc* __restrict__ descs, int K, int* __restrict__ out) {
+  __shared__ int cnt[64 * 64];
+  const EvalDesc d = descs[blockIdx.y];
+  for (int i = threadIdx.x; i < K * K; i += blockDim.x) cnt[i] = 0;
+  __syncthreads();
+  const int r0 = blockIdx.x * CONF_ROWS, r1 = min(d.n, r0 + CONF_ROWS);
+  for (int r = r0 + threadIdx.x; r < r1; r += blockDim.x) atomicAdd(&cnt[d.y[r] * K + d.pred[r]], 1);
+  __syncthreads();
+  int* o = out + (size_t)blockIdx.y * K * K;
+  for (int i = threadIdx.x; i < K * K; i += blockDim.x) if (cnt[i]) atomicAdd(&o[i], cnt[i]);
 }
 
 // Means over the epoch's batches (mr_gan.py:215-217) -> epoch_stats[f][0..3]; [4] = batch-wise test error.

@@ -326,11 +326,12 @@ __global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* _
 
 // ---------------------------------------------------------------- decision values and vote (svm.cpp:2865-2897)
 #define SVM_VOTE_THREADS 256
-// one CTA per (test row, fold): jobs of the fold are jobs[fold * npairs ...]; Kt = the fold's test x labeled matrix
+// one CTA per (test row, fold): jobs of the fold are jobs[fold * npairs ...]; Kt = the fold's test x labeled matrix.
+// wrong (with yte) and pred may be null: rows without labels (mrgan_predict_rows) store only the voted class.
 __global__ void __launch_bounds__(SVM_VOTE_THREADS) k_svm_vote(const SvmPairJob* __restrict__ jobs, int npairs, int n_classes,
                                                                const float* const* __restrict__ Kt, const int* const* __restrict__ yte,
                                                                const int* __restrict__ n_test, float* const* __restrict__ dec_out,
-                                                               int* const* __restrict__ wrong) {
+                                                               int* const* __restrict__ wrong, int* const* __restrict__ pred) {
   const int f = blockIdx.y, t = blockIdx.x;
   if (t >= n_test[f]) return;
   const SvmPairJob* jf = jobs + (size_t)f * npairs;
@@ -358,7 +359,8 @@ __global__ void __launch_bounds__(SVM_VOTE_THREADS) k_svm_vote(const SvmPairJob*
     for (int p = 0; p < npairs; ++p) ++votes[dec_s[p] > 0.5f ? jf[p].ca : jf[p].cb];
     int best = 0;
     for (int c = 1; c < n_classes; ++c) if (votes[c] > votes[best]) best = c;   // the first class with most votes
-    wrong[f][t] = best != yte[f][t];
+    if (wrong) wrong[f][t] = best != yte[f][t];
+    if (pred) pred[f][t] = best;
   }
 }
 

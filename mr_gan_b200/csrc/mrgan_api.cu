@@ -64,6 +64,7 @@ struct FoldBuffers {
   float *a[6], *hb[6], *dz[6], *lg, *dlg, *dfake, *zb, *h1g, *xhat, *istd, *u, *h2g, *dz2g, *du, *dz1g;
   float *stage_x, *stage_z, *ex_stage, *xte, *eh[6], *elg, *xtr, *eval_out, *eval_out_s;
   int *stage_y, *labels_cur, *ey_stage, *ytr, *yte, *idx;
+  int *pred, *pred_s;            // predicted classes of the resident test set / of the staged rows (mrgan_predict*)
   int *lab_rows, *unl_rows;      // device-side epoch permutations: labeled / unlabeled row subsets (mrgan_set_epoch_rows)
   int n_lab = 0, n_unl = 0;
   int lda[6], ldz[6];   // pitches of a/h (with ones column) and dz
@@ -110,6 +111,7 @@ struct mrgan_handle {
   GemmDesc* d_descs = nullptr; std::vector<GemmDesc> h_descs;
   PermDesc* d_perm = nullptr;
   BnDesc* d_bn = nullptr; LossDesc* d_loss = nullptr; EvalDesc *d_eval = nullptr, *d_eval_s = nullptr;
+  int* d_conf = nullptr;              // [nf][K][K] confusion counts (mrgan_confusion)
   AdamRange* d_ranges[2] = {nullptr, nullptr};
   OpInfo ops[NUM_OPS];
   float *d_step_stats = nullptr, *d_epoch_stats = nullptr, *h_epoch_stats = nullptr;
@@ -165,7 +167,12 @@ struct mrgan_handle {
     std::vector<int*> wrong;
     int *d_iters = nullptr, *d_capped = nullptr, *d_count = nullptr, *d_nte = nullptr;
     SvmSplitOp* d_split = nullptr; SvmGemmOp* d_gemm = nullptr; SvmPairJob* d_jobs = nullptr;
-    float** d_Kt = nullptr; float** d_dec = nullptr; int** d_yte = nullptr; int** d_wrong = nullptr;
+    float** d_Kt = nullptr; float** d_dec = nullptr; int** d_yte = nullptr; int** d_wrong = nullptr; int** d_pred = nullptr;
+    // mrgan_predict_rows: up to max_nte new rows of one fold, staged, split, kernel matrix, decision values and vote
+    std::vector<SvmGemmOp> h_gemm;      // host copies of the descriptors in d_gemm
+    float *Xs = nullptr, *Hs = nullptr, *Ls = nullptr, *Ks = nullptr, *decs = nullptr; double* ns = nullptr; int* preds = nullptr;
+    SvmSplitOp* d_split_s = nullptr; SvmGemmOp* d_gemm_s = nullptr;
+    float** d_Ks = nullptr; float** d_decs = nullptr; int** d_preds = nullptr; int* d_ns = nullptr;   // one-fold pointer tables
   } svm;
 #endif
 };
@@ -263,7 +270,10 @@ void layout_buffers(mrgan_handle* h, Arena& ar) {
       b.xtr = ar.take<float>((size_t)h->shapes[f].n_train * pitch8(D));
       b.ytr = ar.take<int>(h->shapes[f].n_train);
       b.yte = ar.take<int>(h->shapes[f].n_test);
+      b.pred = ar.take<int>(h->shapes[f].n_test);
     }
+    h->d_eval = ar.take<EvalDesc>(nf);
+    h->d_conf = ar.take<int>((size_t)nf * K * K);
     return;
   }
   h->P = ar.take<float>(h->n_flat);
@@ -327,7 +337,10 @@ void layout_buffers(mrgan_handle* h, Arena& ar) {
     b.idx = ar.take<int>((size_t)3 * ntr);
     b.lab_rows = ar.take<int>(ntr);
     b.unl_rows = ar.take<int>(ntr);
+    b.pred = ar.take<int>(nte);
+    b.pred_s = ar.take<int>(NE);
   }
+  h->d_conf = ar.take<int>((size_t)nf * K * K);
 }
 
 GemmDesc make_desc(const float* A, int lda, const float* Bm, int ldb, float* C, int ldc, int M, int N, int K, int epi,
@@ -402,8 +415,8 @@ int build_descs(mrgan_handle* h) {
     }
     rg0[f] = AdamRange{LD.off, LD.n};
     ls[f] = LossDesc{b.lg, b.dlg, pitch8(K), b.labels_cur, b.hb[5], b.dz[5], b.lda[5], b.ldz[5], kDW[4]};
-    ev[f] = EvalDesc{b.elg, pitch8(K), b.yte, h->shapes[f].n_test, (h->shapes[f].n_test / B) * B, b.eval_out};
-    evs[f] = EvalDesc{b.elg, pitch8(K), b.ey_stage, h->shapes[f].n_test, 0, b.eval_out_s};
+    ev[f] = EvalDesc{b.elg, pitch8(K), b.yte, h->shapes[f].n_test, (h->shapes[f].n_test / B) * B, b.eval_out, b.pred};
+    evs[f] = EvalDesc{b.elg, pitch8(K), b.ey_stage, h->shapes[f].n_test, 0, b.eval_out_s, b.pred_s};
     if (gan) {
       const NetLayout& LG = h->net[1][f];
       float* PG = h->P + LG.off; float* GG = h->Gr + LG.off;
@@ -873,13 +886,28 @@ void enqueue_nn_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage, in
   launch_adam(h, f0, nfl, 0, false);
 }
 
-// test_batch (mr_gan.py:171): phase 0, no noise
-void enqueue_eval(mrgan_handle* h, int f0, int nfl, bool staged, int n_override) {
+// test_batch (mr_gan.py:171): phase 0, no noise; with_pred: also the predicted class of every row (fb[f].pred / pred_s)
+void enqueue_eval(mrgan_handle* h, int f0, int nfl, bool staged, int n_override, bool with_pred = false) {
   join_side(h);
   launch_gemm(h, staged ? OP_E1S : OP_E1, f0, nfl, n_override);
   for (int l = 1; l < 6; ++l) launch_gemm(h, OP_E2 + l - 1, f0, nfl, n_override);
   launch_k(h, k_argmax_err, dim3(1, 1, nfl), dim3(256), 0, h->stream, (const EvalDesc*)((staged ? h->d_eval_s : h->d_eval) + f0), n_override,
-           h->cfg.n_classes);
+           h->cfg.n_classes, (int)with_pred);
+}
+
+// confusion counts of folds [0, nf) from the EvalDesc rows (y, pred) -> h->d_conf
+void enqueue_confusion(mrgan_handle* h) {
+  const int K = h->cfg.n_classes;
+  int nmax = 1;
+  for (int f = 0; f < h->nf; ++f) nmax = std::max(nmax, h->shapes[f].n_test);
+  cudaMemsetAsync(h->d_conf, 0, (size_t)h->nf * K * K * sizeof(int), h->stream);
+  launch_k(h, k_confusion, dim3((nmax + CONF_ROWS - 1) / CONF_ROWS, h->nf), dim3(256), 0, h->stream, (const EvalDesc*)h->d_eval, K, h->d_conf);
+}
+
+// prediction entry points: the single-GPU handle only (data-parallel replicas are out of their scope)
+int need_local(mrgan_handle* h, const char* fn) {
+  if (h->dp_world > 1 || h->dp_virtual || h->nccl_comm) return fail(h, MRGAN_ERR_STATE, std::string(fn) + ": not available on a data-parallel handle");
+  return MRGAN_OK;
 }
 
 int check_fold(mrgan_handle* h, int fold) {
@@ -1525,6 +1553,11 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
   if (cfg->model != MRGAN_MODEL_SVM) {
     const int rc = build_descs(h); if (rc != MRGAN_OK) return cleanup(rc);
     init_ones(h);
+  } else {      // the confusion rows of an SVM fold: (y_test, voted class)
+    std::vector<EvalDesc> ev(h->nf);
+    for (int f = 0; f < h->nf; ++f) ev[f] = EvalDesc{nullptr, 0, h->fb[f].yte, folds[f].n_test, 0, nullptr, h->fb[f].pred};
+    if (cudaMemcpy(h->d_eval, ev.data(), h->nf * sizeof(EvalDesc), cudaMemcpyHostToDevice) != cudaSuccess)
+      return cleanup(fail(nullptr, MRGAN_ERR_CUDA, "create: descriptor upload failed"));
   }
   if (cfg->model == MRGAN_MODEL_GAN && cfg->batch > 256) {   // large batch: row-parallel split BatchNorm / feature-matching kernels
     int rc = alloc_split_bufs(h);
@@ -2388,7 +2421,7 @@ static void svm_launch(mrgan_handle* h, int phase) {
     h->launches += 1;
   } else {
     k_svm_vote<<<dim3(S.max_nte, nf), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs, S.npairs, h->cfg.n_classes, S.d_Kt, S.d_yte, S.d_nte,
-                                                                         S.d_dec, S.d_wrong);
+                                                                         S.d_dec, S.d_wrong, S.d_pred);
     k_svm_count<<<nf, 256, 0, h->stream>>>(S.d_wrong, S.d_nte, S.d_count);
     h->launches += 2;
   }
@@ -2435,8 +2468,8 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
   }
   // workspace
   mrgan_handle::Svm& S = h->svm;
-  int max_nte = 0;
-  for (int f = 0; f < nf; ++f) max_nte = std::max(max_nte, h->shapes[f].n_test);
+  int max_nte = 0, max_kp = 32;
+  for (int f = 0; f < nf; ++f) { max_nte = std::max(max_nte, h->shapes[f].n_test); max_kp = std::max(max_kp, round_up(h->shapes[f].D, 32)); }
   std::vector<float*> Hl(nf), Ll(nf), Ht(nf), Lt(nf), Klab(nf), Kte(nf), dec(nf);
   std::vector<double*> nl(nf), nt(nf), coef(nf), rho(nf);
   std::vector<int*> wrong(nf);
@@ -2456,6 +2489,12 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
     S.d_count = ar.take<int>(nf); S.d_nte = ar.take<int>(nf);
     S.d_split = ar.take<SvmSplitOp>(2 * nf); S.d_gemm = ar.take<SvmGemmOp>(2 * nf); S.d_jobs = ar.take<SvmPairJob>((size_t)nf * npairs);
     S.d_Kt = ar.take<float*>(nf); S.d_dec = ar.take<float*>(nf); S.d_yte = ar.take<int*>(nf); S.d_wrong = ar.take<int*>(nf);
+    S.d_pred = ar.take<int*>(nf);
+    S.Xs = ar.take<float>((size_t)max_nte * max_kp); S.Hs = ar.take<float>((size_t)max_nte * max_kp); S.Ls = ar.take<float>((size_t)max_nte * max_kp);
+    S.ns = ar.take<double>(max_nte); S.Ks = ar.take<float>((size_t)max_nte * n_lab); S.decs = ar.take<float>((size_t)max_nte * npairs);
+    S.preds = ar.take<int>(max_nte);
+    S.d_split_s = ar.take<SvmSplitOp>(1); S.d_gemm_s = ar.take<SvmGemmOp>(1);
+    S.d_Ks = ar.take<float*>(1); S.d_decs = ar.take<float*>(1); S.d_preds = ar.take<int*>(1); S.d_ns = ar.take<int>(1);
   };
   Arena sizing;
   layout(sizing);
@@ -2477,7 +2516,7 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
   std::vector<SvmGemmOp> gm(2 * nf);
   std::vector<SvmPairJob> jobs((size_t)nf * npairs);
   std::vector<int> nte_v(nf);
-  std::vector<int*> yte_v(nf);
+  std::vector<int*> yte_v(nf), pred_v(nf);
   memset(gm.data(), 0, sizeof(SvmGemmOp) * gm.size());
   for (int f = 0; f < nf; ++f) {
     const FoldBuffers& b = h->fb[f];
@@ -2506,8 +2545,9 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
         jb.coef = coef[f] + (size_t)p * npmax; jb.rho = rho[f] + p;
         jb.n_iter = S.d_iters + (size_t)f * npairs + p; jb.capped = S.d_capped + (size_t)f * npairs + p;
       }
-    nte_v[f] = nte; yte_v[f] = b.yte;
+    nte_v[f] = nte; yte_v[f] = b.yte; pred_v[f] = b.pred;
   }
+  S.h_gemm = gm;
   CK(cudaMemcpyAsync(d_lab, lab_rows, (size_t)nf * n_lab * sizeof(int), cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(S.d_split, sp.data(), sizeof(SvmSplitOp) * sp.size(), cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(S.d_gemm, gm.data(), sizeof(SvmGemmOp) * gm.size(), cudaMemcpyHostToDevice, h->stream));
@@ -2517,6 +2557,10 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
   CK(cudaMemcpyAsync(S.d_dec, dec.data(), sizeof(float*) * nf, cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(S.d_yte, yte_v.data(), sizeof(int*) * nf, cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(S.d_wrong, wrong.data(), sizeof(int*) * nf, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_pred, pred_v.data(), sizeof(int*) * nf, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_Ks, &S.Ks, sizeof(float*), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_decs, &S.decs, sizeof(float*), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(S.d_preds, &S.preds, sizeof(int*), cudaMemcpyHostToDevice, h->stream));
   CK(cudaFuncSetAttribute(k_svm_kmat, cudaFuncAttributeMaxDynamicSharedMemorySize, SVM_KMAT_SMEM));
   CK(cudaFuncSetAttribute(k_svm_smo, cudaFuncAttributeMaxDynamicSharedMemorySize, 20 * SVM_MAX_PAIR));
   svm_launch(h, MRGAN_TIME_SVM_KMAT);
@@ -2585,6 +2629,122 @@ static int svm_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
   *ms_avg = ms / reps;
   return MRGAN_OK;
 #endif
+}
+
+// ------------------------------------------------------------------ predictions and confusion counts
+int mrgan_predict(mrgan_handle* h, int fold, int32_t* pred, float* scores) {
+  int rc = check_fold(h, fold); if (rc) return rc;
+  if (!pred) return fail(h, MRGAN_ERR_ARG, "predict: null pointer");
+  rc = need_local(h, "predict"); if (rc) return rc;
+  const int n = h->shapes[fold].n_test, K = h->cfg.n_classes;
+  const FoldBuffers& b = h->fb[fold];
+  if (h->cfg.model == MRGAN_MODEL_SVM) {
+#ifndef MRGAN_WITH_TC
+    return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
+#else
+    if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "predict before mrgan_svm_fit");
+    CK(cudaSetDevice(h->cfg.device));
+    CK(cudaMemcpyAsync(pred, b.pred, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));     // voted by mrgan_svm_fit
+    if (scores) CK(cudaMemcpyAsync(scores, h->svm.dec[fold], (size_t)n * h->svm.npairs * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+#endif
+  } else {
+    if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "predict before mrgan_load_fold");
+    CK(cudaSetDevice(h->cfg.device));
+    rc = finish_pending(h); if (rc) return rc;
+    enqueue_eval(h, fold, 1, false, 0, true);
+    CK(cudaMemcpyAsync(pred, b.pred, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (scores)
+      CK(cudaMemcpy2DAsync(scores, (size_t)K * sizeof(float), b.elg, (size_t)pitch8(K) * sizeof(float), (size_t)K * sizeof(float), n,
+                           cudaMemcpyDeviceToHost, h->stream));
+  }
+  CK(cudaStreamSynchronize(h->stream));
+  CKS();
+  return MRGAN_OK;
+}
+
+int mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t* pred, float* scores) {
+  int rc = check_fold(h, fold); if (rc) return rc;
+  if (!x || !pred) return fail(h, MRGAN_ERR_ARG, "predict_rows: null pointer");
+  if (n < 1 || n > h->shapes[fold].n_test) return fail(h, MRGAN_ERR_ARG, "predict_rows: n must be in [1, n_test of the fold]");
+  rc = need_local(h, "predict_rows"); if (rc) return rc;
+  const int D = h->shapes[fold].D, K = h->cfg.n_classes;
+  const size_t w = (size_t)D * sizeof(float);
+  FoldBuffers& b = h->fb[fold];
+  if (h->cfg.model == MRGAN_MODEL_SVM) {
+#ifndef MRGAN_WITH_TC
+    return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
+#else
+    mrgan_handle::Svm& S = h->svm;
+    if (!S.fitted) return fail(h, MRGAN_ERR_STATE, "predict_rows before mrgan_svm_fit");
+    CK(cudaSetDevice(h->cfg.device));
+    EncodeTiledFn fn = tc_encoder();
+    if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
+    // the new rows replace the fold's test rows in its second kernel-matrix descriptor (labeled rows, norms, gamma kept)
+    const int Kp = round_up(D, 32);
+    SvmSplitOp sp{S.Xs, Kp, nullptr, n, D, Kp, S.Hs, S.Ls, S.ns};
+    SvmGemmOp g = S.h_gemm[2 * fold + 1];
+    if (!make_map(fn, &g.mapAh, S.Hs, Kp, n, Kp, SVM_BN, false) || !make_map(fn, &g.mapAl, S.Ls, Kp, n, Kp, SVM_BN, false))
+      return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
+    g.normA = S.ns; g.C = S.Ks; g.nA = n;
+    CK(cudaMemcpy2DAsync(S.Xs, (size_t)Kp * sizeof(float), x, w, w, n, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(S.d_split_s, &sp, sizeof(sp), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(S.d_gemm_s, &g, sizeof(g), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(S.d_ns, &n, sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    k_svm_split<<<dim3((n + 7) / 8, 1), 256, 0, h->stream>>>(S.d_split_s);
+    k_svm_kmat<<<dim3((S.n_lab + SVM_BM - 1) / SVM_BM, (n + SVM_BN - 1) / SVM_BN, 1), SVM_KMAT_THREADS, SVM_KMAT_SMEM, h->stream>>>(S.d_gemm_s);
+    k_svm_vote<<<dim3(n, 1), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs + (size_t)fold * S.npairs, S.npairs, K, S.d_Ks, nullptr, S.d_ns,
+                                                               S.d_decs, nullptr, S.d_preds);
+    h->launches += 3;
+    CK(cudaMemcpyAsync(pred, S.preds, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (scores) CK(cudaMemcpyAsync(scores, S.decs, (size_t)n * S.npairs * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+#endif
+  } else {
+    if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "predict_rows before mrgan_load_fold");
+    CK(cudaSetDevice(h->cfg.device));
+    rc = finish_pending(h); if (rc) return rc;
+    // the staging path of mrgan_test_batch, without labels (the error it computes on the stale staged labels is unused)
+    CK(cudaMemcpy2DAsync(b.ex_stage, (size_t)b.lda[0] * sizeof(float), x, w, w, n, cudaMemcpyHostToDevice, h->stream));
+    if (h->cfg.precision == MRGAN_PREC_TF32) {
+      k_round_tf32<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0]);
+      h->launches++;
+    } else if (h->om.mode == 2) {
+      k_to_half<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0], h->om);
+      h->launches++;
+    }
+    enqueue_eval(h, fold, 1, true, n, true);
+    CK(cudaMemcpyAsync(pred, b.pred_s, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (scores)
+      CK(cudaMemcpy2DAsync(scores, (size_t)K * sizeof(float), b.elg, (size_t)pitch8(K) * sizeof(float), (size_t)K * sizeof(float), n,
+                           cudaMemcpyDeviceToHost, h->stream));
+  }
+  CK(cudaStreamSynchronize(h->stream));
+  CKS();
+  return MRGAN_OK;
+}
+
+int mrgan_confusion(mrgan_handle* h, int32_t* out) {
+  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  if (!out) return fail(h, MRGAN_ERR_ARG, "confusion: null pointer");
+  int rc = need_local(h, "confusion"); if (rc) return rc;
+  const int K = h->cfg.n_classes;
+  if (h->cfg.model == MRGAN_MODEL_SVM) {
+#ifndef MRGAN_WITH_TC
+    return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
+#else
+    if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "confusion before mrgan_svm_fit");
+#endif
+  } else {
+    for (int f = 0; f < h->nf; ++f)
+      if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "confusion before mrgan_load_fold");
+  }
+  CK(cudaSetDevice(h->cfg.device));
+  rc = finish_pending(h); if (rc) return rc;
+  if (h->cfg.model != MRGAN_MODEL_SVM) enqueue_eval(h, 0, h->nf, false, 0, true);   // every fold in one pass; the SVM voted at fit
+  enqueue_confusion(h);
+  CK(cudaMemcpyAsync(out, h->d_conf, (size_t)h->nf * K * K * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  CKS();
+  return MRGAN_OK;
 }
 
 int64_t mrgan_kernel_launches(const mrgan_handle* h) { return h ? h->launches : -1; }

@@ -323,6 +323,43 @@ class FoldGroup:
         self._chk(self.lib.mrgan_svm_decision(self._h, int(fold), _lib.fptr(out)))
         return out
 
+    # ------------------------------------------------------------------ predictions (all three models)
+    def _n_scores(self):
+        return self.n_pairs if self.model == "svm" else self.cfg.n_classes
+
+    def predict(self, fold):
+        """Predicted classes of the fold's resident test set and their raw scores: (int32 [n_test], float32 [n_test, K])
+        logits (GAN / NN, phase 0) or (.., [n_test, n_pairs]) one-vs-one decision values (SVM)."""
+        n = self.shapes[fold][2]
+        pred = np.empty(n, dtype=np.int32)
+        scores = np.empty((n, self._n_scores()), dtype=np.float32)
+        self._chk(self.lib.mrgan_predict(self._h, int(fold), _lib.iptr(pred), _lib.fptr(scores)))
+        return pred, scores
+
+    def predict_rows(self, fold, x):
+        """predict() for new rows x [n, D] in the fold's SCALED input space (that of the resident X_test), in chunks of at
+        most n_test rows.  Leaves every later result on the resident test set unchanged."""
+        D, _, nte, _ = self.shapes[fold]
+        x = _f32(x)
+        if x.ndim != 2 or x.shape[1] != D or x.shape[0] < 1:
+            raise ValueError("predict_rows: x must be [n >= 1, %d]" % D)
+        n = x.shape[0]
+        pred = np.empty(n, dtype=np.int32)
+        scores = np.empty((n, self._n_scores()), dtype=np.float32)
+        for a in range(0, n, nte):
+            b = min(n, a + nte)
+            xc, pc, sc = x[a:b], pred[a:b], scores[a:b]       # contiguous row slices: the library writes straight into them
+            self._chk(self.lib.mrgan_predict_rows(self._h, int(fold), _lib.fptr(xc), b - a, _lib.iptr(pc), _lib.fptr(sc)))
+        return pred, scores
+
+    def confusion(self):
+        """Confusion counts of every fold's resident test set in one pass: int32 [n_folds, K, K], rows = true class,
+        columns = predicted class."""
+        K = self.cfg.n_classes
+        out = np.zeros((self.n_folds, K, K), dtype=np.int32)
+        self._chk(self.lib.mrgan_confusion(self._h, _lib.iptr(out)))
+        return out
+
     # ------------------------------------------------------------------ utilities
     def fill_normal(self, fold, step, tensor_id, rows, cols, row0=0):
         out = np.empty((rows, cols), dtype=np.float32)

@@ -11,7 +11,7 @@ import time
 import numpy as np
 from sklearn.model_selection import StratifiedKFold
 
-from . import foldprep, sweep, synthetic
+from . import foldprep, results, sweep, synthetic
 from .engine import FoldGroup
 from .model import MATERIALS, fold_key, init_disc, init_gen
 
@@ -39,14 +39,16 @@ def dataset(modalities=0, forcetempTime=4, contactmicTime=0.2, leaveObjectOut=Fa
 
 
 def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16', device=0, batch=50,
-                    eval_each_epoch=True, shared_t=True, return_group=False, device_perm=False):
+                    eval_each_epoch=True, shared_t=True, return_group=False, device_perm=False, details=False):
     """Train a GROUP of independent folds side by side on one GPU.
 
     jobs: list of dicts with keys ``trainTestSets`` (or ``X``, ``y``), ``percentlabeled``,
     ``percentunlabeled`` (optional), ``job_id`` (optional, seeds the fold's streams).
     device_perm: draw the epoch permutations of mr_gan.py:189-202 on the device (the host then sends one epoch number per
     epoch instead of 3 x int32[n_train] per fold); same distribution, different draws than the host's numpy generator.
-    Returns the list of test errors (mr_gan.py:230,234), one per job."""
+    Returns the list of test errors (mr_gan.py:230,234), one per job; details=True: one dict per job instead,
+    ``{'error': <the same float>, 'confusion': int32 [K, K]}`` (rows = true class, columns = predicted), from one extra
+    forward pass over every fold's test set."""
     folds, rngs, slots = [], [], {}
     for i, job in enumerate(jobs):
         rng = np.random.default_rng([int(seed), int(job.get('job_id', i))])
@@ -120,6 +122,8 @@ def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16',
         for e in errors:
             print('Test error:', e)
         sys.stdout.flush()
+    if details:
+        errors = [dict(error=e, confusion=c) for e, c in zip(errors, fg.confusion())]
     if return_group:
         return errors, fg
     fg.close()
@@ -195,6 +199,7 @@ def main(argv=None):
     parser.add_argument('--data-dir', default='data_processed')
     parser.add_argument('--synthetic', action='store_true', help='synthetic data of the MREO shape instead of the processed pickles')
     parser.add_argument('--host-perm', action='store_true', help='draw the epoch permutations on the host (numpy) instead of on the device')
+    results.add_arguments(parser)
     args = parser.parse_args(argv)
     rank, world, local = sweep.dist_env()
     seed = sweep.shared_seed(args.seed)          # one seed for every rank: same dataset, same splits, same job streams
@@ -202,6 +207,7 @@ def main(argv=None):
     if rank == 0:
         sys.stderr.write('seed: %d%s\n' % (seed, '   [SYNTHETIC data of the MREO shape: not the paper\'s dataset]' if args.synthetic else ''))
     jid = [0]
+    rep = results.Report(args, 'mr_gan', rank, say, seed=seed, precision=args.precision, epochs=args.epochs)
 
     def run(jobs):
         for j in jobs:
@@ -209,7 +215,8 @@ def main(argv=None):
             jid[0] += 1
         res = sweep.run_sharded(
             jobs, lambda js, dev: train_gan_folds(js, epochs=args.epochs, verbose=args.verbose, seed=seed,
-                                                  precision=args.precision, device=dev, device_perm=not args.host_perm),
+                                                  precision=args.precision, device=dev, device_perm=not args.host_perm,
+                                                  details=rep.details),
             group_size=args.group, key=job_rows, cost=job_cost)
         return res
 
@@ -225,17 +232,20 @@ def main(argv=None):
         for modality in range(len(MODALITIES)):
             X, y = dataset(modalities=modality, seed=seed, data_dir=args.data_dir, synthetic_data=args.synthetic)
             jobs += [j for p in percents for j in _kfold_jobs(X, y, seed + p, percentlabeled=p)]
-        errors = run(jobs)
+        res = run(jobs)
+        errors = results.errors(res)
         say('\n', '-' * 25, 'Testing various amounts of labeled training data', '-' * 25)
         say('-' * 100)
         for modality in range(len(MODALITIES)):
             say('-' * 25, MODALITIES[modality], 'modality', '-' * 25)
             for k, p in enumerate(percents):
                 say('-' * 15, 'Percentage of training data labeled: %d%%' % p, '-' * 15)
-                e = errors[42 * modality + 6 * k:42 * modality + 6 * k + 6]
+                a = 42 * modality + 6 * k
+                e = errors[a:a + 6]
                 for v in e:
                     say('Test error:', v, 'Test accuracy:', 1.0 - v)
                 report(e)
+                rep.setting(jobs[a:a + 6], res[a:a + 6], table=1, modality=MODALITIES[modality])
 
     if '3' in args.tables:                      # mr_gan.py:263-283
         say('\n', '-' * 25, 'Testing generalization with leave-one-object-out validation', '-' * 25)
@@ -245,13 +255,15 @@ def main(argv=None):
             objects = dataset(modalities=modality, leaveObjectOut=True, seed=seed, data_dir=args.data_dir, synthetic_data=args.synthetic)
             percents = [1, 4, 16, 50, 100]
             jobs = [j for p in percents for j in _loo_jobs(objects, percentlabeled=p)]
-            errors = run(jobs)
+            res = run(jobs)
+            errors = results.errors(res)
             n = len(objects)
             for k, p in enumerate(percents):
                 say('-' * 15, 'Percentage of training data labeled: %d%%' % p, '-' * 15)
                 for j, e in zip(jobs[n * k:n * k + n], errors[n * k:n * k + n]):
                     say(j['name'], 'Test error:', e, 'Test accuracy:', 1.0 - e)
                 report(errors[n * k:n * k + n], 'Average leave-one-object-out error:')
+                rep.setting(jobs[n * k:n * k + n], res[n * k:n * k + n], table=3, modality=MODALITIES[modality])
 
     if '5' in args.tables:                      # mr_gan.py:285-318
         for header_mods, times, is_contact in (([0, 1, 2], [4, 3, 2, 1, 0.5, 0.2, 0.1], False),
@@ -265,12 +277,14 @@ def main(argv=None):
                     kw = dict(contactmicTime=tm) if is_contact else dict(forcetempTime=tm)
                     X, y = dataset(modalities=modality, seed=seed, data_dir=args.data_dir, synthetic_data=args.synthetic, **kw)
                     jobs += _kfold_jobs(X, y, seed, percentlabeled=100)
-                errors = run(jobs)
+                res = run(jobs)
+                errors = results.errors(res)
                 for k, tm in enumerate(times):
                     say('-' * 15, 'Length of training data: %.1fs' % tm, '-' * 15)
                     for e in errors[6 * k:6 * k + 6]:
                         say('Test error:', e, 'Test accuracy:', 1.0 - e)
                     report(errors[6 * k:6 * k + 6])
+                    rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], table=5, modality=MODALITIES[modality], time=tm)
 
     if '6' in args.tables:                      # mr_gan.py:320-341
         say('\n', '-' * 25, 'Testing performance as quantity of unlabeled data increases', '-' * 25)
@@ -282,12 +296,15 @@ def main(argv=None):
                 say('-' * 15, 'Percentage of training data labeled: %d%%' % percentlabeled, '-' * 15)
                 unl = [0, 4, 8, 16, 32, 64, 100 - percentlabeled]
                 jobs = [j for pu in unl for j in _kfold_jobs(X, y, seed + pu, percentlabeled=percentlabeled, percentunlabeled=pu)]
-                errors = run(jobs)
+                res = run(jobs)
+                errors = results.errors(res)
                 for k, pu in enumerate(unl):
                     say('-' * 15, 'Percentage of training data unlabeled: %d%%' % pu, '-' * 15)
                     for e in errors[6 * k:6 * k + 6]:
                         say('Test error:', e, 'Test accuracy:', 1.0 - e)
                     report(errors[6 * k:6 * k + 6])
+                    rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], table=6, modality=MODALITIES[modality])
+    rep.close()
     return 0
 
 

@@ -12,7 +12,7 @@ import sys
 
 import numpy as np
 
-from . import foldprep, sweep
+from . import foldprep, results, sweep
 from .engine import FoldGroup
 from .model import MATERIALS, fold_key
 from .mr_gan import MODALITIES, _kfold_jobs, _loo_jobs, dataset, job_rows
@@ -31,11 +31,15 @@ def prepare_folds(jobs, seed):
     return folds
 
 
-def train_svm_folds(jobs, verbose=False, *, seed=0, device=0, C=1.0, gamma=None):
-    """Fit a group of independent mr_svm folds side by side; returns their test errors."""
+def train_svm_folds(jobs, verbose=False, *, seed=0, device=0, C=1.0, gamma=None, details=False):
+    """Fit a group of independent mr_svm folds side by side; returns their test errors, or with details=True one dict per
+    job, ``{'error': <the same float>, 'confusion': int32 [K, K]}`` (rows = true class, columns = predicted)."""
     fg, _ = fit_group(jobs, verbose, seed=seed, device=device, C=C, gamma=gamma)
     try:
-        return [fg.svm_eval(i) for i in range(len(jobs))]
+        errors = [fg.svm_eval(i) for i in range(len(jobs))]
+        if details:
+            errors = [dict(error=e, confusion=c) for e, c in zip(errors, fg.confusion())]
+        return errors
     finally:
         fg.close()
 
@@ -116,16 +120,18 @@ def main(argv=None):
     parser.add_argument('--group', type=int, default=42)
     parser.add_argument('--data-dir', default='data_processed')
     parser.add_argument('--synthetic', action='store_true', help='synthetic data of the MREO shape instead of the processed pickles')
+    results.add_arguments(parser)
     args = parser.parse_args(argv)
     rank, world, local = sweep.dist_env()
     seed = sweep.shared_seed(args.seed)
     say = print if rank == 0 else (lambda *a, **k: None)
     if rank == 0:
         sys.stderr.write('seed: %d%s\n' % (seed, '   [SYNTHETIC data of the MREO shape: not the paper\'s dataset]' if args.synthetic else ''))
+    rep = results.Report(args, 'mr_svm', rank, say, seed=seed)
 
     def run(jobs):
         return sweep.run_sharded(
-            jobs, lambda js, dev: train_svm_folds(js, verbose=args.verbose, seed=seed, device=dev),
+            jobs, lambda js, dev: train_svm_folds(js, verbose=args.verbose, seed=seed, device=dev, details=rep.details),
             group_size=args.group,
             key=lambda j: job_rows(j) + (j['percentlabeled'],),
             cost=lambda j: float(60 * j['percentlabeled']) ** 2)          # n_lab^2: kernel matrix and SMO row traffic
@@ -140,12 +146,14 @@ def main(argv=None):
                 say('\n', '-' * 25, 'Testing generalization with leave-one-object-out validation', '-' * 25)
             say('-' * 100)
         say('-' * 25, MODALITIES[modality], 'modality', '-' * 25)
-        errors = run(jobs)
+        res = run(jobs)
+        errors = results.errors(res)
         if t == '2':
             for k, p in enumerate(percents):
                 say('-' * 15, 'Percentage of training data labeled: %d%%' % p, '-' * 15)
                 e = errors[6 * k:6 * k + 6]
                 say('Average error:', np.mean(e), 'Average accuracy:', np.mean(1.0 - np.array(e)))
+                rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], table=2, modality=MODALITIES[modality])
                 sys.stdout.flush()
         else:
             n = len(objects)
@@ -155,7 +163,9 @@ def main(argv=None):
                     say(j['name'], 'Test error:', e, 'Test accuracy:', 1.0 - e)
                 e = errors[n * k:n * k + n]
                 say('Average leave-one-object-out error:', np.mean(e), 'Average accuracy:', np.mean(1.0 - np.array(e)))
+                rep.setting(jobs[n * k:n * k + n], res[n * k:n * k + n], table=4, modality=MODALITIES[modality])
                 sys.stdout.flush()
+    rep.close()
     return 0
 
 
