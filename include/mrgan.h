@@ -207,6 +207,20 @@ int  mrgan_predict(mrgan_handle* h, int fold, int32_t* pred, float* scores);
 int  mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t* pred, float* scores);
 int  mrgan_confusion(mrgan_handle* h, int32_t* out);
 
+/* Input gradients of a trained GAN / NN fold (the activation maps of the reference's others/mr_nn_activation_map.py):
+ *   grad[r][j] = d log softmax(l(x_r))[t_r] / d x_r[j], l = the phase-0 logits of mrgan_predict, x in the fold's SCALED space.
+ *   x: rows [n][D_fold], or NULL = the fold's resident X_test (then n must equal its n_test); 1 <= n <= n_test
+ *   target: [n] classes in [0, K), or NULL = each row's predicted class (first maximal logit)
+ *   grad: [n][D_fold] */
+int  mrgan_input_grad(mrgan_handle* h, int fold, const float* x, int n, const int32_t* target, float* grad);
+/* Every fold of the handle in one pass over its resident test set, target = the true class:
+ *   profile [n_folds][K][D_max] = mean over the test rows of true class c of |grad[r][j]|; 0 beyond a fold's D and for a
+ *   class without test rows.  Fixed summation order: bitwise reproducible and independent of the grouping.
+ * MRGAN_ERR_ARG: null grad / profile, fold or n out of range, x == NULL with n != n_test, a target outside [0, K).
+ * MRGAN_ERR_STATE: an SVM handle, a fold not loaded, or a data-parallel handle.  Like mrgan_predict, each call first completes
+ * a pending asynchronous epoch, whose statistics it leaves unchanged, and changes no later result of the handle. */
+int  mrgan_saliency(mrgan_handle* h, float* profile);
+
 /* Utilities used by tests and bench */
 int  mrgan_fill_normal(mrgan_handle* h, int fold, int step, int tensor_id, int rows, int cols,
                        int row0, float* dst /* host [rows, cols] */);
@@ -221,7 +235,9 @@ enum { MRGAN_TIME_ADAM_D = 0, MRGAN_TIME_ADAM_G = 1, MRGAN_TIME_DW1 = 2, MRGAN_T
        /* SVM handles, after mrgan_svm_fit (re-running a phase reproduces its results bitwise): */
        MRGAN_TIME_SVM_KMAT = 7,     /* both kernel matrices of all folds (operand split + tcgen05 GEMM + RBF) */
        MRGAN_TIME_SVM_SMO = 8,      /* the SMO solver of every (fold, class pair) */
-       MRGAN_TIME_SVM_PREDICT = 9 };/* decision values, vote and error count of every test row */
+       MRGAN_TIME_SVM_PREDICT = 9, /* decision values, vote and error count of every test row */
+       /* GAN / NN handles, read-only (the training state is unchanged): */
+       MRGAN_TIME_SALIENCY = 10 }; /* mrgan_saliency's pass: eval forward, seed, dX chain and profile of every fold */
 int  mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg);
 /* Debug/test hook: copy an intermediate buffer of the last step of one fold to the host
  * (dst is [rows, cols] dense).  which: 0..5 = noisy layer inputs a[l], 10+l = post-ReLU h[l],

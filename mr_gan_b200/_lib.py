@@ -73,6 +73,8 @@ SYMBOLS = {
     "mrgan_predict": (C.c_int, [_H, C.c_int, _ip, _fp]),
     "mrgan_predict_rows": (C.c_int, [_H, C.c_int, _fp, C.c_int, _ip, _fp]),
     "mrgan_confusion": (C.c_int, [_H, _ip]),
+    "mrgan_input_grad": (C.c_int, [_H, C.c_int, _fp, C.c_int, _ip, _fp]),
+    "mrgan_saliency": (C.c_int, [_H, _fp]),
     "mrgan_fill_normal": (C.c_int, [_H, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _fp]),
     "mrgan_adam_flat": (C.c_int, [_H, _fp, _fp, _fp, _fp, C.c_int64, C.c_int]),
     "mrgan_time_op": (C.c_int, [_H, C.c_int, C.c_int, _fp]),

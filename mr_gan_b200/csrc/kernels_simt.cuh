@@ -772,6 +772,62 @@ __global__ void __launch_bounds__(256) k_confusion(const EvalDesc* __restrict__ 
   for (int i = threadIdx.x; i < K * K; i += blockDim.x) if (cnt[i]) atomicAdd(&o[i], cnt[i]);
 }
 
+// ------------------------------------------------------------------ input gradients (mrgan_input_grad / mrgan_saliency)
+// Seed of the backward pass of log softmax(l)_t: d/dl = e_t - softmax(l), written over the row's phase-0 logits (read by
+// nothing after the eval) in the dX operand format of the handle, like the logit gradients of k_loss_disc.  t = d.y[r], or with
+// use_pred the row's predicted class (row_argmax).  One thread per row; grid (row blocks, 1, folds).
+__global__ void __launch_bounds__(256)
+k_logprob_seed(const EvalDesc* __restrict__ descs, int n_override, int K, int use_pred, OperandMode om) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const EvalDesc d = descs[blockIdx.z];
+  const int n = n_override > 0 ? n_override : d.n;
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  float* const l = const_cast<float*>(d.logits) + (size_t)r * d.ld;
+  const int t = use_pred ? row_argmax(l, K) : d.y[r];
+  float mx = l[0];
+  for (int k = 1; k < K; ++k) mx = fmaxf(mx, l[k]);
+  float se = 0.f;
+  for (int k = 0; k < K; ++k) se += expf(l[k] - mx);
+  const float inv = 1.0f / se;
+  for (int k = 0; k < K; ++k) put_grad_operand(l + k, (k == t ? 1.f : 0.f) - expf(l[k] - mx) * inv, om);   // reads l[k] first
+}
+
+// f16 mode: the fp32 input gradients of OP_EX1 (C [M][ldc], N = D columns) carry the loss scale of the dX operands; ginv divides
+// it out in place (a power of two: exact).  grid (blocks, 1, folds).
+__global__ void __launch_bounds__(256) k_unscale_grad(const GemmDesc* __restrict__ descs, int rows_override, float ginv) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const GemmDesc g = descs[blockIdx.z];
+  const int M = rows_override > 0 ? rows_override : g.M;
+  const size_t n = (size_t)M * g.N;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+    g.C[(i / g.N) * g.ldc + i % g.N] *= ginv;
+}
+
+// Saliency profile of every fold: out[f][c][j] = (1 / N_c) sum over the fold's test rows r with y_r = c of |grad[r][j]|, grad =
+// the OP_EX1 output (descs[f].C, d.n rows), N_c = the number of such rows; 0 for a class without rows and for j >= D.  One
+// thread per (fold, feature) and class, summing in double in row order: no atomics, so the result is bitwise reproducible and
+// independent of the grouping of the folds.  grid (feature blocks, folds).
+__global__ void __launch_bounds__(128)
+k_saliency(const GemmDesc* __restrict__ gx, const EvalDesc* __restrict__ ev, int K, int Dmax, float* __restrict__ out) {
+  pdl_wait();
+  const int f = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= Dmax) return;
+  const GemmDesc g = gx[f];
+  const EvalDesc e = ev[f];
+  float* const o = out + (size_t)f * K * Dmax + j;
+  for (int c = 0; c < K; ++c) {
+    double s = 0.0;
+    int nc = 0;
+    if (j < g.N)
+      for (int r = 0; r < e.n; ++r)
+        if (e.y[r] == c) { s += fabs((double)g.C[(size_t)r * g.ldc + j]); ++nc; }
+    o[(size_t)c * Dmax] = nc > 0 ? (float)(s / nc) : 0.f;
+  }
+}
+
 // Means over the epoch's batches (mr_gan.py:215-217) -> epoch_stats[f][0..3]; [4] = batch-wise test error.
 __global__ void k_epoch_reduce(const float* __restrict__ step_stats, const EvalDesc* __restrict__ evals,
                                float* __restrict__ epoch_stats, int nf, int nb, int with_eval) {

@@ -36,8 +36,14 @@ enum Op {
   OP_DX2G, OP_DX3G, OP_DX4G, OP_DX5G,          // G step: dX chain over the B fake rows
   OP_GW1, OP_GW2, OP_GW3, OP_GX2, OP_GX3,
   OP_E1, OP_E1S, OP_E2, OP_E3, OP_E4, OP_E5, OP_E6,
-  NUM_OPS
+  NUM_OPS,
+  // eval backward (mrgan_input_grad / mrgan_saliency), the twins of OP_DX2..6 / OP_DX1G over the phase-0 activations.  Their
+  // device descriptors live in a workspace made on first use (SalWork), outside the arena's [NUM_OPS][nf] table.
+  OP_EX2 = NUM_OPS, OP_EX3, OP_EX4, OP_EX5, OP_EX6,   // OP_EXl: dZ[l] -> dZ[l-1], written over eh[l-1]
+  OP_EX1,                                            // dZ[1] -> d/dx, fp32 into ex_stage
+  NUM_OPS_ALL
 };
+constexpr int NUM_EX = NUM_OPS_ALL - NUM_OPS;
 
 struct OpInfo { bool at = false, bt = false, used = false; int maxM = 0, maxN = 0; };
 
@@ -77,6 +83,7 @@ struct mrgan_handle;
 #ifdef MRGAN_WITH_TC
 namespace {
 int tc_setup(mrgan_handle* h);
+int tc_ex_setup(mrgan_handle* h, TcOp* dst);
 void tc_teardown(mrgan_handle* h);
 bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st);
 void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cudaStream_t st);
@@ -112,8 +119,17 @@ struct mrgan_handle {
   PermDesc* d_perm = nullptr;
   BnDesc* d_bn = nullptr; LossDesc* d_loss = nullptr; EvalDesc *d_eval = nullptr, *d_eval_s = nullptr;
   int* d_conf = nullptr;              // [nf][K][K] confusion counts (mrgan_confusion)
+  // mrgan_input_grad / mrgan_saliency: one allocation on first use (a handle that never calls them allocates nothing more)
+  struct SalWork {
+    char* mem = nullptr;
+    GemmDesc* descs = nullptr;        // [NUM_EX][nf] device copies of the OP_EX* descriptors
+    float* profile = nullptr;         // [nf][K][D_max]
+#ifdef MRGAN_WITH_TC
+    TcOp* tcops = nullptr;            // [NUM_EX][nf] their tcgen05 views (tf32 / f16 handles)
+#endif
+  } sal;
   AdamRange* d_ranges[2] = {nullptr, nullptr};
-  OpInfo ops[NUM_OPS];
+  OpInfo ops[NUM_OPS_ALL];
   float *d_step_stats = nullptr, *d_epoch_stats = nullptr, *h_epoch_stats = nullptr;
   int* h_idx_pinned[2] = {nullptr, nullptr}; cudaEvent_t idx_free[2] = {nullptr, nullptr}; int idx_slot = 0;
   float* h_scratch = nullptr;   // pinned scalars for the step API
@@ -143,9 +159,9 @@ struct mrgan_handle {
   float* dp_losspart = nullptr; unsigned* dp_lossctr = nullptr;    // k_loss_disc block partials [nf][4*64] and arrival counters [nf]
 #ifdef MRGAN_WITH_TC
   TcOp* d_tcops = nullptr;            // [NUM_OPS][nf] tensor maps + epilogue descriptors
-  int tc_bn[NUM_OPS] = {0}, tc_maxME[NUM_OPS] = {0}, tc_maxNE[NUM_OPS] = {0};
+  int tc_bn[NUM_OPS_ALL] = {0}, tc_maxME[NUM_OPS_ALL] = {0}, tc_maxNE[NUM_OPS_ALL] = {0};
   int tc_ksplit[NUM_OPS] = {0};       // large-batch dW: contraction slices per tile (deterministic split-K), 0/1 = off
-  bool tc_mt1[NUM_OPS] = {false};     // large-batch forward / dX whose 256 x 256 tiling would leave SMs idle: 128-feature CTAs (tc_pick_tile)
+  bool tc_mt1[NUM_OPS_ALL] = {false}; // large-batch forward / dX whose 256 x 256 tiling would leave SMs idle: 128-feature CTAs (tc_pick_tile)
   float* d_tcws = nullptr;            // ... and their partial-product workspace
   bool tc_fused_adam = true;          // dW epilogue applies Adam in place (no gradient round trip)
   bool tc_mt2 = true;                 // forward / dX: 256 features per CTA where the layer is wide enough (MRGAN_MT2=0 disables)
@@ -356,7 +372,7 @@ int build_descs(mrgan_handle* h) {
   const mrgan_config& c = h->cfg;
   const int B = c.batch, R = h->R, K = c.n_classes, nd = c.noise_dim, nf = h->nf;
   const bool gan = c.model == MRGAN_MODEL_GAN;
-  h->h_descs.assign((size_t)NUM_OPS * nf, GemmDesc{});
+  h->h_descs.assign((size_t)NUM_OPS_ALL * nf, GemmDesc{});
   h->h_folds.assign(nf, FoldState{});
   std::vector<BnDesc> bn(nf); std::vector<LossDesc> ls(nf); std::vector<EvalDesc> ev(nf), evs(nf);
   std::vector<AdamRange> rg0(nf), rg1(nf);
@@ -411,8 +427,19 @@ int build_descs(mrgan_handle* h) {
         x.aux = (dropout && l - 1 <= 4) ? b.a[l - 1] : b.hb[l - 1]; x.ldaux = b.lda[l - 1]; x.tid = (l - 1 <= 4) ? l - 1 : 0;
         setop(OP_DX2 + l - 2, f, x, false, true, 1);
         if (gan && l <= 5) { GemmDesc xg = x; xg.M = B; setop(OP_DX2G + l - 2, f, xg, false, true, 1); }
+        // eval twin: the fold's test rows, act' from the clean activation (phase 0 has no Dropout), and dZ[l-1] written over
+        // that activation in place -- the epilogue reads h and writes dZ at the same element, and h is no operand of the GEMM
+        // (the ones column at index win[l-1] is outside N and stays)
+        GemmDesc ex = make_desc(EC, ldc, PD + W.off, W.pitch, b.eh[l - 1], b.lda[l - 1], h->shapes[f].n_test, win[l - 1], wout[l - 1],
+                                EPI_DX, hact, f);
+        ex.aux = b.eh[l - 1]; ex.ldaux = b.lda[l - 1]; ex.tid = 0;
+        setop(OP_EX2 + l - 2, f, ex, false, true, 1);
       }
     }
+    // d/dx = dZ[1] @ W1^T in fp32 (no activation: x is the input), over the staging rows
+    const TensorLayout& EW1 = LD.t[0];
+    setop(OP_EX1, f, make_desc(b.eh[1], b.lda[1], PD + EW1.off, EW1.pitch, b.ex_stage, b.lda[0], h->shapes[f].n_test, D, kDW[0], EPI_DX,
+                               ACT_NONE, f), false, true);
     rg0[f] = AdamRange{LD.off, LD.n};
     ls[f] = LossDesc{b.lg, b.dlg, pitch8(K), b.labels_cur, b.hb[5], b.dz[5], b.lda[5], b.ldz[5], kDW[4]};
     ev[f] = EvalDesc{b.elg, pitch8(K), b.yte, h->shapes[f].n_test, (h->shapes[f].n_test / B) * B, b.eval_out, b.pred};
@@ -453,7 +480,7 @@ int build_descs(mrgan_handle* h) {
     fs.a0 = b.a[0]; fs.lda0 = b.lda[0]; fs.z = gan ? b.zb : nullptr; fs.ldz = pitch8(nd + 1);
     fs.labels_cur = b.labels_cur;
   }
-  CK(cudaMemcpy(h->d_descs, h->h_descs.data(), h->h_descs.size() * sizeof(GemmDesc), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(h->d_descs, h->h_descs.data(), (size_t)NUM_OPS * nf * sizeof(GemmDesc), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(h->d_folds, h->h_folds.data(), nf * sizeof(FoldState), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(h->d_loss, ls.data(), nf * sizeof(LossDesc), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(h->d_eval, ev.data(), nf * sizeof(EvalDesc), cudaMemcpyHostToDevice));
@@ -674,7 +701,7 @@ void launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cu
   const OpInfo& oi = h->ops[op];
   int M = oi.maxM;
   if (rows_override > 0 && !oi.at) M = rows_override;
-  const GemmDesc* d = h->d_descs + (size_t)op * h->nf + f0;
+  const GemmDesc* d = (op < NUM_OPS ? h->d_descs + (size_t)op * h->nf : h->sal.descs + (size_t)(op - NUM_OPS) * h->nf) + f0;
 #ifdef MRGAN_WITH_TC
   if (h->cfg.precision != MRGAN_PREC_FP32 && tc_launch_gemm(h, op, f0, nfl, rows_override, st)) return;
 #endif
@@ -902,6 +929,63 @@ void enqueue_confusion(mrgan_handle* h) {
   for (int f = 0; f < h->nf; ++f) nmax = std::max(nmax, h->shapes[f].n_test);
   cudaMemsetAsync(h->d_conf, 0, (size_t)h->nf * K * K * sizeof(int), h->stream);
   launch_k(h, k_confusion, dim3((nmax + CONF_ROWS - 1) / CONF_ROWS, h->nf), dim3(256), 0, h->stream, (const EvalDesc*)h->d_eval, K, h->d_conf);
+}
+
+// Input gradients d log softmax(l)_t / dx of the phase-0 logits l of folds [f0, f0 + nfl) (mrgan_input_grad / mrgan_saliency):
+// the eval forward, the seed e_t - softmax(l) over the logits, then the dX chain OP_EX6 .. OP_EX2 over the eval activations (each
+// dZ over the activation it came from) and OP_EX1 into ex_stage, fp32.  Targets: the rows' predicted classes (TGT_PRED), the
+// resident test labels (TGT_TEST) or the staged labels (TGT_STAGED).  Needs saliency_setup.
+enum { TGT_PRED = 0, TGT_TEST = 1, TGT_STAGED = 2 };
+void enqueue_input_grad(mrgan_handle* h, int f0, int nfl, bool staged, int n_override, int tgt) {
+  enqueue_eval(h, f0, nfl, staged, n_override);
+  int n = n_override;
+  for (int f = f0; f < f0 + nfl && n_override <= 0; ++f) n = std::max(n, h->shapes[f].n_test);
+  launch_k(h, k_logprob_seed, dim3((n + 255) / 256, 1, nfl), dim3(256), 0, h->stream,
+           (const EvalDesc*)((tgt == TGT_STAGED ? h->d_eval_s : h->d_eval) + f0), n_override, h->cfg.n_classes, (int)(tgt == TGT_PRED), h->om);
+  for (int l = 6; l >= 1; --l) launch_gemm(h, l >= 2 ? OP_EX2 + l - 2 : OP_EX1, f0, nfl, n_override);
+  if (h->om.mode == 2)
+    launch_k(h, k_unscale_grad, dim3(std::min((n * max_D(h, f0, nfl) + 255) / 256, 1184), 1, nfl), dim3(256), 0, h->stream,
+             (const GemmDesc*)(h->sal.descs + (size_t)(OP_EX1 - NUM_OPS) * h->nf + f0), n_override, 1.0f / h->om.gscale);
+}
+
+// mrgan_saliency's pass over every fold's resident test set: input gradients for the true classes, then the class means
+void enqueue_saliency(mrgan_handle* h) {
+  const int Dmax = max_D(h, 0, h->nf);
+  enqueue_input_grad(h, 0, h->nf, false, 0, TGT_TEST);
+  launch_k(h, k_saliency, dim3((Dmax + 127) / 128, h->nf), dim3(128), 0, h->stream,
+           (const GemmDesc*)(h->sal.descs + (size_t)(OP_EX1 - NUM_OPS) * h->nf), (const EvalDesc*)h->d_eval, h->cfg.n_classes, Dmax, h->sal.profile);
+}
+
+// the workspace of the input-gradient entry points (descriptors of the OP_EX* ops, the profile), on first use
+int saliency_setup(mrgan_handle* h) {
+  mrgan_handle::SalWork& S = h->sal;
+  if (S.mem) return MRGAN_OK;
+  const int nf = h->nf;
+  const bool tc = h->cfg.precision != MRGAN_PREC_FP32;
+  auto layout = [&](Arena& ar) {
+    S.descs = ar.take<GemmDesc>((size_t)NUM_EX * nf);
+    S.profile = ar.take<float>((size_t)nf * h->cfg.n_classes * max_D(h, 0, nf));
+#ifdef MRGAN_WITH_TC
+    S.tcops = tc ? ar.take<TcOp>((size_t)NUM_EX * nf) : nullptr;
+#endif
+  };
+  Arena sizing;
+  layout(sizing);
+  char* mem = nullptr;
+  CK(cudaMalloc(&mem, sizing.off + 256));
+  Arena real; real.base = mem;
+  layout(real);
+  int rc = MRGAN_OK;
+  if (cudaMemcpy(S.descs, h->h_descs.data() + (size_t)NUM_OPS * nf, (size_t)NUM_EX * nf * sizeof(GemmDesc), cudaMemcpyHostToDevice) != cudaSuccess)
+    rc = fail(h, MRGAN_ERR_CUDA, "saliency workspace: descriptor upload failed");
+#ifdef MRGAN_WITH_TC
+  if (rc == MRGAN_OK && tc) rc = tc_ex_setup(h, S.tcops);
+#else
+  (void)tc;
+#endif
+  if (rc != MRGAN_OK) { cudaFree(mem); return rc; }
+  S.mem = mem;
+  return MRGAN_OK;
 }
 
 // prediction entry points: the single-GPU handle only (data-parallel replicas are out of their scope)
@@ -1183,6 +1267,46 @@ int tc_debug_gemm(mrgan_handle* h, int mode, const GemmDesc& g, int esz) {
   return MRGAN_OK;
 }
 
+// the tcgen05 views of op's descriptors, one per fold (t[0 .. nf)), and the op's tile geometry; no-op for an unused op
+int tc_make_op(mrgan_handle* h, EncodeTiledFn fn, int op, TcOp* ts) {
+  const OpInfo& oi = h->ops[op];
+  if (!oi.used) return MRGAN_OK;
+  const int nf = h->nf;
+  for (int f = 0; f < nf; ++f) {
+    const GemmDesc& g = h->h_descs[(size_t)op * nf + f];
+    TcOp& t = ts[f];
+    const int mode = (!oi.at && !oi.bt) ? 0 : ((!oi.at && oi.bt) ? 1 : 2);
+    int bn_big = 256;
+    if (mode != 2 && oi.maxM > 256) { bool m1; tc_pick_tile(oi.maxM, oi.maxN, nf, &bn_big, &m1); h->tc_mt1[op] = m1; }
+    if (h->om.mode == 2) {    // operands come from the fp16 copies (same element offsets and pitches as the fp32 buffers)
+      GemmDesc gh = g;
+      gh.A = reinterpret_cast<const float*>(h->harena + (g.A - h->om.fbase));
+      gh.B = reinterpret_cast<const float*>(h->harena + (g.B - h->om.fbase));
+      if (!tc_fill_op(fn, t, gh, mode, 2, bn_big)) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled (fp16 operands) failed");
+      t.g = g;                // the epilogue keeps addressing the fp32 buffers (and derives the copies' addresses itself)
+    } else if (!tc_fill_op(fn, t, g, mode, 4, bn_big)) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
+    t.net = (op == OP_GW1 || op == OP_GW2 || op == OP_GW3) ? 1 : 0;
+    if (h->tc_heads) {
+      t.stats = h->d_step_stats + (size_t)f * 4;
+      t.stats_stride = nf * 4;
+      t.mo_off = h->Mo - h->P; t.vo_off = h->Vo - h->P;
+      if (op == OP_D6 && (h->tc_heads & 1)) { t.head = HEAD_DISC; t.hd = h->d_loss + f; t.advance = 1; }
+      else if (op == OP_D5G && (h->tc_heads & 2)) { t.head = HEAD_FM; t.hd = h->d_loss + f; t.advance = (h->tc_heads & 8) ? 1 : 0; }
+      else if (op == OP_G1 && (h->tc_heads & 4)) { t.head = HEAD_BN; t.hd = h->d_bn + f; }
+      else if (op == OP_GX2 && (h->tc_heads & 8)) { t.head = HEAD_BN_BWD; t.hd = h->d_bn + f; }
+    }
+    if (mode == 2) {
+      if (h->tc_fused_adam) t.epi = EPI_ADAM;
+      const size_t off = (size_t)(g.C - h->Gr);
+      t.P = h->P + off; t.Mo = h->Mo + off; t.Vo = h->Vo + off;
+    }
+    if (t.bn > h->tc_bn[op]) h->tc_bn[op] = t.bn;
+    if (t.ME > h->tc_maxME[op]) h->tc_maxME[op] = t.ME;
+    if (t.NE > h->tc_maxNE[op]) h->tc_maxNE[op] = t.NE;
+  }
+  return MRGAN_OK;
+}
+
 int tc_setup(mrgan_handle* h) {
   EncodeTiledFn fn = tc_encoder();
   if (!fn) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
@@ -1202,40 +1326,8 @@ int tc_setup(mrgan_handle* h) {
   std::vector<TcOp> ops((size_t)NUM_OPS * nf);
   memset(ops.data(), 0, ops.size() * sizeof(TcOp));
   for (int op = 0; op < NUM_OPS; ++op) {
-    const OpInfo& oi = h->ops[op];
-    if (!oi.used) continue;
-    for (int f = 0; f < nf; ++f) {
-      const GemmDesc& g = h->h_descs[(size_t)op * nf + f];
-      TcOp& t = ops[(size_t)op * nf + f];
-      const int mode = (!oi.at && !oi.bt) ? 0 : ((!oi.at && oi.bt) ? 1 : 2);
-      int bn_big = 256;
-      if (mode != 2 && oi.maxM > 256) { bool m1; tc_pick_tile(oi.maxM, oi.maxN, nf, &bn_big, &m1); h->tc_mt1[op] = m1; }
-      if (h->om.mode == 2) {    // operands come from the fp16 copies (same element offsets and pitches as the fp32 buffers)
-        GemmDesc gh = g;
-        gh.A = reinterpret_cast<const float*>(h->harena + (g.A - h->om.fbase));
-        gh.B = reinterpret_cast<const float*>(h->harena + (g.B - h->om.fbase));
-        if (!tc_fill_op(fn, t, gh, mode, 2, bn_big)) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled (fp16 operands) failed");
-        t.g = g;                // the epilogue keeps addressing the fp32 buffers (and derives the copies' addresses itself)
-      } else if (!tc_fill_op(fn, t, g, mode, 4, bn_big)) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-      t.net = (op == OP_GW1 || op == OP_GW2 || op == OP_GW3) ? 1 : 0;
-      if (h->tc_heads) {
-        t.stats = h->d_step_stats + (size_t)f * 4;
-        t.stats_stride = nf * 4;
-        t.mo_off = h->Mo - h->P; t.vo_off = h->Vo - h->P;
-        if (op == OP_D6 && (h->tc_heads & 1)) { t.head = HEAD_DISC; t.hd = h->d_loss + f; t.advance = 1; }
-        else if (op == OP_D5G && (h->tc_heads & 2)) { t.head = HEAD_FM; t.hd = h->d_loss + f; t.advance = (h->tc_heads & 8) ? 1 : 0; }
-        else if (op == OP_G1 && (h->tc_heads & 4)) { t.head = HEAD_BN; t.hd = h->d_bn + f; }
-        else if (op == OP_GX2 && (h->tc_heads & 8)) { t.head = HEAD_BN_BWD; t.hd = h->d_bn + f; }
-      }
-      if (mode == 2) {
-        if (h->tc_fused_adam) t.epi = EPI_ADAM;
-        const size_t off = (size_t)(g.C - h->Gr);
-        t.P = h->P + off; t.Mo = h->Mo + off; t.Vo = h->Vo + off;
-      }
-      if (t.bn > h->tc_bn[op]) h->tc_bn[op] = t.bn;
-      if (t.ME > h->tc_maxME[op]) h->tc_maxME[op] = t.ME;
-      if (t.NE > h->tc_maxNE[op]) h->tc_maxNE[op] = t.NE;
-    }
+    const int rc = tc_make_op(h, fn, op, &ops[(size_t)op * nf]);
+    if (rc != MRGAN_OK) return rc;
   }
   // Large-batch dW without the fused Adam: the narrow layers' gradients are a handful of 256x256 tiles with a contraction of
   // thousands of rows -> split the contraction over ~2 CTAs per SM, partial products to a workspace, summed in slice order.
@@ -1325,6 +1417,20 @@ int tc_setup(mrgan_handle* h) {
   return MRGAN_OK;
 }
 
+// the tcgen05 views of the eval-backward ops (OP_EX*), made on the first mrgan_input_grad / mrgan_saliency -> dst [NUM_EX][nf]
+int tc_ex_setup(mrgan_handle* h, TcOp* dst) {
+  EncodeTiledFn fn = tc_encoder();
+  if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
+  std::vector<TcOp> ops((size_t)NUM_EX * h->nf);
+  memset(ops.data(), 0, ops.size() * sizeof(TcOp));
+  for (int op = NUM_OPS; op < NUM_OPS_ALL; ++op) {
+    const int rc = tc_make_op(h, fn, op, &ops[(size_t)(op - NUM_OPS) * h->nf]);
+    if (rc != MRGAN_OK) return rc;
+  }
+  CK(cudaMemcpy(dst, ops.data(), ops.size() * sizeof(TcOp), cudaMemcpyHostToDevice));
+  return MRGAN_OK;
+}
+
 void tc_teardown(mrgan_handle* h) {
   if (h->d_tcops) cudaFree(h->d_tcops);
   if (h->d_tcadam) cudaFree(h->d_tcadam);
@@ -1367,7 +1473,7 @@ bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override,
   int NE = h->tc_maxNE[op];
   if (rows_override > 0 && !oi.at) NE = rows_override;
   dim3 grid((h->tc_maxME[op] + 127) / 128, (NE + bn - 1) / bn, nfl);
-  const TcOp* d = h->d_tcops + (size_t)op * h->nf + f0;
+  const TcOp* d = (op < NUM_OPS ? h->d_tcops + (size_t)op * h->nf : h->sal.tcops + (size_t)(op - NUM_OPS) * h->nf) + f0;
   if (bn == 256 && (oi.at || h->tc_maxME[op] >= 500) && !h->tc_mt1[op]) {     // large-batch regime
     grid.x = (h->tc_maxME[op] + 255) / 256;
     const size_t smem = tc_smem_bytes(256, TC_BIG_STAGES, 2);
@@ -1592,6 +1698,7 @@ int mrgan_destroy(mrgan_handle* h) {
     }
   if (h->d_dpmem) cudaFree(h->d_dpmem);
   if (h->d_dpbufs) cudaFree(h->d_dpbufs);
+  if (h->sal.mem) cudaFree(h->sal.mem);
 #ifdef MRGAN_WITH_TC
   tc_teardown(h);
   if (h->svm.mem) cudaFree(h->svm.mem);
@@ -2092,14 +2199,16 @@ int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
   if (!ms_avg || reps < 1) return fail(h, MRGAN_ERR_ARG, "time_op: bad argument");
   const bool svm = h->cfg.model == MRGAN_MODEL_SVM;
   if (svm != (which >= MRGAN_TIME_SVM_KMAT && which <= MRGAN_TIME_SVM_PREDICT))
-    return fail(h, which < 0 || which > MRGAN_TIME_SVM_PREDICT ? MRGAN_ERR_ARG : MRGAN_ERR_STATE, "time_op: op does not exist for this model");
+    return fail(h, which < 0 || which > MRGAN_TIME_SALIENCY ? MRGAN_ERR_ARG : MRGAN_ERR_STATE, "time_op: op does not exist for this model");
   if (svm) return svm_time_op(h, which, reps, ms_avg);
   const bool gan = h->cfg.model == MRGAN_MODEL_GAN;
   if (!gan && (which == MRGAN_TIME_ADAM_G || which == MRGAN_TIME_GEN_STEP || which == MRGAN_TIME_DX1)) return fail(h, MRGAN_ERR_STATE, "time_op: no generator in this model");
   for (int f = 0; f < h->nf; ++f)
     if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "time_op before mrgan_load_fold");
+  if (which == MRGAN_TIME_SALIENCY) { const int rc0 = need_local(h, "time_op"); if (rc0) return rc0; }
   CK(cudaSetDevice(h->cfg.device));
   int rc = finish_pending(h); if (rc) return rc;
+  if (which == MRGAN_TIME_SALIENCY) { rc = saliency_setup(h); if (rc) return rc; }
   auto once = [&]() {
     switch (which) {
       case MRGAN_TIME_ADAM_D: launch_adam(h, 0, h->nf, 0, false); break;
@@ -2109,10 +2218,11 @@ int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
       case MRGAN_TIME_DISC_STEP: if (gan) enqueue_disc_step(h, 0, h->nf, 0, 0); else enqueue_nn_step(h, 0, h->nf, 0, 0, h->cfg.batch); break;
       case MRGAN_TIME_GEN_STEP: enqueue_gen_step(h, 0, h->nf, 0, 0); break;
       case MRGAN_TIME_DX1: launch_gemm(h, OP_DX1G, 0, h->nf, 0); break;
+      case MRGAN_TIME_SALIENCY: enqueue_saliency(h); break;
       default: break;
     }
   };
-  if (which < 0 || which > MRGAN_TIME_DX1) return fail(h, MRGAN_ERR_ARG, "time_op: unknown op");
+  if (which < 0 || (which > MRGAN_TIME_DX1 && which != MRGAN_TIME_SALIENCY)) return fail(h, MRGAN_ERR_ARG, "time_op: unknown op");
   once();                                   // warm-up
   CK(cudaEventRecord(h->ev0, h->stream));
   for (int i = 0; i < reps; ++i) once();
@@ -2742,6 +2852,59 @@ int mrgan_confusion(mrgan_handle* h, int32_t* out) {
   if (h->cfg.model != MRGAN_MODEL_SVM) enqueue_eval(h, 0, h->nf, false, 0, true);   // every fold in one pass; the SVM voted at fit
   enqueue_confusion(h);
   CK(cudaMemcpyAsync(out, h->d_conf, (size_t)h->nf * K * K * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  CKS();
+  return MRGAN_OK;
+}
+
+// ------------------------------------------------------------------ input gradients and saliency profiles
+int mrgan_input_grad(mrgan_handle* h, int fold, const float* x, int n, const int32_t* target, float* grad) {
+  int rc = check_fold(h, fold); if (rc) return rc;
+  rc = need_nets(h, "input_grad"); if (rc) return rc;
+  if (!grad) return fail(h, MRGAN_ERR_ARG, "input_grad: null pointer");
+  const int D = h->shapes[fold].D, K = h->cfg.n_classes, nte = h->shapes[fold].n_test;
+  if (n < 1 || n > nte) return fail(h, MRGAN_ERR_ARG, "input_grad: n must be in [1, n_test of the fold]");
+  if (!x && n != nte) return fail(h, MRGAN_ERR_ARG, "input_grad: the resident test set (x = NULL) has n_test rows");
+  if (target)
+    for (int i = 0; i < n; ++i)
+      if (target[i] < 0 || target[i] >= K) return fail(h, MRGAN_ERR_ARG, "input_grad: target class out of range");
+  rc = need_local(h, "input_grad"); if (rc) return rc;
+  FoldBuffers& b = h->fb[fold];
+  if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "input_grad before mrgan_load_fold");
+  CK(cudaSetDevice(h->cfg.device));
+  rc = finish_pending(h); if (rc) return rc;
+  rc = saliency_setup(h); if (rc) return rc;
+  const size_t w = (size_t)D * sizeof(float), ld0 = (size_t)b.lda[0] * sizeof(float);
+  if (x) {      // the staging path of mrgan_test_batch / mrgan_predict_rows
+    CK(cudaMemcpy2DAsync(b.ex_stage, ld0, x, w, w, n, cudaMemcpyHostToDevice, h->stream));
+    if (h->cfg.precision == MRGAN_PREC_TF32) {
+      k_round_tf32<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0]);
+      h->launches++;
+    } else if (h->om.mode == 2) {
+      k_to_half<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0], h->om);
+      h->launches++;
+    }
+  }
+  if (target) CK(cudaMemcpyAsync(b.ey_stage, target, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+  enqueue_input_grad(h, fold, 1, x != nullptr, x ? n : 0, target ? TGT_STAGED : TGT_PRED);
+  CK(cudaMemcpy2DAsync(grad, w, b.ex_stage, ld0, w, n, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  CKS();
+  return MRGAN_OK;
+}
+
+int mrgan_saliency(mrgan_handle* h, float* profile) {
+  int rc = need_nets(h, "saliency"); if (rc) return rc;
+  if (!profile) return fail(h, MRGAN_ERR_ARG, "saliency: null pointer");
+  rc = need_local(h, "saliency"); if (rc) return rc;
+  for (int f = 0; f < h->nf; ++f)
+    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "saliency before mrgan_load_fold");
+  CK(cudaSetDevice(h->cfg.device));
+  rc = finish_pending(h); if (rc) return rc;
+  rc = saliency_setup(h); if (rc) return rc;
+  enqueue_saliency(h);
+  CK(cudaMemcpyAsync(profile, h->sal.profile, (size_t)h->nf * h->cfg.n_classes * max_D(h, 0, h->nf) * sizeof(float), cudaMemcpyDeviceToHost,
+                     h->stream));
   CK(cudaStreamSynchronize(h->stream));
   CKS();
   return MRGAN_OK;

@@ -360,6 +360,40 @@ class FoldGroup:
         self._chk(self.lib.mrgan_confusion(self._h, _lib.iptr(out)))
         return out
 
+    # ------------------------------------------------------------------ input gradients (GAN / NN)
+    def input_grad(self, fold, x=None, target=None):
+        """d log softmax(l(x))[t] / dx of the fold's phase-0 logits l (those of predict), float32 [n, D], x in the fold's
+        SCALED input space.  x: rows [n, D] (in chunks of at most n_test rows), or None = the resident X_test.  target: int
+        [n] classes, or None = each row's predicted class.  Leaves every later result of the group unchanged."""
+        D, _, nte, _ = self.shapes[fold]
+        if x is None:
+            n = nte
+        else:
+            x = _f32(x)
+            if x.ndim != 2 or x.shape[1] != D or x.shape[0] < 1:
+                raise ValueError("input_grad: x must be [n >= 1, %d]" % D)
+            n = x.shape[0]
+        if target is not None:
+            target = _i32(target)
+            if target.shape != (n,):
+                raise ValueError("input_grad: target must be [%d]" % n)
+        grad = np.empty((n, D), dtype=np.float32)
+        for a in range(0, n, nte):
+            b = min(n, a + nte)
+            xp = None if x is None else _lib.fptr(x[a:b])
+            tp = None if target is None else _lib.iptr(target[a:b])
+            self._chk(self.lib.mrgan_input_grad(self._h, int(fold), xp, b - a, tp, _lib.fptr(grad[a:b])))
+        return grad
+
+    def saliency(self):
+        """Saliency profile of every fold in one pass over its resident test set: a list of float32 [K, D_f], row c = the mean
+        of |input_grad(f, target=y_test)| over the test rows of class c (zero for a class without test rows).  Bitwise
+        reproducible and independent of the fold grouping."""
+        K, Dmax = self.cfg.n_classes, max(s[0] for s in self.shapes)
+        out = np.empty((self.n_folds, K, Dmax), dtype=np.float32)
+        self._chk(self.lib.mrgan_saliency(self._h, _lib.fptr(out)))
+        return [out[f, :, :D].copy() for f, (D, _, _, _) in enumerate(self.shapes)]
+
     # ------------------------------------------------------------------ utilities
     def fill_normal(self, fold, step, tensor_id, rows, cols, row0=0):
         out = np.empty((rows, cols), dtype=np.float32)
@@ -396,10 +430,10 @@ class FoldGroup:
         return float(out[0])
 
     TIME_OPS = {"adam_d": 0, "adam_g": 1, "dw1": 2, "fwd1": 3, "disc_step": 4, "gen_step": 5, "dx1": 6,
-                "svm_kmat": 7, "svm_smo": 8, "svm_predict": 9}
+                "svm_kmat": 7, "svm_smo": 8, "svm_predict": 9, "saliency": 10}
 
     def time_op(self, which, reps=20):
-        """Average device ms of one kernel (or one whole step) over all folds; mutates training state."""
+        """Average device ms of one kernel (or one whole step) over all folds; mutates training state (but 'saliency')."""
         out = np.zeros(1, dtype=np.float32)
         self._chk(self.lib.mrgan_time_op(self._h, self.TIME_OPS[which], reps, _lib.fptr(out)))
         return float(out[0])

@@ -39,7 +39,7 @@ def dataset(modalities=0, forcetempTime=4, contactmicTime=0.2, leaveObjectOut=Fa
 
 
 def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16', device=0, batch=50,
-                    eval_each_epoch=True, shared_t=True, return_group=False, device_perm=False, details=False):
+                    eval_each_epoch=True, shared_t=True, return_group=False, device_perm=False, details=False, saliency=False):
     """Train a GROUP of independent folds side by side on one GPU.
 
     jobs: list of dicts with keys ``trainTestSets`` (or ``X``, ``y``), ``percentlabeled``,
@@ -48,7 +48,7 @@ def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16',
     epoch instead of 3 x int32[n_train] per fold); same distribution, different draws than the host's numpy generator.
     Returns the list of test errors (mr_gan.py:230,234), one per job; details=True: one dict per job instead,
     ``{'error': <the same float>, 'confusion': int32 [K, K]}`` (rows = true class, columns = predicted), from one extra
-    forward pass over every fold's test set."""
+    forward pass over every fold's test set; saliency=True: those dicts with ``'saliency'``, float32 [K, D] (FoldGroup.saliency)."""
     folds, rngs, slots = [], [], {}
     for i, job in enumerate(jobs):
         rng = np.random.default_rng([int(seed), int(job.get('job_id', i))])
@@ -122,8 +122,11 @@ def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16',
         for e in errors:
             print('Test error:', e)
         sys.stdout.flush()
-    if details:
+    if details or saliency:
         errors = [dict(error=e, confusion=c) for e, c in zip(errors, fg.confusion())]
+    if saliency:
+        for r, p in zip(errors, fg.saliency()):
+            r['saliency'] = p
     if return_group:
         return errors, fg
     fg.close()
@@ -199,7 +202,7 @@ def main(argv=None):
     parser.add_argument('--data-dir', default='data_processed')
     parser.add_argument('--synthetic', action='store_true', help='synthetic data of the MREO shape instead of the processed pickles')
     parser.add_argument('--host-perm', action='store_true', help='draw the epoch permutations on the host (numpy) instead of on the device')
-    results.add_arguments(parser)
+    results.add_arguments(parser, saliency=True)
     args = parser.parse_args(argv)
     rank, world, local = sweep.dist_env()
     seed = sweep.shared_seed(args.seed)          # one seed for every rank: same dataset, same splits, same job streams
@@ -216,7 +219,7 @@ def main(argv=None):
         res = sweep.run_sharded(
             jobs, lambda js, dev: train_gan_folds(js, epochs=args.epochs, verbose=args.verbose, seed=seed,
                                                   precision=args.precision, device=dev, device_perm=not args.host_perm,
-                                                  details=rep.details),
+                                                  details=rep.details, saliency=rep.saliency),
             group_size=args.group, key=job_rows, cost=job_cost)
         return res
 
@@ -245,7 +248,7 @@ def main(argv=None):
                 for v in e:
                     say('Test error:', v, 'Test accuracy:', 1.0 - v)
                 report(e)
-                rep.setting(jobs[a:a + 6], res[a:a + 6], table=1, modality=MODALITIES[modality])
+                rep.setting(jobs[a:a + 6], res[a:a + 6], synthetic.block_widths(modality), table=1, modality=MODALITIES[modality])
 
     if '3' in args.tables:                      # mr_gan.py:263-283
         say('\n', '-' * 25, 'Testing generalization with leave-one-object-out validation', '-' * 25)
@@ -263,7 +266,8 @@ def main(argv=None):
                 for j, e in zip(jobs[n * k:n * k + n], errors[n * k:n * k + n]):
                     say(j['name'], 'Test error:', e, 'Test accuracy:', 1.0 - e)
                 report(errors[n * k:n * k + n], 'Average leave-one-object-out error:')
-                rep.setting(jobs[n * k:n * k + n], res[n * k:n * k + n], table=3, modality=MODALITIES[modality])
+                rep.setting(jobs[n * k:n * k + n], res[n * k:n * k + n], synthetic.block_widths(modality), table=3,
+                            modality=MODALITIES[modality])
 
     if '5' in args.tables:                      # mr_gan.py:285-318
         for header_mods, times, is_contact in (([0, 1, 2], [4, 3, 2, 1, 0.5, 0.2, 0.1], False),
@@ -284,7 +288,9 @@ def main(argv=None):
                     for e in errors[6 * k:6 * k + 6]:
                         say('Test error:', e, 'Test accuracy:', 1.0 - e)
                     report(errors[6 * k:6 * k + 6])
-                    rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], table=5, modality=MODALITIES[modality], time=tm)
+                    kw = dict(contactmicTime=tm) if is_contact else dict(forcetempTime=tm)
+                    rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], synthetic.block_widths(modality, **kw), table=5,
+                                modality=MODALITIES[modality], time=tm)
 
     if '6' in args.tables:                      # mr_gan.py:320-341
         say('\n', '-' * 25, 'Testing performance as quantity of unlabeled data increases', '-' * 25)
@@ -303,7 +309,8 @@ def main(argv=None):
                     for e in errors[6 * k:6 * k + 6]:
                         say('Test error:', e, 'Test accuracy:', 1.0 - e)
                     report(errors[6 * k:6 * k + 6])
-                    rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], table=6, modality=MODALITIES[modality])
+                    rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], synthetic.block_widths(modality), table=6,
+                                modality=MODALITIES[modality])
     rep.close()
     return 0
 

@@ -6,15 +6,16 @@ import sys
 
 import numpy as np
 
-from . import foldprep, results, sweep
+from . import foldprep, results, sweep, synthetic
 from .engine import FoldGroup
 from .model import MATERIALS, fold_key, init_disc
 from .mr_gan import MODALITIES, _kfold_jobs, _loo_jobs, dataset, job_rows, job_width
 
 
-def train_nn_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16', device=0, batch=20, details=False):
+def train_nn_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16', device=0, batch=20, details=False, saliency=False):
     """Train a group of independent mr_nn folds side by side; returns test errors (mr_nn.py:118-119), or with details=True
-    one dict per job, ``{'error': <the same float>, 'confusion': int32 [K, K]}`` (rows = true class, columns = predicted)."""
+    one dict per job, ``{'error': <the same float>, 'confusion': int32 [K, K]}`` (rows = true class, columns = predicted);
+    saliency=True: those dicts with ``'saliency'``, float32 [K, D] (FoldGroup.saliency)."""
     folds, rngs, slots = [], [], {}
     for i, job in enumerate(jobs):
         rng = np.random.default_rng([int(seed), int(job.get('job_id', i))])
@@ -61,8 +62,11 @@ def train_nn_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16', 
         if epoch + 1 < epochs:
             nxt = draw()
     errors = [1.0 - float(fg.nn_evaluate(i)[1]) for i in range(len(jobs))]     # mr_nn.py:118
-    if details:
+    if details or saliency:
         errors = [dict(error=e, confusion=c) for e, c in zip(errors, fg.confusion())]
+    if saliency:
+        for r, p in zip(errors, fg.saliency()):
+            r['saliency'] = p
     fg.close()
     return errors
 
@@ -88,7 +92,7 @@ def main(argv=None):
     parser.add_argument('--group', type=int, default=42)
     parser.add_argument('--data-dir', default='data_processed')
     parser.add_argument('--synthetic', action='store_true', help='synthetic data of the MREO shape instead of the processed pickles')
-    results.add_arguments(parser)
+    results.add_arguments(parser, saliency=True)
     args = parser.parse_args(argv)
     rank, world, local = sweep.dist_env()
     seed = sweep.shared_seed(args.seed)          # one seed for every rank: same dataset, same splits, same job streams
@@ -104,7 +108,8 @@ def main(argv=None):
             jid[0] += 1
         return sweep.run_sharded(
             jobs, lambda js, dev: train_nn_folds(js, epochs=args.epochs, verbose=args.verbose, seed=seed,
-                                                 precision=args.precision, device=dev, details=rep.details),
+                                                 precision=args.precision, device=dev, details=rep.details,
+                                                 saliency=rep.saliency),
             group_size=args.group,
             key=lambda j: job_rows(j) + (j['percentlabeled'],),
             cost=lambda j: job_width(j) * j['percentlabeled'])
@@ -123,7 +128,8 @@ def main(argv=None):
                 say('-' * 15, 'Percentage of training data labeled: %d%%' % p, '-' * 15)
                 e = errors[6 * k:6 * k + 6]
                 say('Average error:', np.mean(e), 'Average accuracy:', np.mean(1.0 - np.array(e)))
-                rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], table=2, modality=MODALITIES[modality])
+                rep.setting(jobs[6 * k:6 * k + 6], res[6 * k:6 * k + 6], synthetic.block_widths(modality), table=2,
+                            modality=MODALITIES[modality])
                 sys.stdout.flush()
 
     if '4' in args.tables:                      # mr_nn.py:148-168
@@ -143,7 +149,8 @@ def main(argv=None):
                     say(j['name'], 'Test error:', e, 'Test accuracy:', 1.0 - e)
                 e = errors[n * k:n * k + n]
                 say('Average leave-one-object-out error:', np.mean(e), 'Average accuracy:', np.mean(1.0 - np.array(e)))
-                rep.setting(jobs[n * k:n * k + n], res[n * k:n * k + n], table=4, modality=MODALITIES[modality])
+                rep.setting(jobs[n * k:n * k + n], res[n * k:n * k + n], synthetic.block_widths(modality), table=4,
+                            modality=MODALITIES[modality])
                 sys.stdout.flush()
     rep.close()
     return 0

@@ -1,10 +1,12 @@
 """Per-fold results of the three CLIs (mr_gan.py, mr_nn.py, mr_svm.py): the JSON Lines record of one fold-training
-(``--results FILE``) and the printed confusion block (``--confusion``).
+(``--results FILE``), the printed confusion block (``--confusion``) and, for the GAN / NN CLIs, the saliency profiles
+(``--saliency FILE``: an .npz file, and one printed line of block shares per setting).
 
 The trainers return one float per job by default, or with ``details=True`` one dict per job,
-``{'error': <the same float>, 'confusion': int [K, K]}`` (rows = true class, columns = predicted class).  A ``Report``
-turns a setting's results into what the flags ask for; without either flag it prints and writes nothing, so the CLIs'
-stdout stays the reference's."""
+``{'error': <the same float>, 'confusion': int [K, K]}`` (rows = true class, columns = predicted class); with
+``saliency=True`` the dict also holds ``'saliency'``, float32 [K, D] (mean |d log p(true class) / dx| over the test rows of
+each class, x in the fold's scaled input space).  A ``Report`` turns a setting's results into what the flags ask for;
+without a flag it prints and writes nothing, so the CLIs' stdout stays the reference's."""
 import json
 
 import numpy as np
@@ -12,11 +14,15 @@ import numpy as np
 from .model import MATERIALS
 
 
-def add_arguments(parser):
+def add_arguments(parser, saliency=False):
     parser.add_argument('--confusion', action='store_true',
                         help="after each setting's average, print its confusion matrix summed over the setting's fold-trainings")
     parser.add_argument('--results', metavar='FILE', default=None,
                         help='write one JSON Lines record per fold-training (rank 0)')
+    if saliency:
+        parser.add_argument('--saliency', metavar='FILE', default=None,
+                            help="write every fold-training's input-gradient saliency profile [K, D] to one .npz file (rank 0) and "
+                                 "print each feature block's share of a setting's summed profile after its average")
 
 
 def errors(results):
@@ -35,9 +41,9 @@ def confusion_lines(conf, names=MATERIALS):
     return lines
 
 
-def record(tool, job, result, index, **fields):
-    """The JSON record of one fold-training: the given fields, the job's labeled / unlabeled shares and id, its fold index
-    within the setting (k-fold) or held-out object (leave-one-object-out), n_test, error and confusion."""
+def setting_fields(tool, job, index, **fields):
+    """What identifies one fold-training: the given fields, the job's labeled / unlabeled shares, its fold index within the
+    setting (k-fold) or held-out object (leave-one-object-out), and its id."""
     rec = dict(tool=tool)
     rec.update(fields)
     rec['percentlabeled'] = job['percentlabeled']
@@ -48,6 +54,12 @@ def record(tool, job, result, index, **fields):
     else:
         rec['fold'] = index
     rec['job_id'] = job.get('job_id')
+    return rec
+
+
+def record(tool, job, result, index, **fields):
+    """The JSON record of one fold-training: its setting_fields, n_test, error and confusion."""
+    rec = setting_fields(tool, job, index, **fields)
     conf = np.asarray(result['confusion'])
     rec['n_test'] = int(conf.sum())
     rec['error'] = result['error']
@@ -55,22 +67,46 @@ def record(tool, job, result, index, **fields):
     return rec
 
 
+def block_shares(profiles, blocks):
+    """Each feature block's share of the summed profiles (over folds, classes and the block's features): a mass share, so
+    wider blocks hold more features.  blocks: [(name, width)] in row order."""
+    tot = np.sum([np.asarray(p, dtype=np.float64).sum(axis=0) for p in profiles], axis=0)    # [D]
+    edges = np.cumsum([0] + [w for _, w in blocks])
+    mass = np.array([tot[a:b].sum() for a, b in zip(edges[:-1], edges[1:])])
+    return mass / mass.sum()
+
+
+def share_line(shares, blocks):
+    return 'Saliency share: ' + ' '.join('%s %.3f' % (name, v) for (name, _), v in zip(blocks, shares))
+
+
 class Report:
-    """What --confusion and --results add to a CLI; inactive (details=False) when neither flag is given."""
+    """What --confusion, --results and --saliency add to a CLI; inactive (details=False, saliency=False) without them."""
 
     def __init__(self, args, tool, rank, say, **fields):
         self.show = bool(args.confusion)
+        sal = getattr(args, 'saliency', None)
+        self.saliency = bool(sal)
         self.details = self.show or bool(args.results)
         self.tool, self.say, self.fields = tool, say, fields
         self.fh = open(args.results, 'w') if args.results and rank == 0 else None
+        self.sal_path = sal if sal and rank == 0 else None
+        self.sal_arrays, self.sal_index = {}, []
 
-    def setting(self, jobs, results, **fields):
-        """Call after a setting's average line, with the setting's jobs and trainer results in printed order."""
-        if not self.details:
+    def setting(self, jobs, results, blocks=None, **fields):
+        """Call after a setting's average line, with the setting's jobs and trainer results in printed order; blocks: the
+        [(name, width)] feature blocks of the setting's rows (needed with --saliency)."""
+        if not (self.details or self.saliency):
             return
         if self.show:
             for line in confusion_lines(np.sum([np.asarray(r['confusion']) for r in results], axis=0)):
                 self.say(line)
+        if self.saliency:
+            self.say(share_line(block_shares([r['saliency'] for r in results], blocks), blocks))
+            for k, (j, r) in enumerate(zip(jobs, results)):
+                self.sal_arrays['job_%d' % j['job_id']] = np.asarray(r['saliency'], dtype=np.float32)
+                self.sal_index.append(dict(setting_fields(self.tool, j, k, **dict(self.fields, **fields)),
+                                           blocks=[[name, int(w)] for name, w in blocks]))
         if self.fh:
             for k, (j, r) in enumerate(zip(jobs, results)):
                 self.fh.write(json.dumps(record(self.tool, j, r, k, **dict(self.fields, **fields))) + '\n')
@@ -80,3 +116,7 @@ class Report:
         if self.fh:
             self.fh.close()
             self.fh = None
+        if self.sal_path:
+            with open(self.sal_path, 'wb') as f:       # the name as given (np.savez would append .npz to a path)
+                np.savez(f, index=np.array(json.dumps(self.sal_index)), **self.sal_arrays)
+            self.sal_path = None
