@@ -164,7 +164,7 @@ int  mrgan_dp_init(mrgan_handle* h, int rank, int world, const void* id128);
  * (CUDA IPC handles of its arenas), the host exchanges them with any transport, and every rank opens all of them.  From
  * then on the per-step exchange is ONE kernel per rank -- reduce-scatter of the flat gradient by peer loads, Adam on the
  * owned 1/W shard, all-gather of the updated weights by peer stores -- instead of ncclAllReduce + a full-size Adam
- * (which remains the path when the handles are not opened, or with MRGAN_DP_FUSED=0).
+ * (which remains the path when the handles are not opened).
  *   handles: world x 128 bytes, rank-major. */
 int  mrgan_dp_ipc_export(mrgan_handle* h, void* out128);
 int  mrgan_dp_ipc_open(mrgan_handle* h, const void* handles, int world);

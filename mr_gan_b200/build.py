@@ -20,7 +20,7 @@ LOCK = os.path.join(HERE, ".build.lock")
 SOURCES = ["mrgan_api.cu"]
 HEADERS = ["common.cuh", "kernels_simt.cuh", "kernels_tc.cuh", "kernels_svm.cuh", "kernels_dp.cuh", os.path.join("..", "..", "include", "mrgan.h")]
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
-         "-Xcompiler", "-fPIC", "-shared", "-ldl", "-DMRGAN_WITH_TC", "-lcuda"]
+         "-Xcompiler", "-fPIC", "-shared", "-ldl", "-lcuda"]
 
 
 def source_hash():

@@ -73,19 +73,8 @@ __host__ __device__ inline int global_row(int L, const AdamHyper& hp, int fold =
   return sec * hp.dp_bg + (hp.dp_rank < 0 ? fold : hp.dp_rank) * hp.dp_bloc + (L - sec * hp.dp_bloc);
 }
 
-// Programmatic dependent launch: every kernel of the step chain lets its successor be scheduled as soon as all of its own
-// CTAs are running (launch_dependents at the top) and orders itself after its predecessor with griddepcontrol.wait, which
-// returns once the predecessor grid has completed and its writes are visible.  What a kernel does BEFORE the wait (barrier
-// init, TMEM allocation, descriptor fetch) overlaps the predecessor's tail.  Without the launch attribute both are no-ops.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
 // row pitch in elements: a multiple of 8 so that both the fp32 rows and their fp16 operand copies have 16-byte strides (TMA)
-#ifdef MRGAN_PITCH4_EXPERIMENT
-__host__ __device__ inline int pitch8(int w) { return (w + 3) & ~3; }
-#else
 __host__ __device__ inline int pitch8(int w) { return (w + 7) & ~7; }
-#endif
 
 // ---------------------------------------------------------------- Philox4x32-10
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {

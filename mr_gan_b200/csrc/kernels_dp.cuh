@@ -1,9 +1,10 @@
 // kernels_dp.cuh -- data-parallel gradient exchange fused with the optimizer, over NVLink peer memory.
 //
 // The data-parallel large-batch mode (BASELINE config 5; mr_gan.py:165-167 is the update being distributed) needs, once per
-// D or G step, sum-over-ranks of the flat gradient followed by Keras Adam on every parameter.  The NCCL baseline
-// (MRGAN_DP_FUSED=0) all-reduces the whole gradient (2 (W-1)/W x 4 B per parameter over the links) and then every rank runs
-// the full Adam (28 B per parameter of HBM traffic on EVERY rank).  k_dp_exchange does both in ONE kernel per rank:
+// D or G step, sum-over-ranks of the flat gradient followed by Keras Adam on every parameter.  The NCCL path (a handle
+// whose IPC handles were not opened) all-reduces the whole gradient (2 (W-1)/W x 4 B per parameter over the links) and
+// then every rank runs the full Adam (28 B per parameter of HBM traffic on EVERY rank).  k_dp_exchange does both in ONE
+// kernel per rank:
 //
 //   reduce-scatter by peer LOADS : rank r owns the r-th 1/W of the flat range; it reads that shard of every rank's gradient
 //                                  buffer straight out of the peers' HBM (NVLink P2P loads, summed in rank order)

@@ -18,8 +18,6 @@ __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpre
 template <bool AT, bool BT>
 __global__ void __launch_bounds__(256)
 k_gemm_simt(const GemmDesc* __restrict__ descs, const FoldState* __restrict__ folds, int rows_override, AdamHyper hp) {
-  pdl_launch_dependents();
-  pdl_wait();
   const GemmDesc d = descs[blockIdx.z];
   int M = d.M, K = d.K;
   const int N = d.N;
@@ -181,8 +179,6 @@ template <int PG>
 __global__ void __launch_bounds__(128)
 k_prep(FoldState* __restrict__ folds, int fold_base, int mode, int from_stage, int t, int B, int nrows,
        int noise_dim, float sigma_in, AdamHyper hp, OperandMode om) {
-  pdl_launch_dependents();
-  pdl_wait();
   FoldState& fs = folds[fold_base + blockIdx.z];
   const int c = blockIdx.x * 128 + threadIdx.x;
   const uint32_t step = (uint32_t)fs.rng_step;
@@ -351,8 +347,6 @@ struct BnDesc {
 #define BN_COLS 32
 #define BN_MAX_SLICES 32
 __global__ void __launch_bounds__(1024) k_bn_fwd(const BnDesc* __restrict__ descs, float eps, OperandMode om) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float red[2][BN_MAX_SLICES][BN_COLS];
   const BnDesc d = descs[blockIdx.z];
   const int BN_SLICES = blockDim.x / BN_COLS;
@@ -386,8 +380,6 @@ __global__ void __launch_bounds__(1024) k_bn_fwd(const BnDesc* __restrict__ desc
 
 // BN backward + softplus' of the layer in front of it (G layer 1): du -> dgamma, dbeta, dz1.
 __global__ void __launch_bounds__(1024) k_bn_bwd(const BnDesc* __restrict__ descs, OperandMode om) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float red[2][BN_MAX_SLICES][BN_COLS];
   const BnDesc d = descs[blockIdx.z];
   const int BN_SLICES = blockDim.x / BN_COLS;
@@ -436,8 +428,6 @@ struct LossDesc {
 __global__ void __launch_bounds__(256)
 k_loss_disc(const LossDesc* __restrict__ descs, float* __restrict__ step_stats, int fold_base, int nf_total,
             int t, int B, int K, float w_unl, OperandMode om, int Bg, float* __restrict__ part, unsigned* __restrict__ ctr) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float sh[32];
   const LossDesc d = descs[blockIdx.z];   // B rows per section on this rank, Bg in the global batch (means are over Bg)
   float s_lab = 0.f, s_unl = 0.f, s_err = 0.f;
@@ -497,8 +487,6 @@ k_loss_disc(const LossDesc* __restrict__ descs, float* __restrict__ step_stats, 
 __global__ void __launch_bounds__(1024)
 k_fm(const LossDesc* __restrict__ descs, float* __restrict__ step_stats, int fold_base, int nf_total, int t, int B,
      OperandMode om, float alpha) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float sh[32];
   __shared__ float red[2][4][256];
   const LossDesc d = descs[blockIdx.z];
@@ -529,8 +517,6 @@ k_fm(const LossDesc* __restrict__ descs, float* __restrict__ step_stats, int fol
 __global__ void __launch_bounds__(256)
 k_loss_mse(const LossDesc* __restrict__ descs, float* __restrict__ step_stats, int fold_base, int nf_total,
            int t, int n, int rows_total, int K, OperandMode om) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float sh[32];
   const LossDesc d = descs[blockIdx.z];
   float s_loss = 0.f, s_acc = 0.f;
@@ -733,8 +719,6 @@ __device__ __forceinline__ int row_argmax(const float* l, int K) {
 // out[2] = mse vs one-hot over all rows (mr_nn.py:118 evaluate()[0]).  with_pred: also store every row's class in d.pred.
 __global__ void __launch_bounds__(256)
 k_argmax_err(const EvalDesc* __restrict__ descs, int n_override, int K, int with_pred) {
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float sh[32];
   const EvalDesc d = descs[blockIdx.z];
   const int n = n_override > 0 ? n_override : d.n;
@@ -778,8 +762,6 @@ __global__ void __launch_bounds__(256) k_confusion(const EvalDesc* __restrict__ 
 // use_pred the row's predicted class (row_argmax).  One thread per row; grid (row blocks, 1, folds).
 __global__ void __launch_bounds__(256)
 k_logprob_seed(const EvalDesc* __restrict__ descs, int n_override, int K, int use_pred, OperandMode om) {
-  pdl_launch_dependents();
-  pdl_wait();
   const EvalDesc d = descs[blockIdx.z];
   const int n = n_override > 0 ? n_override : d.n;
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
@@ -797,8 +779,6 @@ k_logprob_seed(const EvalDesc* __restrict__ descs, int n_override, int K, int us
 // f16 mode: the fp32 input gradients of OP_EX1 (C [M][ldc], N = D columns) carry the loss scale of the dX operands; ginv divides
 // it out in place (a power of two: exact).  grid (blocks, 1, folds).
 __global__ void __launch_bounds__(256) k_unscale_grad(const GemmDesc* __restrict__ descs, int rows_override, float ginv) {
-  pdl_launch_dependents();
-  pdl_wait();
   const GemmDesc g = descs[blockIdx.z];
   const int M = rows_override > 0 ? rows_override : g.M;
   const size_t n = (size_t)M * g.N;
@@ -812,7 +792,6 @@ __global__ void __launch_bounds__(256) k_unscale_grad(const GemmDesc* __restrict
 // independent of the grouping of the folds.  grid (feature blocks, folds).
 __global__ void __launch_bounds__(128)
 k_saliency(const GemmDesc* __restrict__ gx, const EvalDesc* __restrict__ ev, int K, int Dmax, float* __restrict__ out) {
-  pdl_wait();
   const int f = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= Dmax) return;
   const GemmDesc g = gx[f];
@@ -831,8 +810,6 @@ k_saliency(const GemmDesc* __restrict__ gx, const EvalDesc* __restrict__ ev, int
 // Means over the epoch's batches (mr_gan.py:215-217) -> epoch_stats[f][0..3]; [4] = batch-wise test error.
 __global__ void k_epoch_reduce(const float* __restrict__ step_stats, const EvalDesc* __restrict__ evals,
                                float* __restrict__ epoch_stats, int nf, int nb, int with_eval) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int f = blockIdx.x, j = threadIdx.x;
   if (j < 4) {
     float s = 0.f;
@@ -853,8 +830,6 @@ __global__ void __launch_bounds__(256)
 k_adam(float* __restrict__ P, float* __restrict__ Mo, float* __restrict__ Vo, const float* __restrict__ G,
        const AdamRange* __restrict__ ranges, FoldState* __restrict__ folds, int fold_base, int net, AdamHyper hp,
        float ginv, __half* __restrict__ Ph) {      // ginv: 1 / loss scale of the gradient buffer; Ph: fp16 operand copy of P or null
-  pdl_launch_dependents();
-  pdl_wait();
   const int f = fold_base + blockIdx.y;
   const AdamRange rg = ranges[f];
   FoldState& fs = folds[f];

@@ -16,38 +16,32 @@
 //
 // Pipeline: warp 0 = TMA producer (4-stage mbarrier ring, 32 contraction elements per stage),
 // warp 1 = TMEM allocator + single-thread tcgen05.mma issuer, warps 2..5 = epilogue
-// (tcgen05.ld 32x32b -> bias-free activation + Philox GaussianNoise | act' mask | fused Adam).
+// (tcgen05.ld 32x32b -> bias-free activation + Philox GaussianNoise | act' mask | dW store).
 #pragma once
 #include <cuda.h>
 #include "common.cuh"
 
-enum { EPI_ADAM = 3 };
 // Reductions fused into the epilogue of the GEMM that produces their input (thread = feature, the batch is in TMEM columns,
 // so batch statistics are thread-local):
 //   HEAD_DISC    forward of the logit layer: Salimans supervised / unsupervised losses, training error, logit gradients
 //                (mr_gan.py:146-149,161), and K.update_add(iterations, 1) of the discriminator step
 //   HEAD_FM      forward of D layer 5 in the generator step: feature-matching loss and its gradient (mr_gan.py:152-154)
 //   HEAD_BN      forward of G layer 1: BatchNormalization with batch statistics (mr_gan.py:112)
-//   HEAD_BN_BWD  dX into G layer 1: BatchNorm backward, softplus', and the Adam update of gamma / beta
-enum { HEAD_NONE = 0, HEAD_DISC = 1, HEAD_FM = 2, HEAD_BN = 3, HEAD_BN_BWD = 4 };
+enum { HEAD_NONE = 0, HEAD_DISC = 1, HEAD_FM = 2, HEAD_BN = 3 };
 
 struct alignas(64) TcOp {
   CUtensorMap mapA, mapB;
   GemmDesc g;                 // epilogue description shared with the fp32 path (C, C2, aux, act, noise ...)
-  float *P, *Mo, *Vo;         // fused Adam (EPI_ADAM): tensor base inside the flat buffers
   int ME, NE, KE;             // extents: MMA-M (features), MMA-N, contraction
   int bn;                     // MMA-N per tile (multiple of 16, <= 256; multiple of 32 when B is MN-major)
-  int epi;                    // EPI_FWD / EPI_DX / EPI_STORE / EPI_ADAM
-  int net;                    // 0 = discriminator, 1 = generator (which lr_t the fused Adam uses)
+  int net;                    // 0 = discriminator, 1 = generator (which lr_t k_dw_adam_tc uses)
   int ws_stride;              // split-K (large-batch dW): floats between the partial products of two contraction slices
   float* ws;                  // ... and their workspace, laid out like C; k_splitk_reduce sums the slices in a fixed order
   int esz;                    // operand element size: 4 (or 0) = fp32 read as tf32, 2 = fp16 copies (kind::f16, fp32 accumulation)
   int head;                   // HEAD_*: reduction fused into this GEMM's epilogue
-  int advance;                // the head also advances the fold's step counters (no k_adam launch follows)
   int stats_stride;           // floats between the statistics blocks of two batches of the epoch
-  const void* hd;             // the fold's LossDesc (HEAD_DISC / HEAD_FM) or BnDesc (HEAD_BN / HEAD_BN_BWD)
+  const void* hd;             // the fold's LossDesc (HEAD_DISC / HEAD_FM) or BnDesc (HEAD_BN)
   float* stats;               // the fold's block of 4 step statistics at batch 0
-  long long mo_off, vo_off;   // Adam slots of a parameter p: p + mo_off, p + vo_off (HEAD_BN_BWD: gamma / beta)
 };
 
 #define TC_KBLK 32            // contraction elements per stage (one 128-byte swizzle row of fp32)
@@ -402,57 +396,8 @@ __device__ __forceinline__ void head_bn(uint32_t trow, int cbeg, int ncols, int 
   }
 }
 
-// HEAD_BN_BWD: the accumulator is dU (gradient w.r.t. the BatchNorm output) of this thread's feature: BatchNorm backward,
-// softplus' of G layer 1 for rows [cbeg, ncols), and Keras Adam on gamma_f, beta_f (their gradients are the two
-// thread-local sums over all nall rows; the warp group with cbeg == 0 applies the update).
-template <bool F16>
-__device__ __forceinline__ void head_bn_bwd(uint32_t trow, int cbeg, int ncols, int nall, int f, bool f_ok, const BnDesc& Bd,
-                                            const AdamHyper& hp, const OperandMode& om, float lr_t, long long mo_off, long long vo_off) {
-  const float ginv = F16 ? 1.0f / om.gscale : 1.0f;            // the dZ operand carried the loss scale into the accumulator
-  float s1 = 0.f, s2 = 0.f;
-  for (int c0 = 0; c0 < nall; c0 += 16) {
-    float du[16];
-    head_chunk<F16, ACT_NONE>(trow + (uint32_t)c0, du);
-    if (!f_ok) continue;
-#pragma unroll
-    for (int j = 0; j < 16; ++j) {
-      const int r = c0 + j;
-      if (r >= nall) break;
-      const float d = du[j] * ginv;
-      s1 += d;
-      s2 = fmaf(d, Bd.xhat[(size_t)r * Bd.ld + f], s2);
-    }
-  }
-  float ga = 0.f, istd = 0.f;
-  if (f_ok) { ga = Bd.gamma[f]; istd = Bd.istd[f]; }
-  const float invB = 1.0f / nall;
-  for (int c0 = cbeg; c0 < ncols; c0 += 16) {
-    float du[16];
-    head_chunk<F16, ACT_NONE>(trow + (uint32_t)c0, du);
-    if (!f_ok) continue;
-#pragma unroll
-    for (int j = 0; j < 16; ++j) {
-      const int r = c0 + j;
-      if (r >= ncols) break;
-      const float xh = Bd.xhat[(size_t)r * Bd.ld + f];
-      const float dxh = du[j] * ginv * ga;
-      const float dh1 = istd * (dxh - invB * ga * s1 - xh * invB * ga * s2);
-      put_grad_operand(Bd.dz1 + (size_t)r * Bd.ld + f, dh1 * (1.0f - expf(-Bd.h1[(size_t)r * Bd.ld + f])), om);
-    }
-  }
-  if (f_ok && cbeg == 0) {      // Adam.get_updates for gamma (gradient s2) and beta (gradient s1), mr_gan.py:167
-    const float b1 = hp.b1, b2 = hp.b2, c1 = 1.0f - hp.b1, c2 = 1.0f - hp.b2;
-    float* const pg = const_cast<float*>(Bd.gamma) + f;
-    float* const pb = const_cast<float*>(Bd.beta) + f;
-    float m = fmaf(b1, pg[mo_off], c1 * s2), v = fmaf(b2, pg[vo_off], c2 * s2 * s2);
-    pg[mo_off] = m; pg[vo_off] = v; *pg = ga - lr_t * m / (sqrtf(v) + hp.eps);
-    m = fmaf(b1, pb[mo_off], c1 * s1); v = fmaf(b2, pb[vo_off], c2 * s1 * s1);
-    pb[mo_off] = m; pb[vo_off] = v; *pb -= lr_t * m / (sqrtf(v) + hp.eps);
-  }
-}
-
 // A_MN / B_MN: operand is MN-major (its MMA M/N dimension is the memory-contiguous one).  The pair also selects the role:
-//   A_MN && !B_MN  forward   (EPI_FWD)      !A_MN && !B_MN  dX (EPI_DX)      A_MN && B_MN  dW (EPI_ADAM or EPI_STORE)
+//   A_MN && !B_MN  forward   (EPI_FWD)      !A_MN && !B_MN  dX (EPI_DX)      A_MN && B_MN  dW (EPI_STORE)
 // STAGES: depth of the TMA->MMA ring; TMEM_COLS: TMEM columns allocated (power of 2 >= MT x bn);
 // MINB: CTAs per SM the register allocation must allow; EPW: epilogue warps (4 or 8; with 8 and MT == 1 the accumulator
 // columns are split between two warp groups).
@@ -471,7 +416,6 @@ template <bool A_MN, bool B_MN, int STAGES, int TMEM_COLS, int MINB, int EPW, in
 __global__ void __launch_bounds__(64 + 32 * EPW, MINB)
 k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_override, AdamHyper hp, OperandMode om) {
   using namespace tc;
-  pdl_launch_dependents();
 #ifdef MRGAN_PHASE_TIMING
   const unsigned long long pt_t0 = gtimer();
 #endif
@@ -482,7 +426,7 @@ k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_
   // tiles, which would leave a large-batch contraction of thousands of rows on one or two SMs)
   const int ksplit = (B_MN && rows_override > 1) ? rows_override : 1;
   const int kslice = (int)blockIdx.z % ksplit;
-  const TcOp& op = ops[blockIdx.z / ksplit];      // descriptor tables are written once at handle creation: safe before pdl_wait()
+  const TcOp& op = ops[blockIdx.z / ksplit];
   const int ME = op.ME, KE = op.KE, bn = op.bn;
   int NE = op.NE;
   if (rows_override > 0 && !B_MN) NE = rows_override;      // fewer batch rows (G step)
@@ -524,7 +468,6 @@ k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_
   __syncthreads();
   fence_after();
   const uint32_t tmem_base = *tmem_holder;
-  pdl_wait();                             // everything above overlapped the previous kernel's tail
   if (threadIdx.x == 0) PT_MARK(1);
 
   if (warp == 0) {
@@ -609,70 +552,20 @@ k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_
     const int npark = max(min(flen >> 4, nchunks), 0);          // chunks whose noise / h values fit the free columns
 
     if constexpr (B_MN) {
-      // ------------------------------------------------------------------ dW: fused Adam (LSU variant) or plain store
-      const int epi = op.epi;
-      if (epi == EPI_ADAM) {
-        // Keras-2.0.9 Adam fused into the dW epilogue: the gradient never leaves the SM.  Accumulator D[n = f, k];
-        // the weight tensor is [k, n] row-major, so for a fixed k the 32 lanes touch one 128-byte line of each of
-        // W, m, v.  The three streams are register double-buffered one 8-column chunk ahead, and the first chunk
-        // is requested BEFORE the accumulator is ready, so HBM latency overlaps the TMA/MMA phase.  (A/B variant of
-        // k_dw_adam_tc, which stages the optimizer state by TMA instead: MRGAN_ADAM_TMA=0.)
-        float* const adamP = op.P; float* const adamM = op.Mo; float* const adamV = op.Vo;
-        const float lr_t = folds[g.fold].lr_t[op.net];
-        const float b1 = hp.b1, b2 = hp.b2, c1 = 1.0f - hp.b1, c2 = 1.0f - hp.b2, eps = hp.eps;
-        const float ginv_a = F16 ? 1.0f / om.gscale : 1.0f;      // the dZ operand carries the loss scale
-        auto fetch = [&](int c0, float (&pw)[8], float (&pm)[8], float (&pv)[8]) {
+      // ------------------------------------------------------------------ dW: EPI_STORE into the flat gradient buffer
+      // (large-batch / data-parallel mode: Adam follows on the all-reduced gradient; the reference batch uses k_dw_adam_tc)
+      mbar_wait(tmem_full, 0);
+      fence_after();
+      float* const dst = ksplit > 1 ? op.ws + (size_t)kslice * op.ws_stride : g.C;
+      for (int c0 = cbeg; c0 < ncols; c0 += 16) {
+        float v[16];
+        tmem_ld16(trow + (uint32_t)c0, v);                   // warp-collective: every lane takes part
+        if (!f_ok) continue;
 #pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            if (f_ok && c0 + j < ncols) {
-              const size_t idx = (size_t)(n0 + c0 + j) * g.ldc + f;
-              pw[j] = __ldcs(adamP + idx); pm[j] = __ldcs(adamM + idx); pv[j] = __ldcs(adamV + idx);
-            }
-          }
-        };
-        auto apply = [&](int c0, const float (&v)[8], const float (&pw)[8], const float (&pm)[8], const float (&pv)[8]) {
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            if (f_ok && c0 + j < ncols) {
-              const size_t idx = (size_t)(n0 + c0 + j) * g.ldc + f;
-              const float gr = v[j] * ginv_a;
-              const float m = fmaf(b1, pm[j], c1 * gr), vv = fmaf(b2, pv[j], c2 * gr * gr);
-              __stcs(adamM + idx, m); __stcs(adamV + idx, vv);
-              const float w = pw[j] - lr_t * __fdividef(m, sqrtf(vv) + eps);
-              __stcs(adamP + idx, w);
-              if (F16) om.hbase[adamP + idx - om.fbase] = __float2half_rn(w);
-            }
-          }
-        };
-        float pwA[8], pmA[8], pvA[8], pwB[8], pmB[8], pvB[8], v[8];
-        fetch(cbeg, pwA, pmA, pvA);
-        fetch(cbeg + 8, pwB, pmB, pvB);
-        mbar_wait(tmem_full, 0);
-        fence_after();
-        for (int c0 = cbeg; c0 < ncols; c0 += 16) {
-          tmem_ld8(trow + (uint32_t)c0, v);
-          apply(c0, v, pwA, pmA, pvA);
-          if (c0 + 16 < ncols) fetch(c0 + 16, pwA, pmA, pvA);
-          if (c0 + 8 < ncols) {
-            tmem_ld8(trow + (uint32_t)(c0 + 8), v);
-            apply(c0 + 8, v, pwB, pmB, pvB);
-            if (c0 + 24 < ncols) fetch(c0 + 24, pwB, pmB, pvB);
-          }
-        }
-      } else {   // EPI_STORE: dW into the flat gradient buffer (data-parallel / large-batch mode: all-reduced before Adam)
-        mbar_wait(tmem_full, 0);
-        fence_after();
-        float* const dst = ksplit > 1 ? op.ws + (size_t)kslice * op.ws_stride : g.C;
-        for (int c0 = cbeg; c0 < ncols; c0 += 16) {
-          float v[16];
-          tmem_ld16(trow + (uint32_t)c0, v);                   // warp-collective: every lane takes part
-          if (!f_ok) continue;
-#pragma unroll
-          for (int j = 0; j < 16; ++j) {
-            const int k = n0 + c0 + j;
-            if (k >= NE) break;
-            dst[(size_t)k * g.ldc + f] = v[j];
-          }
+        for (int j = 0; j < 16; ++j) {
+          const int k = n0 + c0 + j;
+          if (k >= NE) break;
+          dst[(size_t)k * g.ldc + f] = v[j];
         }
       }
     } else if constexpr (!A_MN) {
@@ -747,9 +640,6 @@ k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_
         if (nrows >= 16) DX_ACT(true); else DX_ACT(false);
 #undef DX_ACT
       }
-      if (op.head == HEAD_BN_BWD)
-        head_bn_bwd<F16>(trow, cbeg, ncols, min(bn, NE - n0), f, f_ok, *static_cast<const BnDesc*>(op.hd), hp, om, folds[g.fold].lr_t[1],
-                         op.mo_off, op.vo_off);
     } else {
       // ------------------------------------------------------------------ forward: act, optional clean copy, noisy copy
       // GaussianNoise of the next layer's input (C2): the draws do not depend on the accumulator, and the epilogue warps are
@@ -818,11 +708,7 @@ k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_
 #endif
         tmem_ld16_issue(trow + (uint32_t)c0, va);
         if (ch < npk) tmem_ld16_issue(tfree + 16u * (uint32_t)ch, vn);
-#ifdef MRGAN_EXP_NODRAW
-        else if (noisy) { for (int j = 0; j < 16; ++j) nz[j] = 0.f; }
-#else
         else if (noisy) draw16(c0, nz);                        // overlaps the accumulator load
-#endif
         tmem_wait_ld();
 #ifdef MRGAN_PHASE_TIMING
         if (ch < 12) tch[2 * ch + 1] = gtimer();
@@ -895,8 +781,8 @@ k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TMEM_COLS) : "memory");
   }
   if (!B_MN && A_MN && threadIdx.x == 0 && (op.head == HEAD_DISC || op.head == HEAD_FM)) {
-    // publish the step statistics (partials added in a fixed order) and, when no k_adam launch follows, advance
-    // K.update_add(iterations, 1) and the noise step: nothing later in this step reads either
+    // publish the step statistics (partials added in a fixed order); HEAD_DISC also advances the discriminator step's
+    // K.update_add(iterations, 1) and noise step, since no k_adam launch follows it: nothing later in this step reads either
     float* const st = op.stats + (size_t)hp.t * op.stats_stride;
     if (op.head == HEAD_DISC) {
       const float Bg = (float)hp.dp_bg;
@@ -904,15 +790,13 @@ k_gemm_tc(const TcOp* __restrict__ ops, FoldState* __restrict__ folds, int rows_
       float a0 = 0.f, a1 = 0.f, a2 = 0.f;
       for (int w = 0; w < EPW; ++w) { a0 += part[3 * w]; a1 += part[3 * w + 1]; a2 += part[3 * w + 2]; }
       st[0] = a0 / Bg; st[1] = a1 / Bg; st[2] = a2 / Bg;
+      FoldState& fs = folds[op.g.fold];
+      if (hp.shared_t) fs.iterations += 1; else fs.it_net[0] += 1;
+      fs.rng_step += 1;
     } else {
       float sum = 0.f;
       for (int w = 0; w < EPW; ++w) sum += red[w];
       st[3] = sum / static_cast<const LossDesc*>(op.hd)->Wmid;
-    }
-    if (op.advance) {
-      FoldState& fs = folds[op.g.fold];
-      if (hp.shared_t) fs.iterations += 1; else fs.it_net[op.head == HEAD_DISC ? 0 : 1] += 1;
-      fs.rng_step += 1;
     }
   }
 #ifdef MRGAN_PHASE_TIMING
@@ -949,9 +833,9 @@ __global__ void __launch_bounds__(256) k_splitk_reduce(const TcOp* __restrict__ 
 // chunks with cp.async.bulk.tensor (full 128-byte lines, deep queues); the 4 epilogue warps combine each chunk
 // with the matching 8 accumulator columns from TMEM in shared memory.  24 B per parameter of HBM traffic, which
 // is the algorithmic minimum for Adam; the gradient never leaves the SM.  F16 (operand-copy mode): the operands are the
-// 16-bit copies (64 contraction rows per stage) and every chunk also carries the fp16 copy of the UPDATED weights that the
-// next forward / dX pass reads (written to smem by the epilogue, stored by TMA: +2 B per parameter).
-//   smem: 2 operand stages x 32 KB + NB chunk buffers x (3 x KC x 512 B [+ KC x 256 B]); 2 CTAs per SM.
+// 16-bit copies and every chunk also carries the fp16 copy of the UPDATED weights that the next forward / dX pass reads
+// (written to smem by the epilogue, stored by TMA: +2 B per parameter).
+//   smem: 2 operand stages x 16 KB + 3 chunk buffers x (3 x KC x 512 B [+ KC x 256 B]); 3 CTAs per SM.
 // ====================================================================================================
 struct alignas(64) TcAdamOp {
   CUtensorMap mapA, mapB;          // dZ[r, n] and A[r, k], both MN-major operands
@@ -964,7 +848,6 @@ struct alignas(64) TcAdamOp {
 };
 
 #define TCA_KC 8
-#define TCA_NB 4                   // dedicated chunk buffers (tf32); the F16 variant's chunks are 2 KB larger and it takes 3
 
 namespace tc {
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* src, int c0, int c1) {
@@ -979,14 +862,13 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 }  // namespace tc
 
-// KROWS: contraction rows (batch rows) per operand stage.  F16 with KROWS = 32 halves the operand stages (2 x 16 KB), which
-// lets THREE CTAs share an SM: a CTA spends its first microseconds on TMEM allocation, barrier set-up and the operand round
-// trips while only its first chunk buffers are in flight -- with three co-resident CTAs two of them are always streaming.
+// KROWS: contraction rows (batch rows) per operand stage, 32 fp16 / 16 fp32: 16 KB operand stages, which let THREE CTAs
+// share an SM: a CTA spends its first microseconds on TMEM allocation, barrier set-up and the operand round trips while only
+// its first chunk buffers are in flight -- with three co-resident CTAs two of them are always streaming.
 template <bool F16, int KROWS> struct TcAdamCfg {
-  static_assert(F16 ? (KROWS == 64 || KROWS == 32) : (KROWS == 32 || KROWS == 16), "operand stage geometry");
-  static constexpr bool SMALL = F16 ? KROWS == 32 : KROWS == 16;            // 16 KB operand stages
-  static constexpr int STAGES = 2, KC = TCA_KC, NB = (F16 || SMALL) ? 3 : TCA_NB;
-  static constexpr int MINB = SMALL ? 3 : 2;                                // CTAs per SM
+  static_assert(KROWS == (F16 ? 32 : 16), "operand stage geometry: 16 KB stages");
+  static constexpr int STAGES = 2, KC = TCA_KC, NB = 3;
+  static constexpr int MINB = 3;                                            // CTAs per SM
   static constexpr uint32_t MN_BOX = 128u * KROWS;                          // one MN-major box: 128 bytes (64 fp16 / 32 fp32) x KROWS rows
   static constexpr uint32_t STAGE_BYTES = (F16 ? 4 : 8) * MN_BOX;           // A + B operand tiles (128 features each)
   static constexpr uint32_t ARR_BYTES = KC * 128 * 4;                       // one array (W, m or v) of one chunk
@@ -1004,7 +886,6 @@ k_dw_adam_tc(const TcAdamOp* __restrict__ ops, FoldState* __restrict__ folds, Ad
   // the narrow layers' own grids are too small to keep HBM busy (60 % of peak against 89 % for the wide ones)
   using namespace tc;
   using Cfg = TcAdamCfg<F16, KROWS>;
-  pdl_launch_dependents();
   constexpr int STAGES = Cfg::STAGES, KC = Cfg::KC, NB = Cfg::NB, NBUF = Cfg::NBUF;
   constexpr uint32_t STAGE_BYTES = Cfg::STAGE_BYTES, ARR_BYTES = Cfg::ARR_BYTES, CHUNK_BYTES = Cfg::CHUNK_BYTES;
   constexpr int KBLK = KROWS;
@@ -1050,7 +931,6 @@ k_dw_adam_tc(const TcAdamOp* __restrict__ ops, FoldState* __restrict__ folds, Ad
   __syncthreads();
   fence_after();
   const uint32_t tmem_base = *tmem_holder;
-  pdl_wait();
 
   if (warp == 0) {
     if (lane == 0) {

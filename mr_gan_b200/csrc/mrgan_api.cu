@@ -15,10 +15,8 @@
 
 #include "../../include/mrgan.h"
 #include "kernels_simt.cuh"
-#ifdef MRGAN_WITH_TC
 #include "kernels_tc.cuh"
 #include "kernels_svm.cuh"
-#endif
 #include "kernels_dp.cuh"
 
 namespace {
@@ -80,7 +78,6 @@ struct FoldBuffers {
 }  // namespace
 
 struct mrgan_handle;
-#ifdef MRGAN_WITH_TC
 namespace {
 int tc_setup(mrgan_handle* h);
 int tc_ex_setup(mrgan_handle* h, TcOp* dst);
@@ -88,10 +85,8 @@ void tc_teardown(mrgan_handle* h);
 bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st);
 void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cudaStream_t st);
 bool tc_dw_merge(const mrgan_handle* h);
-void tc_params_changed(mrgan_handle* h, int fold, int net);
 int tc_debug_gemm(mrgan_handle* h, int mode, const GemmDesc& g, int esz);
 }
-#endif
 
 constexpr int kMaxChains = 16;
 struct mrgan_handle {
@@ -103,8 +98,6 @@ struct mrgan_handle {
   cudaStream_t stream = nullptr;
   cudaStream_t side = nullptr;        // dW (+Adam) kernels run here, concurrently with the latency-bound dX chain
   cudaEvent_t ev_pool[16] = {nullptr}; int ev_next = 0;
-  bool use_pdl = false;               // programmatic dependent launch between the kernels of a step: opt-in (MRGAN_PDL=1);
-                                      // measured neutral at 74 folds/GPU and -17 % at 12 (early-resident dependents hold SM resources)
   bool side_open = false;             // work forked to `side` since the last join (joins are no-ops otherwise)
   // the folds of a group are independent, so an epoch is captured as `nchains` parallel chains of kernels (disjoint fold
   // ranges, own main + side stream): one chain's latency-bound small kernels fill the SMs another chain leaves idle
@@ -124,9 +117,7 @@ struct mrgan_handle {
     char* mem = nullptr;
     GemmDesc* descs = nullptr;        // [NUM_EX][nf] device copies of the OP_EX* descriptors
     float* profile = nullptr;         // [nf][K][D_max]
-#ifdef MRGAN_WITH_TC
     TcOp* tcops = nullptr;            // [NUM_EX][nf] their tcgen05 views (tf32 / f16 handles)
-#endif
   } sal;
   AdamRange* d_ranges[2] = {nullptr, nullptr};
   OpInfo ops[NUM_OPS_ALL];
@@ -157,20 +148,14 @@ struct mrgan_handle {
   float* d_dpmem = nullptr; DpBufs* d_dpbufs = nullptr;
   float *dp_bnf = nullptr, *dp_bnb = nullptr, *dp_fm = nullptr;   // [nf][2*500], [nf][2*500], [nf][2*250]
   float* dp_losspart = nullptr; unsigned* dp_lossctr = nullptr;    // k_loss_disc block partials [nf][4*64] and arrival counters [nf]
-#ifdef MRGAN_WITH_TC
   TcOp* d_tcops = nullptr;            // [NUM_OPS][nf] tensor maps + epilogue descriptors
   int tc_bn[NUM_OPS_ALL] = {0}, tc_maxME[NUM_OPS_ALL] = {0}, tc_maxNE[NUM_OPS_ALL] = {0};
   int tc_ksplit[NUM_OPS] = {0};       // large-batch dW: contraction slices per tile (deterministic split-K), 0/1 = off
   bool tc_mt1[NUM_OPS_ALL] = {false}; // large-batch forward / dX whose 256 x 256 tiling would leave SMs idle: 128-feature CTAs (tc_pick_tile)
   float* d_tcws = nullptr;            // ... and their partial-product workspace
-  bool tc_fused_adam = true;          // dW epilogue applies Adam in place (no gradient round trip)
-  bool tc_mt2 = true;                 // forward / dX: 256 features per CTA where the layer is wide enough (MRGAN_MT2=0 disables)
-  bool tc_adam_tma = true;            // ... with W/m/v staged through smem by TMA (k_dw_adam_tc) instead of the LSU
-  bool tc_dw_merge = true;            // dW+Adam of the narrow layers (D 3..6; G 1, 2) in one launch each; MRGAN_DW_MERGE=0: one launch per layer
-  bool tc_dw_small = true;            // dW+Adam: 16 KB operand stages (32 fp16 / 16 fp32 batch rows) -> three CTAs per SM; MRGAN_DW_SMALL=0: two
+  bool tc_fused_adam = true;          // dW and Adam in one kernel, k_dw_adam_tc (no gradient round trip)
   int tc_heads = 0;                   // losses / feature matching / BatchNorm fused into GEMM epilogues (set by tc_setup), bit mask:
-                                      // 1 = HEAD_DISC (no k_loss_disc, no k_adam of D), 2 = HEAD_FM (no k_fm), 4 = HEAD_BN (no k_bn_fwd),
-                                      // 8 = HEAD_BN_BWD (no k_bn_bwd); 2 and 8 together also retire the generator's k_adam
+                                      // 1 = HEAD_DISC (no k_loss_disc, no k_adam of D), 2 = HEAD_FM (no k_fm), 4 = HEAD_BN (no k_bn_fwd)
   TcAdamOp* d_tcadam = nullptr;       // [NUM_OPS][nf]
   AdamRange* d_ranges_tc[2] = {nullptr, nullptr};   // what is left for k_adam: BN gamma/beta (G), nothing (D)
   // MRGAN_MODEL_SVM: workspace of mrgan_svm_fit (one allocation, reused while it is large enough)
@@ -190,7 +175,6 @@ struct mrgan_handle {
     SvmSplitOp* d_split_s = nullptr; SvmGemmOp* d_gemm_s = nullptr;
     float** d_Ks = nullptr; float** d_decs = nullptr; int** d_preds = nullptr; int* d_ns = nullptr;   // one-fold pointer tables
   } svm;
-#endif
 };
 
 namespace {
@@ -521,17 +505,12 @@ void init_ones(mrgan_handle* h) {
 }
 
 
-// ------------------------------------------------------------------ kernel launch with programmatic stream serialization
+// ------------------------------------------------------------------ kernel launch (a failure is kept as the handle's sticky error)
 template <typename... KArgs, typename... Args>
 void launch_k(mrgan_handle* h, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = h->use_pdl ? 1 : 0;
   const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
   if (e != cudaSuccess && !h->sticky) { h->sticky = MRGAN_ERR_CUDA; h->err = std::string("kernel launch: ") + cudaGetErrorString(e); }
   h->launches++;
@@ -607,7 +586,7 @@ void dp_allreduce_grads(mrgan_handle* h, int net) {
   dp_allreduce(h, h->Gr + h->net[net][0].off, (size_t)n);      // the nets of all folds are contiguous in the flat buffer
 }
 
-void launch_adam(mrgan_handle* h, int f0, int nfl, int net, bool counters_only);
+void launch_adam(mrgan_handle* h, int f0, int nfl, int net);
 
 // Pointer sets of the fused exchange.  Real ranks: the same offsets inside every rank's (IPC-mapped) arena.  Virtual ranks:
 // fold r's net inside this handle's own flat buffers.
@@ -660,7 +639,7 @@ void dp_exchange(mrgan_handle* h, int net) {
 void dp_update(mrgan_handle* h, int f0, int nfl, int net) {
   if (h->dp_fused) { dp_exchange(h, net); return; }
   dp_allreduce_grads(h, net);
-  launch_adam(h, f0, nfl, net, false);
+  launch_adam(h, f0, nfl, net);
 }
 
 // Scratch of the split (statistics -> [all-reduce] -> apply) BatchNorm / feature-matching kernels: used by the data-parallel
@@ -702,9 +681,7 @@ void launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cu
   int M = oi.maxM;
   if (rows_override > 0 && !oi.at) M = rows_override;
   const GemmDesc* d = (op < NUM_OPS ? h->d_descs + (size_t)op * h->nf : h->sal.descs + (size_t)(op - NUM_OPS) * h->nf) + f0;
-#ifdef MRGAN_WITH_TC
   if (h->cfg.precision != MRGAN_PREC_FP32 && tc_launch_gemm(h, op, f0, nfl, rows_override, st)) return;
-#endif
   dim3 grid((oi.maxN + 63) / 64, (M + 63) / 64, nfl);
   if (!oi.at && !oi.bt) launch_k(h, k_gemm_simt<false, false>, grid, dim3(256), 0, st, d, (const FoldState*)h->d_folds, rows_override, h->hp);
   else if (!oi.at && oi.bt) launch_k(h, k_gemm_simt<false, true>, grid, dim3(256), 0, st, d, (const FoldState*)h->d_folds, rows_override, h->hp);
@@ -747,16 +724,14 @@ void launch_prep(mrgan_handle* h, int f0, int nfl, int mode, int from_stage, int
 #undef LAUNCH_PREP
 }
 
-void launch_adam(mrgan_handle* h, int f0, int nfl, int net, bool counters_only) {
+void launch_adam(mrgan_handle* h, int f0, int nfl, int net) {
   long long nmax = 0;
   for (int f = f0; f < f0 + nfl; ++f) nmax = h->net[net][f].n > nmax ? h->net[net][f].n : nmax;
   int blocks = (int)((nmax / 4 + 255) / 256);
   if (blocks > 2048) blocks = 2048;
   if (blocks < 1) blocks = 1;
   const AdamRange* ranges = h->d_ranges[net];
-#ifdef MRGAN_WITH_TC
-  if (h->cfg.precision != MRGAN_PREC_FP32 && h->tc_fused_adam) { ranges = h->d_ranges_tc[counters_only ? 0 : net]; blocks = 1; }
-#endif
+  if (h->cfg.precision != MRGAN_PREC_FP32 && h->tc_fused_adam) { ranges = h->d_ranges_tc[net]; blocks = 1; }
   // f16 mode: the gradient buffer carries the loss scale, and every parameter update refreshes the fp16 operand copy
   const float ginv = h->om.mode == 2 ? 1.0f / h->om.gscale : 1.0f;
   __half* Ph = h->om.mode == 2 ? h->harena + (h->P - reinterpret_cast<float*>(h->arena)) : nullptr;
@@ -764,22 +739,9 @@ void launch_adam(mrgan_handle* h, int f0, int nfl, int net, bool counters_only) 
            ginv, Ph);
 }
 
-// The side stream's dW kernels read the step's activation buffers (a[l], dZ[l]), which the NEXT step's batch assembly
-// and forward pass overwrite: every step therefore joins the side stream before it ends (measured: deferring the join
-// past the next step's generator forward gains nothing once several fold chains run concurrently, and would need
-// double-buffered activations).
-bool deferred_join(const mrgan_handle*) { return false; }
-
-int heads_on(const mrgan_handle* h) {
-#ifdef MRGAN_WITH_TC
-  return h->cfg.precision != MRGAN_PREC_FP32 ? h->tc_heads : 0;
-#else
-  return 0;
-#endif
-}
+int heads_on(const mrgan_handle* h) { return h->cfg.precision != MRGAN_PREC_FP32 ? h->tc_heads : 0; }
 
 void enqueue_gen_fwd(mrgan_handle* h, int f0, int nfl, int op_g3) {
-  if (deferred_join(h)) join_side(h);          // generator weights of the previous G step (GW1..3 on the side stream)
   launch_gemm(h, OP_G1, f0, nfl, 0);
   if (heads_on(h) & 4) {                       // BatchNorm ran in G1's epilogue
     launch_gemm(h, OP_G2, f0, nfl, 0);
@@ -817,23 +779,21 @@ void enqueue_disc_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) 
     launch_k(h, k_loss_disc, dim3(lb, 1, nfl), dim3(256), 0, h->stream, (const LossDesc*)(h->d_loss + f0), h->d_step_stats, f0, h->nf, t, B,
              c.n_classes, c.unlabeled_weight, h->om, h->hp.dp_bg, h->dp_losspart, h->dp_lossctr);
   }
-#ifdef MRGAN_WITH_TC
   const bool merge = tc_dw_merge(h);
-#else
-  const bool merge = false;
-#endif
   for (int l = 6; l >= 1; --l) {      // dX first: it reads W_l, which the fused-Adam dW epilogue overwrites
     if (l >= 2) launch_gemm(h, OP_DX2 + l - 2, f0, nfl, 0);
     if (merge && l > 3) continue;     // the narrow layers 3..6 share ONE dW+Adam launch, after the last dX that reads their weights
     fork_side(h);                     // dW_l (+Adam) streams HBM on the side while main continues the dX chain
-#ifdef MRGAN_WITH_TC
     if (merge && l == 3) { tc_launch_dw_adam(h, OP_DW3, 4, f0, nfl, h->side); continue; }
-#endif
     launch_gemm(h, OP_DW1 + l - 1, f0, nfl, 0, h->side);
   }
-  if (!deferred_join(h) || from_stage) join_side(h);   // deferred: dW1+Adam overlaps the next G step's generator forward
+  // The side stream's dW kernels read the step's activation buffers (a[l], dZ[l]), which the NEXT step's batch assembly
+  // and forward pass overwrite: every step joins the side stream before it ends (measured: deferring the join past the
+  // next step's generator forward gains nothing once several fold chains run concurrently, and would need
+  // double-buffered activations).
+  join_side(h);
   if (h->dp_world > 1) dp_update(h, f0, nfl, 0);
-  else if (!heads) launch_adam(h, f0, nfl, 0, false);
+  else if (!heads) launch_adam(h, f0, nfl, 0);
   if (from_stage) dp_allreduce(h, h->d_step_stats + ((size_t)t * h->nf + f0) * 4, (size_t)nfl * 4);
 }
 
@@ -845,7 +805,6 @@ void enqueue_gen_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
   h->hp.t = t;
   launch_prep(h, f0, nfl, 1, from_stage, t, 2 * B);
   enqueue_gen_fwd(h, f0, nfl, OP_G3G);
-  if (deferred_join(h)) join_side(h);          // discriminator weights updated by the D step's dW+Adam kernels
   for (int l = 0; l < 5; ++l) launch_gemm(h, OP_D1G + l, f0, nfl, 0);
   if (h->d_dpbufs) {
     const dim3 fmg((kDW[4] + BN_COLS - 1) / BN_COLS, split_chunks(B), nfl), fmt(B > 256 ? 1024 : 256);
@@ -864,11 +823,7 @@ void enqueue_gen_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
   fork_side(h);
   launch_gemm(h, OP_GW3, f0, nfl, 0, h->side);
   launch_gemm(h, OP_GX2, f0, nfl, 0);
-#ifdef MRGAN_WITH_TC
   const bool merge = tc_dw_merge(h);
-#else
-  const bool merge = false;
-#endif
   if (!merge) {
     fork_side(h);
     launch_gemm(h, OP_GW2, f0, nfl, 0, h->side);
@@ -879,18 +834,15 @@ void enqueue_gen_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
     dp_allreduce(h, h->dp_bnb + (size_t)f0 * 2 * kGH, (size_t)nfl * 2 * kGH);
     k_bn_bwd_apply<<<bng, bnt, 0, h->stream>>>(h->d_bn + f0, h->d_dpbufs + f0, h->om, h->hp.dp_bg);
     h->launches += 2;
-  } else if (!(hm & 8)) {   // otherwise GX2's epilogue did BatchNorm backward and the Adam update of gamma / beta
+  } else {
     launch_k(h, k_bn_bwd, bng, bnt, 0, h->stream, (const BnDesc*)(h->d_bn + f0), h->om);
   }
   fork_side(h);
-#ifdef MRGAN_WITH_TC
   if (merge) tc_launch_dw_adam(h, OP_GW1, 2, f0, nfl, h->side);      // G layers 1 and 2 share one dW+Adam launch
-  else
-#endif
-  launch_gemm(h, OP_GW1, f0, nfl, 0, h->side);
-  if (!deferred_join(h) || from_stage) join_side(h);
+  else launch_gemm(h, OP_GW1, f0, nfl, 0, h->side);
+  join_side(h);
   if (h->dp_world > 1) dp_update(h, f0, nfl, 1);
-  else if ((hm & 10) != 10) launch_adam(h, f0, nfl, 1, (hm & 8) != 0);      // gamma / beta and the counters, unless heads took both over
+  else launch_adam(h, f0, nfl, 1);      // gamma / beta and the generator's step counters
   dp_allreduce(h, h->d_step_stats + ((size_t)t * h->nf + f0) * 4, (size_t)nfl * 4);
 }
 
@@ -910,7 +862,7 @@ void enqueue_nn_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage, in
     launch_gemm(h, OP_DW1 + l - 1, f0, nfl, 0, h->side);
   }
   join_side(h);
-  launch_adam(h, f0, nfl, 0, false);
+  launch_adam(h, f0, nfl, 0);
 }
 
 // test_batch (mr_gan.py:171): phase 0, no noise; with_pred: also the predicted class of every row (fb[f].pred / pred_s)
@@ -965,9 +917,7 @@ int saliency_setup(mrgan_handle* h) {
   auto layout = [&](Arena& ar) {
     S.descs = ar.take<GemmDesc>((size_t)NUM_EX * nf);
     S.profile = ar.take<float>((size_t)nf * h->cfg.n_classes * max_D(h, 0, nf));
-#ifdef MRGAN_WITH_TC
     S.tcops = tc ? ar.take<TcOp>((size_t)NUM_EX * nf) : nullptr;
-#endif
   };
   Arena sizing;
   layout(sizing);
@@ -978,11 +928,7 @@ int saliency_setup(mrgan_handle* h) {
   int rc = MRGAN_OK;
   if (cudaMemcpy(S.descs, h->h_descs.data() + (size_t)NUM_OPS * nf, (size_t)NUM_EX * nf * sizeof(GemmDesc), cudaMemcpyHostToDevice) != cudaSuccess)
     rc = fail(h, MRGAN_ERR_CUDA, "saliency workspace: descriptor upload failed");
-#ifdef MRGAN_WITH_TC
   if (rc == MRGAN_OK && tc) rc = tc_ex_setup(h, S.tcops);
-#else
-  (void)tc;
-#endif
   if (rc != MRGAN_OK) { cudaFree(mem); return rc; }
   S.mem = mem;
   return MRGAN_OK;
@@ -1044,7 +990,7 @@ void pack_params(const mrgan_handle* h, int fold, int net, const float* src, std
   }
 }
 
-int build_graph(mrgan_handle* h, int key, int nb, int n_idx_nn) {
+int build_graph(mrgan_handle* h, int key, int nb) {
   if (h->graphs.count(key)) return MRGAN_OK;
   const mrgan_config& c = h->cfg;
   const long long before = h->launches;
@@ -1092,7 +1038,6 @@ int build_graph(mrgan_handle* h, int key, int nb, int n_idx_nn) {
   h->graphs[key] = ge;
   h->graph_nodes[key] = h->launches - before;
   h->launches = before;
-  (void)n_idx_nn;
   return MRGAN_OK;
 }
 
@@ -1115,7 +1060,6 @@ int upload_indices(mrgan_handle* h, const int32_t* const* streams, int n_streams
 }  // namespace
 
 
-#ifdef MRGAN_WITH_TC
 // ------------------------------------------------------------------ tcgen05 path: host side
 namespace {
 
@@ -1126,7 +1070,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 // 2D fp32 tensor [rows, cols] with `pitch` floats per row; box = 32 columns (one 128B swizzle row) x box_rows
 // L2 promotion of the TMA loads: every box row is one 128-byte line of a row-major matrix, so neighbouring boxes /
 // k-blocks touch the adjacent 128 bytes of the same DRAM page; fetching 256 B per miss halves the DRAM activations.
-CUtensorMapL2promotion g_l2_promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+constexpr CUtensorMapL2promotion kL2Promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
 
 // esz = 4: fp32 elements (read as tf32); esz = 2: fp16 elements (`base` then points at __half data, pitch in elements).
 // The swizzled box is always one 128-byte row wide (32 fp32 / 64 fp16 elements); MN-major 32-bit operands need the
@@ -1143,7 +1087,7 @@ bool make_map(EncodeTiledFn fn, CUtensorMap* m, const void* base, int cols, int 
             strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
             box_cols != row_elems ? CU_TENSOR_MAP_SWIZZLE_NONE
                                   : ((mn_major && esz == 4) ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B),
-            g_l2_promo,
+            kL2Promo,
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
@@ -1203,10 +1147,7 @@ template <bool F, bool V> void tc_set_smem_attr_fmt() {
   cudaFuncSetAttribute(K_TC_FWD2(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   cudaFuncSetAttribute(K_TC_DX2(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   cudaFuncSetAttribute(K_TC_DW(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(128, TC_DW_STAGES));
-  if (!V) {
-    cudaFuncSetAttribute(k_dw_adam_tc<F, (F ? 64 : 32)>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcAdamCfg<F, (F ? 64 : 32)>::SMEM);
-    cudaFuncSetAttribute(k_dw_adam_tc<F, (F ? 32 : 16)>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcAdamCfg<F, (F ? 32 : 16)>::SMEM);
-  }
+  if (!V) cudaFuncSetAttribute(k_dw_adam_tc<F, (F ? 32 : 16)>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcAdamCfg<F, (F ? 32 : 16)>::SMEM);
 }
 void tc_set_smem_attr() {
   tc_set_smem_attr_fmt<false, false>(); tc_set_smem_attr_fmt<true, false>();
@@ -1233,16 +1174,14 @@ bool tc_fill_op(EncodeTiledFn fn, TcOp& t, const GemmDesc& g, int mode, int esz 
   t.ME = g.N; t.NE = g.M; t.KE = g.K;
   const int kb = 128 / esz;   // contraction rows of an MN-major box = elements of one 128-byte row
   if (mode == 0) {            // forward: C[M rows, N feats] = act[M, K] @ W[K, N]
-    t.epi = EPI_FWD;
     t.bn = g.M <= 256 ? round_up(g.M, 16) : bn_big;
     return make_map(fn, &t.mapA, g.B, g.N, g.K, g.ldb, kb, true, 0, esz) && make_map(fn, &t.mapB, g.A, g.K, g.M, g.lda, t.bn, false, 0, esz);
   }
   if (mode == 1) {            // dX: C[M rows, N in-feats] = dZ[M, K] @ W[N, K]^T
-    t.epi = EPI_DX;
     t.bn = g.M <= 256 ? round_up(g.M, 16) : bn_big;
     return make_map(fn, &t.mapA, g.B, g.K, g.N, g.ldb, 128, false, 0, esz) && make_map(fn, &t.mapB, g.A, g.K, g.M, g.lda, t.bn, false, 0, esz);
   }
-  t.epi = EPI_STORE;          // dW: C[M in-feats(+1), N out-feats] = act[K rows, M]^T @ dZ[K rows, N]
+  // dW: C[M in-feats(+1), N out-feats] = act[K rows, M]^T @ dZ[K rows, N]
   t.bn = g.K > 512 ? 256 : 128;   // a long contraction (large batch) is a regular big GEMM: 256 x 256 tiles
   return make_map(fn, &t.mapA, g.B, g.N, g.K, g.ldb, kb, true, 0, esz) && make_map(fn, &t.mapB, g.A, g.M, g.K, g.lda, kb, true, 0, esz);
 }
@@ -1289,16 +1228,9 @@ int tc_make_op(mrgan_handle* h, EncodeTiledFn fn, int op, TcOp* ts) {
     if (h->tc_heads) {
       t.stats = h->d_step_stats + (size_t)f * 4;
       t.stats_stride = nf * 4;
-      t.mo_off = h->Mo - h->P; t.vo_off = h->Vo - h->P;
-      if (op == OP_D6 && (h->tc_heads & 1)) { t.head = HEAD_DISC; t.hd = h->d_loss + f; t.advance = 1; }
-      else if (op == OP_D5G && (h->tc_heads & 2)) { t.head = HEAD_FM; t.hd = h->d_loss + f; t.advance = (h->tc_heads & 8) ? 1 : 0; }
+      if (op == OP_D6 && (h->tc_heads & 1)) { t.head = HEAD_DISC; t.hd = h->d_loss + f; }
+      else if (op == OP_D5G && (h->tc_heads & 2)) { t.head = HEAD_FM; t.hd = h->d_loss + f; }
       else if (op == OP_G1 && (h->tc_heads & 4)) { t.head = HEAD_BN; t.hd = h->d_bn + f; }
-      else if (op == OP_GX2 && (h->tc_heads & 8)) { t.head = HEAD_BN_BWD; t.hd = h->d_bn + f; }
-    }
-    if (mode == 2) {
-      if (h->tc_fused_adam) t.epi = EPI_ADAM;
-      const size_t off = (size_t)(g.C - h->Gr);
-      t.P = h->P + off; t.Mo = h->Mo + off; t.Vo = h->Vo + off;
     }
     if (t.bn > h->tc_bn[op]) h->tc_bn[op] = t.bn;
     if (t.ME > h->tc_maxME[op]) h->tc_maxME[op] = t.ME;
@@ -1311,18 +1243,11 @@ int tc_setup(mrgan_handle* h) {
   EncodeTiledFn fn = tc_encoder();
   if (!fn) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
   if (h->R > 512) h->tc_fused_adam = false;   // large batch: dW is tensor-bound -> big-tile GEMM + flat Adam instead of the fused kernel
-  if (const char* pr = getenv("MRGAN_L2PROMO"))
-    g_l2_promo = atoi(pr) == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : (atoi(pr) == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                 : (atoi(pr) == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
   const int nf = h->nf;
-  // reductions fused into GEMM epilogues: the reference batch regime (one batch tile, batch statistics local to the GPU)
+  // reductions fused into GEMM epilogues: the reference batch regime (one batch tile, batch statistics local to the GPU).
+  // BatchNorm backward stays the stand-alone k_bn_bwd: fused into GX2's epilogue it measured 1-2 % slower (a thread per
+  // feature walks all 50 rows twice behind a GEMM whose own work is tiny).
   h->tc_heads = (h->cfg.model == MRGAN_MODEL_GAN && h->tc_fused_adam && !h->d_dpbufs && h->R <= 256 && h->cfg.n_classes <= 32) ? 7 : 0;
-  // default: loss, feature-matching and BatchNorm-forward heads.  HEAD_BN_BWD (bit 8) is implemented and parity-tested but
-  // measured 1-2 % slower than the stand-alone k_bn_bwd (a thread per feature walks all 50 rows twice behind a GEMM whose
-  // own work is tiny), so it is opt-in: MRGAN_HEADS=15.  MRGAN_HEADS=0 runs every reduction as its own kernel (A/B).
-  if (const char* hv = getenv("MRGAN_HEADS")) h->tc_heads = h->tc_heads ? (atoi(hv) & 15) : 0;
-  if (const char* kr = getenv("MRGAN_DW_SMALL")) h->tc_dw_small = atoi(kr) != 0;
-  if (const char* kr = getenv("MRGAN_DW_MERGE")) h->tc_dw_merge = atoi(kr) != 0;
   std::vector<TcOp> ops((size_t)NUM_OPS * nf);
   memset(ops.data(), 0, ops.size() * sizeof(TcOp));
   for (int op = 0; op < NUM_OPS; ++op) {
@@ -1364,7 +1289,7 @@ int tc_setup(mrgan_handle* h) {
   }
   if (cudaMalloc(&h->d_tcops, ops.size() * sizeof(TcOp)) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMalloc tc ops");
   if (cudaMemcpy(h->d_tcops, ops.data(), ops.size() * sizeof(TcOp), cudaMemcpyHostToDevice) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMemcpy tc ops");
-  if (h->tc_fused_adam && h->tc_adam_tma) {
+  if (h->tc_fused_adam) {
     std::vector<TcAdamOp> aops((size_t)NUM_OPS * nf);
     memset(aops.data(), 0, aops.size() * sizeof(TcAdamOp));
     for (int op = 0; op < NUM_OPS; ++op) {
@@ -1373,27 +1298,29 @@ int tc_setup(mrgan_handle* h) {
       for (int f = 0; f < nf; ++f) {
         const TcOp& t = ops[(size_t)op * nf + f];
         TcAdamOp& a = aops[(size_t)op * nf + f];
-        a.mapA = t.mapA; a.mapB = t.mapB; a.ME = t.ME; a.NE = t.NE; a.KE = t.KE; a.fold = t.g.fold; a.net = t.net;
-        if (h->tc_dw_small) {      // operand boxes of 32 (fp16) / 16 (fp32) batch rows: 16 KB stages
-          const GemmDesc& g = t.g;
-          bool ok;
-          if (h->om.mode == 2) {
-            const __half* hA = h->harena + (g.A - h->om.fbase);
-            const __half* hB = h->harena + (g.B - h->om.fbase);
-            ok = make_map(fn, &a.mapA, hB, g.N, g.K, g.ldb, 32, true, 0, 2) && make_map(fn, &a.mapB, hA, g.M, g.K, g.lda, 32, true, 0, 2);
-          } else {
-            ok = make_map(fn, &a.mapA, g.B, g.N, g.K, g.ldb, 16, true) && make_map(fn, &a.mapB, g.A, g.M, g.K, g.lda, 16, true);
-          }
-          if (!ok) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled (dW operands) failed");
+        const GemmDesc& g = t.g;
+        a.ME = t.ME; a.NE = t.NE; a.KE = t.KE; a.fold = g.fold; a.net = t.net;
+        // operand boxes of 32 (fp16) / 16 (fp32) batch rows: 16 KB stages
+        bool ok;
+        if (h->om.mode == 2) {
+          const __half* hA = h->harena + (g.A - h->om.fbase);
+          const __half* hB = h->harena + (g.B - h->om.fbase);
+          ok = make_map(fn, &a.mapA, hB, g.N, g.K, g.ldb, 32, true, 0, 2) && make_map(fn, &a.mapB, hA, g.M, g.K, g.lda, 32, true, 0, 2);
+        } else {
+          ok = make_map(fn, &a.mapA, g.B, g.N, g.K, g.ldb, 16, true) && make_map(fn, &a.mapB, g.A, g.M, g.K, g.lda, 16, true);
         }
+        if (!ok) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled (dW operands) failed");
         a.ginv = h->om.mode == 2 ? 1.0f / h->om.gscale : 1.0f;
+        // the layer's weights and Adam slots: the gradient tensor's offset inside the flat buffers
+        const size_t off = (size_t)(g.C - h->Gr);
+        float *P = h->P + off, *Mo = h->Mo + off, *Vo = h->Vo + off;
         // fp16 operand copy of W (refreshed with every update), same geometry as the fp32 tensor
-        if (h->om.mode == 2 && !make_map(fn, &a.mapH, h->harena + (t.P - h->om.fbase), t.ME, t.NE, t.g.ldc, TCA_KC, false, 128, 2))
+        if (h->om.mode == 2 && !make_map(fn, &a.mapH, h->harena + (P - h->om.fbase), t.ME, t.NE, g.ldc, TCA_KC, false, 128, 2))
           return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled (fp16 weight copy) failed");
         // W / m / v as [rows = in+1, cols = out] with the tensor's pitch; box 128 cols x KC rows, clipped at the logical extents
-        if (!make_map(fn, &a.mapP, t.P, t.ME, t.NE, t.g.ldc, TCA_KC, false, 128) ||
-            !make_map(fn, &a.mapM, t.Mo, t.ME, t.NE, t.g.ldc, TCA_KC, false, 128) ||
-            !make_map(fn, &a.mapV, t.Vo, t.ME, t.NE, t.g.ldc, TCA_KC, false, 128))
+        if (!make_map(fn, &a.mapP, P, t.ME, t.NE, g.ldc, TCA_KC, false, 128) ||
+            !make_map(fn, &a.mapM, Mo, t.ME, t.NE, g.ldc, TCA_KC, false, 128) ||
+            !make_map(fn, &a.mapV, Vo, t.ME, t.NE, g.ldc, TCA_KC, false, 128))
           return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled (optimizer state) failed");
       }
     }
@@ -1443,8 +1370,6 @@ void tc_teardown(mrgan_handle* h) {
   h->d_tcops = nullptr;
 }
 
-void tc_params_changed(mrgan_handle*, int, int) {}   // fp32 master weights are the MMA operands: nothing to refresh
-
 // dW + fused Adam of `nlayers` consecutive ops (op, op + 1, ...) of folds [f0, f0 + nfl) in ONE launch (grid.z = layer x fold;
 // CTAs beyond a layer's extents exit at once)
 void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cudaStream_t st) {
@@ -1456,15 +1381,12 @@ void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cu
   }
   const dim3 grid(gx, gy, nlayers * nfl);
   const TcAdamOp* ad = h->d_tcadam + (size_t)op * h->nf + f0;
-  // small operand stages: three CTAs per SM (default); MRGAN_DW_SMALL=0: the two-CTA configuration (A/B)
-  if (f16 && h->tc_dw_small) launch_k(h, k_dw_adam_tc<true, 32>, grid, dim3(192), TcAdamCfg<true, 32>::SMEM, st, ad, h->d_folds, h->hp, nfl, h->nf);
-  else if (f16) launch_k(h, k_dw_adam_tc<true, 64>, grid, dim3(192), TcAdamCfg<true, 64>::SMEM, st, ad, h->d_folds, h->hp, nfl, h->nf);
-  else if (h->tc_dw_small) launch_k(h, k_dw_adam_tc<false, 16>, grid, dim3(192), TcAdamCfg<false, 16>::SMEM, st, ad, h->d_folds, h->hp, nfl, h->nf);
-  else launch_k(h, k_dw_adam_tc<false, 32>, grid, dim3(192), TcAdamCfg<false, 32>::SMEM, st, ad, h->d_folds, h->hp, nfl, h->nf);
+  if (f16) launch_k(h, k_dw_adam_tc<true, 32>, grid, dim3(192), TcAdamCfg<true, 32>::SMEM, st, ad, h->d_folds, h->hp, nfl, h->nf);
+  else launch_k(h, k_dw_adam_tc<false, 16>, grid, dim3(192), TcAdamCfg<false, 16>::SMEM, st, ad, h->d_folds, h->hp, nfl, h->nf);
 }
 
 // the fused-Adam dW path is active (tcgen05 precision, reference batch regime): narrow layers may share launches
-bool tc_dw_merge(const mrgan_handle* h) { return h->cfg.precision != MRGAN_PREC_FP32 && h->d_tcadam != nullptr && h->tc_dw_merge; }
+bool tc_dw_merge(const mrgan_handle* h) { return h->cfg.precision != MRGAN_PREC_FP32 && h->d_tcadam != nullptr; }
 
 bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st) {
   const OpInfo& oi = h->ops[op];
@@ -1490,7 +1412,7 @@ bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override,
     return true;
   }
   const bool head_mt2 = (h->tc_heads & 2) && op == OP_D5G;      // feature matching: one CTA sums the loss over all 250 features
-  if (!oi.at && !h->tc_mt1[op] && ((h->tc_mt2 && tc_use_mt2(h->tc_maxME[op], bn)) || head_mt2)) {
+  if (!oi.at && !h->tc_mt1[op] && (tc_use_mt2(h->tc_maxME[op], bn) || head_mt2)) {
     grid.x = (h->tc_maxME[op] + 255) / 256;
     const size_t smem = tc_smem_bytes(bn, TC_FWD_STAGES, 2);
     if (!oi.bt) TC_LAUNCH(h, f16, K_TC_FWD2, grid, dim3(TC_FWD_THREADS), smem, st, d, h->d_folds, rows_override, h->hp, h->om);
@@ -1516,7 +1438,6 @@ bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override,
 }
 
 }  // namespace
-#endif  // MRGAN_WITH_TC
 
 // ====================================================================== C-ABI
 extern "C" {
@@ -1575,9 +1496,6 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
   if (cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess || prop.major != 10 || prop.minor != 0)
     return fail(nullptr, MRGAN_ERR_NO_DEVICE, "device is not sm_100 (B200): the library holds sm_100a code only and has no CPU fallback");
   if (cfg->precision < MRGAN_PREC_FP32 || cfg->precision > MRGAN_PREC_F16) return fail(nullptr, MRGAN_ERR_ARG, "bad config (precision)");
-#ifndef MRGAN_WITH_TC
-  if (cfg->precision != MRGAN_PREC_FP32) return fail(nullptr, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#endif
   h = new mrgan_handle();
   h->cfg = *cfg;
   h->nf = cfg->n_folds;
@@ -1630,12 +1548,6 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
   ok = ok && cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking) == cudaSuccess;
   for (int i = 0; i < 16 && ok; ++i) ok = cudaEventCreateWithFlags(&h->ev_pool[i], cudaEventDisableTiming) == cudaSuccess;
   {
-#ifdef MRGAN_WITH_TC
-    if (const char* mt2 = getenv("MRGAN_MT2")) h->tc_mt2 = atoi(mt2) != 0;
-    if (const char* at = getenv("MRGAN_ADAM_TMA")) h->tc_adam_tma = atoi(at) != 0;    // 0: LSU epilogue of k_gemm_tc (A/B switch)
-#endif
-    const char* pdl = getenv("MRGAN_PDL");
-    if (pdl) h->use_pdl = atoi(pdl) != 0;
     const char* env = getenv("MRGAN_CHAINS");
     int nch = env ? atoi(env) : (h->nf >= 32 ? 4 : (h->nf >= 8 ? 2 : 1));
     if (nch < 1) nch = 1;
@@ -1669,12 +1581,10 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
     int rc = alloc_split_bufs(h);
     if (rc != MRGAN_OK) return cleanup(rc);
   }
-#ifdef MRGAN_WITH_TC
   if (cfg->precision != MRGAN_PREC_FP32) {
     int rc = tc_setup(h);
     if (rc != MRGAN_OK) return cleanup(rc);
   }
-#endif
   e = cudaStreamSynchronize(h->stream);
   if (e == cudaSuccess) e = cudaGetLastError();
   if (e != cudaSuccess) return cleanup(fail(nullptr, MRGAN_ERR_CUDA, std::string("create: ") + cudaGetErrorString(e)));
@@ -1699,10 +1609,8 @@ int mrgan_destroy(mrgan_handle* h) {
   if (h->d_dpmem) cudaFree(h->d_dpmem);
   if (h->d_dpbufs) cudaFree(h->d_dpbufs);
   if (h->sal.mem) cudaFree(h->sal.mem);
-#ifdef MRGAN_WITH_TC
   tc_teardown(h);
   if (h->svm.mem) cudaFree(h->svm.mem);
-#endif
   if (h->arena) cudaFree(h->arena);
   if (h->harena) cudaFree(h->harena);
   if (h->h_epoch_stats) cudaFreeHost(h->h_epoch_stats);
@@ -1750,9 +1658,6 @@ int mrgan_set_params(mrgan_handle* h, int fold, int net, const float* src, int64
     h->launches++;
   }
   CK(cudaStreamSynchronize(h->stream));
-#ifdef MRGAN_WITH_TC
-  if (h->cfg.precision != MRGAN_PREC_FP32) tc_params_changed(h, fold, net);
-#endif
   return MRGAN_OK;
 }
 
@@ -2054,25 +1959,14 @@ int mrgan_train_epoch(mrgan_handle* h, const int32_t* idx_lab, const int32_t* id
   return launch_epoch(h, nb, stats);
 }
 
-// the epoch itself (index arrays already on their way on the handle's stream): one graph launch, or step by step
+// the epoch itself (index arrays already on their way on the handle's stream): one graph launch.  Data-parallel epochs are
+// captured like the others (NCCL collectives and the fused exchange are stream-ordered graph nodes; one chain, so every
+// rank issues them in the same order).
 static int launch_epoch(mrgan_handle* h, int nb, mrgan_epoch_stats* stats) {
-  // data-parallel epochs are captured like the others (NCCL collectives and the fused exchange are stream-ordered graph
-  // nodes; one chain, so every rank issues them in the same order); MRGAN_DP_GRAPH=0 enqueues them step by step instead
-  static const bool dp_graph = !(getenv("MRGAN_DP_GRAPH") && atoi(getenv("MRGAN_DP_GRAPH")) == 0);
-  const bool eager = h->dp_world > 1 && !dp_graph;
-  int rc = MRGAN_OK;
-  if (!eager) { rc = build_graph(h, nb, nb, 0); if (rc) return rc; }
+  const int rc = build_graph(h, nb, nb); if (rc) return rc;
   CK(cudaEventRecord(h->ev0, h->stream));
-  if (eager) {
-    for (int t = 0; t < nb; ++t) { enqueue_disc_step(h, 0, h->nf, t, 0); enqueue_gen_step(h, 0, h->nf, t, 0); }
-    if (h->cfg.eval_each_epoch) enqueue_eval(h, 0, h->nf, false, 0);
-    k_epoch_reduce<<<h->nf, 32, 0, h->stream>>>(h->d_step_stats, h->d_eval, h->d_epoch_stats, h->nf, nb, h->cfg.eval_each_epoch);
-    h->launches++;
-    CK(cudaMemcpyAsync(h->h_epoch_stats, h->d_epoch_stats, (size_t)h->nf * 8 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  } else {
-    CK(cudaGraphLaunch(h->graphs[nb], h->stream));
-    h->launches += h->graph_nodes[nb];
-  }
+  CK(cudaGraphLaunch(h->graphs[nb], h->stream));
+  h->launches += h->graph_nodes[nb];
   CK(cudaEventRecord(h->ev1, h->stream));
   h->epoch_pending = true;
   { const int sk = take_sticky(h); if (sk) return sk; }
@@ -2114,7 +2008,7 @@ int mrnn_train_epoch(mrgan_handle* h, const int32_t* idx, int n_idx, float* loss
   CK(cudaSetDevice(h->cfg.device));
   int rc = finish_pending(h); if (rc) return rc;
   const int nb = n_idx / h->cfg.batch;
-  rc = build_graph(h, nb, nb, n_idx); if (rc) return rc;
+  rc = build_graph(h, nb, nb); if (rc) return rc;
   const int32_t* streams[1] = {idx};
   rc = upload_indices(h, streams, 1, n_idx); if (rc) return rc;
   CK(cudaEventRecord(h->ev0, h->stream));
@@ -2211,8 +2105,8 @@ int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
   if (which == MRGAN_TIME_SALIENCY) { rc = saliency_setup(h); if (rc) return rc; }
   auto once = [&]() {
     switch (which) {
-      case MRGAN_TIME_ADAM_D: launch_adam(h, 0, h->nf, 0, false); break;
-      case MRGAN_TIME_ADAM_G: launch_adam(h, 0, h->nf, 1, false); break;
+      case MRGAN_TIME_ADAM_D: launch_adam(h, 0, h->nf, 0); break;
+      case MRGAN_TIME_ADAM_G: launch_adam(h, 0, h->nf, 1); break;
       case MRGAN_TIME_DW1: launch_gemm(h, OP_DW1, 0, h->nf, 0); break;
       case MRGAN_TIME_FWD1: launch_gemm(h, OP_D1, 0, h->nf, 0); break;
       case MRGAN_TIME_DISC_STEP: if (gan) enqueue_disc_step(h, 0, h->nf, 0, 0); else enqueue_nn_step(h, 0, h->nf, 0, 0, h->cfg.batch); break;
@@ -2262,13 +2156,11 @@ int mrgan_dp_init(mrgan_handle* h, int rank, int world, const void* id128) {
   rc = alloc_split_bufs(h); if (rc) return rc;
   h->dp_world = world; h->dp_rank = rank;
   h->hp.dp_bloc = h->cfg.batch; h->hp.dp_bg = h->cfg.batch * world; h->hp.dp_rank = rank;
-#ifdef MRGAN_WITH_TC
   if (h->cfg.precision != MRGAN_PREC_FP32) {   // gradients must be all-reduced before Adam: dW stores them, k_adam applies
     tc_teardown(h);
     h->tc_fused_adam = false;
     rc = tc_setup(h); if (rc) return rc;
   }
-#endif
   for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
   h->graphs.clear(); h->graph_nodes.clear();
   CK(cudaDeviceSynchronize());
@@ -2309,7 +2201,7 @@ int mrgan_dp_ipc_open(mrgan_handle* h, const void* handles, int world) {
       h->peer_harena[p] = static_cast<__half*>(ptr);
     }
   }
-  h->dp_fused = !(getenv("MRGAN_DP_FUSED") && atoi(getenv("MRGAN_DP_FUSED")) == 0);
+  h->dp_fused = true;
   dp_build_peers(h);
   for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
   h->graphs.clear(); h->graph_nodes.clear();
@@ -2331,15 +2223,13 @@ int mrgan_dp_init_virtual(mrgan_handle* h, int world) {
   if (world > DP_MAX_RANKS) return fail(h, MRGAN_ERR_ARG, "dp_init_virtual: at most 8 ranks");
   h->dp_world = world; h->dp_rank = 0; h->dp_virtual = true;
   h->hp.dp_bloc = h->cfg.batch; h->hp.dp_bg = h->cfg.batch * world; h->hp.dp_rank = -1;     // -1: rank = fold index (common.cuh)
-  h->dp_fused = !(getenv("MRGAN_DP_FUSED") && atoi(getenv("MRGAN_DP_FUSED")) == 0);
+  h->dp_fused = true;
   dp_build_peers(h);
-#ifdef MRGAN_WITH_TC
   if (h->cfg.precision != MRGAN_PREC_FP32) {   // gradients must be all-reduced before Adam: dW stores them, k_adam applies
     tc_teardown(h);
     h->tc_fused_adam = false;
     rc = tc_setup(h); if (rc) return rc;
   }
-#endif
   for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
   h->graphs.clear(); h->graph_nodes.clear();
   CK(cudaDeviceSynchronize());
@@ -2357,13 +2247,11 @@ int mrgan_debug_buffer(mrgan_handle* h, int fold, int which, float* dst, int row
   const float* src = nullptr; int ld = 0;
   if (h->cfg.model == MRGAN_MODEL_SVM) {
     if (which != 50 && which != 51 && which != 60 && which != 61) return fail(h, MRGAN_ERR_STATE, "debug_buffer: an SVM handle has fold data and kernel matrices only");
-#ifdef MRGAN_WITH_TC
     if (which >= 60) {
       if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "debug_buffer: kernel matrices before mrgan_svm_fit");
       if (rows > (which == 60 ? h->svm.n_lab : h->shapes[fold].n_test)) return fail(h, MRGAN_ERR_ARG, "debug_buffer: too many rows");
       src = which == 60 ? h->svm.Klab[fold] : h->svm.Kte[fold]; ld = h->svm.n_lab;
     }
-#endif
   }
   if (which >= 0 && which <= 5) { src = b.a[which]; ld = b.lda[which]; }
   else if (which >= 11 && which <= 15) { src = b.hb[which - 10]; ld = b.lda[which - 10]; }
@@ -2424,8 +2312,6 @@ int mrgan_debug_gemm(mrgan_handle* h, int mode, int M, int N, int K, const float
   CK(cudaMemcpy2DAsync(dB, (size_t)ldb * 4, B, (size_t)bc * 4, (size_t)bc * 4, br, cudaMemcpyHostToDevice, h->stream));
   GemmDesc g = make_desc(dA, lda, dB, ldb, dC, ldc, M, N, K, mode == 0 ? EPI_FWD : (mode == 1 ? EPI_DX : EPI_STORE), ACT_NONE, 0);
   CK(cudaMemcpyAsync(dd, &g, sizeof(g), cudaMemcpyHostToDevice, h->stream));
-  bool done = false;
-#ifdef MRGAN_WITH_TC
   __half *hA = nullptr, *hB = nullptr;
   if (use_tc == 2) {          // fp16 operand copies (kind::f16): host conversion, pitch rounded to 8 elements (16-byte TMA strides)
     const int lha = (ac + 7) & ~7, lhb = (bc + 7) & ~7;
@@ -2440,15 +2326,10 @@ int mrgan_debug_gemm(mrgan_handle* h, int mode, int M, int N, int K, const float
     rc = tc_debug_gemm(h, mode, gh, 2);
     cudaFree(hA); cudaFree(hB);
     if (rc) return rc;
-    done = true;
   } else if (use_tc) {
     rc = tc_debug_gemm(h, mode, g, 4);
     if (rc) return rc;
-    done = true;
-  }
-#endif
-  if (use_tc && !done) return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-  if (!done) {
+  } else {
     dim3 grid((N + 63) / 64, (M + 63) / 64, 1);
     if (mode == 0) k_gemm_simt<false, false><<<grid, 256, 0, h->stream>>>(dd, h->d_folds, 0, h->hp);
     else if (mode == 1) k_gemm_simt<false, true><<<grid, 256, 0, h->stream>>>(dd, h->d_folds, 0, h->hp);
@@ -2467,9 +2348,6 @@ int mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int gr
   if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
   { const int rc0 = need_nets(h, "debug_gemm_time"); if (rc0) return rc0; }
   if (mode < 0 || mode > 2 || M < 1 || N < 1 || K < 1 || groups < 1 || reps < 1 || !ms) return fail(h, MRGAN_ERR_ARG, "debug_gemm_time: bad argument");
-#ifndef MRGAN_WITH_TC
-  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
   CK(cudaSetDevice(h->cfg.device));
   int rc = finish_pending(h); if (rc) return rc;
   const int ar = mode == 2 ? K : M, ac = mode == 2 ? M : K;
@@ -2512,12 +2390,10 @@ int mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int gr
   h->launches += reps + 1;
   cudaFree(buf); cudaFree(dops);
   return MRGAN_OK;
-#endif
 }
 
 
 // ------------------------------------------------------------------ RBF C-SVC (MRGAN_MODEL_SVM, csrc/kernels_svm.cuh)
-#ifdef MRGAN_WITH_TC
 static void svm_launch(mrgan_handle* h, int phase) {
   mrgan_handle::Svm& S = h->svm;
   const int nf = h->nf;
@@ -2536,14 +2412,10 @@ static void svm_launch(mrgan_handle* h, int phase) {
     h->launches += 2;
   }
 }
-#endif
 
 int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, const float* gamma, float tol, int32_t* n_iter) {
   if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
   if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_fit needs an SVM handle");
-#ifndef MRGAN_WITH_TC
-  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
   if (!lab_rows || !gamma || n_lab < 2 || !(C > 0.0f) || !(tol > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_fit: bad argument");
   const int nf = h->nf, K = h->cfg.n_classes, npairs = K * (K - 1) / 2;
   for (int f = 0; f < nf; ++f)
@@ -2687,16 +2559,12 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
     if (cap[q]) return fail(h, MRGAN_ERR_STATE, "svm_fit: fold " + std::to_string(q / npairs) + ", class pair " + std::to_string(q % npairs) +
                                                     " hit the iteration cap max(1e7, 100 n)");
   return MRGAN_OK;
-#endif
 }
 
 int mrgan_svm_eval(mrgan_handle* h, int fold, float* err) {
   int rc = check_fold(h, fold); if (rc) return rc;
   if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_eval needs an SVM handle");
   if (!err) return fail(h, MRGAN_ERR_ARG, "svm_eval: null pointer");
-#ifndef MRGAN_WITH_TC
-  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
   if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "svm_eval before mrgan_svm_fit");
   CK(cudaSetDevice(h->cfg.device));
   int c = 0;
@@ -2704,28 +2572,20 @@ int mrgan_svm_eval(mrgan_handle* h, int fold, float* err) {
   CK(cudaStreamSynchronize(h->stream));
   *err = (float)c / (float)h->shapes[fold].n_test;     // np.mean(predicted != y_test)
   return MRGAN_OK;
-#endif
 }
 
 int mrgan_svm_decision(mrgan_handle* h, int fold, float* dst) {
   int rc = check_fold(h, fold); if (rc) return rc;
   if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_decision needs an SVM handle");
   if (!dst) return fail(h, MRGAN_ERR_ARG, "svm_decision: null pointer");
-#ifndef MRGAN_WITH_TC
-  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
   if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "svm_decision before mrgan_svm_fit");
   CK(cudaSetDevice(h->cfg.device));
   CK(cudaMemcpyAsync(dst, h->svm.dec[fold], sizeof(float) * h->shapes[fold].n_test * h->svm.npairs, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   return MRGAN_OK;
-#endif
 }
 
 static int svm_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
-#ifndef MRGAN_WITH_TC
-  return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
   if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "time_op: SVM phases before mrgan_svm_fit");
   CK(cudaSetDevice(h->cfg.device));
   svm_launch(h, which);                     // warm-up
@@ -2738,7 +2598,6 @@ static int svm_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
   CK(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
   *ms_avg = ms / reps;
   return MRGAN_OK;
-#endif
 }
 
 // ------------------------------------------------------------------ predictions and confusion counts
@@ -2749,14 +2608,10 @@ int mrgan_predict(mrgan_handle* h, int fold, int32_t* pred, float* scores) {
   const int n = h->shapes[fold].n_test, K = h->cfg.n_classes;
   const FoldBuffers& b = h->fb[fold];
   if (h->cfg.model == MRGAN_MODEL_SVM) {
-#ifndef MRGAN_WITH_TC
-    return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
     if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "predict before mrgan_svm_fit");
     CK(cudaSetDevice(h->cfg.device));
     CK(cudaMemcpyAsync(pred, b.pred, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));     // voted by mrgan_svm_fit
     if (scores) CK(cudaMemcpyAsync(scores, h->svm.dec[fold], (size_t)n * h->svm.npairs * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-#endif
   } else {
     if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "predict before mrgan_load_fold");
     CK(cudaSetDevice(h->cfg.device));
@@ -2781,9 +2636,6 @@ int mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t
   const size_t w = (size_t)D * sizeof(float);
   FoldBuffers& b = h->fb[fold];
   if (h->cfg.model == MRGAN_MODEL_SVM) {
-#ifndef MRGAN_WITH_TC
-    return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
     mrgan_handle::Svm& S = h->svm;
     if (!S.fitted) return fail(h, MRGAN_ERR_STATE, "predict_rows before mrgan_svm_fit");
     CK(cudaSetDevice(h->cfg.device));
@@ -2807,7 +2659,6 @@ int mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t
     h->launches += 3;
     CK(cudaMemcpyAsync(pred, S.preds, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (scores) CK(cudaMemcpyAsync(scores, S.decs, (size_t)n * S.npairs * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-#endif
   } else {
     if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "predict_rows before mrgan_load_fold");
     CK(cudaSetDevice(h->cfg.device));
@@ -2838,11 +2689,7 @@ int mrgan_confusion(mrgan_handle* h, int32_t* out) {
   int rc = need_local(h, "confusion"); if (rc) return rc;
   const int K = h->cfg.n_classes;
   if (h->cfg.model == MRGAN_MODEL_SVM) {
-#ifndef MRGAN_WITH_TC
-    return fail(h, MRGAN_ERR_ARG, "library built without the tcgen05 kernels");
-#else
     if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "confusion before mrgan_svm_fit");
-#endif
   } else {
     for (int f = 0; f < h->nf; ++f)
       if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "confusion before mrgan_load_fold");

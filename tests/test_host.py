@@ -218,6 +218,23 @@ def test_scheduler_mirrors_the_library_chain_rule(monkeypatch):
     assert sweep.chain_count(74) == kmax
 
 
+def test_library_has_one_code_path_per_decision():
+    """The library is built one way and measured one way: no build-time variant, no environment switch that selects an
+    alternative kernel path, no programmatic-dependent-launch hooks, no opt-in BatchNorm-backward head.  The two variables
+    it does read are a scheduling parameter (MRGAN_CHAINS) and a numeric one (MRGAN_LOSS_SCALE)."""
+    csrc = os.path.join(ROOT, "mr_gan_b200", "csrc")
+    names = sorted(os.listdir(csrc))
+    assert "mrgan_api.cu" in names and "kernels_tc.cuh" in names
+    for fn in names:
+        src = open(os.path.join(csrc, fn)).read()
+        for word in ("MRGAN_WITH_TC", "griddepcontrol", "HEAD_BN_BWD"):
+            assert word not in src, (fn, word)
+        calls = re.findall(r"\bgetenv\s*\(", src)
+        read = re.findall(r"\bgetenv\s*\(\s*\"(\w+)\"\s*\)", src)
+        assert len(read) == len(calls), (fn, "getenv of a non-literal name")
+        assert set(read) <= {"MRGAN_CHAINS", "MRGAN_LOSS_SCALE"}, (fn, read)
+
+
 def test_logmel_front_end_against_scipy_stft_and_slaney_landmarks():
     """librosa is absent, so the restated front end (mr_gan.py:45-47) is pinned piecewise: the framing / window / FFT against
     scipy.signal.stft (an independent implementation; centred frames = reflect padding, periodic Hann, hop 512), the mel
