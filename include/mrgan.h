@@ -188,6 +188,21 @@ int  mrnn_evaluate(mrgan_handle* h, int fold, float out[2]);
  *   tol: libsvm eps.  A class pair has at most 8192 rows.
  *   n_iter [n_folds][K(K-1)/2] or NULL; returns MRGAN_ERR_STATE if a pair hit the iteration cap max(1e7, 100 n). */
 int  mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, const float* gamma, float tol, int32_t* n_iter);
+/* mrgan_svm_fit with its own C per fold: C [n_folds] (mrgan_svm_fit is this call with C broadcast). */
+int  mrgan_svm_fit_folds(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const float* C, const float* gamma, float tol,
+                         int32_t* n_iter);
+/* The inner cross-validation of GridSearchCV(SVC(kernel='rbf', tol), {'C': C, 'gamma': gamma}, cv) for every fold: one SVC fit
+ * per (fold, gamma, C, split) on the split's inner-training rows (labeled rows with split index != s, in the labeled order),
+ * voted on its validation rows (split index == s).  Same labeled rows and checks as mrgan_svm_fit; also
+ *   split [n_folds][n_lab] in [0, n_splits), n_splits >= 2, every split with a validation row and every class among its
+ *   inner-training rows; C [nC] > 0; gamma [n_folds][nG] > 0 (absolute); otherwise MRGAN_ERR_ARG.
+ *   wrong [n_folds][nG][nC][n_splits]: misclassified validation rows (integers, bitwise reproducible).
+ * One gamma column at a time in the fit's labeled x labeled buffers.  MRGAN_ERR_STATE if a problem hits the iteration cap (the
+ * message names fold, gamma, C, split and class pair).  A call that passes the argument checks invalidates a previous fit:
+ * mrgan_svm_eval, mrgan_svm_decision, mrgan_predict*, mrgan_confusion and the SVM phases of mrgan_time_op return
+ * MRGAN_ERR_STATE until the next mrgan_svm_fit*.  A call rejected with MRGAN_ERR_ARG leaves the previous fit valid. */
+int  mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int32_t* split, int n_splits, const float* C, int nC,
+                  const float* gamma, int nG, float tol, int32_t* wrong);
 int  mrgan_svm_eval(mrgan_handle* h, int fold, float* err);                 /* full resident X_test, ovo vote */
 int  mrgan_svm_decision(mrgan_handle* h, int fold, float* dst);             /* test hook: [n_test][K(K-1)/2] */
 

@@ -68,6 +68,8 @@ SYMBOLS = {
     "mrnn_train_epoch": (C.c_int, [_H, _ip, C.c_int, _fp]),
     "mrnn_evaluate": (C.c_int, [_H, C.c_int, _fp]),
     "mrgan_svm_fit": (C.c_int, [_H, _ip, C.c_int, C.c_float, _fp, C.c_float, _ip]),
+    "mrgan_svm_fit_folds": (C.c_int, [_H, _ip, C.c_int, _fp, _fp, C.c_float, _ip]),
+    "mrgan_svm_cv": (C.c_int, [_H, _ip, C.c_int, _ip, C.c_int, _fp, C.c_int, _fp, C.c_int, C.c_float, _ip]),
     "mrgan_svm_eval": (C.c_int, [_H, C.c_int, _fp]),
     "mrgan_svm_decision": (C.c_int, [_H, C.c_int, _fp]),
     "mrgan_predict": (C.c_int, [_H, C.c_int, _ip, _fp]),

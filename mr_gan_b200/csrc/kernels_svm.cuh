@@ -3,8 +3,9 @@
 // Specification: the libsvm source shipped with sklearn, sklearn/svm/src/libsvm/svm.cpp (cited as svm.cpp:<line>).
 //   k_svm_split  tf32 hi / lo parts of every labeled and test row, and their row norms
 //   k_svm_kmat   kernel matrices on tcgen05 (labeled x labeled, test x labeled), RBF transform in the epilogue
-//   k_svm_smo    Solver::Solve without shrinking, one CTA per (fold, class pair), alpha / G in double in shared memory
-//   k_svm_vote   svm_predict_values' one-vs-one decision values and vote; k_svm_count the fold's error count
+//   k_svm_smo    Solver::Solve without shrinking, one CTA per problem (fold, class pair; for mrgan_svm_cv also C and inner
+//                split), alpha / G in double in shared memory
+//   k_svm_vote   svm_predict_values' one-vs-one decision values and vote; k_svm_count the error count of a row set
 #pragma once
 #include "kernels_tc.cuh"
 
@@ -168,20 +169,26 @@ __global__ void __launch_bounds__(SVM_KMAT_THREADS, 1) k_svm_kmat(const SvmGemmO
 
 // ---------------------------------------------------------------- batched SMO
 #define SVM_SMO_THREADS 512
-#define SVM_MAX_PAIR 8192                              // rows of one class pair: 20 bytes each in shared memory
+#define SVM_MAX_PAIR 8192                              // rows of one class pair: 24 bytes each in shared memory
+#define SVM_SMO_SMEM_PER_ROW 24                        // alpha, G (double), QD (float), row map (int)
 #define SVM_PER (SVM_MAX_PAIR / SVM_SMO_THREADS)
 #define SVM_TAU 1e-12                                  // svm.cpp:105
 
 struct SvmPairJob {
   const float* K; int ld;           // the fold's labeled x labeled matrix
-  int a_off, na, b_off, nb;         // rows of class a (y = +1) and b (y = -1) in the labeled set
+  int a_off, na, b_off, nb;         // rows of class a (y = +1) and b (y = -1) in the labeled set (a_off / b_off: no row map)
+  const int* rows;                  // [na + nb] row map into the labeled set (the class-a rows, then the class-b rows), or
+                                    // nullptr: the contiguous segments a_off.. and b_off.. (mrgan_svm_fit)
+  double C;                         // box constraint of this problem
   int ca, cb;                       // the two classes
   double* coef;                     // [na + nb]: alpha_k y_k (sv_coef)
   double* rho;
   int* n_iter; int* capped;
 };
 
-__device__ __forceinline__ int svm_row(const SvmPairJob& jb, int k) { return k < jb.na ? jb.a_off + k : jb.b_off + (k - jb.na); }
+__device__ __forceinline__ int svm_row(const SvmPairJob& jb, int k) {
+  return jb.rows ? jb.rows[k] : k < jb.na ? jb.a_off + k : jb.b_off + (k - jb.na);
+}
 
 // (value, index) arg-max with libsvm's scan order: on equal values the larger index wins (svm.cpp:964,973 use >=)
 __device__ __forceinline__ void svm_max_last(double& v, int& i, double v2, int i2) {
@@ -196,13 +203,16 @@ __device__ __forceinline__ void svm_min_last(double& v, int& i, double v2, int i
 // (value, index) with a total order, so the result does not depend on the reduction tree: bitwise reproducible.
 // Double arithmetic is written with _rn intrinsics so that no product is contracted into an FMA (libsvm's host build
 // rounds every product).
-__global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* __restrict__ jobs, double C, double eps) {
+// The row map is read once into shared memory, so the scans below load only K from global memory.
+__global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* __restrict__ jobs, double eps) {
   const SvmPairJob jb = jobs[blockIdx.x];
   const int n = jb.na + jb.nb;
+  const double C = jb.C;
   extern __shared__ double svm_smem[];
   double* alpha = svm_smem;                            // [n]
   double* G = alpha + n;                               // [n]
   float* QD = reinterpret_cast<float*>(G + n);         // [n]: K(k, k)
+  int* row = reinterpret_cast<int*>(QD + n);           // [n]: row of problem row k in the labeled set
   __shared__ double r1v[SVM_SMO_THREADS / 32], r2v[SVM_SMO_THREADS / 32], r2m[SVM_SMO_THREADS / 32];
   __shared__ int r1i[SVM_SMO_THREADS / 32], r2i[SVM_SMO_THREADS / 32];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -210,6 +220,7 @@ __global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* _
   for (int k = tid; k < n; k += SVM_SMO_THREADS) {
     alpha[k] = 0.0; G[k] = -1.0;                       // alpha = 0, G = p = -1 (svm.cpp:703)
     const int r = svm_row(jb, k);
+    row[k] = r;
     QD[k] = jb.K[(size_t)r * jb.ld + r];
   }
   __syncthreads();
@@ -237,13 +248,13 @@ __global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* _
     // ---- j: second-order rule over I_low (svm.cpp:985-1035)
     double g2 = -INFINITY, om = INFINITY; int oj = -1;
     const double yi = i < jb.na ? 1.0 : -1.0;
-    const float* Ki = jb.K + (size_t)svm_row(jb, i >= 0 ? i : 0) * jb.ld;
+    const float* Ki = jb.K + (size_t)row[i >= 0 ? i : 0] * jb.ld;
     const double QDi = i >= 0 ? (double)QD[i] : 0.0;
 #pragma unroll
     for (int s = 0; s < SVM_PER; ++s) {
       const int k = tid + s * SVM_SMO_THREADS;
       if (k >= n) break;
-      qi[s] = i >= 0 ? Ki[svm_row(jb, k)] : 0.0f;
+      qi[s] = i >= 0 ? Ki[row[k]] : 0.0f;
       const double a = alpha[k], yk = k < jb.na ? 1.0 : -1.0;
       if (yk > 0 ? a > 0.0 : a < C) {
         const double yG = yk * G[k];
@@ -269,7 +280,7 @@ __global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* _
     ++iter;
     // ---- two-variable update with box clipping (svm.cpp:761-855); every thread computes it, identically
     const double yj = j < jb.na ? 1.0 : -1.0;
-    const double Kij = (double)Ki[svm_row(jb, j)], QDj = (double)QD[j];
+    const double Kij = (double)Ki[row[j]], QDj = (double)QD[j];
     const double ai = alpha[i], aj = alpha[j], Gi = G[i], Gj = G[j];
     double ni, nj;
     if (yi != yj) {
@@ -294,7 +305,7 @@ __global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* _
       else { if (ni < 0) { ni = 0; nj = sum; } }
     }
     const double dai = __dsub_rn(ni, ai), daj = __dsub_rn(nj, aj);
-    const float* Kj = jb.K + (size_t)svm_row(jb, j) * jb.ld;
+    const float* Kj = jb.K + (size_t)row[j] * jb.ld;
     __syncthreads();                                   // everybody has read alpha / G of i and j
     if (tid == 0) { alpha[i] = ni; alpha[j] = nj; }
 #pragma unroll
@@ -302,7 +313,7 @@ __global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* _
       const int k = tid + s * SVM_SMO_THREADS;
       if (k >= n) break;
       const double yk = k < jb.na ? 1.0 : -1.0;
-      const double Qik = yi * yk * (double)qi[s], Qjk = yj * yk * (double)Kj[svm_row(jb, k)];
+      const double Qik = yi * yk * (double)qi[s], Qjk = yj * yk * (double)Kj[row[k]];
       G[k] = __dadd_rn(G[k], __dadd_rn(__dmul_rn(Qik, dai), __dmul_rn(Qjk, daj)));
     }
     __syncthreads();                                   // alpha[i], alpha[j] visible to the owners' next scan
@@ -326,17 +337,20 @@ __global__ void __launch_bounds__(SVM_SMO_THREADS) k_svm_smo(const SvmPairJob* _
 
 // ---------------------------------------------------------------- decision values and vote (svm.cpp:2865-2897)
 #define SVM_VOTE_THREADS 256
-// one CTA per (test row, fold): jobs of the fold are jobs[fold * npairs ...]; Kt = the fold's test x labeled matrix.
-// wrong (with yte) and pred may be null: rows without labels (mrgan_predict_rows) store only the voted class.
+// one CTA per (row t, row set f): the models of set f are jobs[f * npairs ...]; Kt[f] = its rows x labeled kernel matrix,
+// whose row t is the voted row, or row trow[f][t] when trow is given (the validation rows of mrgan_svm_cv's inner splits,
+// rows of the labeled x labeled matrix).  dec_out, wrong (with yte) and pred may be null: rows without labels
+// (mrgan_predict_rows) store only the voted class, the validation rows only their wrong flags.
 __global__ void __launch_bounds__(SVM_VOTE_THREADS) k_svm_vote(const SvmPairJob* __restrict__ jobs, int npairs, int n_classes,
-                                                               const float* const* __restrict__ Kt, const int* const* __restrict__ yte,
-                                                               const int* __restrict__ n_test, float* const* __restrict__ dec_out,
-                                                               int* const* __restrict__ wrong, int* const* __restrict__ pred) {
+                                                               const float* const* __restrict__ Kt, const int* const* __restrict__ trow,
+                                                               const int* const* __restrict__ yte, const int* __restrict__ n_test,
+                                                               float* const* __restrict__ dec_out, int* const* __restrict__ wrong,
+                                                               int* const* __restrict__ pred) {
   const int f = blockIdx.y, t = blockIdx.x;
   if (t >= n_test[f]) return;
   const SvmPairJob* jf = jobs + (size_t)f * npairs;
   const int ld = jf[0].ld;
-  const float* row = Kt[f] + (size_t)t * ld;
+  const float* row = Kt[f] + (size_t)(trow ? trow[f][t] : t) * ld;
   __shared__ float dec_s[2048];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int p = warp; p < npairs; p += SVM_VOTE_THREADS / 32) {
@@ -348,7 +362,7 @@ __global__ void __launch_bounds__(SVM_VOTE_THREADS) k_svm_vote(const SvmPairJob*
     for (int o = 16; o > 0; o >>= 1) s = __dadd_rn(s, __shfl_xor_sync(0xffffffffu, s, o));
     if (lane == 0) {
       const double d = s - *jb.rho;
-      dec_out[f][(size_t)t * npairs + p] = (float)d;
+      if (dec_out) dec_out[f][(size_t)t * npairs + p] = (float)d;
       dec_s[p] = d > 0 ? 1.0f : 0.0f;                  // the vote only needs the sign
     }
   }
@@ -364,7 +378,7 @@ __global__ void __launch_bounds__(SVM_VOTE_THREADS) k_svm_vote(const SvmPairJob*
   }
 }
 
-// error count of each fold (blockIdx.x), summed in a fixed order
+// error count of each row set (blockIdx.x: a fold's test rows, or a validation split), summed in a fixed order
 __global__ void __launch_bounds__(256) k_svm_count(int* const* __restrict__ wrong, const int* __restrict__ n_test, int* __restrict__ count) {
   const int f = blockIdx.x, n = n_test[f];
   __shared__ int part[256];

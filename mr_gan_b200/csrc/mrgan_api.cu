@@ -162,7 +162,7 @@ struct mrgan_handle {
   struct Svm {
     char* mem = nullptr; size_t bytes = 0;
     int n_lab = 0, npairs = 0, npmax = 0, max_rows = 0, max_nte = 0;
-    double C = 1.0, eps = 1e-3;
+    double eps = 1e-3;
     bool fitted = false;
     std::vector<float*> Klab, Kte, dec;
     std::vector<int*> wrong;
@@ -174,6 +174,8 @@ struct mrgan_handle {
     float *Xs = nullptr, *Hs = nullptr, *Ls = nullptr, *Ks = nullptr, *decs = nullptr; double* ns = nullptr; int* preds = nullptr;
     SvmSplitOp* d_split_s = nullptr; SvmGemmOp* d_gemm_s = nullptr;
     float** d_Ks = nullptr; float** d_decs = nullptr; int** d_preds = nullptr; int* d_ns = nullptr;   // one-fold pointer tables
+    // mrgan_svm_cv: problems, row maps, validation rows and counts of every (fold, C, inner split), beside the fit's workspace
+    char* cv_mem = nullptr; size_t cv_bytes = 0;
   } svm;
 };
 
@@ -1611,6 +1613,7 @@ int mrgan_destroy(mrgan_handle* h) {
   if (h->sal.mem) cudaFree(h->sal.mem);
   tc_teardown(h);
   if (h->svm.mem) cudaFree(h->svm.mem);
+  if (h->svm.cv_mem) cudaFree(h->svm.cv_mem);
   if (h->arena) cudaFree(h->arena);
   if (h->harena) cudaFree(h->harena);
   if (h->h_epoch_stats) cudaFreeHost(h->h_epoch_stats);
@@ -2403,52 +2406,73 @@ static void svm_launch(mrgan_handle* h, int phase) {
                  h->stream>>>(S.d_gemm);
     h->launches += 2;
   } else if (phase == MRGAN_TIME_SVM_SMO) {
-    k_svm_smo<<<nf * S.npairs, SVM_SMO_THREADS, (size_t)20 * S.npmax, h->stream>>>(S.d_jobs, S.C, S.eps);
+    k_svm_smo<<<nf * S.npairs, SVM_SMO_THREADS, (size_t)SVM_SMO_SMEM_PER_ROW * S.npmax, h->stream>>>(S.d_jobs, S.eps);
     h->launches += 1;
   } else {
-    k_svm_vote<<<dim3(S.max_nte, nf), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs, S.npairs, h->cfg.n_classes, S.d_Kt, S.d_yte, S.d_nte,
-                                                                         S.d_dec, S.d_wrong, S.d_pred);
+    k_svm_vote<<<dim3(S.max_nte, nf), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs, S.npairs, h->cfg.n_classes, S.d_Kt, nullptr, S.d_yte,
+                                                                         S.d_nte, S.d_dec, S.d_wrong, S.d_pred);
     k_svm_count<<<nf, 256, 0, h->stream>>>(S.d_wrong, S.d_nte, S.d_count);
     h->launches += 2;
   }
 }
 
-int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, const float* gamma, float tol, int32_t* n_iter) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_fit needs an SVM handle");
-  if (!lab_rows || !gamma || n_lab < 2 || !(C > 0.0f) || !(tol > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_fit: bad argument");
-  const int nf = h->nf, K = h->cfg.n_classes, npairs = K * (K - 1) / 2;
+// The labeled rows of every fold: class c is the segment [start[f][c], start[f][c] + cnt[f][c]); ylab [nf][n_lab] their labels
+struct SvmLabels {
+  std::vector<int> ylab, start, cnt;
+  int npmax = 0;                      // rows of the largest class pair
+};
+
+// Checks the labeled rows of every fold (loaded, in range, class-major, every class present, class pairs within SVM_MAX_PAIR)
+// and reads their labels.  Changes no SVM state.  The caller has checked the scalars.
+static int svm_labels(mrgan_handle* h, const char* fn, const int32_t* lab_rows, int n_lab, SvmLabels& L) {
+  const std::string pre = std::string(fn) + ": ";
+  const int nf = h->nf, K = h->cfg.n_classes;
   for (int f = 0; f < nf; ++f)
-    if (!(gamma[f] > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_fit: gamma must be positive");
-  for (int f = 0; f < nf; ++f)
-    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "svm_fit before the fold data is loaded (mrgan_load_fold / mrgan_prepare_fold)");
+    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, pre + "the fold data is not loaded (mrgan_load_fold / mrgan_prepare_fold)");
   CK(cudaSetDevice(h->cfg.device));
   int rc = finish_pending(h); if (rc) return rc;
-  // class-major labeled rows: class c is the segment [start[f][c], start[f][c] + cnt[f][c])
-  std::vector<int> ytr(h->n_train), start((size_t)nf * K), cnt((size_t)nf * K, 0);
-  int npmax = 0;
+  std::vector<int> ytr(h->n_train);
+  std::vector<int>& ylab = L.ylab;
+  std::vector<int>& start = L.start;
+  std::vector<int>& cnt = L.cnt;
+  ylab.assign((size_t)nf * n_lab, 0);
+  start.assign((size_t)nf * K, 0);
+  cnt.assign((size_t)nf * K, 0);
+  int& npmax = L.npmax;
+  npmax = 0;
   for (int f = 0; f < nf; ++f) {
     CK(cudaMemcpy(ytr.data(), h->fb[f].ytr, (size_t)h->n_train * sizeof(int), cudaMemcpyDeviceToHost));
     const int32_t* lr = lab_rows + (size_t)f * n_lab;
     int prev = -1;
     for (int r = 0; r < n_lab; ++r) {
-      if (lr[r] < 0 || lr[r] >= h->n_train) return fail(h, MRGAN_ERR_ARG, "svm_fit: labeled row out of range");
+      if (lr[r] < 0 || lr[r] >= h->n_train) return fail(h, MRGAN_ERR_ARG, pre + "labeled row out of range");
       const int c = ytr[lr[r]];
-      if (c < prev) return fail(h, MRGAN_ERR_ARG, "svm_fit: labeled rows must be class-major (labels non-decreasing)");
+      if (c < prev) return fail(h, MRGAN_ERR_ARG, pre + "labeled rows must be class-major (labels non-decreasing)");
       if (c != prev) start[(size_t)f * K + c] = r;
       cnt[(size_t)f * K + c]++;
+      ylab[(size_t)f * n_lab + r] = c;
       prev = c;
     }
     for (int c = 0; c < K; ++c)
-      if (cnt[(size_t)f * K + c] == 0) return fail(h, MRGAN_ERR_ARG, "svm_fit: every class needs a labeled row");
+      if (cnt[(size_t)f * K + c] == 0) return fail(h, MRGAN_ERR_ARG, pre + "every class needs a labeled row");
     for (int a = 0; a < K; ++a)
       for (int b = a + 1; b < K; ++b) {
         const int np = cnt[(size_t)f * K + a] + cnt[(size_t)f * K + b];
-        if (np > SVM_MAX_PAIR) return fail(h, MRGAN_ERR_ARG, "svm_fit: a class pair has more than 8192 labeled rows (shared-memory limit of the solver)");
+        if (np > SVM_MAX_PAIR) return fail(h, MRGAN_ERR_ARG, pre + "a class pair has more than 8192 labeled rows (shared-memory limit of the solver)");
         npmax = std::max(npmax, np);
       }
   }
-  // workspace
+  return MRGAN_OK;
+}
+
+// Lays out the fit's workspace for checked labeled rows and uploads its descriptors: the operand split and both kernel
+// matrices of every fold at gamma[f], and one problem per (fold, class pair) at C[f] over the fold's contiguous class
+// segments.  Launches nothing; the previous fit is invalid from here on.
+static int svm_setup(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const SvmLabels& L, const float* C, const float* gamma,
+                     float tol) {
+  const int nf = h->nf, K = h->cfg.n_classes, npairs = K * (K - 1) / 2, npmax = L.npmax;
+  const std::vector<int>& start = L.start;
+  const std::vector<int>& cnt = L.cnt;
   mrgan_handle::Svm& S = h->svm;
   int max_nte = 0, max_kp = 32;
   for (int f = 0; f < nf; ++f) { max_nte = std::max(max_nte, h->shapes[f].n_test); max_kp = std::max(max_kp, round_up(h->shapes[f].D, 32)); }
@@ -2489,11 +2513,11 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
   Arena real; real.base = S.mem;
   layout(real);
   S.n_lab = n_lab; S.npairs = npairs; S.npmax = npmax; S.max_nte = max_nte; S.max_rows = std::max(n_lab, max_nte);
-  S.C = C; S.eps = tol;
+  S.eps = tol;
   S.Klab = Klab; S.Kte = Kte; S.dec = dec; S.wrong = wrong;
   // descriptors
-  EncodeTiledFn fn = tc_encoder();
-  if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
+  EncodeTiledFn enc = tc_encoder();
+  if (!enc) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
   std::vector<SvmSplitOp> sp(2 * nf);
   std::vector<SvmGemmOp> gm(2 * nf);
   std::vector<SvmPairJob> jobs((size_t)nf * npairs);
@@ -2508,9 +2532,9 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
     for (int w = 0; w < 2; ++w) {
       SvmGemmOp& g = gm[2 * f + w];
       const int nA = w == 0 ? n_lab : nte;
-      bool ok = make_map(fn, &g.mapBh, Hl[f], Kp, n_lab, Kp, SVM_BM, false) && make_map(fn, &g.mapBl, Ll[f], Kp, n_lab, Kp, SVM_BM, false) &&
-                make_map(fn, &g.mapAh, w == 0 ? Hl[f] : Ht[f], Kp, nA, Kp, SVM_BN, false) &&
-                make_map(fn, &g.mapAl, w == 0 ? Ll[f] : Lt[f], Kp, nA, Kp, SVM_BN, false);
+      bool ok = make_map(enc, &g.mapBh, Hl[f], Kp, n_lab, Kp, SVM_BM, false) && make_map(enc, &g.mapBl, Ll[f], Kp, n_lab, Kp, SVM_BM, false) &&
+                make_map(enc, &g.mapAh, w == 0 ? Hl[f] : Ht[f], Kp, nA, Kp, SVM_BN, false) &&
+                make_map(enc, &g.mapAl, w == 0 ? Ll[f] : Lt[f], Kp, nA, Kp, SVM_BN, false);
       if (!ok) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
       g.normA = w == 0 ? nl[f] : nt[f]; g.normB = nl[f];
       g.C = w == 0 ? Klab[f] : Kte[f]; g.ldc = n_lab;
@@ -2523,6 +2547,7 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
         jb.K = Klab[f]; jb.ld = n_lab;
         jb.a_off = start[(size_t)f * K + a]; jb.na = cnt[(size_t)f * K + a];
         jb.b_off = start[(size_t)f * K + c]; jb.nb = cnt[(size_t)f * K + c];
+        jb.rows = nullptr; jb.C = C[f];
         jb.ca = a; jb.cb = c;
         jb.coef = coef[f] + (size_t)p * npmax; jb.rho = rho[f] + p;
         jb.n_iter = S.d_iters + (size_t)f * npairs + p; jb.capped = S.d_capped + (size_t)f * npairs + p;
@@ -2544,7 +2569,27 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
   CK(cudaMemcpyAsync(S.d_decs, &S.decs, sizeof(float*), cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(S.d_preds, &S.preds, sizeof(int*), cudaMemcpyHostToDevice, h->stream));
   CK(cudaFuncSetAttribute(k_svm_kmat, cudaFuncAttributeMaxDynamicSharedMemorySize, SVM_KMAT_SMEM));
-  CK(cudaFuncSetAttribute(k_svm_smo, cudaFuncAttributeMaxDynamicSharedMemorySize, 20 * SVM_MAX_PAIR));
+  CK(cudaFuncSetAttribute(k_svm_smo, cudaFuncAttributeMaxDynamicSharedMemorySize, SVM_SMO_SMEM_PER_ROW * SVM_MAX_PAIR));
+  return MRGAN_OK;
+}
+
+static bool all_positive(const float* v, size_t n) {
+  for (size_t i = 0; i < n; ++i)
+    if (!(v[i] > 0.0f)) return false;
+  return true;
+}
+
+int mrgan_svm_fit_folds(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const float* C, const float* gamma, float tol, int32_t* n_iter) {
+  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_fit needs an SVM handle");
+  if (!lab_rows || !C || !gamma || n_lab < 2 || !(tol > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_fit: bad argument");
+  const int nf = h->nf, npairs = h->cfg.n_classes * (h->cfg.n_classes - 1) / 2;
+  if (!all_positive(C, nf)) return fail(h, MRGAN_ERR_ARG, "svm_fit: C must be positive");
+  if (!all_positive(gamma, nf)) return fail(h, MRGAN_ERR_ARG, "svm_fit: gamma must be positive");
+  SvmLabels L;
+  int rc = svm_labels(h, "svm_fit", lab_rows, n_lab, L); if (rc) return rc;
+  rc = svm_setup(h, lab_rows, n_lab, L, C, gamma, tol); if (rc) return rc;
+  mrgan_handle::Svm& S = h->svm;
   svm_launch(h, MRGAN_TIME_SVM_KMAT);
   svm_launch(h, MRGAN_TIME_SVM_SMO);
   svm_launch(h, MRGAN_TIME_SVM_PREDICT);
@@ -2558,6 +2603,159 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
   for (size_t q = 0; q < cap.size(); ++q)
     if (cap[q]) return fail(h, MRGAN_ERR_STATE, "svm_fit: fold " + std::to_string(q / npairs) + ", class pair " + std::to_string(q % npairs) +
                                                     " hit the iteration cap max(1e7, 100 n)");
+  return MRGAN_OK;
+}
+
+int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, const float* gamma, float tol, int32_t* n_iter) {
+  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  std::vector<float> Cf(h->nf, C);
+  return mrgan_svm_fit_folds(h, lab_rows, n_lab, Cf.data(), gamma, tol, n_iter);
+}
+
+// Inner cross-validation (GridSearchCV's fits and scores): for every gamma column g, the labeled x labeled kernel matrices
+// of all folds are recomputed in the fit's buffers, then one SMO problem per (fold, C, split, class pair) is solved on the
+// split's inner-training rows (a row map into the labeled set) and the split's validation rows are voted from the same
+// matrix and counted.
+int mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int32_t* split, int n_splits, const float* C, int nC,
+                 const float* gamma, int nG, float tol, int32_t* wrong) {
+  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_cv needs an SVM handle");
+  if (!lab_rows || !split || !C || !gamma || !wrong || n_lab < 2 || !(tol > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_cv: bad argument");
+  if (n_splits < 2 || nC < 1 || nG < 1) return fail(h, MRGAN_ERR_ARG, "svm_cv: need n_splits >= 2, nC >= 1 and nG >= 1");
+  const int nf = h->nf, K = h->cfg.n_classes, npairs = K * (K - 1) / 2, ns = n_splits;
+  if (!all_positive(C, nC)) return fail(h, MRGAN_ERR_ARG, "svm_cv: C must be positive");
+  if (!all_positive(gamma, (size_t)nf * nG)) return fail(h, MRGAN_ERR_ARG, "svm_cv: gamma must be positive");
+  for (size_t r = 0; r < (size_t)nf * n_lab; ++r)
+    if (split[r] < 0 || split[r] >= ns) return fail(h, MRGAN_ERR_ARG, "svm_cv: split index outside [0, n_splits)");
+  std::vector<float> g0(nf), C0(nf, C[0]);
+  for (int f = 0; f < nf; ++f) g0[f] = gamma[(size_t)f * nG];
+  SvmLabels L;
+  int rc = svm_labels(h, "svm_cv", lab_rows, n_lab, L); if (rc) return rc;
+  const std::vector<int>& ylab = L.ylab;
+  // the problems: validation rows of (f, s) and the inner-training rows of (f, s, pair), in the labeled order; a rejected
+  // split leaves the previous fit valid
+  const int nQ = nf * nC * ns, nJobs = nQ * npairs;
+  std::vector<int> vrows, vy, voff((size_t)nf * ns), nval((size_t)nf * ns, 0), maps, moff((size_t)nf * ns * npairs), mna(moff.size()), mnb(moff.size());
+  int max_nval = 0, npmax = 0;
+  for (int f = 0; f < nf; ++f) {
+    const int32_t* sf = split + (size_t)f * n_lab;
+    const int* yf = ylab.data() + (size_t)f * n_lab;
+    for (int s = 0; s < ns; ++s) {
+      const size_t fs = (size_t)f * ns + s;
+      voff[fs] = (int)vrows.size();
+      std::vector<int> train_cnt(K, 0);
+      for (int r = 0; r < n_lab; ++r) {
+        if (sf[r] == s) { vrows.push_back(r); vy.push_back(yf[r]); }
+        else train_cnt[yf[r]]++;
+      }
+      nval[fs] = (int)vrows.size() - voff[fs];
+      if (nval[fs] == 0) return fail(h, MRGAN_ERR_ARG, "svm_cv: fold " + std::to_string(f) + ", split " + std::to_string(s) + " has no validation row");
+      for (int c = 0; c < K; ++c)
+        if (train_cnt[c] == 0)
+          return fail(h, MRGAN_ERR_ARG, "svm_cv: fold " + std::to_string(f) + ", split " + std::to_string(s) + ": the inner-training rows lack class " + std::to_string(c));
+      max_nval = std::max(max_nval, nval[fs]);
+      int p = 0;
+      for (int a = 0; a < K; ++a)
+        for (int b = a + 1; b < K; ++b, ++p) {
+          const size_t m = fs * npairs + p;
+          moff[m] = (int)maps.size();
+          for (int r = 0; r < n_lab; ++r) if (sf[r] != s && yf[r] == a) maps.push_back(r);
+          mna[m] = (int)maps.size() - moff[m];
+          for (int r = 0; r < n_lab; ++r) if (sf[r] != s && yf[r] == b) maps.push_back(r);
+          mnb[m] = (int)maps.size() - moff[m] - mna[m];
+          npmax = std::max(npmax, mna[m] + mnb[m]);
+        }
+    }
+  }
+  rc = svm_setup(h, lab_rows, n_lab, L, C0.data(), g0.data(), tol); if (rc) return rc;
+  mrgan_handle::Svm& S = h->svm;
+  // second allocation: kept while large enough, freed by mrgan_destroy
+  int *d_maps = nullptr, *d_vrows = nullptr, *d_vy = nullptr, *d_nval = nullptr, *d_flags = nullptr, *d_count = nullptr, *d_iters = nullptr, *d_capped = nullptr;
+  double *d_coef = nullptr, *d_rho = nullptr;
+  SvmPairJob* d_jobs = nullptr; SvmGemmOp* d_gemm = nullptr;
+  const float** d_Kq = nullptr; const int** d_trow = nullptr; const int** d_yq = nullptr; int** d_wq = nullptr;
+  auto layout = [&](Arena& ar) {
+    d_maps = ar.take<int>(maps.size()); d_vrows = ar.take<int>(vrows.size()); d_vy = ar.take<int>(vy.size());
+    d_nval = ar.take<int>(nQ); d_flags = ar.take<int>((size_t)nQ * max_nval); d_count = ar.take<int>((size_t)nG * nQ);
+    d_iters = ar.take<int>(nJobs); d_capped = ar.take<int>(nJobs);
+    d_coef = ar.take<double>((size_t)nJobs * npmax); d_rho = ar.take<double>(nJobs);
+    d_jobs = ar.take<SvmPairJob>(nJobs); d_gemm = ar.take<SvmGemmOp>((size_t)nG * nf);
+    d_Kq = ar.take<const float*>(nQ); d_trow = ar.take<const int*>(nQ); d_yq = ar.take<const int*>(nQ); d_wq = ar.take<int*>(nQ);
+  };
+  Arena sizing;
+  layout(sizing);
+  if (sizing.off + 256 > S.cv_bytes) {
+    if (S.cv_mem) { cudaFree(S.cv_mem); S.cv_mem = nullptr; S.cv_bytes = 0; }
+    CK(cudaMalloc(&S.cv_mem, sizing.off + 256));
+    S.cv_bytes = sizing.off + 256;
+  }
+  Arena real; real.base = S.cv_mem;
+  layout(real);
+  // problem q = (f * nC + c) * ns + s; its class pairs are jobs q * npairs ...
+  std::vector<SvmPairJob> jobs(nJobs);
+  std::vector<const float*> Kq(nQ); std::vector<const int*> trow(nQ), yq(nQ); std::vector<int*> wq(nQ); std::vector<int> nq(nQ);
+  for (int f = 0; f < nf; ++f)
+    for (int c = 0; c < nC; ++c)
+      for (int s = 0; s < ns; ++s) {
+        const int q = (f * nC + c) * ns + s;
+        const size_t fs = (size_t)f * ns + s;
+        Kq[q] = S.Klab[f]; trow[q] = d_vrows + voff[fs]; yq[q] = d_vy + voff[fs]; wq[q] = d_flags + (size_t)q * max_nval; nq[q] = nval[fs];
+        int p = 0;
+        for (int a = 0; a < K; ++a)
+          for (int b = a + 1; b < K; ++b, ++p) {
+            const size_t m = fs * npairs + p, j = (size_t)q * npairs + p;
+            SvmPairJob& jb = jobs[j];
+            jb.K = S.Klab[f]; jb.ld = n_lab;
+            jb.rows = d_maps + moff[m]; jb.na = mna[m]; jb.nb = mnb[m];
+            jb.C = C[c]; jb.ca = a; jb.cb = b;
+            jb.coef = d_coef + j * npmax; jb.rho = d_rho + j;
+            jb.n_iter = d_iters + j; jb.capped = d_capped + j;
+          }
+      }
+  std::vector<SvmGemmOp> gm((size_t)nG * nf);
+  for (int g = 0; g < nG; ++g)
+    for (int f = 0; f < nf; ++f) {
+      gm[(size_t)g * nf + f] = S.h_gemm[2 * f];
+      gm[(size_t)g * nf + f].gamma = gamma[(size_t)f * nG + g];
+    }
+  CK(cudaMemcpyAsync(d_maps, maps.data(), sizeof(int) * maps.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_vrows, vrows.data(), sizeof(int) * vrows.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_vy, vy.data(), sizeof(int) * vy.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_nval, nq.data(), sizeof(int) * nQ, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_jobs, jobs.data(), sizeof(SvmPairJob) * jobs.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_gemm, gm.data(), sizeof(SvmGemmOp) * gm.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_Kq, Kq.data(), sizeof(float*) * nQ, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_trow, trow.data(), sizeof(int*) * nQ, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_yq, yq.data(), sizeof(int*) * nQ, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(d_wq, wq.data(), sizeof(int*) * nQ, cudaMemcpyHostToDevice, h->stream));
+  // the operand split does not depend on gamma: once (the fit's launch, which also splits the test rows)
+  k_svm_split<<<dim3((S.max_rows + 7) / 8, 2 * nf), 256, 0, h->stream>>>(S.d_split);
+  h->launches += 1;
+  std::vector<int> cap(nJobs), cnt((size_t)nG * nQ);
+  for (int g = 0; g < nG; ++g) {
+    k_svm_kmat<<<dim3((n_lab + SVM_BM - 1) / SVM_BM, (n_lab + SVM_BN - 1) / SVM_BN, nf), SVM_KMAT_THREADS, SVM_KMAT_SMEM, h->stream>>>(
+        d_gemm + (size_t)g * nf);
+    k_svm_smo<<<nJobs, SVM_SMO_THREADS, (size_t)SVM_SMO_SMEM_PER_ROW * npmax, h->stream>>>(d_jobs, S.eps);
+    k_svm_vote<<<dim3(max_nval, nQ), SVM_VOTE_THREADS, 0, h->stream>>>(d_jobs, npairs, K, d_Kq, d_trow, d_yq, d_nval, nullptr, d_wq, nullptr);
+    k_svm_count<<<nQ, 256, 0, h->stream>>>(d_wq, d_nval, d_count + (size_t)g * nQ);
+    h->launches += 4;
+    CK(cudaMemcpyAsync(cap.data(), d_capped, sizeof(int) * nJobs, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaGetLastError());
+    for (int j = 0; j < nJobs; ++j)
+      if (cap[j]) {
+        const int q = j / npairs, s = q % ns, c = (q / ns) % nC, f = q / (ns * nC);
+        return fail(h, MRGAN_ERR_STATE, "svm_cv: fold " + std::to_string(f) + ", gamma " + std::to_string(g) + ", C " + std::to_string(c) +
+                                         ", split " + std::to_string(s) + ", class pair " + std::to_string(j % npairs) +
+                                         " hit the iteration cap max(1e7, 100 n)");
+      }
+  }
+  CK(cudaMemcpyAsync(cnt.data(), d_count, sizeof(int) * cnt.size(), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  for (int f = 0; f < nf; ++f)
+    for (int g = 0; g < nG; ++g)
+      for (int c = 0; c < nC; ++c)
+        for (int s = 0; s < ns; ++s) wrong[(((size_t)f * nG + g) * nC + c) * ns + s] = cnt[(size_t)g * nQ + (f * nC + c) * ns + s];
   return MRGAN_OK;
 }
 
@@ -2654,8 +2852,8 @@ int mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t
     CK(cudaMemcpyAsync(S.d_ns, &n, sizeof(int), cudaMemcpyHostToDevice, h->stream));
     k_svm_split<<<dim3((n + 7) / 8, 1), 256, 0, h->stream>>>(S.d_split_s);
     k_svm_kmat<<<dim3((S.n_lab + SVM_BM - 1) / SVM_BM, (n + SVM_BN - 1) / SVM_BN, 1), SVM_KMAT_THREADS, SVM_KMAT_SMEM, h->stream>>>(S.d_gemm_s);
-    k_svm_vote<<<dim3(n, 1), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs + (size_t)fold * S.npairs, S.npairs, K, S.d_Ks, nullptr, S.d_ns,
-                                                               S.d_decs, nullptr, S.d_preds);
+    k_svm_vote<<<dim3(n, 1), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs + (size_t)fold * S.npairs, S.npairs, K, S.d_Ks, nullptr, nullptr,
+                                                               S.d_ns, S.d_decs, nullptr, S.d_preds);
     h->launches += 3;
     CK(cudaMemcpyAsync(pred, S.preds, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (scores) CK(cudaMemcpyAsync(scores, S.decs, (size_t)n * S.npairs * sizeof(float), cudaMemcpyDeviceToHost, h->stream));

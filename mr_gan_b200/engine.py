@@ -297,19 +297,44 @@ class FoldGroup:
         K = self.cfg.n_classes
         return K * (K - 1) // 2
 
-    def svm_fit(self, lab_rows, C=1.0, gamma=None, tol=1e-3):
-        """mr_svm.py:106 ``SVC(kernel='rbf', C).fit`` for every fold, then the prediction of every fold's test set.
-        lab_rows: int32 [n_folds, n_lab] class-major rows of X_train; gamma: per-fold list / scalar (None: 1 / D).
-        Returns the SMO iterations, int32 [n_folds, n_pairs]."""
+    def _svm_lab(self, fn, lab_rows):
         lab = _i32(lab_rows)
         if lab.ndim != 2 or lab.shape[0] != self.n_folds:
-            raise ValueError("svm_fit: lab_rows must be [n_folds, n_lab]")
+            raise ValueError(fn + ": lab_rows must be [n_folds, n_lab]")
+        return lab
+
+    def svm_fit(self, lab_rows, C=1.0, gamma=None, tol=1e-3):
+        """mr_svm.py:106 ``SVC(kernel='rbf', C).fit`` for every fold, then the prediction of every fold's test set.
+        lab_rows: int32 [n_folds, n_lab] class-major rows of X_train; C, gamma: per-fold list / scalar (gamma None: 1 / D).
+        Returns the SMO iterations, int32 [n_folds, n_pairs]."""
+        lab = self._svm_lab("svm_fit", lab_rows)
         if gamma is None:
             gamma = [1.0 / D for D, _, _, _ in self.shapes]
         g = _f32(np.broadcast_to(np.asarray(gamma, dtype=np.float32), (self.n_folds,)))
+        c = _f32(np.broadcast_to(np.asarray(C, dtype=np.float32), (self.n_folds,)))
         it = np.zeros((self.n_folds, self.n_pairs), dtype=np.int32)
-        self._chk(self.lib.mrgan_svm_fit(self._h, _lib.iptr(lab), lab.shape[1], float(C), _lib.fptr(g), float(tol), _lib.iptr(it)))
+        self._chk(self.lib.mrgan_svm_fit_folds(self._h, _lib.iptr(lab), lab.shape[1], _lib.fptr(c), _lib.fptr(g), float(tol), _lib.iptr(it)))
         return it
+
+    def svm_cv(self, lab_rows, split, C_grid, gamma, tol=1e-3):
+        """The inner cross-validation of ``GridSearchCV(SVC(kernel='rbf'), {'C': C_grid, 'gamma': ...}, cv)`` for every fold:
+        split: int [n_folds, n_lab], the inner split of each labeled row (0 .. n_splits - 1, n_splits = split.max() + 1);
+        C_grid: [nC]; gamma: [n_folds, nG] (or [nG] for every fold), absolute.  Returns the misclassified validation rows,
+        int32 [n_folds, nG, nC, n_splits].  Invalidates a previous svm_fit (svm_eval etc. fail until the next one)."""
+        lab = self._svm_lab("svm_cv", lab_rows)
+        sp = _i32(split)
+        if sp.shape != lab.shape:
+            raise ValueError("svm_cv: split must have the shape of lab_rows")
+        c = _f32(np.atleast_1d(np.asarray(C_grid, dtype=np.float32)))
+        g = np.asarray(gamma, dtype=np.float32)
+        g = _f32(np.broadcast_to(g, (self.n_folds,) + g.shape[-1:]) if g.ndim == 1 else g)
+        if g.ndim != 2 or g.shape[0] != self.n_folds:
+            raise ValueError("svm_cv: gamma must be [nG] or [n_folds, nG]")
+        ns = int(sp.max()) + 1 if sp.size else 0
+        out = np.zeros((self.n_folds, g.shape[1], len(c), max(ns, 1)), dtype=np.int32)
+        self._chk(self.lib.mrgan_svm_cv(self._h, _lib.iptr(lab), lab.shape[1], _lib.iptr(sp), ns, _lib.fptr(c), len(c), _lib.fptr(g),
+                                        g.shape[1], float(tol), _lib.iptr(out)))
+        return out
 
     def svm_eval(self, fold):
         """Error of the one-vs-one vote on the fold's full test set (np.mean(predicted != y_test))."""

@@ -58,12 +58,18 @@ def setting_fields(tool, job, index, **fields):
 
 
 def record(tool, job, result, index, **fields):
-    """The JSON record of one fold-training: its setting_fields, n_test, error and confusion."""
+    """The JSON record of one fold-training: its setting_fields, n_test, error and confusion, and for a tuned SVM fold
+    (mr_svm.py --tune) the selected C, gamma_D and the cv_accuracy grid [nC][nG]."""
     rec = setting_fields(tool, job, index, **fields)
     conf = np.asarray(result['confusion'])
     rec['n_test'] = int(conf.sum())
     rec['error'] = result['error']
     rec['confusion'] = conf.tolist()
+    for k in ('C', 'gamma_D'):
+        if k in result:
+            rec[k] = float(result[k])
+    if 'cv_accuracy' in result:
+        rec['cv_accuracy'] = np.asarray(result['cv_accuracy'], dtype=np.float64).tolist()
     return rec
 
 
