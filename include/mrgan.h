@@ -52,8 +52,9 @@ enum { MRGAN_MODEL_GAN = 0,   /* mr_gan.py: G + D, feature matching          */
 enum { MRGAN_PREC_FP32 = 0,   /* FFMA kernels, fp32 operands (parity mode)                  */
        MRGAN_PREC_TF32 = 1,   /* tcgen05 kind::tf32 tensor-core kernels, fp32 accumulate    */
        MRGAN_PREC_F16 = 2 };  /* tcgen05 kind::f16 on 16-bit operand COPIES: fp16 weights and activations (the same
-                                 10-bit mantissa as tf32, rounded to nearest), bf16 gradients (fp32's exponent
-                                 range, no loss scale); fp32 master weights, fp32 accumulation and Adam. */
+                                 10-bit mantissa as tf32, rounded to nearest), fp16 gradients times a loss scale
+                                 (4096, saturating; MRGAN_LOSS_SCALE overrides it); fp32 master weights, fp32
+                                 accumulation and Adam. */
 
 /* Hyper-parameters; mrgan_default_config() fills the reference's values. */
 typedef struct {

@@ -479,8 +479,24 @@ int build_descs(mrgan_handle* h) {
   return MRGAN_OK;
 }
 
+// ------------------------------------------------------------------ kernel launch (a failure is kept as the handle's sticky error)
+// Every kernel of the library is launched here, so h->launches counts them all.
+template <typename... KArgs, typename... Args>
+void launch_k(mrgan_handle* h, void (*kern)(KArgs...), const cudaLaunchConfig_t& cfg, Args... args) {
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+  if (e != cudaSuccess && !h->sticky) { h->sticky = MRGAN_ERR_CUDA; h->err = std::string("kernel launch: ") + cudaGetErrorString(e); }
+  h->launches++;
+}
+template <typename... KArgs, typename... Args>
+void launch_k(mrgan_handle* h, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  launch_k(h, kern, cfg, args...);
+}
+
 void set_ones(mrgan_handle* h, float* p, int ld, int rows, int col) {
-  k_set_col<<<(rows + 127) / 128, 128, 0, h->stream>>>(p, ld, rows, col, 1.0f, h->om);
+  launch_k(h, k_set_col, (rows + 127) / 128, 128, 0, h->stream, p, ld, rows, col, 1.0f, h->om);
 }
 
 void init_ones(mrgan_handle* h) {
@@ -506,17 +522,6 @@ void init_ones(mrgan_handle* h) {
   }
 }
 
-
-// ------------------------------------------------------------------ kernel launch (a failure is kept as the handle's sticky error)
-template <typename... KArgs, typename... Args>
-void launch_k(mrgan_handle* h, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-  if (e != cudaSuccess && !h->sticky) { h->sticky = MRGAN_ERR_CUDA; h->err = std::string("kernel launch: ") + cudaGetErrorString(e); }
-  h->launches++;
-}
 
 // status of everything enqueued since the last check (launch_k / dp_allreduce record the first failure)
 int take_sticky(mrgan_handle* h) {
@@ -570,8 +575,7 @@ void dp_allreduce(mrgan_handle* h, float* buf, size_t n) {
   if (h->dp_virtual) {
     const size_t seg = n / (size_t)h->dp_world;
     const int blocks = (int)std::min<size_t>((seg + 255) / 256, 1184);
-    k_virtual_allreduce<<<blocks, 256, 0, h->stream>>>(buf, seg, h->dp_world);
-    h->launches++;
+    launch_k(h, k_virtual_allreduce, blocks, 256, 0, h->stream, buf, seg, h->dp_world);
     return;
   }
   const int rc = g_nccl.AllReduce(buf, buf, n, 7, 0, h->nccl_comm, h->stream);
@@ -631,10 +635,7 @@ void dp_exchange(mrgan_handle* h, int net) {
   attr[0].val.cooperative = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   const float ginv = h->om.mode == 2 ? 1.0f / h->om.gscale : 1.0f;
-  const cudaError_t e = cudaLaunchKernelEx(&cfg, k_dp_exchange, h->dp_peers[net], W, h->dp_virtual ? -1 : h->dp_rank, off, len, h->d_folds,
-                                           h->nf, net, h->hp, ginv);
-  if (e != cudaSuccess && !h->sticky) { h->sticky = MRGAN_ERR_CUDA; h->err = std::string("k_dp_exchange launch: ") + cudaGetErrorString(e); }
-  h->launches++;
+  launch_k(h, k_dp_exchange, cfg, h->dp_peers[net], W, h->dp_virtual ? -1 : h->dp_rank, off, len, h->d_folds, h->nf, net, h->hp, ginv);
 }
 
 // gradient exchange + optimizer of one net in the data-parallel mode
@@ -754,10 +755,9 @@ void enqueue_gen_fwd(mrgan_handle* h, int f0, int nfl, int op_g3) {
   const dim3 bnt(h->cfg.batch > 256 ? 1024 : 256);     // 32 columns x 8 (reference batch) or 32 (large batch) row slices
   const OperandMode tf32 = h->om;
   if (h->d_dpbufs) {          // batch statistics over the GLOBAL batch: local sums -> NVLink all-reduce -> apply
-    k_bn_stats<<<bnf, bnt, 0, h->stream>>>(h->d_bn + f0, h->d_dpbufs + f0);
+    launch_k(h, k_bn_stats, bnf, bnt, 0, h->stream, h->d_bn + f0, h->d_dpbufs + f0);
     dp_allreduce(h, h->dp_bnf + (size_t)f0 * 2 * kGH, (size_t)nfl * 2 * kGH);
-    k_bn_apply<<<bnf, bnt, 0, h->stream>>>(h->d_bn + f0, h->d_dpbufs + f0, h->cfg.bn_eps, tf32, h->hp.dp_bg);
-    h->launches += 2;
+    launch_k(h, k_bn_apply, bnf, bnt, 0, h->stream, h->d_bn + f0, h->d_dpbufs + f0, h->cfg.bn_eps, tf32, h->hp.dp_bg);
   } else {
     launch_k(h, k_bn_fwd, bnf, bnt, 0, h->stream, (const BnDesc*)(h->d_bn + f0), h->cfg.bn_eps, tf32);
   }
@@ -810,11 +810,10 @@ void enqueue_gen_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
   for (int l = 0; l < 5; ++l) launch_gemm(h, OP_D1G + l, f0, nfl, 0);
   if (h->d_dpbufs) {
     const dim3 fmg((kDW[4] + BN_COLS - 1) / BN_COLS, split_chunks(B), nfl), fmt(B > 256 ? 1024 : 256);
-    k_fm_stats<<<fmg, fmt, 0, h->stream>>>(h->d_loss + f0, h->d_dpbufs + f0, B);
+    launch_k(h, k_fm_stats, fmg, fmt, 0, h->stream, h->d_loss + f0, h->d_dpbufs + f0, B);
     dp_allreduce(h, h->dp_fm + (size_t)f0 * 2 * kDW[4], (size_t)nfl * 2 * kDW[4]);
-    k_fm_apply<<<fmg, fmt, 0, h->stream>>>(h->d_loss + f0, h->d_dpbufs + f0, h->d_step_stats, f0, h->nf, t, B,
-                                           h->om, h->hp.dp_bg, h->dp_world, h->hp.alpha);
-    h->launches += 2;
+    launch_k(h, k_fm_apply, fmg, fmt, 0, h->stream, h->d_loss + f0, h->d_dpbufs + f0, h->d_step_stats, f0, h->nf, t, B,
+             h->om, h->hp.dp_bg, h->dp_world, h->hp.alpha);
   } else if (!(hm & 2)) {   // otherwise D layer 5's epilogue computed the feature-matching loss, its gradient, and advanced the counters
     launch_k(h, k_fm, dim3(1, 1, nfl), dim3(1024), 0, h->stream, (const LossDesc*)(h->d_loss + f0), h->d_step_stats, f0, h->nf, t, B,
              h->om, h->hp.alpha);
@@ -832,10 +831,9 @@ void enqueue_gen_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
   }
   const dim3 bng((kGH + BN_COLS - 1) / BN_COLS, h->d_dpbufs ? split_chunks(B) : 1, nfl), bnt(B > 256 ? 1024 : 256);
   if (h->d_dpbufs) {
-    k_bn_bwd_stats<<<bng, bnt, 0, h->stream>>>(h->d_bn + f0, h->d_dpbufs + f0, h->om);
+    launch_k(h, k_bn_bwd_stats, bng, bnt, 0, h->stream, h->d_bn + f0, h->d_dpbufs + f0, h->om);
     dp_allreduce(h, h->dp_bnb + (size_t)f0 * 2 * kGH, (size_t)nfl * 2 * kGH);
-    k_bn_bwd_apply<<<bng, bnt, 0, h->stream>>>(h->d_bn + f0, h->d_dpbufs + f0, h->om, h->hp.dp_bg);
-    h->launches += 2;
+    launch_k(h, k_bn_bwd_apply, bng, bnt, 0, h->stream, h->d_bn + f0, h->d_dpbufs + f0, h->om, h->hp.dp_bg);
   } else {
     launch_k(h, k_bn_bwd, bng, bnt, 0, h->stream, (const BnDesc*)(h->d_bn + f0), h->om);
   }
@@ -936,25 +934,6 @@ int saliency_setup(mrgan_handle* h) {
   return MRGAN_OK;
 }
 
-// prediction entry points: the single-GPU handle only (data-parallel replicas are out of their scope)
-int need_local(mrgan_handle* h, const char* fn) {
-  if (h->dp_world > 1 || h->dp_virtual || h->nccl_comm) return fail(h, MRGAN_ERR_STATE, std::string(fn) + ": not available on a data-parallel handle");
-  return MRGAN_OK;
-}
-
-int check_fold(mrgan_handle* h, int fold) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (fold < 0 || fold >= h->nf) return fail(h, MRGAN_ERR_ARG, "fold index out of range");
-  return MRGAN_OK;
-}
-
-// GAN / NN entry points: an SVM handle has no nets
-int need_nets(mrgan_handle* h, const char* fn) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model == MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, std::string(fn) + ": not available on an SVM handle");
-  return MRGAN_OK;
-}
-
 int finish_pending(mrgan_handle* h) {
   if (h->epoch_pending) {
     CK(cudaStreamSynchronize(h->stream));
@@ -965,6 +944,120 @@ int finish_pending(mrgan_handle* h) {
   }
   return MRGAN_OK;
 }
+
+#define TRY(expr)                                                                                  \
+  do {                                                                                             \
+    const int _rc = (expr);                                                                        \
+    if (_rc) return _rc;                                                                           \
+  } while (0)
+
+// What a C-ABI entry point needs of its handle.  Every entry point that takes a handle and returns a status calls
+// enter() first and ready() after its own argument checks, so the checks run in one order (enter reads FOLD and the
+// model flags, ready reads FOLD and the state flags):
+//   enter: null handle, fold index (MRGAN_ERR_ARG); model (MRGAN_ERR_STATE)
+//   ... the call's own argument checks (MRGAN_ERR_ARG) ...
+//   ready: data-parallel mode, loaded folds, fitted SVM (MRGAN_ERR_STATE); then the handle's device and a pending epoch.
+enum : unsigned {
+  FOLD = 1u,          // the call takes a fold index
+  GAN = 2u, NN = 4u, SVM = 8u,
+  NETS = 16u,         // GAN or NN: an SVM handle has no nets
+  LOADED = 32u,       // the call's fold, or every fold of the handle, has its data (mrgan_load_fold / mrgan_prepare_fold)
+  FITTED = 64u,       // mrgan_svm_fit* ran since the last invalidation
+  LOCAL = 128u,       // not a data-parallel handle (mrgan_dp_init / mrgan_dp_init_virtual)
+  NOT_VIRTUAL = 256u, // not a handle whose folds play virtual ranks
+};
+
+int enter(mrgan_handle* h, const char* fn, unsigned need, int fold = 0) {
+  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  if ((need & FOLD) && (fold < 0 || fold >= h->nf)) return fail(h, MRGAN_ERR_ARG, "fold index out of range");
+  const int m = h->cfg.model;
+  if ((need & GAN) && m != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, std::string(fn) + " needs a GAN handle");
+  if ((need & NN) && m != MRGAN_MODEL_NN) return fail(h, MRGAN_ERR_STATE, std::string(fn) + " needs an NN handle");
+  if ((need & SVM) && m != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, std::string(fn) + " needs an SVM handle");
+  if ((need & NETS) && m == MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, std::string(fn) + ": not available on an SVM handle");
+  return MRGAN_OK;
+}
+
+int ready(mrgan_handle* h, const char* fn, unsigned need, int fold = 0) {
+  if ((need & LOCAL) && (h->dp_world > 1 || h->dp_virtual || h->nccl_comm))
+    return fail(h, MRGAN_ERR_STATE, std::string(fn) + ": not available on a data-parallel handle");
+  if ((need & NOT_VIRTUAL) && h->dp_virtual)
+    return fail(h, MRGAN_ERR_STATE, std::string(fn) + ": virtual ranks step together: use mrgan_train_epoch");
+  if (need & LOADED)
+    for (int f = (need & FOLD) ? fold : 0; f < ((need & FOLD) ? fold + 1 : h->nf); ++f)
+      if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, std::string(fn) + " before mrgan_load_fold");
+  if ((need & FITTED) && !h->svm.fitted) return fail(h, MRGAN_ERR_STATE, std::string(fn) + " before mrgan_svm_fit");
+  CK(cudaSetDevice(h->cfg.device));
+  return finish_pending(h);
+}
+
+// The end of an entry point that enqueued work: wait for it, then report a failed launch or collective.
+int complete(mrgan_handle* h) {
+  CK(cudaStreamSynchronize(h->stream));
+  CKS();
+  return MRGAN_OK;
+}
+
+// Average device ms of `reps` calls of once() on the handle's stream, after one warm-up call.
+template <typename Once>
+int time_reps(mrgan_handle* h, int reps, Once once, float* ms_avg) {
+  once();
+  CK(cudaEventRecord(h->ev0, h->stream));
+  for (int i = 0; i < reps; ++i) once();
+  CK(cudaEventRecord(h->ev1, h->stream));
+  TRY(complete(h));
+  float ms = 0.f;
+  CK(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+  *ms_avg = ms / reps;
+  return MRGAN_OK;
+}
+
+// Rows that feed the first eval MMA directly get their operand form: rounded onto the tf32 grid (RN), or their fp16 copy.
+void to_operand(mrgan_handle* h, float* p, size_t n) {
+  if (h->cfg.precision == MRGAN_PREC_TF32) launch_k(h, k_round_tf32, 256, 256, 0, h->stream, p, n);
+  else if (h->om.mode == 2) launch_k(h, k_to_half, 256, 256, 0, h->stream, p, n, h->om);
+}
+
+// Host rows x [n][D] of a fold -> its eval staging rows (ex_stage), in operand form.
+int stage_rows(mrgan_handle* h, int fold, const float* x, int n) {
+  FoldBuffers& b = h->fb[fold];
+  const size_t w = (size_t)h->shapes[fold].D * sizeof(float);
+  CK(cudaMemcpy2DAsync(b.ex_stage, (size_t)b.lda[0] * sizeof(float), x, w, w, n, cudaMemcpyHostToDevice, h->stream));
+  to_operand(h, b.ex_stage, (size_t)n * b.lda[0]);
+  return MRGAN_OK;
+}
+
+// The captured epochs bake in the handle's mode: a mode change drops them, and the next epoch captures again.
+void drop_graphs(mrgan_handle* h) {
+  for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
+  h->graphs.clear(); h->graph_nodes.clear();
+}
+
+// The handle becomes a data-parallel replica of `world` ranks (rank < 0: its folds play the ranks).
+int dp_switch(mrgan_handle* h, int world, int rank) {
+  TRY(alloc_split_bufs(h));
+  h->dp_world = world; h->dp_rank = std::max(rank, 0); h->dp_virtual = rank < 0;
+  h->hp.dp_bloc = h->cfg.batch; h->hp.dp_bg = h->cfg.batch * world; h->hp.dp_rank = rank;     // -1: rank = fold index (common.cuh)
+  if (h->cfg.precision != MRGAN_PREC_FP32) {   // gradients must be all-reduced before Adam: dW stores them, k_adam applies
+    tc_teardown(h);
+    h->tc_fused_adam = false;
+    TRY(tc_setup(h));
+  }
+  drop_graphs(h);
+  CK(cudaDeviceSynchronize());
+  return MRGAN_OK;
+}
+
+// Device temporaries of one call, freed on every return path.
+struct Temps {
+  std::vector<void*> p;
+  template <typename T> cudaError_t alloc(T** ptr, size_t bytes) {
+    const cudaError_t e = cudaMalloc(ptr, bytes);
+    if (e == cudaSuccess) p.push_back(*ptr);
+    return e;
+  }
+  ~Temps() { for (void* q : p) cudaFree(q); }
+};
 
 // reference-order <-> internal (augmented, padded) parameter layout
 void pack_params(const mrgan_handle* h, int fold, int net, const float* src, std::vector<float>& dst, bool to_internal,
@@ -1028,9 +1121,8 @@ int build_graph(mrgan_handle* h, int key, int nb) {
       cudaStreamWaitEvent(origin, j, 0);
     }
   }
-  k_epoch_reduce<<<h->nf, 32, 0, h->stream>>>(h->d_step_stats, h->d_eval, h->d_epoch_stats, h->nf, nb,
-                                              c.model == MRGAN_MODEL_GAN && c.eval_each_epoch);
-  h->launches++;
+  launch_k(h, k_epoch_reduce, h->nf, 32, 0, h->stream, h->d_step_stats, h->d_eval, h->d_epoch_stats, h->nf, nb,
+           (int)(c.model == MRGAN_MODEL_GAN && c.eval_each_epoch));
   CK(cudaMemcpyAsync(h->h_epoch_stats, h->d_epoch_stats, (size_t)h->nf * 8 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamEndCapture(h->stream, &g));
   { const int sk = take_sticky(h); if (sk) { cudaGraphDestroy(g); return sk; } }
@@ -1193,8 +1285,9 @@ int tc_debug_gemm(mrgan_handle* h, int mode, const GemmDesc& g, int esz) {
   if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
   TcOp t; memset(&t, 0, sizeof(t));
   if (!tc_fill_op(fn, t, g, mode, esz)) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
+  Temps tmp;
   TcOp* d = nullptr;
-  CK(cudaMalloc(&d, sizeof(TcOp)));
+  CK(tmp.alloc(&d, sizeof(TcOp)));
   CK(cudaMemcpyAsync(d, &t, sizeof(t), cudaMemcpyHostToDevice, h->stream));
   tc_set_smem_attr();
   dim3 grid((t.ME + 127) / 128, (t.NE + t.bn - 1) / t.bn, 1);
@@ -1204,7 +1297,6 @@ int tc_debug_gemm(mrgan_handle* h, int mode, const GemmDesc& g, int esz) {
   else if (mode == 1) TC_LAUNCH(h, f16, K_TC_DX, grid, dim3(TC_FWD_THREADS), tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream, (const TcOp*)d, h->d_folds, 0, h->hp, om0);
   else TC_LAUNCH(h, f16, K_TC_DW, grid, dim3(TC_DW_THREADS), tc_smem_bytes(t.bn, TC_DW_STAGES), h->stream, (const TcOp*)d, h->d_folds, 0, h->hp, om0);
   CK(cudaStreamSynchronize(h->stream));
-  cudaFree(d);
   return MRGAN_OK;
 }
 
@@ -1587,6 +1679,10 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
     int rc = tc_setup(h);
     if (rc != MRGAN_OK) return cleanup(rc);
   }
+  if (cfg->model == MRGAN_MODEL_GAN) {     // the device-side epoch permutations sort in shared memory
+    e = cudaFuncSetAttribute(k_epoch_perm, cudaFuncAttributeMaxDynamicSharedMemorySize, PERM_MAX * 8);
+    if (e != cudaSuccess) return cleanup(fail(nullptr, MRGAN_ERR_CUDA, std::string("create: k_epoch_perm: ") + cudaGetErrorString(e)));
+  }
   e = cudaStreamSynchronize(h->stream);
   if (e == cudaSuccess) e = cudaGetLastError();
   if (e != cudaSuccess) return cleanup(fail(nullptr, MRGAN_ERR_CUDA, std::string("create: ") + cudaGetErrorString(e)));
@@ -1598,7 +1694,7 @@ int mrgan_destroy(mrgan_handle* h) {
   if (!h) return MRGAN_OK;
   cudaSetDevice(h->cfg.device);
   if (h->stream) cudaStreamSynchronize(h->stream);
-  for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
+  drop_graphs(h);
   for (auto& ds : h->datasets) { if (ds.x) cudaFree(ds.x); if (ds.y) cudaFree(ds.y); }
   if (h->d_prep_stats) cudaFree(h->d_prep_stats);
   if (h->d_prep_rows) cudaFree(h->d_prep_rows);
@@ -1633,10 +1729,8 @@ int mrgan_destroy(mrgan_handle* h) {
 }
 
 int mrgan_sync(mrgan_handle* h) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h);
-  if (rc) return rc;
+  TRY(enter(h, "sync", 0));
+  TRY(ready(h, "sync", 0));
   CK(cudaStreamSynchronize(h->stream));
   return MRGAN_OK;
 }
@@ -1647,21 +1741,17 @@ int64_t mrgan_num_params(const mrgan_handle* h, int fold, int net) {
 }
 
 int mrgan_set_params(mrgan_handle* h, int fold, int net, const float* src, int64_t n) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "set_params"); if (rc) return rc;
+  TRY(enter(h, "set_params", FOLD | NETS, fold));
   if (net < 0 || net > 1 || h->net[net].empty()) return fail(h, MRGAN_ERR_ARG, "no such net in this model");
   const NetLayout& L = h->net[net][fold];
   if (!src || n != L.n_ref) return fail(h, MRGAN_ERR_ARG, "set_params: length does not match mrgan_num_params");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "set_params", FOLD | NETS, fold));
   std::vector<float> buf((size_t)L.n, 0.f);
   pack_params(h, fold, net, src, buf, true, nullptr);
   CK(cudaMemcpyAsync(h->P + L.off, buf.data(), (size_t)L.n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-  if (h->om.mode == 2) {      // refresh the fp16 operand copy of the uploaded weights
-    k_to_half<<<256, 256, 0, h->stream>>>(h->P + L.off, (size_t)L.n, h->om);
-    h->launches++;
-  }
-  CK(cudaStreamSynchronize(h->stream));
-  return MRGAN_OK;
+  // refresh the fp16 operand copy of the uploaded weights (the tf32 path reads the fp32 master weights unrounded)
+  if (h->om.mode == 2) launch_k(h, k_to_half, 256, 256, 0, h->stream, h->P + L.off, (size_t)L.n, h->om);
+  return complete(h);
 }
 
 static int get_flat(mrgan_handle* h, int fold, int net, const float* dev, float* dst, int64_t n) {
@@ -1675,26 +1765,23 @@ static int get_flat(mrgan_handle* h, int fold, int net, const float* dev, float*
 }
 
 int mrgan_get_params(mrgan_handle* h, int fold, int net, float* dst, int64_t n) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "get_params"); if (rc) return rc;
+  TRY(enter(h, "get_params", FOLD | NETS, fold));
   if (net < 0 || net > 1 || h->net[net].empty()) return fail(h, MRGAN_ERR_ARG, "no such net in this model");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "get_params", FOLD | NETS, fold));
   return get_flat(h, fold, net, h->P, dst, n);
 }
 
 int mrgan_get_adam(mrgan_handle* h, int fold, int net, float* m, float* v, int64_t n) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "get_adam"); if (rc) return rc;
+  TRY(enter(h, "get_adam", FOLD | NETS, fold));
   if (net < 0 || net > 1 || h->net[net].empty()) return fail(h, MRGAN_ERR_ARG, "no such net in this model");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
-  rc = get_flat(h, fold, net, h->Mo, m, n); if (rc) return rc;
+  TRY(ready(h, "get_adam", FOLD | NETS, fold));
+  TRY(get_flat(h, fold, net, h->Mo, m, n));
   return get_flat(h, fold, net, h->Vo, v, n);
 }
 
 int mrgan_get_counters(mrgan_handle* h, int fold, int* iterations, int* rng_step) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "get_counters"); if (rc) return rc;
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(enter(h, "get_counters", FOLD | NETS, fold));
+  TRY(ready(h, "get_counters", FOLD | NETS, fold));
   FoldState fs;
   CK(cudaMemcpyAsync(&fs, h->d_folds + fold, sizeof(fs), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
@@ -1705,40 +1792,32 @@ int mrgan_get_counters(mrgan_handle* h, int fold, int* iterations, int* rng_step
 
 int mrgan_load_fold(mrgan_handle* h, int fold, const float* x_train, const int32_t* y_train, const float* x_test,
                     const int32_t* y_test) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  TRY(enter(h, "load_fold", FOLD, fold));
   if (!x_train || !y_train || !x_test || !y_test) return fail(h, MRGAN_ERR_ARG, "load_fold: null pointer");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
   const mrgan_fold_shape& s = h->shapes[fold];
   for (int i = 0; i < s.n_train; ++i)
     if (y_train[i] < 0 || y_train[i] >= h->cfg.n_classes) return fail(h, MRGAN_ERR_ARG, "load_fold: y_train label out of range");
   for (int i = 0; i < s.n_test; ++i)
     if (y_test[i] < 0 || y_test[i] >= h->cfg.n_classes) return fail(h, MRGAN_ERR_ARG, "load_fold: y_test label out of range");
+  TRY(ready(h, "load_fold", FOLD, fold));
   FoldBuffers& b = h->fb[fold];
   const size_t w = (size_t)s.D * sizeof(float);
   CK(cudaMemcpy2DAsync(b.xtr, (size_t)pitch8(s.D) * sizeof(float), x_train, w, w, s.n_train, cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpy2DAsync(b.xte, (size_t)b.lda[0] * sizeof(float), x_test, w, w, s.n_test, cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(b.ytr, y_train, (size_t)s.n_train * sizeof(int), cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(b.yte, y_test, (size_t)s.n_test * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-  if (h->cfg.precision == MRGAN_PREC_TF32) {   // X_test feeds the first eval MMA directly: put it on the tf32 grid (RN) once
-    k_round_tf32<<<256, 256, 0, h->stream>>>(b.xte, (size_t)s.n_test * b.lda[0]);
-    h->launches++;
-  } else if (h->om.mode == 2) {                // ... or make its fp16 operand copy (ones column included)
-    k_to_half<<<256, 256, 0, h->stream>>>(b.xte, (size_t)s.n_test * b.lda[0], h->om);
-    h->launches++;
-  }
-  CK(cudaStreamSynchronize(h->stream));
+  to_operand(h, b.xte, (size_t)s.n_test * b.lda[0]);      // X_test feeds the first eval MMA directly (ones column included)
+  TRY(complete(h));
   b.loaded = true;
   return MRGAN_OK;
 }
 
 int mrgan_load_dataset(mrgan_handle* h, int slot, const float* x, const int32_t* y, int n_rows, int D) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  TRY(enter(h, "load_dataset", 0));
   if (slot < 0 || slot >= 8 || !x || !y || n_rows < 1 || D < 1) return fail(h, MRGAN_ERR_ARG, "load_dataset: bad argument");
   for (int i = 0; i < n_rows; ++i)
     if (y[i] < 0 || y[i] >= h->cfg.n_classes) return fail(h, MRGAN_ERR_ARG, "load_dataset: label out of range");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "load_dataset", 0));
   mrgan_handle::Dataset& ds = h->datasets[slot];
   if (ds.x && (ds.n != n_rows || ds.D != D)) { cudaFree(ds.x); cudaFree(ds.y); ds.x = nullptr; ds.y = nullptr; }
   ds.n = n_rows; ds.D = D; ds.ld = pitch8(D);
@@ -1749,12 +1828,11 @@ int mrgan_load_dataset(mrgan_handle* h, int slot, const float* x, const int32_t*
   CK(cudaMemcpy2DAsync(ds.x, (size_t)ds.ld * sizeof(float), x, (size_t)D * sizeof(float), (size_t)D * sizeof(float), n_rows,
                        cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(ds.y, y, (size_t)n_rows * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  return MRGAN_OK;
+  return complete(h);
 }
 
 int mrgan_prepare_fold(mrgan_handle* h, int fold, int slot, const int32_t* train_rows, const int32_t* test_rows) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  TRY(enter(h, "prepare_fold", FOLD, fold));
   if (slot < 0 || slot >= 8 || !h->datasets[slot].x) return fail(h, MRGAN_ERR_STATE, "prepare_fold: dataset slot is empty");
   if (!train_rows || !test_rows) return fail(h, MRGAN_ERR_ARG, "prepare_fold: null pointer");
   const mrgan_handle::Dataset& ds = h->datasets[slot];
@@ -1762,8 +1840,7 @@ int mrgan_prepare_fold(mrgan_handle* h, int fold, int slot, const int32_t* train
   if (ds.D != s.D) return fail(h, MRGAN_ERR_ARG, "prepare_fold: dataset width differs from the fold's D");
   for (int i = 0; i < s.n_train; ++i) if ((unsigned)train_rows[i] >= (unsigned)ds.n) return fail(h, MRGAN_ERR_ARG, "prepare_fold: train row out of range");
   for (int i = 0; i < s.n_test; ++i) if ((unsigned)test_rows[i] >= (unsigned)ds.n) return fail(h, MRGAN_ERR_ARG, "prepare_fold: test row out of range");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "prepare_fold", FOLD, fold));
   const int nrows = s.n_train + s.n_test;
   if (nrows > h->prep_rows_cap) {
     if (h->d_prep_rows) cudaFree(h->d_prep_rows);
@@ -1779,29 +1856,24 @@ int mrgan_prepare_fold(mrgan_handle* h, int fold, int slot, const int32_t* train
   CK(cudaMemcpyAsync(h->d_prep_rows, train_rows, (size_t)s.n_train * sizeof(int), cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(h->d_prep_rows + s.n_train, test_rows, (size_t)s.n_test * sizeof(int), cudaMemcpyHostToDevice, h->stream));
   const int gx = (s.D + 127) / 128;
-  k_col_stats<<<dim3(gx, PREP_SLICES), 128, 0, h->stream>>>(ds.x, ds.ld, h->d_prep_rows, s.n_train, s.D, h->d_prep_stats);
-  k_scale_gather<<<dim3(gx, 64), 128, 0, h->stream>>>(ds.x, ds.ld, h->d_prep_rows, s.n_train, s.D, h->d_prep_stats, PREP_SLICES, s.n_train,
-                                                     b.xtr, pitch8(s.D), ds.y, b.ytr, OperandMode{0, 1.0f, nullptr, nullptr});
-  k_scale_gather<<<dim3(gx, 64), 128, 0, h->stream>>>(ds.x, ds.ld, h->d_prep_rows + s.n_train, s.n_test, s.D, h->d_prep_stats, PREP_SLICES, s.n_train,
-                                                     b.xte, b.lda[0], ds.y, b.yte, h->om);
-  h->launches += 3;
-  CK(cudaStreamSynchronize(h->stream));     // the pageable index arrays are borrowed only for the call
-  CKS();
+  launch_k(h, k_col_stats, dim3(gx, PREP_SLICES), 128, 0, h->stream, ds.x, ds.ld, h->d_prep_rows, s.n_train, s.D, h->d_prep_stats);
+  launch_k(h, k_scale_gather, dim3(gx, 64), 128, 0, h->stream, ds.x, ds.ld, h->d_prep_rows, s.n_train, s.D, h->d_prep_stats, PREP_SLICES,
+           s.n_train, b.xtr, pitch8(s.D), ds.y, b.ytr, OperandMode{0, 1.0f, nullptr, nullptr});
+  launch_k(h, k_scale_gather, dim3(gx, 64), 128, 0, h->stream, ds.x, ds.ld, h->d_prep_rows + s.n_train, s.n_test, s.D, h->d_prep_stats,
+           PREP_SLICES, s.n_train, b.xte, b.lda[0], ds.y, b.yte, h->om);
+  TRY(complete(h));     // the pageable index arrays are borrowed only for the call
   b.loaded = true;
   return MRGAN_OK;
 }
 
 int mrgan_disc_step(mrgan_handle* h, int fold, const float* x_lab, const int32_t* labels, const float* x_unl,
                     const float* z, float out[3]) {
-  int rc = check_fold(h, fold); if (rc) return rc;
-  if (h->cfg.model != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, "disc_step needs a GAN handle");
+  TRY(enter(h, "disc_step", FOLD | GAN, fold));
   if (!x_lab || !labels || !x_unl || !z || !out) return fail(h, MRGAN_ERR_ARG, "disc_step: null pointer");
-  if (h->dp_virtual) return fail(h, MRGAN_ERR_STATE, "disc_step: virtual ranks step together: use mrgan_train_epoch");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
   const int B = h->cfg.batch, D = h->shapes[fold].D, nd = h->cfg.noise_dim;
   for (int i = 0; i < B; ++i)
     if (labels[i] < 0 || labels[i] >= h->cfg.n_classes) return fail(h, MRGAN_ERR_ARG, "disc_step: label out of range");
+  TRY(ready(h, "disc_step", FOLD | GAN | NOT_VIRTUAL, fold));
   FoldBuffers& b = h->fb[fold];
   const size_t w = (size_t)D * sizeof(float), ld = (size_t)pitch8(D) * sizeof(float);
   CK(cudaMemcpy2DAsync(b.stage_x, ld, x_lab, w, w, B, cudaMemcpyHostToDevice, h->stream));
@@ -1810,19 +1882,15 @@ int mrgan_disc_step(mrgan_handle* h, int fold, const float* x_lab, const int32_t
   CK(cudaMemcpyAsync(b.stage_z, z, (size_t)B * nd * sizeof(float), cudaMemcpyHostToDevice, h->stream));
   enqueue_disc_step(h, fold, 1, 0, 1);
   CK(cudaMemcpyAsync(h->h_scratch, h->d_step_stats + (size_t)fold * 4, 4 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
+  TRY(complete(h));
   out[0] = h->h_scratch[0]; out[1] = h->h_scratch[1]; out[2] = h->h_scratch[2];
   return MRGAN_OK;
 }
 
 int mrgan_gen_step(mrgan_handle* h, int fold, const float* x_unl, const float* z, float out[1]) {
-  int rc = check_fold(h, fold); if (rc) return rc;
-  if (h->cfg.model != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, "gen_step needs a GAN handle");
+  TRY(enter(h, "gen_step", FOLD | GAN, fold));
   if (!x_unl || !z || !out) return fail(h, MRGAN_ERR_ARG, "gen_step: null pointer");
-  if (h->dp_virtual) return fail(h, MRGAN_ERR_STATE, "gen_step: virtual ranks step together: use mrgan_train_epoch");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "gen_step", FOLD | GAN | NOT_VIRTUAL, fold));
   const int B = h->cfg.batch, D = h->shapes[fold].D, nd = h->cfg.noise_dim;
   FoldBuffers& b = h->fb[fold];
   const size_t w = (size_t)D * sizeof(float), ld = (size_t)pitch8(D) * sizeof(float);
@@ -1830,59 +1898,42 @@ int mrgan_gen_step(mrgan_handle* h, int fold, const float* x_unl, const float* z
   CK(cudaMemcpyAsync(b.stage_z, z, (size_t)B * nd * sizeof(float), cudaMemcpyHostToDevice, h->stream));
   enqueue_gen_step(h, fold, 1, 0, 1);
   CK(cudaMemcpyAsync(h->h_scratch, h->d_step_stats + (size_t)fold * 4, 4 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
+  TRY(complete(h));
   out[0] = h->h_scratch[3];
   return MRGAN_OK;
 }
 
 int mrgan_test_batch(mrgan_handle* h, int fold, const float* x, const int32_t* y, int n, float* err) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "test_batch"); if (rc) return rc;
+  TRY(enter(h, "test_batch", FOLD | NETS, fold));
   if (!x || !y || !err) return fail(h, MRGAN_ERR_ARG, "test_batch: null pointer");
   if (n < 1 || n > h->NE) return fail(h, MRGAN_ERR_ARG, "test_batch: n exceeds max(n_test, rows of a train step)");
   for (int i = 0; i < n; ++i)
     if (y[i] < 0 || y[i] >= h->cfg.n_classes) return fail(h, MRGAN_ERR_ARG, "test_batch: label out of range");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "test_batch", FOLD | NETS, fold));
   FoldBuffers& b = h->fb[fold];
-  const int D = h->shapes[fold].D;
-  const size_t w = (size_t)D * sizeof(float);
-  CK(cudaMemcpy2DAsync(b.ex_stage, (size_t)b.lda[0] * sizeof(float), x, w, w, n, cudaMemcpyHostToDevice, h->stream));
+  TRY(stage_rows(h, fold, x, n));
   CK(cudaMemcpyAsync(b.ey_stage, y, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-  if (h->cfg.precision == MRGAN_PREC_TF32) {
-    k_round_tf32<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0]);
-    h->launches++;
-  } else if (h->om.mode == 2) {
-    k_to_half<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0], h->om);
-    h->launches++;
-  }
   enqueue_eval(h, fold, 1, true, n);
   CK(cudaMemcpyAsync(h->h_scratch, b.eval_out_s, 4 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
+  TRY(complete(h));
   err[0] = h->h_scratch[1];
   return MRGAN_OK;
 }
 
 int mrgan_eval(mrgan_handle* h, int fold, float* err) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "eval"); if (rc) return rc;
+  TRY(enter(h, "eval", FOLD | NETS, fold));
   if (!err) return fail(h, MRGAN_ERR_ARG, "eval: null pointer");
-  if (!h->fb[fold].loaded) return fail(h, MRGAN_ERR_STATE, "eval before mrgan_load_fold");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "eval", FOLD | NETS | LOADED, fold));
   enqueue_eval(h, fold, 1, false, 0);
   CK(cudaMemcpyAsync(h->h_scratch, h->fb[fold].eval_out, 4 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
+  TRY(complete(h));
   err[0] = h->h_scratch[1];
   return MRGAN_OK;
 }
 
 int mrgan_epoch_result(mrgan_handle* h, mrgan_epoch_stats* stats) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  { const int rc0 = need_nets(h, "epoch_result"); if (rc0) return rc0; }
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(enter(h, "epoch_result", NETS));
+  TRY(ready(h, "epoch_result", NETS));
   CKS();
   if (stats)
     for (int f = 0; f < h->nf; ++f) {
@@ -1893,16 +1944,14 @@ int mrgan_epoch_result(mrgan_handle* h, mrgan_epoch_stats* stats) {
 }
 
 int mrgan_set_epoch_rows(mrgan_handle* h, int fold, const int32_t* lab_rows, int n_lab, const int32_t* unl_rows, int n_unl) {
-  int rc = check_fold(h, fold); if (rc) return rc;
-  if (h->cfg.model != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, "set_epoch_rows needs a GAN handle");
+  TRY(enter(h, "set_epoch_rows", FOLD | GAN, fold));
   const int N = h->n_train;
   if (!lab_rows || n_lab < 1 || n_lab > N || n_lab > PERM_MAX) return fail(h, MRGAN_ERR_ARG, "set_epoch_rows: 1 <= n_lab <= min(n_train, 8192)");
   if (unl_rows ? (n_unl < 1 || n_unl > N || n_unl > PERM_MAX) : (n_unl != 0 || N > PERM_MAX))
     return fail(h, MRGAN_ERR_ARG, "set_epoch_rows: unlabeled subset must have 1..min(n_train, 8192) rows (none: n_train <= 8192)");
   for (int i = 0; i < n_lab; ++i) if ((unsigned)lab_rows[i] >= (unsigned)N) return fail(h, MRGAN_ERR_ARG, "set_epoch_rows: labeled row out of range");
   for (int i = 0; i < n_unl; ++i) if ((unsigned)unl_rows[i] >= (unsigned)N) return fail(h, MRGAN_ERR_ARG, "set_epoch_rows: unlabeled row out of range");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "set_epoch_rows", FOLD | GAN, fold));
   FoldBuffers& b = h->fb[fold];
   CK(cudaMemcpyAsync(b.lab_rows, lab_rows, (size_t)n_lab * sizeof(int), cudaMemcpyHostToDevice, h->stream));
   if (unl_rows) CK(cudaMemcpyAsync(b.unl_rows, unl_rows, (size_t)n_unl * sizeof(int), cudaMemcpyHostToDevice, h->stream));
@@ -1910,82 +1959,65 @@ int mrgan_set_epoch_rows(mrgan_handle* h, int fold, const int32_t* lab_rows, int
   PermDesc pd{b.lab_rows, unl_rows ? b.unl_rows : nullptr, b.idx, n_lab, b.n_unl, N,
               (uint32_t)(h->shapes[fold].seed & 0xFFFFFFFFull), (uint32_t)(h->shapes[fold].seed >> 32)};
   CK(cudaMemcpyAsync(h->d_perm + fold, &pd, sizeof(pd), cudaMemcpyHostToDevice, h->stream));
-  CK(cudaStreamSynchronize(h->stream));     // the pageable row arrays are borrowed only for the call
-  return MRGAN_OK;
+  return complete(h);       // the pageable row arrays are borrowed only for the call
 }
 
 static int launch_epoch(mrgan_handle* h, int nb, mrgan_epoch_stats* stats);
 
 int mrgan_train_epoch_seeded(mrgan_handle* h, uint32_t epoch, mrgan_epoch_stats* stats) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, "train_epoch_seeded needs a GAN handle");
-  for (int f = 0; f < h->nf; ++f) {
-    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "train_epoch_seeded before mrgan_load_fold");
+  TRY(enter(h, "train_epoch_seeded", GAN));
+  TRY(ready(h, "train_epoch_seeded", GAN | LOADED));
+  for (int f = 0; f < h->nf; ++f)
     if (h->fb[f].n_lab < 1) return fail(h, MRGAN_ERR_STATE, "train_epoch_seeded before mrgan_set_epoch_rows");
-  }
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
-  static bool attr_set = false;
-  if (!attr_set) { cudaFuncSetAttribute(k_epoch_perm, cudaFuncAttributeMaxDynamicSharedMemorySize, PERM_MAX * 8); attr_set = true; }
-  k_epoch_perm<<<dim3(3, h->nf), 1024, PERM_MAX * 8, h->stream>>>(h->d_perm, epoch);
-  h->launches++;
+  launch_k(h, k_epoch_perm, dim3(3, h->nf), 1024, PERM_MAX * 8, h->stream, h->d_perm, epoch);
   return launch_epoch(h, h->n_train / h->cfg.batch, stats);
 }
 
 int mrgan_debug_epoch_indices(mrgan_handle* h, int fold, int32_t* dst) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "debug_epoch_indices"); if (rc) return rc;
+  TRY(enter(h, "debug_epoch_indices", FOLD | NETS, fold));
   if (!dst) return fail(h, MRGAN_ERR_ARG, "debug_epoch_indices: null pointer");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "debug_epoch_indices", FOLD | NETS, fold));
   CK(cudaMemcpyAsync(dst, h->fb[fold].idx, (size_t)3 * h->n_train * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  return MRGAN_OK;
+  return complete(h);
 }
 
 int mrgan_train_epoch(mrgan_handle* h, const int32_t* idx_lab, const int32_t* idx_unl, const int32_t* idx_unl2,
                       mrgan_epoch_stats* stats) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, "train_epoch needs a GAN handle");
+  TRY(enter(h, "train_epoch", GAN));
   if (!idx_lab || !idx_unl || !idx_unl2) return fail(h, MRGAN_ERR_ARG, "train_epoch: null index array");
-  for (int f = 0; f < h->nf; ++f)
-    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "train_epoch before mrgan_load_fold");
-  const int nb = h->n_train / h->cfg.batch;
   const size_t tot = (size_t)h->nf * h->n_train;
   for (size_t i = 0; i < tot; ++i)
     if ((unsigned)idx_lab[i] >= (unsigned)h->n_train || (unsigned)idx_unl[i] >= (unsigned)h->n_train ||
         (unsigned)idx_unl2[i] >= (unsigned)h->n_train)
       return fail(h, MRGAN_ERR_ARG, "train_epoch: row index out of range");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "train_epoch", GAN | LOADED));
   const int32_t* streams[3] = {idx_lab, idx_unl, idx_unl2};
-  rc = upload_indices(h, streams, 3, h->n_train); if (rc) return rc;
-  return launch_epoch(h, nb, stats);
+  TRY(upload_indices(h, streams, 3, h->n_train));
+  return launch_epoch(h, h->n_train / h->cfg.batch, stats);
 }
 
 // the epoch itself (index arrays already on their way on the handle's stream): one graph launch.  Data-parallel epochs are
 // captured like the others (NCCL collectives and the fused exchange are stream-ordered graph nodes; one chain, so every
 // rank issues them in the same order).
 static int launch_epoch(mrgan_handle* h, int nb, mrgan_epoch_stats* stats) {
-  const int rc = build_graph(h, nb, nb); if (rc) return rc;
+  TRY(build_graph(h, nb, nb));
   CK(cudaEventRecord(h->ev0, h->stream));
   CK(cudaGraphLaunch(h->graphs[nb], h->stream));
   h->launches += h->graph_nodes[nb];
   CK(cudaEventRecord(h->ev1, h->stream));
   h->epoch_pending = true;
-  { const int sk = take_sticky(h); if (sk) return sk; }
+  TRY(take_sticky(h));
   if (stats) return mrgan_epoch_result(h, stats);
   return MRGAN_OK;
 }
 
 int mrnn_step(mrgan_handle* h, int fold, const float* x, const int32_t* labels, int n, float out[2]) {
-  int rc = check_fold(h, fold); if (rc) return rc;
-  if (h->cfg.model != MRGAN_MODEL_NN) return fail(h, MRGAN_ERR_STATE, "mrnn_step needs an NN handle");
+  TRY(enter(h, "mrnn_step", FOLD | NN, fold));
   if (!x || !labels || !out) return fail(h, MRGAN_ERR_ARG, "mrnn_step: null pointer");
   if (n < 1 || n > h->cfg.batch) return fail(h, MRGAN_ERR_ARG, "mrnn_step: n must be in [1, batch]");
   for (int i = 0; i < n; ++i)
     if (labels[i] < 0 || labels[i] >= h->cfg.n_classes) return fail(h, MRGAN_ERR_ARG, "mrnn_step: label out of range");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "mrnn_step", FOLD | NN, fold));
   FoldBuffers& b = h->fb[fold];
   const int D = h->shapes[fold].D;
   const size_t w = (size_t)D * sizeof(float);
@@ -1993,34 +2025,23 @@ int mrnn_step(mrgan_handle* h, int fold, const float* x, const int32_t* labels, 
   CK(cudaMemcpyAsync(b.stage_y, labels, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
   enqueue_nn_step(h, fold, 1, 0, 1, n);
   CK(cudaMemcpyAsync(h->h_scratch, h->d_step_stats + (size_t)fold * 4, 4 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
+  TRY(complete(h));
   out[0] = h->h_scratch[0]; out[1] = h->h_scratch[1];
   return MRGAN_OK;
 }
 
 int mrnn_train_epoch(mrgan_handle* h, const int32_t* idx, int n_idx, float* loss_acc) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model != MRGAN_MODEL_NN) return fail(h, MRGAN_ERR_STATE, "mrnn_train_epoch needs an NN handle");
+  TRY(enter(h, "mrnn_train_epoch", NN));
   if (!idx || n_idx < h->cfg.batch || n_idx > h->n_train || n_idx % h->cfg.batch)
     return fail(h, MRGAN_ERR_ARG, "mrnn_train_epoch: n_idx must be a multiple of batch in [batch, n_train]");
-  for (int f = 0; f < h->nf; ++f)
-    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "mrnn_train_epoch before mrgan_load_fold");
   for (size_t i = 0; i < (size_t)h->nf * n_idx; ++i)
     if ((unsigned)idx[i] >= (unsigned)h->n_train) return fail(h, MRGAN_ERR_ARG, "mrnn_train_epoch: row index out of range");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
-  const int nb = n_idx / h->cfg.batch;
-  rc = build_graph(h, nb, nb); if (rc) return rc;
+  TRY(ready(h, "mrnn_train_epoch", NN | LOADED));
   const int32_t* streams[1] = {idx};
-  rc = upload_indices(h, streams, 1, n_idx); if (rc) return rc;
-  CK(cudaEventRecord(h->ev0, h->stream));
-  CK(cudaGraphLaunch(h->graphs[nb], h->stream));
-  CK(cudaEventRecord(h->ev1, h->stream));
-  h->launches += h->graph_nodes[nb];
-  h->epoch_pending = true;
+  TRY(upload_indices(h, streams, 1, n_idx));
+  TRY(launch_epoch(h, n_idx / h->cfg.batch, nullptr));
   if (loss_acc) {
-    rc = finish_pending(h); if (rc) return rc;
+    TRY(finish_pending(h));
     CKS();
     for (int f = 0; f < h->nf; ++f) { loss_acc[2 * f] = h->h_epoch_stats[f * 8]; loss_acc[2 * f + 1] = h->h_epoch_stats[f * 8 + 1]; }
   }
@@ -2028,85 +2049,68 @@ int mrnn_train_epoch(mrgan_handle* h, const int32_t* idx, int n_idx, float* loss
 }
 
 int mrnn_evaluate(mrgan_handle* h, int fold, float out[2]) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "evaluate"); if (rc) return rc;
+  TRY(enter(h, "evaluate", FOLD | NETS, fold));
   if (!out) return fail(h, MRGAN_ERR_ARG, "evaluate: null pointer");
-  if (!h->fb[fold].loaded) return fail(h, MRGAN_ERR_STATE, "evaluate before mrgan_load_fold");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "evaluate", FOLD | NETS | LOADED, fold));
   enqueue_eval(h, fold, 1, false, 0);
   CK(cudaMemcpyAsync(h->h_scratch, h->fb[fold].eval_out, 4 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
+  TRY(complete(h));
   out[0] = h->h_scratch[2]; out[1] = 1.0f - h->h_scratch[1];
   return MRGAN_OK;
 }
 
 int mrgan_fill_normal(mrgan_handle* h, int fold, int step, int tensor_id, int rows, int cols, int row0, float* dst) {
-  int rc = check_fold(h, fold); if (rc) return rc; rc = need_nets(h, "fill_normal"); if (rc) return rc;
+  TRY(enter(h, "fill_normal", FOLD | NETS, fold));
   if (!dst || rows < 1 || cols < 1) return fail(h, MRGAN_ERR_ARG, "fill_normal: bad argument");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "fill_normal", FOLD | NETS, fold));
+  Temps tmp;
   float* d = nullptr;
   const size_t n = (size_t)rows * cols;
-  CK(cudaMalloc(&d, n * sizeof(float)));
-  k_fill_normal<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(d, h->d_folds, fold, step, tensor_id, rows, cols, row0);
-  h->launches++;
-  cudaError_t e = cudaMemcpyAsync(dst, d, n * sizeof(float), cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  cudaFree(d);
-  if (e != cudaSuccess) return fail(h, MRGAN_ERR_CUDA, cudaGetErrorString(e));
-  return MRGAN_OK;
+  CK(tmp.alloc(&d, n * sizeof(float)));
+  launch_k(h, k_fill_normal, (unsigned)((n + 255) / 256), 256, 0, h->stream, d, h->d_folds, fold, step, tensor_id, rows, cols, row0);
+  CK(cudaMemcpyAsync(dst, d, n * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  return complete(h);
 }
 
 int mrgan_adam_flat(mrgan_handle* h, float* p, float* m, float* v, const float* g, int64_t n, int t) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  { const int rc0 = need_nets(h, "adam_flat"); if (rc0) return rc0; }
+  TRY(enter(h, "adam_flat", NETS));
   if (!p || !m || !v || !g || n < 1 || t < 1) return fail(h, MRGAN_ERR_ARG, "adam_flat: bad argument");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "adam_flat", NETS));
   const int64_t n4 = (n + 3) / 4;
+  Temps tmp;
   float* d = nullptr;
-  CK(cudaMalloc(&d, (size_t)n4 * 16 * 4));
+  CK(tmp.alloc(&d, (size_t)n4 * 16 * 4));
   CK(cudaMemsetAsync(d, 0, (size_t)n4 * 16 * 4, h->stream));
   float *dp = d, *dm = d + n4 * 4, *dv = d + n4 * 8, *dg = d + n4 * 12;
-  cudaMemcpyAsync(dp, p, n * 4, cudaMemcpyHostToDevice, h->stream);
-  cudaMemcpyAsync(dm, m, n * 4, cudaMemcpyHostToDevice, h->stream);
-  cudaMemcpyAsync(dv, v, n * 4, cudaMemcpyHostToDevice, h->stream);
-  cudaMemcpyAsync(dg, g, n * 4, cudaMemcpyHostToDevice, h->stream);
+  CK(cudaMemcpyAsync(dp, p, n * 4, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(dm, m, n * 4, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(dv, v, n * 4, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(dg, g, n * 4, cudaMemcpyHostToDevice, h->stream));
   const double b1t = pow((double)h->hp.b1, (double)t), b2t = pow((double)h->hp.b2, (double)t);
   const float lr_t = (float)((double)h->hp.lr * sqrt(1.0 - b2t) / (1.0 - b1t));
   int blocks = (int)((n4 + 255) / 256); if (blocks > 4096) blocks = 4096;
-  k_adam_plain<<<blocks, 256, 0, h->stream>>>((float4*)dp, (float4*)dm, (float4*)dv, (const float4*)dg, n4, lr_t,
-                                              h->hp.b1, h->hp.b2, h->hp.eps);
-  h->launches++;
-  cudaMemcpyAsync(p, dp, n * 4, cudaMemcpyDeviceToHost, h->stream);
-  cudaMemcpyAsync(m, dm, n * 4, cudaMemcpyDeviceToHost, h->stream);
-  cudaError_t e = cudaMemcpyAsync(v, dv, n * 4, cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  if (e == cudaSuccess) e = cudaGetLastError();
-  cudaFree(d);
-  if (e != cudaSuccess) return fail(h, MRGAN_ERR_CUDA, cudaGetErrorString(e));
-  return MRGAN_OK;
+  launch_k(h, k_adam_plain, blocks, 256, 0, h->stream, (float4*)dp, (float4*)dm, (float4*)dv, (const float4*)dg, n4, lr_t,
+           h->hp.b1, h->hp.b2, h->hp.eps);
+  CK(cudaMemcpyAsync(p, dp, n * 4, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(m, dm, n * 4, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(v, dv, n * 4, cudaMemcpyDeviceToHost, h->stream));
+  return complete(h);
 }
 
-static int svm_time_op(mrgan_handle* h, int which, int reps, float* ms_avg);
+static void svm_launch(mrgan_handle* h, int phase);
 
 int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  TRY(enter(h, "time_op", 0));
   if (!ms_avg || reps < 1) return fail(h, MRGAN_ERR_ARG, "time_op: bad argument");
-  const bool svm = h->cfg.model == MRGAN_MODEL_SVM;
+  const bool svm = h->cfg.model == MRGAN_MODEL_SVM, gan = h->cfg.model == MRGAN_MODEL_GAN;
   if (svm != (which >= MRGAN_TIME_SVM_KMAT && which <= MRGAN_TIME_SVM_PREDICT))
     return fail(h, which < 0 || which > MRGAN_TIME_SALIENCY ? MRGAN_ERR_ARG : MRGAN_ERR_STATE, "time_op: op does not exist for this model");
-  if (svm) return svm_time_op(h, which, reps, ms_avg);
-  const bool gan = h->cfg.model == MRGAN_MODEL_GAN;
+  if (which < 0 || which > MRGAN_TIME_SALIENCY) return fail(h, MRGAN_ERR_ARG, "time_op: unknown op");
   if (!gan && (which == MRGAN_TIME_ADAM_G || which == MRGAN_TIME_GEN_STEP || which == MRGAN_TIME_DX1)) return fail(h, MRGAN_ERR_STATE, "time_op: no generator in this model");
-  for (int f = 0; f < h->nf; ++f)
-    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "time_op before mrgan_load_fold");
-  if (which == MRGAN_TIME_SALIENCY) { const int rc0 = need_local(h, "time_op"); if (rc0) return rc0; }
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
-  if (which == MRGAN_TIME_SALIENCY) { rc = saliency_setup(h); if (rc) return rc; }
-  auto once = [&]() {
+  TRY(ready(h, "time_op", svm ? FITTED : (LOADED | (which == MRGAN_TIME_SALIENCY ? LOCAL : 0u))));
+  if (svm) return time_reps(h, reps, [&]() { svm_launch(h, which); }, ms_avg);
+  if (which == MRGAN_TIME_SALIENCY) TRY(saliency_setup(h));
+  return time_reps(h, reps, [&]() {
     switch (which) {
       case MRGAN_TIME_ADAM_D: launch_adam(h, 0, h->nf, 0); break;
       case MRGAN_TIME_ADAM_G: launch_adam(h, 0, h->nf, 1); break;
@@ -2118,18 +2122,7 @@ int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
       case MRGAN_TIME_SALIENCY: enqueue_saliency(h); break;
       default: break;
     }
-  };
-  if (which < 0 || (which > MRGAN_TIME_DX1 && which != MRGAN_TIME_SALIENCY)) return fail(h, MRGAN_ERR_ARG, "time_op: unknown op");
-  once();                                   // warm-up
-  CK(cudaEventRecord(h->ev0, h->stream));
-  for (int i = 0; i < reps; ++i) once();
-  CK(cudaEventRecord(h->ev1, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
-  float ms = 0.f;
-  CK(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-  *ms_avg = ms / reps;
-  return MRGAN_OK;
+  }, ms_avg);
 }
 
 int mrgan_nccl_unique_id(void* id128) {
@@ -2143,36 +2136,24 @@ int mrgan_nccl_unique_id(void* id128) {
 }
 
 int mrgan_dp_init(mrgan_handle* h, int rank, int world, const void* id128) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  TRY(enter(h, "dp_init", GAN));
   if (world < 1 || rank < 0 || rank >= world || !id128) return fail(h, MRGAN_ERR_ARG, "dp_init: bad rank / world / id");
   if (world > DP_MAX_RANKS) return fail(h, MRGAN_ERR_ARG, "dp_init: at most 8 ranks (one NVSwitch domain)");
-  if (h->cfg.model != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, "dp_init: data-parallel mode is implemented for the GAN model");
   if (h->dp_world > 1 || h->nccl_comm) return fail(h, MRGAN_ERR_STATE, "dp_init called twice");
   if (world == 1) return MRGAN_OK;
   if (h->cfg.batch % 4) return fail(h, MRGAN_ERR_ARG, "dp_init: the local batch must be a multiple of 4 (noise row groups)");
   if (!nccl_load()) return fail(h, MRGAN_ERR_STATE, "libnccl.so.2 not found");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "dp_init", GAN));
   NcclId id; memcpy(id.b, id128, 128);
   const int nrc = g_nccl.CommInitRank(&h->nccl_comm, world, id, rank);
   if (nrc != 0) return fail(h, MRGAN_ERR_CUDA, std::string("ncclCommInitRank: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(nrc) : "error"));
-  rc = alloc_split_bufs(h); if (rc) return rc;
-  h->dp_world = world; h->dp_rank = rank;
-  h->hp.dp_bloc = h->cfg.batch; h->hp.dp_bg = h->cfg.batch * world; h->hp.dp_rank = rank;
-  if (h->cfg.precision != MRGAN_PREC_FP32) {   // gradients must be all-reduced before Adam: dW stores them, k_adam applies
-    tc_teardown(h);
-    h->tc_fused_adam = false;
-    rc = tc_setup(h); if (rc) return rc;
-  }
-  for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
-  h->graphs.clear(); h->graph_nodes.clear();
-  CK(cudaDeviceSynchronize());
-  return MRGAN_OK;
+  return dp_switch(h, world, rank);
 }
 
 int mrgan_dp_ipc_export(mrgan_handle* h, void* out128) {
-  if (!h || !out128) return fail(h, MRGAN_ERR_ARG, "dp_ipc_export: null argument");
-  CK(cudaSetDevice(h->cfg.device));
+  TRY(enter(h, "dp_ipc_export", 0));
+  if (!out128) return fail(h, MRGAN_ERR_ARG, "dp_ipc_export: null argument");
+  TRY(ready(h, "dp_ipc_export", 0));
   memset(out128, 0, 128);
   cudaIpcMemHandle_t a;
   CK(cudaIpcGetMemHandle(&a, h->arena));
@@ -2185,11 +2166,11 @@ int mrgan_dp_ipc_export(mrgan_handle* h, void* out128) {
 }
 
 int mrgan_dp_ipc_open(mrgan_handle* h, const void* handles, int world) {
-  if (!h || !handles) return fail(h, MRGAN_ERR_ARG, "dp_ipc_open: null argument");
+  TRY(enter(h, "dp_ipc_open", 0));
+  if (!handles) return fail(h, MRGAN_ERR_ARG, "dp_ipc_open: null argument");
   if (h->dp_world != world || world < 2 || world > DP_MAX_RANKS || h->dp_virtual)
     return fail(h, MRGAN_ERR_STATE, "dp_ipc_open: call after mrgan_dp_init with the same world size (at most 8 ranks)");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "dp_ipc_open", 0));
   const char* hb = static_cast<const char*>(handles);
   for (int p = 0; p < world; ++p) {
     if (p == h->dp_rank) { h->peer_arena[p] = h->arena; h->peer_harena[p] = h->harena; continue; }
@@ -2206,44 +2187,30 @@ int mrgan_dp_ipc_open(mrgan_handle* h, const void* handles, int world) {
   }
   h->dp_fused = true;
   dp_build_peers(h);
-  for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
-  h->graphs.clear(); h->graph_nodes.clear();
+  drop_graphs(h);
   return MRGAN_OK;
 }
 
 int mrgan_dp_init_virtual(mrgan_handle* h, int world) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model != MRGAN_MODEL_GAN) return fail(h, MRGAN_ERR_STATE, "dp_init_virtual: data-parallel mode is implemented for the GAN model");
+  TRY(enter(h, "dp_init_virtual", GAN));
   if (h->dp_world > 1 || h->nccl_comm) return fail(h, MRGAN_ERR_STATE, "dp_init called twice");
   if (world < 2 || world != h->nf) return fail(h, MRGAN_ERR_ARG, "dp_init_virtual: the handle must hold exactly `world` folds (one per virtual rank)");
+  if (world > DP_MAX_RANKS) return fail(h, MRGAN_ERR_ARG, "dp_init_virtual: at most 8 ranks");
   if (h->cfg.batch % 4) return fail(h, MRGAN_ERR_ARG, "dp_init_virtual: the local batch must be a multiple of 4 (noise row groups)");
   for (int f = 1; f < h->nf; ++f)
     if (h->shapes[f].D != h->shapes[0].D || h->shapes[f].seed != h->shapes[0].seed)
       return fail(h, MRGAN_ERR_ARG, "dp_init_virtual: virtual ranks are replicas: same input width and noise key");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
-  rc = alloc_split_bufs(h); if (rc) return rc;
-  if (world > DP_MAX_RANKS) return fail(h, MRGAN_ERR_ARG, "dp_init_virtual: at most 8 ranks");
-  h->dp_world = world; h->dp_rank = 0; h->dp_virtual = true;
-  h->hp.dp_bloc = h->cfg.batch; h->hp.dp_bg = h->cfg.batch * world; h->hp.dp_rank = -1;     // -1: rank = fold index (common.cuh)
+  TRY(ready(h, "dp_init_virtual", GAN));
+  TRY(dp_switch(h, world, -1));
   h->dp_fused = true;
   dp_build_peers(h);
-  if (h->cfg.precision != MRGAN_PREC_FP32) {   // gradients must be all-reduced before Adam: dW stores them, k_adam applies
-    tc_teardown(h);
-    h->tc_fused_adam = false;
-    rc = tc_setup(h); if (rc) return rc;
-  }
-  for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
-  h->graphs.clear(); h->graph_nodes.clear();
-  CK(cudaDeviceSynchronize());
   return MRGAN_OK;
 }
 
 int mrgan_debug_buffer(mrgan_handle* h, int fold, int which, float* dst, int rows, int cols) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  TRY(enter(h, "debug_buffer", FOLD, fold));
   if (!dst || rows < 1 || cols < 1) return fail(h, MRGAN_ERR_ARG, "debug_buffer: bad argument");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "debug_buffer", FOLD, fold));
   const FoldBuffers& b = h->fb[fold];
   const int K = h->cfg.n_classes, D = h->shapes[fold].D, nd = h->cfg.noise_dim;
   const bool gan = h->cfg.model == MRGAN_MODEL_GAN;
@@ -2272,96 +2239,84 @@ int mrgan_debug_buffer(mrgan_handle* h, int fold, int which, float* dst, int row
   else if (gan && which == 45) { src = b.du; ld = pitch8(kGH); }
   else if (gan && which == 46) { src = b.dz1g; ld = pitch8(kGH); }
   if (!src || cols > ld) return fail(h, MRGAN_ERR_ARG, "debug_buffer: unknown buffer or too many columns");
-  float* tmp = nullptr;
+  Temps tmp;
   if (h->om.mode == 2) {
     // f16 mode: noisy activations / inputs and every dZ exist only as fp16 operand copies (dZ times the loss scale)
     const bool act_only = (which >= 0 && which <= 4) || which == 40 || which == 42;
     const bool grad_only = (which >= 21 && which <= 25) || which == 31 || which == 32 || which == 44 || which == 46;
+    float* t = nullptr;
     if (act_only || grad_only) {
-      CK(cudaMalloc(&tmp, (size_t)rows * ld * sizeof(float)));
-      k_from_half<<<256, 256, 0, h->stream>>>(src, tmp, (size_t)rows * ld, grad_only ? 1.0f / h->om.gscale : 1.0f, h->om);
-      src = tmp;
+      CK(tmp.alloc(&t, (size_t)rows * ld * sizeof(float)));
+      launch_k(h, k_from_half, 256, 256, 0, h->stream, src, t, (size_t)rows * ld, grad_only ? 1.0f / h->om.gscale : 1.0f, h->om);
+      src = t;
     } else if (which == 45) {   // du stays fp32 but carries the loss scale
-      CK(cudaMalloc(&tmp, (size_t)rows * ld * sizeof(float)));
-      CK(cudaMemcpyAsync(tmp, src, (size_t)rows * ld * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
-      k_scale_buf<<<256, 256, 0, h->stream>>>(tmp, (size_t)rows * ld, 1.0f / h->om.gscale);
-      src = tmp;
+      CK(tmp.alloc(&t, (size_t)rows * ld * sizeof(float)));
+      CK(cudaMemcpyAsync(t, src, (size_t)rows * ld * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
+      launch_k(h, k_scale_buf, 256, 256, 0, h->stream, t, (size_t)rows * ld, 1.0f / h->om.gscale);
+      src = t;
     }
   }
-  cudaError_t ce = cudaMemcpy2DAsync(dst, (size_t)cols * sizeof(float), src, (size_t)ld * sizeof(float), (size_t)cols * sizeof(float), rows,
-                                     cudaMemcpyDeviceToHost, h->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(h->stream);
-  if (tmp) cudaFree(tmp);
-  if (ce != cudaSuccess) return fail(h, MRGAN_ERR_CUDA, std::string("debug_buffer: ") + cudaGetErrorString(ce));
-  return MRGAN_OK;
+  CK(cudaMemcpy2DAsync(dst, (size_t)cols * sizeof(float), src, (size_t)ld * sizeof(float), (size_t)cols * sizeof(float), rows,
+                       cudaMemcpyDeviceToHost, h->stream));
+  return complete(h);
 }
 
 int mrgan_debug_gemm(mrgan_handle* h, int mode, int M, int N, int K, const float* A, const float* B, float* C, int use_tc) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  { const int rc0 = need_nets(h, "debug_gemm"); if (rc0) return rc0; }
+  TRY(enter(h, "debug_gemm", NETS));
   if (mode < 0 || mode > 2 || M < 1 || N < 1 || K < 1 || !A || !B || !C) return fail(h, MRGAN_ERR_ARG, "debug_gemm: bad argument");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "debug_gemm", NETS));
   // operand shapes (rows, cols) as stored
   const int ar = mode == 2 ? K : M, ac = mode == 2 ? M : K;
   const int br = mode == 1 ? N : K, bc = mode == 1 ? K : N;
   const int lda = pitch8(ac), ldb = pitch8(bc), ldc = pitch8(N);
+  Temps tmp;
   float *dA = nullptr, *dB = nullptr, *dC = nullptr; GemmDesc* dd = nullptr;
-  CK(cudaMalloc(&dA, (size_t)ar * lda * 4)); CK(cudaMalloc(&dB, (size_t)br * ldb * 4)); CK(cudaMalloc(&dC, (size_t)M * ldc * 4));
-  CK(cudaMalloc(&dd, sizeof(GemmDesc)));
+  CK(tmp.alloc(&dA, (size_t)ar * lda * 4)); CK(tmp.alloc(&dB, (size_t)br * ldb * 4)); CK(tmp.alloc(&dC, (size_t)M * ldc * 4));
+  CK(tmp.alloc(&dd, sizeof(GemmDesc)));
   CK(cudaMemsetAsync(dA, 0, (size_t)ar * lda * 4, h->stream)); CK(cudaMemsetAsync(dB, 0, (size_t)br * ldb * 4, h->stream));
   CK(cudaMemsetAsync(dC, 0, (size_t)M * ldc * 4, h->stream));
   CK(cudaMemcpy2DAsync(dA, (size_t)lda * 4, A, (size_t)ac * 4, (size_t)ac * 4, ar, cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpy2DAsync(dB, (size_t)ldb * 4, B, (size_t)bc * 4, (size_t)bc * 4, br, cudaMemcpyHostToDevice, h->stream));
   GemmDesc g = make_desc(dA, lda, dB, ldb, dC, ldc, M, N, K, mode == 0 ? EPI_FWD : (mode == 1 ? EPI_DX : EPI_STORE), ACT_NONE, 0);
   CK(cudaMemcpyAsync(dd, &g, sizeof(g), cudaMemcpyHostToDevice, h->stream));
-  __half *hA = nullptr, *hB = nullptr;
   if (use_tc == 2) {          // fp16 operand copies (kind::f16): host conversion, pitch rounded to 8 elements (16-byte TMA strides)
     const int lha = (ac + 7) & ~7, lhb = (bc + 7) & ~7;
     std::vector<__half> ha((size_t)ar * lha, __float2half(0.f)), hb((size_t)br * lhb, __float2half(0.f));
     for (int r = 0; r < ar; ++r) for (int c2 = 0; c2 < ac; ++c2) ha[(size_t)r * lha + c2] = __float2half_rn(A[(size_t)r * ac + c2]);
     for (int r = 0; r < br; ++r) for (int c2 = 0; c2 < bc; ++c2) hb[(size_t)r * lhb + c2] = __float2half_rn(B[(size_t)r * bc + c2]);
-    CK(cudaMalloc(&hA, ha.size() * sizeof(__half))); CK(cudaMalloc(&hB, hb.size() * sizeof(__half)));
+    __half *hA = nullptr, *hB = nullptr;
+    CK(tmp.alloc(&hA, ha.size() * sizeof(__half))); CK(tmp.alloc(&hB, hb.size() * sizeof(__half)));
     CK(cudaMemcpy(hA, ha.data(), ha.size() * sizeof(__half), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(hB, hb.data(), hb.size() * sizeof(__half), cudaMemcpyHostToDevice));
     GemmDesc gh = g;
     gh.A = reinterpret_cast<const float*>(hA); gh.lda = lha; gh.B = reinterpret_cast<const float*>(hB); gh.ldb = lhb;
-    rc = tc_debug_gemm(h, mode, gh, 2);
-    cudaFree(hA); cudaFree(hB);
-    if (rc) return rc;
+    TRY(tc_debug_gemm(h, mode, gh, 2));
   } else if (use_tc) {
-    rc = tc_debug_gemm(h, mode, g, 4);
-    if (rc) return rc;
+    TRY(tc_debug_gemm(h, mode, g, 4));
   } else {
-    dim3 grid((N + 63) / 64, (M + 63) / 64, 1);
-    if (mode == 0) k_gemm_simt<false, false><<<grid, 256, 0, h->stream>>>(dd, h->d_folds, 0, h->hp);
-    else if (mode == 1) k_gemm_simt<false, true><<<grid, 256, 0, h->stream>>>(dd, h->d_folds, 0, h->hp);
-    else k_gemm_simt<true, false><<<grid, 256, 0, h->stream>>>(dd, h->d_folds, 0, h->hp);
-    h->launches++;
+    const dim3 grid((N + 63) / 64, (M + 63) / 64, 1);
+    if (mode == 0) launch_k(h, k_gemm_simt<false, false>, grid, 256, 0, h->stream, dd, h->d_folds, 0, h->hp);
+    else if (mode == 1) launch_k(h, k_gemm_simt<false, true>, grid, 256, 0, h->stream, dd, h->d_folds, 0, h->hp);
+    else launch_k(h, k_gemm_simt<true, false>, grid, 256, 0, h->stream, dd, h->d_folds, 0, h->hp);
   }
-  cudaError_t e = cudaMemcpy2DAsync(C, (size_t)N * 4, dC, (size_t)ldc * 4, (size_t)N * 4, M, cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  if (e == cudaSuccess) e = cudaGetLastError();
-  cudaFree(dA); cudaFree(dB); cudaFree(dC); cudaFree(dd);
-  if (e != cudaSuccess) return fail(h, MRGAN_ERR_CUDA, std::string("debug_gemm: ") + cudaGetErrorString(e));
-  return MRGAN_OK;
+  CK(cudaMemcpy2DAsync(C, (size_t)N * 4, dC, (size_t)ldc * 4, (size_t)N * 4, M, cudaMemcpyDeviceToHost, h->stream));
+  return complete(h);
 }
 
 int mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int groups, int reps, float* ms) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  { const int rc0 = need_nets(h, "debug_gemm_time"); if (rc0) return rc0; }
+  TRY(enter(h, "debug_gemm_time", NETS));
   if (mode < 0 || mode > 2 || M < 1 || N < 1 || K < 1 || groups < 1 || reps < 1 || !ms) return fail(h, MRGAN_ERR_ARG, "debug_gemm_time: bad argument");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
+  TRY(ready(h, "debug_gemm_time", NETS));
+  EncodeTiledFn fn = tc_encoder();
+  if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available");
   const int ar = mode == 2 ? K : M, ac = mode == 2 ? M : K;
   const int br = mode == 1 ? N : K, bc = mode == 1 ? K : N;
   const int lda = pitch8(ac), ldb = pitch8(bc), ldc = pitch8(N);
   const size_t sa = (size_t)ar * lda, sb = (size_t)br * ldb, sc = (size_t)M * ldc;
+  Temps tmp;
   float* buf = nullptr;
-  CK(cudaMalloc(&buf, (sa + sb + sc) * groups * 4));
+  CK(tmp.alloc(&buf, (sa + sb + sc) * groups * 4));
   CK(cudaMemsetAsync(buf, 0, (sa + sb + sc) * groups * 4, h->stream));
-  EncodeTiledFn fn = tc_encoder();
-  if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available");
   std::vector<TcOp> ops(groups);
   memset(ops.data(), 0, sizeof(TcOp) * groups);
   for (int g = 0; g < groups; ++g) {
@@ -2370,29 +2325,17 @@ int mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int gr
     if (!tc_fill_op(fn, ops[g], d, mode)) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
   }
   TcOp* dops = nullptr;
-  CK(cudaMalloc(&dops, sizeof(TcOp) * groups));
+  CK(tmp.alloc(&dops, sizeof(TcOp) * groups));
   CK(cudaMemcpyAsync(dops, ops.data(), sizeof(TcOp) * groups, cudaMemcpyHostToDevice, h->stream));
   tc_set_smem_attr();
   const TcOp& t = ops[0];
-  dim3 grid((t.ME + 127) / 128, (t.NE + t.bn - 1) / t.bn, groups);
-  auto once = [&]() {
-    const OperandMode om0{0, 1.0f, nullptr, nullptr};
-    if (mode == 0) K_TC_FWD(false, false)<<<grid, TC_FWD_THREADS, tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream>>>(dops, h->d_folds, 0, h->hp, om0);
-    else if (mode == 1) K_TC_DX(false, false)<<<grid, TC_FWD_THREADS, tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream>>>(dops, h->d_folds, 0, h->hp, om0);
-    else K_TC_DW(false, false)<<<grid, TC_DW_THREADS, tc_smem_bytes(t.bn, TC_DW_STAGES), h->stream>>>(dops, h->d_folds, 0, h->hp, om0);
-  };
-  once();
-  CK(cudaEventRecord(h->ev0, h->stream));
-  for (int i = 0; i < reps; ++i) once();
-  CK(cudaEventRecord(h->ev1, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
-  float t_ms = 0.f;
-  CK(cudaEventElapsedTime(&t_ms, h->ev0, h->ev1));
-  *ms = t_ms / reps;
-  h->launches += reps + 1;
-  cudaFree(buf); cudaFree(dops);
-  return MRGAN_OK;
+  const dim3 grid((t.ME + 127) / 128, (t.NE + t.bn - 1) / t.bn, groups);
+  const OperandMode om0{0, 1.0f, nullptr, nullptr};
+  return time_reps(h, reps, [&]() {
+    if (mode == 0) launch_k(h, K_TC_FWD(false, false), grid, TC_FWD_THREADS, tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream, dops, h->d_folds, 0, h->hp, om0);
+    else if (mode == 1) launch_k(h, K_TC_DX(false, false), grid, TC_FWD_THREADS, tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream, dops, h->d_folds, 0, h->hp, om0);
+    else launch_k(h, K_TC_DW(false, false), grid, TC_DW_THREADS, tc_smem_bytes(t.bn, TC_DW_STAGES), h->stream, dops, h->d_folds, 0, h->hp, om0);
+  }, ms);
 }
 
 
@@ -2401,18 +2344,15 @@ static void svm_launch(mrgan_handle* h, int phase) {
   mrgan_handle::Svm& S = h->svm;
   const int nf = h->nf;
   if (phase == MRGAN_TIME_SVM_KMAT) {
-    k_svm_split<<<dim3((S.max_rows + 7) / 8, 2 * nf), 256, 0, h->stream>>>(S.d_split);
-    k_svm_kmat<<<dim3((S.n_lab + SVM_BM - 1) / SVM_BM, (S.max_rows + SVM_BN - 1) / SVM_BN, 2 * nf), SVM_KMAT_THREADS, SVM_KMAT_SMEM,
-                 h->stream>>>(S.d_gemm);
-    h->launches += 2;
+    launch_k(h, k_svm_split, dim3((S.max_rows + 7) / 8, 2 * nf), 256, 0, h->stream, S.d_split);
+    launch_k(h, k_svm_kmat, dim3((S.n_lab + SVM_BM - 1) / SVM_BM, (S.max_rows + SVM_BN - 1) / SVM_BN, 2 * nf), SVM_KMAT_THREADS,
+             SVM_KMAT_SMEM, h->stream, S.d_gemm);
   } else if (phase == MRGAN_TIME_SVM_SMO) {
-    k_svm_smo<<<nf * S.npairs, SVM_SMO_THREADS, (size_t)SVM_SMO_SMEM_PER_ROW * S.npmax, h->stream>>>(S.d_jobs, S.eps);
-    h->launches += 1;
+    launch_k(h, k_svm_smo, nf * S.npairs, SVM_SMO_THREADS, (size_t)SVM_SMO_SMEM_PER_ROW * S.npmax, h->stream, S.d_jobs, S.eps);
   } else {
-    k_svm_vote<<<dim3(S.max_nte, nf), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs, S.npairs, h->cfg.n_classes, S.d_Kt, nullptr, S.d_yte,
-                                                                         S.d_nte, S.d_dec, S.d_wrong, S.d_pred);
-    k_svm_count<<<nf, 256, 0, h->stream>>>(S.d_wrong, S.d_nte, S.d_count);
-    h->launches += 2;
+    launch_k(h, k_svm_vote, dim3(S.max_nte, nf), SVM_VOTE_THREADS, 0, h->stream, S.d_jobs, S.npairs, h->cfg.n_classes, S.d_Kt, nullptr,
+             S.d_yte, S.d_nte, S.d_dec, S.d_wrong, S.d_pred);
+    launch_k(h, k_svm_count, nf, 256, 0, h->stream, S.d_wrong, S.d_nte, S.d_count);
   }
 }
 
@@ -2422,15 +2362,11 @@ struct SvmLabels {
   int npmax = 0;                      // rows of the largest class pair
 };
 
-// Checks the labeled rows of every fold (loaded, in range, class-major, every class present, class pairs within SVM_MAX_PAIR)
+// Checks the labeled rows of every loaded fold (in range, class-major, every class present, class pairs within SVM_MAX_PAIR)
 // and reads their labels.  Changes no SVM state.  The caller has checked the scalars.
 static int svm_labels(mrgan_handle* h, const char* fn, const int32_t* lab_rows, int n_lab, SvmLabels& L) {
   const std::string pre = std::string(fn) + ": ";
   const int nf = h->nf, K = h->cfg.n_classes;
-  for (int f = 0; f < nf; ++f)
-    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, pre + "the fold data is not loaded (mrgan_load_fold / mrgan_prepare_fold)");
-  CK(cudaSetDevice(h->cfg.device));
-  int rc = finish_pending(h); if (rc) return rc;
   std::vector<int> ytr(h->n_train);
   std::vector<int>& ylab = L.ylab;
   std::vector<int>& start = L.start;
@@ -2580,15 +2516,15 @@ static bool all_positive(const float* v, size_t n) {
 }
 
 int mrgan_svm_fit_folds(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const float* C, const float* gamma, float tol, int32_t* n_iter) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_fit needs an SVM handle");
+  TRY(enter(h, "svm_fit", SVM));
   if (!lab_rows || !C || !gamma || n_lab < 2 || !(tol > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_fit: bad argument");
   const int nf = h->nf, npairs = h->cfg.n_classes * (h->cfg.n_classes - 1) / 2;
   if (!all_positive(C, nf)) return fail(h, MRGAN_ERR_ARG, "svm_fit: C must be positive");
   if (!all_positive(gamma, nf)) return fail(h, MRGAN_ERR_ARG, "svm_fit: gamma must be positive");
+  TRY(ready(h, "svm_fit", SVM | LOADED));
   SvmLabels L;
-  int rc = svm_labels(h, "svm_fit", lab_rows, n_lab, L); if (rc) return rc;
-  rc = svm_setup(h, lab_rows, n_lab, L, C, gamma, tol); if (rc) return rc;
+  TRY(svm_labels(h, "svm_fit", lab_rows, n_lab, L));
+  TRY(svm_setup(h, lab_rows, n_lab, L, C, gamma, tol));
   mrgan_handle::Svm& S = h->svm;
   svm_launch(h, MRGAN_TIME_SVM_KMAT);
   svm_launch(h, MRGAN_TIME_SVM_SMO);
@@ -2596,8 +2532,7 @@ int mrgan_svm_fit_folds(mrgan_handle* h, const int32_t* lab_rows, int n_lab, con
   std::vector<int> it((size_t)nf * npairs), cap((size_t)nf * npairs);
   CK(cudaMemcpyAsync(it.data(), S.d_iters, sizeof(int) * it.size(), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaMemcpyAsync(cap.data(), S.d_capped, sizeof(int) * cap.size(), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CK(cudaGetLastError());
+  TRY(complete(h));
   if (n_iter) memcpy(n_iter, it.data(), sizeof(int) * it.size());
   S.fitted = true;
   for (size_t q = 0; q < cap.size(); ++q)
@@ -2607,7 +2542,7 @@ int mrgan_svm_fit_folds(mrgan_handle* h, const int32_t* lab_rows, int n_lab, con
 }
 
 int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, const float* gamma, float tol, int32_t* n_iter) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  TRY(enter(h, "svm_fit", 0));
   std::vector<float> Cf(h->nf, C);
   return mrgan_svm_fit_folds(h, lab_rows, n_lab, Cf.data(), gamma, tol, n_iter);
 }
@@ -2618,8 +2553,7 @@ int mrgan_svm_fit(mrgan_handle* h, const int32_t* lab_rows, int n_lab, float C, 
 // matrix and counted.
 int mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int32_t* split, int n_splits, const float* C, int nC,
                  const float* gamma, int nG, float tol, int32_t* wrong) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
-  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_cv needs an SVM handle");
+  TRY(enter(h, "svm_cv", SVM));
   if (!lab_rows || !split || !C || !gamma || !wrong || n_lab < 2 || !(tol > 0.0f)) return fail(h, MRGAN_ERR_ARG, "svm_cv: bad argument");
   if (n_splits < 2 || nC < 1 || nG < 1) return fail(h, MRGAN_ERR_ARG, "svm_cv: need n_splits >= 2, nC >= 1 and nG >= 1");
   const int nf = h->nf, K = h->cfg.n_classes, npairs = K * (K - 1) / 2, ns = n_splits;
@@ -2629,8 +2563,9 @@ int mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int3
     if (split[r] < 0 || split[r] >= ns) return fail(h, MRGAN_ERR_ARG, "svm_cv: split index outside [0, n_splits)");
   std::vector<float> g0(nf), C0(nf, C[0]);
   for (int f = 0; f < nf; ++f) g0[f] = gamma[(size_t)f * nG];
+  TRY(ready(h, "svm_cv", SVM | LOADED));
   SvmLabels L;
-  int rc = svm_labels(h, "svm_cv", lab_rows, n_lab, L); if (rc) return rc;
+  TRY(svm_labels(h, "svm_cv", lab_rows, n_lab, L));
   const std::vector<int>& ylab = L.ylab;
   // the problems: validation rows of (f, s) and the inner-training rows of (f, s, pair), in the labeled order; a rejected
   // split leaves the previous fit valid
@@ -2667,7 +2602,7 @@ int mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int3
         }
     }
   }
-  rc = svm_setup(h, lab_rows, n_lab, L, C0.data(), g0.data(), tol); if (rc) return rc;
+  TRY(svm_setup(h, lab_rows, n_lab, L, C0.data(), g0.data(), tol));
   mrgan_handle::Svm& S = h->svm;
   // second allocation: kept while large enough, freed by mrgan_destroy
   int *d_maps = nullptr, *d_vrows = nullptr, *d_vy = nullptr, *d_nval = nullptr, *d_flags = nullptr, *d_count = nullptr, *d_iters = nullptr, *d_capped = nullptr;
@@ -2729,19 +2664,17 @@ int mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int3
   CK(cudaMemcpyAsync(d_yq, yq.data(), sizeof(int*) * nQ, cudaMemcpyHostToDevice, h->stream));
   CK(cudaMemcpyAsync(d_wq, wq.data(), sizeof(int*) * nQ, cudaMemcpyHostToDevice, h->stream));
   // the operand split does not depend on gamma: once (the fit's launch, which also splits the test rows)
-  k_svm_split<<<dim3((S.max_rows + 7) / 8, 2 * nf), 256, 0, h->stream>>>(S.d_split);
-  h->launches += 1;
+  launch_k(h, k_svm_split, dim3((S.max_rows + 7) / 8, 2 * nf), 256, 0, h->stream, S.d_split);
   std::vector<int> cap(nJobs), cnt((size_t)nG * nQ);
   for (int g = 0; g < nG; ++g) {
-    k_svm_kmat<<<dim3((n_lab + SVM_BM - 1) / SVM_BM, (n_lab + SVM_BN - 1) / SVM_BN, nf), SVM_KMAT_THREADS, SVM_KMAT_SMEM, h->stream>>>(
-        d_gemm + (size_t)g * nf);
-    k_svm_smo<<<nJobs, SVM_SMO_THREADS, (size_t)SVM_SMO_SMEM_PER_ROW * npmax, h->stream>>>(d_jobs, S.eps);
-    k_svm_vote<<<dim3(max_nval, nQ), SVM_VOTE_THREADS, 0, h->stream>>>(d_jobs, npairs, K, d_Kq, d_trow, d_yq, d_nval, nullptr, d_wq, nullptr);
-    k_svm_count<<<nQ, 256, 0, h->stream>>>(d_wq, d_nval, d_count + (size_t)g * nQ);
-    h->launches += 4;
+    launch_k(h, k_svm_kmat, dim3((n_lab + SVM_BM - 1) / SVM_BM, (n_lab + SVM_BN - 1) / SVM_BN, nf), SVM_KMAT_THREADS, SVM_KMAT_SMEM,
+             h->stream, d_gemm + (size_t)g * nf);
+    launch_k(h, k_svm_smo, nJobs, SVM_SMO_THREADS, (size_t)SVM_SMO_SMEM_PER_ROW * npmax, h->stream, d_jobs, S.eps);
+    launch_k(h, k_svm_vote, dim3(max_nval, nQ), SVM_VOTE_THREADS, 0, h->stream, d_jobs, npairs, K, d_Kq, d_trow, d_yq, d_nval, nullptr,
+             d_wq, nullptr);
+    launch_k(h, k_svm_count, nQ, 256, 0, h->stream, d_wq, d_nval, d_count + (size_t)g * nQ);
     CK(cudaMemcpyAsync(cap.data(), d_capped, sizeof(int) * nJobs, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaGetLastError());
+    TRY(complete(h));
     for (int j = 0; j < nJobs; ++j)
       if (cap[j]) {
         const int q = j / npairs, s = q % ns, c = (q / ns) % nC, f = q / (ns * nC);
@@ -2751,7 +2684,7 @@ int mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int3
       }
   }
   CK(cudaMemcpyAsync(cnt.data(), d_count, sizeof(int) * cnt.size(), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
+  TRY(complete(h));
   for (int f = 0; f < nf; ++f)
     for (int g = 0; g < nG; ++g)
       for (int c = 0; c < nC; ++c)
@@ -2760,83 +2693,55 @@ int mrgan_svm_cv(mrgan_handle* h, const int32_t* lab_rows, int n_lab, const int3
 }
 
 int mrgan_svm_eval(mrgan_handle* h, int fold, float* err) {
-  int rc = check_fold(h, fold); if (rc) return rc;
-  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_eval needs an SVM handle");
+  TRY(enter(h, "svm_eval", FOLD | SVM, fold));
   if (!err) return fail(h, MRGAN_ERR_ARG, "svm_eval: null pointer");
-  if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "svm_eval before mrgan_svm_fit");
-  CK(cudaSetDevice(h->cfg.device));
+  TRY(ready(h, "svm_eval", FOLD | SVM | FITTED, fold));
   int c = 0;
   CK(cudaMemcpyAsync(&c, h->svm.d_count + fold, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
+  TRY(complete(h));
   *err = (float)c / (float)h->shapes[fold].n_test;     // np.mean(predicted != y_test)
   return MRGAN_OK;
 }
 
 int mrgan_svm_decision(mrgan_handle* h, int fold, float* dst) {
-  int rc = check_fold(h, fold); if (rc) return rc;
-  if (h->cfg.model != MRGAN_MODEL_SVM) return fail(h, MRGAN_ERR_STATE, "svm_decision needs an SVM handle");
+  TRY(enter(h, "svm_decision", FOLD | SVM, fold));
   if (!dst) return fail(h, MRGAN_ERR_ARG, "svm_decision: null pointer");
-  if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "svm_decision before mrgan_svm_fit");
-  CK(cudaSetDevice(h->cfg.device));
+  TRY(ready(h, "svm_decision", FOLD | SVM | FITTED, fold));
   CK(cudaMemcpyAsync(dst, h->svm.dec[fold], sizeof(float) * h->shapes[fold].n_test * h->svm.npairs, cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  return MRGAN_OK;
-}
-
-static int svm_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
-  if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "time_op: SVM phases before mrgan_svm_fit");
-  CK(cudaSetDevice(h->cfg.device));
-  svm_launch(h, which);                     // warm-up
-  CK(cudaEventRecord(h->ev0, h->stream));
-  for (int i = 0; i < reps; ++i) svm_launch(h, which);
-  CK(cudaEventRecord(h->ev1, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CK(cudaGetLastError());
-  float ms = 0.f;
-  CK(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-  *ms_avg = ms / reps;
-  return MRGAN_OK;
+  return complete(h);
 }
 
 // ------------------------------------------------------------------ predictions and confusion counts
 int mrgan_predict(mrgan_handle* h, int fold, int32_t* pred, float* scores) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  TRY(enter(h, "predict", FOLD, fold));
   if (!pred) return fail(h, MRGAN_ERR_ARG, "predict: null pointer");
-  rc = need_local(h, "predict"); if (rc) return rc;
+  const bool svm = h->cfg.model == MRGAN_MODEL_SVM;
+  TRY(ready(h, "predict", FOLD | LOCAL | (svm ? FITTED : LOADED), fold));
   const int n = h->shapes[fold].n_test, K = h->cfg.n_classes;
   const FoldBuffers& b = h->fb[fold];
-  if (h->cfg.model == MRGAN_MODEL_SVM) {
-    if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "predict before mrgan_svm_fit");
-    CK(cudaSetDevice(h->cfg.device));
+  if (svm) {
     CK(cudaMemcpyAsync(pred, b.pred, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));     // voted by mrgan_svm_fit
     if (scores) CK(cudaMemcpyAsync(scores, h->svm.dec[fold], (size_t)n * h->svm.npairs * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   } else {
-    if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "predict before mrgan_load_fold");
-    CK(cudaSetDevice(h->cfg.device));
-    rc = finish_pending(h); if (rc) return rc;
     enqueue_eval(h, fold, 1, false, 0, true);
     CK(cudaMemcpyAsync(pred, b.pred, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (scores)
       CK(cudaMemcpy2DAsync(scores, (size_t)K * sizeof(float), b.elg, (size_t)pitch8(K) * sizeof(float), (size_t)K * sizeof(float), n,
                            cudaMemcpyDeviceToHost, h->stream));
   }
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
-  return MRGAN_OK;
+  return complete(h);
 }
 
 int mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t* pred, float* scores) {
-  int rc = check_fold(h, fold); if (rc) return rc;
+  TRY(enter(h, "predict_rows", FOLD, fold));
   if (!x || !pred) return fail(h, MRGAN_ERR_ARG, "predict_rows: null pointer");
   if (n < 1 || n > h->shapes[fold].n_test) return fail(h, MRGAN_ERR_ARG, "predict_rows: n must be in [1, n_test of the fold]");
-  rc = need_local(h, "predict_rows"); if (rc) return rc;
+  const bool svm = h->cfg.model == MRGAN_MODEL_SVM;
+  TRY(ready(h, "predict_rows", FOLD | LOCAL | (svm ? FITTED : LOADED), fold));
   const int D = h->shapes[fold].D, K = h->cfg.n_classes;
-  const size_t w = (size_t)D * sizeof(float);
   FoldBuffers& b = h->fb[fold];
-  if (h->cfg.model == MRGAN_MODEL_SVM) {
+  if (svm) {
     mrgan_handle::Svm& S = h->svm;
-    if (!S.fitted) return fail(h, MRGAN_ERR_STATE, "predict_rows before mrgan_svm_fit");
-    CK(cudaSetDevice(h->cfg.device));
     EncodeTiledFn fn = tc_encoder();
     if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
     // the new rows replace the fold's test rows in its second kernel-matrix descriptor (labeled rows, norms, gamma kept)
@@ -2846,66 +2751,45 @@ int mrgan_predict_rows(mrgan_handle* h, int fold, const float* x, int n, int32_t
     if (!make_map(fn, &g.mapAh, S.Hs, Kp, n, Kp, SVM_BN, false) || !make_map(fn, &g.mapAl, S.Ls, Kp, n, Kp, SVM_BN, false))
       return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
     g.normA = S.ns; g.C = S.Ks; g.nA = n;
+    const size_t w = (size_t)D * sizeof(float);
     CK(cudaMemcpy2DAsync(S.Xs, (size_t)Kp * sizeof(float), x, w, w, n, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(S.d_split_s, &sp, sizeof(sp), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(S.d_gemm_s, &g, sizeof(g), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(S.d_ns, &n, sizeof(int), cudaMemcpyHostToDevice, h->stream));
-    k_svm_split<<<dim3((n + 7) / 8, 1), 256, 0, h->stream>>>(S.d_split_s);
-    k_svm_kmat<<<dim3((S.n_lab + SVM_BM - 1) / SVM_BM, (n + SVM_BN - 1) / SVM_BN, 1), SVM_KMAT_THREADS, SVM_KMAT_SMEM, h->stream>>>(S.d_gemm_s);
-    k_svm_vote<<<dim3(n, 1), SVM_VOTE_THREADS, 0, h->stream>>>(S.d_jobs + (size_t)fold * S.npairs, S.npairs, K, S.d_Ks, nullptr, nullptr,
-                                                               S.d_ns, S.d_decs, nullptr, S.d_preds);
-    h->launches += 3;
+    launch_k(h, k_svm_split, dim3((n + 7) / 8, 1), 256, 0, h->stream, S.d_split_s);
+    launch_k(h, k_svm_kmat, dim3((S.n_lab + SVM_BM - 1) / SVM_BM, (n + SVM_BN - 1) / SVM_BN, 1), SVM_KMAT_THREADS, SVM_KMAT_SMEM, h->stream,
+             S.d_gemm_s);
+    launch_k(h, k_svm_vote, dim3(n, 1), SVM_VOTE_THREADS, 0, h->stream, S.d_jobs + (size_t)fold * S.npairs, S.npairs, K, S.d_Ks, nullptr,
+             nullptr, S.d_ns, S.d_decs, nullptr, S.d_preds);
     CK(cudaMemcpyAsync(pred, S.preds, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (scores) CK(cudaMemcpyAsync(scores, S.decs, (size_t)n * S.npairs * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   } else {
-    if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "predict_rows before mrgan_load_fold");
-    CK(cudaSetDevice(h->cfg.device));
-    rc = finish_pending(h); if (rc) return rc;
     // the staging path of mrgan_test_batch, without labels (the error it computes on the stale staged labels is unused)
-    CK(cudaMemcpy2DAsync(b.ex_stage, (size_t)b.lda[0] * sizeof(float), x, w, w, n, cudaMemcpyHostToDevice, h->stream));
-    if (h->cfg.precision == MRGAN_PREC_TF32) {
-      k_round_tf32<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0]);
-      h->launches++;
-    } else if (h->om.mode == 2) {
-      k_to_half<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0], h->om);
-      h->launches++;
-    }
+    TRY(stage_rows(h, fold, x, n));
     enqueue_eval(h, fold, 1, true, n, true);
     CK(cudaMemcpyAsync(pred, b.pred_s, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     if (scores)
       CK(cudaMemcpy2DAsync(scores, (size_t)K * sizeof(float), b.elg, (size_t)pitch8(K) * sizeof(float), (size_t)K * sizeof(float), n,
                            cudaMemcpyDeviceToHost, h->stream));
   }
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
-  return MRGAN_OK;
+  return complete(h);
 }
 
 int mrgan_confusion(mrgan_handle* h, int32_t* out) {
-  if (!h) return fail(nullptr, MRGAN_ERR_ARG, "null handle");
+  TRY(enter(h, "confusion", 0));
   if (!out) return fail(h, MRGAN_ERR_ARG, "confusion: null pointer");
-  int rc = need_local(h, "confusion"); if (rc) return rc;
+  const bool svm = h->cfg.model == MRGAN_MODEL_SVM;
+  TRY(ready(h, "confusion", LOCAL | (svm ? FITTED : LOADED)));
   const int K = h->cfg.n_classes;
-  if (h->cfg.model == MRGAN_MODEL_SVM) {
-    if (!h->svm.fitted) return fail(h, MRGAN_ERR_STATE, "confusion before mrgan_svm_fit");
-  } else {
-    for (int f = 0; f < h->nf; ++f)
-      if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "confusion before mrgan_load_fold");
-  }
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
-  if (h->cfg.model != MRGAN_MODEL_SVM) enqueue_eval(h, 0, h->nf, false, 0, true);   // every fold in one pass; the SVM voted at fit
+  if (!svm) enqueue_eval(h, 0, h->nf, false, 0, true);   // every fold in one pass; the SVM voted at fit
   enqueue_confusion(h);
   CK(cudaMemcpyAsync(out, h->d_conf, (size_t)h->nf * K * K * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
-  return MRGAN_OK;
+  return complete(h);
 }
 
 // ------------------------------------------------------------------ input gradients and saliency profiles
 int mrgan_input_grad(mrgan_handle* h, int fold, const float* x, int n, const int32_t* target, float* grad) {
-  int rc = check_fold(h, fold); if (rc) return rc;
-  rc = need_nets(h, "input_grad"); if (rc) return rc;
+  TRY(enter(h, "input_grad", FOLD | NETS, fold));
   if (!grad) return fail(h, MRGAN_ERR_ARG, "input_grad: null pointer");
   const int D = h->shapes[fold].D, K = h->cfg.n_classes, nte = h->shapes[fold].n_test;
   if (n < 1 || n > nte) return fail(h, MRGAN_ERR_ARG, "input_grad: n must be in [1, n_test of the fold]");
@@ -2913,46 +2797,26 @@ int mrgan_input_grad(mrgan_handle* h, int fold, const float* x, int n, const int
   if (target)
     for (int i = 0; i < n; ++i)
       if (target[i] < 0 || target[i] >= K) return fail(h, MRGAN_ERR_ARG, "input_grad: target class out of range");
-  rc = need_local(h, "input_grad"); if (rc) return rc;
+  TRY(ready(h, "input_grad", FOLD | NETS | LOCAL | LOADED, fold));
+  TRY(saliency_setup(h));
   FoldBuffers& b = h->fb[fold];
-  if (!b.loaded) return fail(h, MRGAN_ERR_STATE, "input_grad before mrgan_load_fold");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
-  rc = saliency_setup(h); if (rc) return rc;
   const size_t w = (size_t)D * sizeof(float), ld0 = (size_t)b.lda[0] * sizeof(float);
-  if (x) {      // the staging path of mrgan_test_batch / mrgan_predict_rows
-    CK(cudaMemcpy2DAsync(b.ex_stage, ld0, x, w, w, n, cudaMemcpyHostToDevice, h->stream));
-    if (h->cfg.precision == MRGAN_PREC_TF32) {
-      k_round_tf32<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0]);
-      h->launches++;
-    } else if (h->om.mode == 2) {
-      k_to_half<<<64, 256, 0, h->stream>>>(b.ex_stage, (size_t)n * b.lda[0], h->om);
-      h->launches++;
-    }
-  }
+  if (x) TRY(stage_rows(h, fold, x, n));
   if (target) CK(cudaMemcpyAsync(b.ey_stage, target, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
   enqueue_input_grad(h, fold, 1, x != nullptr, x ? n : 0, target ? TGT_STAGED : TGT_PRED);
   CK(cudaMemcpy2DAsync(grad, w, b.ex_stage, ld0, w, n, cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
-  return MRGAN_OK;
+  return complete(h);
 }
 
 int mrgan_saliency(mrgan_handle* h, float* profile) {
-  int rc = need_nets(h, "saliency"); if (rc) return rc;
+  TRY(enter(h, "saliency", NETS));
   if (!profile) return fail(h, MRGAN_ERR_ARG, "saliency: null pointer");
-  rc = need_local(h, "saliency"); if (rc) return rc;
-  for (int f = 0; f < h->nf; ++f)
-    if (!h->fb[f].loaded) return fail(h, MRGAN_ERR_STATE, "saliency before mrgan_load_fold");
-  CK(cudaSetDevice(h->cfg.device));
-  rc = finish_pending(h); if (rc) return rc;
-  rc = saliency_setup(h); if (rc) return rc;
+  TRY(ready(h, "saliency", NETS | LOCAL | LOADED));
+  TRY(saliency_setup(h));
   enqueue_saliency(h);
   CK(cudaMemcpyAsync(profile, h->sal.profile, (size_t)h->nf * h->cfg.n_classes * max_D(h, 0, h->nf) * sizeof(float), cudaMemcpyDeviceToHost,
                      h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CKS();
-  return MRGAN_OK;
+  return complete(h);
 }
 
 int64_t mrgan_kernel_launches(const mrgan_handle* h) { return h ? h->launches : -1; }

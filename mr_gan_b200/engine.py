@@ -15,7 +15,7 @@ from . import _lib
 from .model import disc_shapes, gen_shapes
 
 MODEL = {"gan": 0, "nn": 1, "svm": 2}
-PRECISION = {"fp32": 0, "tf32": 1, "f16": 2}      # f16: fp16 operand copies, fp32 master weights / accumulation (experimental)
+PRECISION = {"fp32": 0, "tf32": 1, "f16": 2}      # f16 (the trainers' and CLIs' default): fp16 operand copies, fp32 master weights / accumulation
 
 
 class MrganError(RuntimeError):
