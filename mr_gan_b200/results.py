@@ -30,6 +30,24 @@ def errors(results):
     return [r['error'] if isinstance(r, dict) else r for r in results]
 
 
+def collect(fg, errors, details=False, saliency=False, extra=None):
+    """A trainer's results from its group's test errors: the floats as they are, or with details / saliency one dict per
+    fold, ``{'error', 'confusion'}`` from fg.confusion() and with saliency also ``'saliency'`` from fg.saliency(); extra:
+    per-fold fields to add (a tuned SVM's selected point), which makes dicts too."""
+    if not (details or saliency or extra):
+        return errors
+    out = [dict(error=e) for e in errors]
+    if details or saliency:
+        for r, c in zip(out, fg.confusion()):
+            r['confusion'] = c
+    if saliency:
+        for r, p in zip(out, fg.saliency()):
+            r['saliency'] = p
+    for r, x in zip(out, extra or []):
+        r.update(x)
+    return out
+
+
 def confusion_lines(conf, names=MATERIALS):
     """The printed block of one K x K confusion matrix, materials in model.MATERIALS order."""
     conf = np.asarray(conf)
@@ -101,9 +119,8 @@ class Report:
 
     def setting(self, jobs, results, blocks=None, **fields):
         """Call after a setting's average line, with the setting's jobs and trainer results in printed order; blocks: the
-        [(name, width)] feature blocks of the setting's rows (needed with --saliency)."""
-        if not (self.details or self.saliency):
-            return
+        [(name, width)] feature blocks of the setting's rows (needed with --saliency).  Results of a tuned SVM (mr_svm.py
+        --tune) also print the selected C and gamma * D of every fold-training."""
         if self.show:
             for line in confusion_lines(np.sum([np.asarray(r['confusion']) for r in results], axis=0)):
                 self.say(line)
@@ -113,6 +130,9 @@ class Report:
                 self.sal_arrays['job_%d' % j['job_id']] = np.asarray(r['saliency'], dtype=np.float32)
                 self.sal_index.append(dict(setting_fields(self.tool, j, k, **dict(self.fields, **fields)),
                                            blocks=[[name, int(w)] for name, w in blocks]))
+        if results and isinstance(results[0], dict) and 'C' in results[0]:
+            self.say('Selected C: ' + ' '.join('%g' % r['C'] for r in results) +
+                     ' Selected gamma*D: ' + ' '.join('%g' % r['gamma_D'] for r in results))
         if self.fh:
             for k, (j, r) in enumerate(zip(jobs, results)):
                 self.fh.write(json.dumps(record(self.tool, j, r, k, **dict(self.fields, **fields))) + '\n')

@@ -1,14 +1,15 @@
-"""CPU suite, part 4: the drop-in's host orchestration (mr_gan_b200/mr_gan.py, mr_nn.py) against a recording stand-in for
-the C-ABI handle -- order of calls, shapes, index streams, stdout format.  No GPU, no compute."""
+"""CPU suite, part 4: the drop-in's host orchestration (mr_gan_b200/mr_gan.py, mr_nn.py, mr_svm.py) against a recording
+stand-in for the C-ABI handle -- order of calls, shapes, index streams, stdout format.  No GPU, no compute."""
 import importlib
 
 import numpy as np
 import pytest
 
-from mr_gan_b200 import foldprep, synthetic
+from mr_gan_b200 import foldprep, synthetic, tables
 
 mg = importlib.import_module("mr_gan_b200.mr_gan")
 mn = importlib.import_module("mr_gan_b200.mr_nn")
+ms = importlib.import_module("mr_gan_b200.mr_svm")
 
 
 class FakeGroup:
@@ -17,7 +18,7 @@ class FakeGroup:
     def __init__(self, shapes, model="gan", precision="fp32", device=0, batch=None, **kw):
         self.shapes, self.model, self.precision, self.batch = list(shapes), model, precision, batch
         self.n_folds, self.n_train = len(self.shapes), self.shapes[0][1]
-        self.calls, self.params, self.datasets, self.epochs = [], {}, {}, []
+        self.calls, self.params, self.datasets, self.epochs, self.rows, self.lab = [], {}, {}, [], {}, []
         FakeGroup.instances.append(self)
 
     def set_params(self, fold, net, params):
@@ -30,6 +31,7 @@ class FakeGroup:
 
     def prepare_fold(self, fold, slot, train_rows, test_rows):
         self.calls.append(("prepare_fold", fold, slot))
+        self.rows[fold] = (np.array(train_rows), np.array(test_rows))
         D, ntr, nte, _ = self.shapes[fold]
         assert len(train_rows) == ntr and len(test_rows) == nte and not set(train_rows) & set(test_rows)
 
@@ -65,6 +67,26 @@ class FakeGroup:
     def nn_evaluate(self, fold):
         return np.float32(0.2), np.float32(0.75)
 
+    def svm_fit(self, lab_rows, C=1.0, gamma=None):
+        assert lab_rows.shape[0] == self.n_folds and len(np.broadcast_to(gamma, (self.n_folds,))) == self.n_folds
+        self.lab.append(np.array(lab_rows))
+        self.calls.append(("svm_fit",))
+        return np.zeros((self.n_folds, 15), np.int32)
+
+    def svm_cv(self, lab_rows, split, C_grid, gamma):
+        assert split.shape == lab_rows.shape and gamma.shape[0] == self.n_folds
+        self.lab.append(np.array(lab_rows))
+        self.calls.append(("svm_cv",))
+        wrong = np.zeros((self.n_folds, gamma.shape[1], len(C_grid), int(split.max()) + 1), np.int32)
+        wrong[:, 0, 1] = 1                      # every point but (C_grid[1], gamma[0]) is perfect: C_grid[0] is chosen
+        return wrong
+
+    def svm_eval(self, fold):
+        return 0.375
+
+    def confusion(self):
+        return np.ones((self.n_folds, 6, 6), np.int32)
+
     def close(self):
         self.calls.append(("close",))
 
@@ -74,6 +96,7 @@ def fake(monkeypatch):
     FakeGroup.instances.clear()
     monkeypatch.setattr(mg, "FoldGroup", FakeGroup)
     monkeypatch.setattr(mn, "FoldGroup", FakeGroup)
+    monkeypatch.setattr(ms, "FoldGroup", FakeGroup)
     return FakeGroup
 
 
@@ -128,6 +151,39 @@ def test_mr_nn_host_loop(fake):
     assert all(len(set(g.epochs[0][f])) == 120 for f in range(6))                        # model.fit shuffles the labeled rows
     with pytest.raises(ValueError, match="multiple of the batch size"):
         mn.train_nn_folds(mg._kfold_jobs(X, y, 0, percentlabeled=0.3), epochs=1, seed=2)  # 3 rows per class -> 18 rows
+
+
+def test_gan_nn_and_svm_load_the_same_folds(fake):
+    """One loader for the three trainers: the same jobs and seed give every group the same shapes and rows, and the SVM fits
+    the NN's labeled rows.  Per fold, the GAN sets the generator, then the discriminator, then prepares the fold; the NN
+    sets the discriminator; the SVM only prepares the fold."""
+    X, y = synthetic.synthetic_dataset(1, forcetempTime=0.1, pokes=5, seed=0)
+    jobs = tables.kfold_jobs(X, y, 0, percentlabeled=2)
+    for i, j in enumerate(jobs):
+        j['job_id'] = 7 + i
+    assert mg.train_gan_folds(jobs, epochs=1, seed=3) == [pytest.approx(0.125)] * 6
+    assert mn.train_nn_folds(jobs, epochs=1, seed=3) == [pytest.approx(0.25)] * 6
+    assert ms.train_svm_folds(jobs, seed=3, details=True)[0]['confusion'].sum() == 36
+    tuned = ms.train_svm_folds(jobs, seed=3, grid=dict(C=[0.5, 2.0], gamma_D=[1.0]), cv=3)
+    assert [(r['error'], r['C'], r['gamma_D']) for r in tuned] == [(0.375, 0.5, 1.0)] * 6
+    gan, nn, svm, svm_tuned = fake.instances
+    assert [g.model for g in fake.instances] == ["gan", "nn", "svm", "svm"]
+    for g in (nn, svm, svm_tuned):
+        assert g.shapes == gan.shapes
+        for f in range(6):
+            for a, b in zip(g.rows[f], gan.rows[f]):
+                np.testing.assert_array_equal(a, b)
+    nn_lab = np.stack([np.unique(e) for e in nn.epochs[0]])          # the NN's epoch permutes its labeled rows
+    for lab in svm.lab + svm_tuned.lab:                                 # the fit, and the tuned group's CV and refit
+        np.testing.assert_array_equal(np.sort(lab, axis=1), nn_lab)
+    per_fold = {"gan": [("set_params", 1), ("set_params", 0), ("prepare_fold",)], "nn": [("set_params", 0), ("prepare_fold",)],
+                "svm": [("prepare_fold",)]}
+    for g in fake.instances:
+        steps = [c[:1] + c[2:] if c[0] == "set_params" else c[:1] for c in g.calls
+                 if c[0] in ("set_params", "prepare_fold")]
+        assert steps == per_fold[g.model] * 6
+        folds = [c[1] for c in g.calls if c[0] in ("set_params", "prepare_fold")]
+        assert folds == sorted(folds)                                    # fold by fold
 
 
 def test_cli_prints_reference_strings(fake, capsys, monkeypatch):

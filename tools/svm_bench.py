@@ -1,7 +1,8 @@
 """Measures mr_svm's tables 2 and 4 on synthetic data on one GPU and writes one JSON file (default
 profiles/r03_svm_1gpu.json):
 
-  - wall clock of the whole sweep (fold preparation, fit and prediction of every fold, as ``mr_svm.py --tables 2 4``);
+  - wall clock of the sweeps of ``mr_svm.py --tables 2 4 --synthetic`` (fold preparation, fit and prediction of every fold),
+    run through the CLI itself with its stdout discarded;
   - device time per phase (kernel matrices, SMO, prediction) of every group, re-run once through mrgan_time_op;
   - achieved TFLOP/s of the kernel-matrix GEMM (3-term split: 3 x 2 x Kp per matrix element, from shapes) against the
     TF32 rate torch.mm measures on the same GPU in the same run;
@@ -12,6 +13,8 @@ profiles/r03_svm_1gpu.json):
     python tools/svm_bench.py [--out FILE] [--cpu-sample N]
 """
 import argparse
+import contextlib
+import io
 import json
 import multiprocessing
 import os
@@ -26,7 +29,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.dont_write_bytecode = True
 
 from mr_gan_b200 import mr_svm, sweep  # noqa: E402
-from mr_gan_b200.mr_gan import job_rows  # noqa: E402
+from mr_gan_b200.tables import job_rows  # noqa: E402
 
 
 def gpu_info():
@@ -69,6 +72,25 @@ def sk_fold(k):
     return err, time.time() - t
 
 
+def cli_sweeps(seed, group):
+    """(jobs, errors, wall seconds) of every sweep mr_svm.py --tables 2 4 --synthetic runs, in its order."""
+    runs, real = [], sweep.run_sharded
+
+    def timed(jobs, train_group, **kw):
+        t0 = time.time()
+        errors = real(jobs, train_group, **kw)
+        runs.append((jobs, errors, time.time() - t0))
+        return errors
+
+    sweep.run_sharded = timed
+    try:
+        with contextlib.redirect_stdout(io.StringIO()):
+            mr_svm.main(['--tables', '2', '4', '--synthetic', '--seed', str(seed), '--group', str(group)])
+    finally:
+        sweep.run_sharded = real
+    return runs
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument('--out', default='profiles/r03_svm_1gpu.json')
@@ -77,15 +99,13 @@ def main(argv=None):
     ap.add_argument('--cpu-sample', type=int, default=2, help='sklearn folds per (table, modality, labeled %%)')
     args = ap.parse_args(argv)
     res = dict(gpu=gpu_info(), seed=args.seed, group=args.group)
-    tables = mr_svm.table_jobs(['2', '4'], args.seed, synthetic=True)
-    jobs = [j for *_, js in tables for j in js]
-    groups = sweep.plan(jobs, 1, args.group, key=lambda j: job_rows(j) + (j['percentlabeled'],))[0]
-    # 1. the sweep as the CLI runs it
-    t0 = time.time()
-    errors = sweep.run_sharded(jobs, lambda js, dev: mr_svm.train_svm_folds(js, seed=args.seed, device=dev), group_size=args.group,
-                               key=lambda j: job_rows(j) + (j['percentlabeled'],))
-    res['wall_s_tables_2_4'] = time.time() - t0
+    # 1. the sweeps as the CLI runs them
+    runs = cli_sweeps(args.seed, args.group)
+    jobs = [j for js, _, _ in runs for j in js]
+    errors = [e for _, es, _ in runs for e in es]
+    res['wall_s_tables_2_4'] = sum(t for *_, t in runs)
     res['folds'] = len(jobs)
+    groups = sweep.plan(jobs, 1, args.group, key=lambda j: job_rows(j) + (j['percentlabeled'],))[0]
     # 2. per-phase device time of every group
     ph = dict(kmat_ms=0.0, smo_ms=0.0, predict_ms=0.0)
     flops, iters, ctas, smo_by_pct = 0.0, 0, 0, {}
@@ -112,10 +132,11 @@ def main(argv=None):
     res['smo_iters_per_s_per_cta'] = {str(p): (v[1] / v[2]) / (v[0] * 1e-3) for p, v in sorted(smo_by_pct.items())}
     # 3. CPU arm on a labelled sample
     sample = []
-    for t, modality, percents, objects, js in tables:
-        for p in percents:
+    for js, _, _ in runs:                       # one sweep per (table, modality); D names the modality
+        t, D = '4' if 'name' in js[0] else '2', js[0]['X'].shape[1]
+        for p in sorted({j['percentlabeled'] for j in js}):
             sel = [j for j in js if j['percentlabeled'] == p][:args.cpu_sample]
-            sample += [(t, modality, p, j) for j in sel]
+            sample += [(t, D, p, j) for j in sel]
     ncpu = os.cpu_count() or 1
     t0 = time.time()
     _SAMPLE[:] = [(j, args.seed) for *_, j in sample]
@@ -123,12 +144,12 @@ def main(argv=None):
         out = list(ex.map(sk_fold, range(len(sample))))
     res['cpu_arm'] = dict(sample='%d folds per (table, modality, labeled %%)' % args.cpu_sample, host_cores=ncpu,
                           sample_folds=len(sample), sample_wall_s=time.time() - t0,
-                          per_fold_s={'%s/m%d/%d%%' % (t, m, p): [] for t, m, p, _ in sample})
+                          per_fold_s={'%s/D%d/%d%%' % (t, D, p): [] for t, D, p, _ in sample})
     by_id = {j['job_id']: e for j, e in zip(jobs, errors)}
     diffs = []
-    for (t, m, p, j), (e, s) in zip(sample, out):
-        res['cpu_arm']['per_fold_s']['%s/m%d/%d%%' % (t, m, p)].append(s)
-        diffs.append(dict(table=t, modality=m, percent=p, job_id=j['job_id'], gpu_err=by_id[j['job_id']], sklearn_err=e))
+    for (t, D, p, j), (e, s) in zip(sample, out):
+        res['cpu_arm']['per_fold_s']['%s/D%d/%d%%' % (t, D, p)].append(s)
+        diffs.append(dict(table=t, D=D, percent=p, job_id=j['job_id'], gpu_err=by_id[j['job_id']], sklearn_err=e))
     res['errors_gpu_vs_sklearn'] = diffs
     res['mean_error_difference'] = float(np.mean([d['gpu_err'] - d['sklearn_err'] for d in diffs]))
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)

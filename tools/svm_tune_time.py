@@ -20,7 +20,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.dont_write_bytecode = True
 
 from mr_gan_b200 import mr_svm  # noqa: E402
-from mr_gan_b200.mr_gan import _kfold_jobs, dataset  # noqa: E402
+from mr_gan_b200.mr_gan import dataset  # noqa: E402
+from mr_gan_b200.tables import kfold_jobs  # noqa: E402
 
 
 def gpu_info():
@@ -37,15 +38,15 @@ def main(argv=None):
     gpu, grid, cv = gpu_info(), mr_svm.DEFAULT_GRID, 5
     X, y = dataset(modalities=2, seed=a.seed, synthetic_data=True)
     for p in a.percents:
-        jobs = _kfold_jobs(X, y, a.seed + p, percentlabeled=p)
+        jobs = kfold_jobs(X, y, a.seed + p, percentlabeled=p)
         for i, j in enumerate(jobs):
             j['job_id'] = i
         mr_svm.train_svm_folds(jobs, seed=a.seed, grid=grid, cv=cv)           # warm-up: module load, allocations
-        fg, folds, shapes = mr_svm.load_group(jobs, seed=a.seed)
+        fg, folds = mr_svm.load_group(jobs, seed=a.seed)
         try:
             lab = np.stack([f.lab_rows for f in folds])
             split = np.stack([mr_svm.inner_splits(f.y_train[f.lab_rows], cv) for f in folds])
-            gam = np.array(grid['gamma_D'])[None, :] / np.array([s[0] for s in shapes], np.float64)[:, None]
+            gam = np.array(grid['gamma_D'])[None, :] / np.array([s[0] for s in fg.shapes], np.float64)[:, None]
             t0 = time.perf_counter()
             fg.svm_cv(lab, split, grid['C'], gam)
             t_cv = time.perf_counter() - t0
@@ -67,7 +68,7 @@ def main(argv=None):
     if not a.no_sklearn and 100 in a.percents:
         from sklearn.model_selection import GridSearchCV, StratifiedKFold
         from sklearn.svm import SVC
-        jobs = _kfold_jobs(X, y, a.seed + 100, percentlabeled=100)
+        jobs = kfold_jobs(X, y, a.seed + 100, percentlabeled=100)
         f, = mr_svm.prepare_folds(jobs[:1], a.seed)
         tr = X[f.train_rows]
         mu, sd = tr.mean(0), tr.std(0)
