@@ -108,6 +108,24 @@ int  mrgan_get_params(mrgan_handle* h, int fold, int net, float* dst, int64_t n)
 int  mrgan_get_adam(mrgan_handle* h, int fold, int net, float* m, float* v, int64_t n);
 int  mrgan_get_counters(mrgan_handle* h, int fold, int* iterations, int* rng_step);
 
+/* Checkpoints.  The complete training state of a GAN / NN fold between epochs is
+ *   - the parameters of each net (mrgan_get_params / mrgan_set_params),
+ *   - Adam's m and v of each net (mrgan_get_adam / mrgan_set_adam), reference order like the parameters,
+ *   - the four step counters {iterations, it_net[0], it_net[1], rng_step} (mrgan_get_fold_counters /
+ *     mrgan_set_fold_counters): Keras `iterations` (used when shared_t = 1), the per-net counters of D and G (used when
+ *     shared_t = 0; the NN trains net 0 only) and the Philox `step` word of the noise streams;
+ * plus what the caller keeps: the fold key (mrgan_fold_shape.seed) and the epoch number (device permutations are keyed by
+ * both) or its host RNG.  Adam's lr_t is not state: every step derives it from the counters.  Restoring these into a fresh
+ * handle, in any grouping, and training on gives bitwise what the uninterrupted run gives: the epoch graph reads the
+ * counters from device memory, so a restore between epochs needs no recapture.  In f16 mode mrgan_set_params rebuilds the
+ * fp16 operand copy of the weights with the round-to-nearest conversion the fused Adam epilogues use, so the copy is the
+ * one training left.  Restores write zero pad columns, as training leaves them.
+ * Each call first completes a pending asynchronous epoch.  MRGAN_ERR_ARG: a null pointer, a wrong length, a negative
+ * counter.  MRGAN_ERR_STATE: an SVM handle or a data-parallel handle (mrgan_dp_init / mrgan_dp_init_virtual). */
+int  mrgan_set_adam(mrgan_handle* h, int fold, int net, const float* m, const float* v, int64_t n);
+int  mrgan_get_fold_counters(mrgan_handle* h, int fold, int32_t out[4]);
+int  mrgan_set_fold_counters(mrgan_handle* h, int fold, const int32_t in[4]);
+
 /* Fold data made device-resident once (replaces the per-call numpy slices of
  * mr_gan.py:207,213,222): scaled X_train/X_test, labels. */
 int  mrgan_load_fold(mrgan_handle* h, int fold,

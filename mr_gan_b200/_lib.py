@@ -47,6 +47,9 @@ SYMBOLS = {
     "mrgan_get_params": (C.c_int, [_H, C.c_int, C.c_int, _fp, C.c_int64]),
     "mrgan_get_adam": (C.c_int, [_H, C.c_int, C.c_int, _fp, _fp, C.c_int64]),
     "mrgan_get_counters": (C.c_int, [_H, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "mrgan_set_adam": (C.c_int, [_H, C.c_int, C.c_int, _fp, _fp, C.c_int64]),
+    "mrgan_get_fold_counters": (C.c_int, [_H, C.c_int, _ip]),
+    "mrgan_set_fold_counters": (C.c_int, [_H, C.c_int, _ip]),
     "mrgan_load_fold": (C.c_int, [_H, C.c_int, _fp, _ip, _fp, _ip]),
     "mrgan_load_dataset": (C.c_int, [_H, C.c_int, _fp, _ip, C.c_int, C.c_int]),
     "mrgan_prepare_fold": (C.c_int, [_H, C.c_int, C.c_int, _ip, _ip]),

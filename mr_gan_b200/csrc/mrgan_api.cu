@@ -1790,6 +1790,49 @@ int mrgan_get_counters(mrgan_handle* h, int fold, int* iterations, int* rng_step
   return MRGAN_OK;
 }
 
+// ------------------------------------------------------------------ checkpoint state (include/mrgan.h "Checkpoints")
+int mrgan_set_adam(mrgan_handle* h, int fold, int net, const float* m, const float* v, int64_t n) {
+  TRY(enter(h, "set_adam", FOLD | NETS, fold));
+  if (net < 0 || net > 1 || h->net[net].empty()) return fail(h, MRGAN_ERR_ARG, "no such net in this model");
+  const NetLayout& L = h->net[net][fold];
+  if (!m || !v || n != L.n_ref) return fail(h, MRGAN_ERR_ARG, "set_adam: null pointer or length does not match mrgan_num_params");
+  TRY(ready(h, "set_adam", FOLD | NETS | LOCAL, fold));
+  std::vector<float> bm((size_t)L.n, 0.f), bv((size_t)L.n, 0.f);      // pad columns stay zero, as training leaves them
+  pack_params(h, fold, net, m, bm, true, nullptr);
+  pack_params(h, fold, net, v, bv, true, nullptr);
+  CK(cudaMemcpyAsync(h->Mo + L.off, bm.data(), (size_t)L.n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(h->Vo + L.off, bv.data(), (size_t)L.n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  return complete(h);
+}
+
+// {iterations, it_net[0], it_net[1], rng_step}: four consecutive ints of FoldState, copied as one block
+static_assert(offsetof(FoldState, it_net) == offsetof(FoldState, iterations) + sizeof(int) &&
+              offsetof(FoldState, rng_step) == offsetof(FoldState, iterations) + 3 * sizeof(int), "FoldState counter block");
+
+int mrgan_get_fold_counters(mrgan_handle* h, int fold, int32_t out[4]) {
+  TRY(enter(h, "get_fold_counters", FOLD | NETS, fold));
+  if (!out) return fail(h, MRGAN_ERR_ARG, "get_fold_counters: null pointer");
+  TRY(ready(h, "get_fold_counters", FOLD | NETS | LOCAL, fold));
+  CK(cudaMemcpyAsync(h->h_scratch, reinterpret_cast<const char*>(h->d_folds + fold) + offsetof(FoldState, iterations),
+                     4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+  TRY(complete(h));
+  memcpy(out, h->h_scratch, 4 * sizeof(int32_t));
+  return MRGAN_OK;
+}
+
+int mrgan_set_fold_counters(mrgan_handle* h, int fold, const int32_t in[4]) {
+  TRY(enter(h, "set_fold_counters", FOLD | NETS, fold));
+  if (!in) return fail(h, MRGAN_ERR_ARG, "set_fold_counters: null pointer");
+  for (int i = 0; i < 4; ++i)
+    if (in[i] < 0) return fail(h, MRGAN_ERR_ARG, "set_fold_counters: negative counter");
+  TRY(ready(h, "set_fold_counters", FOLD | NETS | LOCAL, fold));
+  // lr_t is not part of the state: k_prep derives it from these counters at the start of every step
+  memcpy(h->h_scratch, in, 4 * sizeof(int32_t));
+  CK(cudaMemcpyAsync(reinterpret_cast<char*>(h->d_folds + fold) + offsetof(FoldState, iterations), h->h_scratch,
+                     4 * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+  return complete(h);
+}
+
 int mrgan_load_fold(mrgan_handle* h, int fold, const float* x_train, const int32_t* y_train, const float* x_test,
                     const int32_t* y_test) {
   TRY(enter(h, "load_fold", FOLD, fold));

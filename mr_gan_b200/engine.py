@@ -51,6 +51,7 @@ class FoldGroup:
                 raise TypeError("unknown hyper-parameter %r" % k)
             setattr(cfg, k, v)
         self.cfg = cfg
+        self.hyper = dict(hyper)     # the config fields the caller set beyond the named arguments (saved with a checkpoint)
         self.model = model
         self.n_folds = len(shapes)
         self.shapes = [(int(D), int(ntr), int(nte), int(seed)) for D, ntr, nte, seed in shapes]
@@ -170,6 +171,62 @@ class FoldGroup:
         self._chk(self.lib.mrgan_get_counters(self._h, fold, C.byref(it), C.byref(rs)))
         return it.value, rs.value
 
+    # ------------------------------------------------------------------ training state (checkpoints, GAN / NN)
+    @property
+    def nets(self):
+        """The nets of a fold: (0, 1) = discriminator and generator (GAN), (0,) = the classifier (NN)."""
+        return (0, 1) if self.model == "gan" else (0,)
+
+    def _check_arrays(self, fold, net, arrs, what):
+        shp = self._shapes(fold, net)
+        if len(arrs) != len(shp) or any(tuple(np.shape(a)) != tuple(s) for a, s in zip(arrs, shp)):
+            raise ValueError("%s does not have the shapes of net %d of fold %d (D=%d)" % (what, net, fold, self.shapes[fold][0]))
+
+    def set_adam(self, fold, net, m, v):
+        """Adam's m and v of one net: lists of arrays in the reference's weight order, like set_params."""
+        flat = []
+        for name, arrs in (("m", m), ("v", v)):
+            self._check_arrays(fold, net, arrs, "set_adam: " + name)
+            flat.append(_f32(np.concatenate([np.asarray(a, dtype=np.float32).ravel() for a in arrs])))
+        self._chk(self.lib.mrgan_set_adam(self._h, fold, net, _lib.fptr(flat[0]), _lib.fptr(flat[1]), flat[0].size))
+
+    def fold_counters(self, fold):
+        """int32 [4]: {iterations, it_net[0], it_net[1], rng_step} (include/mrgan.h, Checkpoints)."""
+        out = np.zeros(4, dtype=np.int32)
+        self._chk(self.lib.mrgan_get_fold_counters(self._h, int(fold), _lib.iptr(out)))
+        return out
+
+    def set_fold_counters(self, fold, counters):
+        c = _i32(counters)
+        if c.shape != (4,):
+            raise ValueError("set_fold_counters: expected 4 counters")
+        self._chk(self.lib.mrgan_set_fold_counters(self._h, int(fold), _lib.iptr(c)))
+
+    def fold_state(self, fold):
+        """The training state of one fold between epochs: ``{'params': [per net: arrays], 'm': [...], 'v': [...],
+        'counters': int32 [4]}``, nets in ``self.nets`` order and arrays in the reference's weight order."""
+        st = dict(params=[], m=[], v=[], counters=self.fold_counters(fold))
+        for net in self.nets:
+            m, v = self.get_adam(fold, net)
+            st["params"].append(self.get_params(fold, net))
+            st["m"].append(m)
+            st["v"].append(v)
+        return st
+
+    def load_fold_state(self, fold, state):
+        """Restore fold_state(); the shapes are checked before anything is written."""
+        for k in ("params", "m", "v"):
+            if len(state[k]) != len(self.nets):
+                raise ValueError("load_fold_state: %s holds %d nets, this %s fold has %d" % (k, len(state[k]), self.model, len(self.nets)))
+            for net, arrs in zip(self.nets, state[k]):
+                self._check_arrays(fold, net, arrs, "load_fold_state: " + k)
+        if np.shape(state["counters"]) != (4,):
+            raise ValueError("load_fold_state: expected 4 counters")
+        for i, net in enumerate(self.nets):
+            self.set_params(fold, net, state["params"][i])
+            self.set_adam(fold, net, state["m"][i], state["v"][i])
+        self.set_fold_counters(fold, state["counters"])
+
     # ------------------------------------------------------------------ data
     def load_fold(self, fold, x_train, y_train, x_test, y_test):
         D, ntr, nte, _ = self.shapes[fold]
@@ -270,6 +327,13 @@ class FoldGroup:
         out = np.zeros(1, dtype=np.float32)
         self._chk(self.lib.mrgan_eval(self._h, fold, _lib.fptr(out)))
         return out[0]
+
+    def test_error(self, fold):
+        """The test error train_gan_folds / train_nn_folds report, computed as they compute it: mrgan_eval's error (GAN,
+        mr_gan.py:230), or 1 - model.evaluate's accuracy (NN, mr_nn.py:118)."""
+        if self.model == "nn":
+            return 1.0 - float(self.nn_evaluate(fold)[1])
+        return float(self.eval(fold))
 
     # ------------------------------------------------------------------ mr_nn twins
     def nn_step(self, fold, x, labels):

@@ -9,7 +9,7 @@ import time
 
 import numpy as np
 
-from . import foldprep, results, synthetic, tables
+from . import checkpoint, foldprep, results, synthetic, tables
 from .engine import FoldGroup
 from .model import MATERIALS, init_disc, init_gen
 from .tables import MODALITIES, job_rows, job_width, kfold_jobs, loo_jobs, stack_objects  # noqa: F401
@@ -37,7 +37,8 @@ def dataset(modalities=0, forcetempTime=4, contactmicTime=0.2, leaveObjectOut=Fa
 
 
 def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16', device=0, batch=50,
-                    eval_each_epoch=True, shared_t=True, return_group=False, device_perm=False, details=False, saliency=False):
+                    eval_each_epoch=True, shared_t=True, return_group=False, device_perm=False, details=False, saliency=False,
+                    start_states=None, on_epoch=None):
     """Train a GROUP of independent folds side by side on one GPU.
 
     jobs: list of dicts with keys ``trainTestSets`` (or ``X``, ``y``), ``percentlabeled``,
@@ -46,14 +47,20 @@ def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16',
     epoch instead of 3 x int32[n_train] per fold); same distribution, different draws than the host's numpy generator.
     Returns the list of test errors (mr_gan.py:230,234), one per job; details=True: one dict per job instead,
     ``{'error': <the same float>, 'confusion': int32 [K, K]}`` (rows = true class, columns = predicted), from one extra
-    forward pass over every fold's test set; saliency=True: those dicts with ``'saliency'``, float32 [K, D] (FoldGroup.saliency)."""
+    forward pass over every fold's test set; saliency=True: those dicts with ``'saliency'``, float32 [K, D] (FoldGroup.saliency).
+    start_states / on_epoch: resume and snapshots (checkpoint.py)."""
+    start = checkpoint.start_epoch(start_states, len(jobs))
+
     def init(fg, i, D, rng):
+        if start_states is not None and start_states[i] is not None:
+            return                                  # the weights come from the state
         fg.set_params(i, 1, init_gen(D, rng))       # generator first, as mr_gan.py:110-114 builds it first
         fg.set_params(i, 0, init_disc(D, rng))
 
     fg, folds, rngs = foldprep.load_folds(jobs, seed, lambda shapes: FoldGroup(
         shapes, model='gan', precision=precision, device=device, batch=batch, eval_each_epoch=eval_each_epoch,
         shared_t=shared_t), init, verbose)
+    checkpoint.restore(fg, rngs, start_states)
     n_train = fg.shapes[0][1]
     if verbose:
         print('Epochs:', epochs)
@@ -71,16 +78,21 @@ def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16',
             fg.set_epoch_rows(i, f.lab_rows, f.unl_rows)
     else:
         device_perm = False
-    nxt = None if device_perm else draw()
-    for epoch in range(1, epochs + 1):
+    nxt = None if device_perm or start >= epochs else draw()
+    for epoch in range(start + 1, epochs + 1):
         begin = time.time()
+        snap = None
         if device_perm:
             fg.train_epoch_seeded(epoch, wait=False)  # permutations drawn on the device from (fold key, epoch)
         else:
             fg.train_epoch(*nxt, wait=False)      # one CUDA-graph launch: the whole epoch, all folds
+            if on_epoch is not None:
+                snap = checkpoint.rng_states(rngs)  # the streams after this epoch's draws, before the next epoch's
             if epoch < epochs:
                 nxt = draw()                      # host permutations of the next epoch overlap the GPU
         st = fg.epoch_result()
+        if on_epoch is not None:
+            on_epoch(epoch, fg, st, snap)
         if verbose:
             for i in range(len(jobs)):
                 print('Epoch %d, time = %ds, loss labeled = %.4f, loss unlabeled = %.4f, train error = %.4f, test error = %.4f'
@@ -120,11 +132,12 @@ def main(argv=None):
     parser.add_argument('--host-perm', action='store_true', help='draw the epoch permutations on the host (numpy) instead of on the device')
     args = parser.parse_args(argv)
 
-    def train(jobs, device, seed, rep):
+    def train(jobs, device, seed, rep, **resume):
         return train_gan_folds(jobs, epochs=args.epochs, verbose=args.verbose, seed=seed, precision=args.precision, device=device,
-                               device_perm=not args.host_perm, details=rep.details, saliency=rep.saliency)
+                               device_perm=not args.host_perm, details=rep.details, saliency=rep.saliency, **resume)
 
-    return tables.run(args, 'mr_gan', train, job_rows, job_cost, ['1', '3', '5', '6'])
+    return tables.run(args, 'mr_gan', train, job_rows, job_cost, ['1', '3', '5', '6'],
+                      checkpoint_fields=dict(model='gan', shared_t=True, batch=50, perm='host' if args.host_perm else 'device'))
 
 
 if __name__ == '__main__':

@@ -7,7 +7,7 @@ import sys
 import numpy as np
 from sklearn.model_selection import StratifiedKFold
 
-from . import results, sweep, synthetic
+from . import checkpoint, results, sweep, synthetic
 
 MODALITIES = ['Force', 'Temperature', 'Force and Temperature', 'Contact mic', 'Temperature and Contact Mic',
               'Force, Temperature, and Contact Mic', 'Force and Contact Mic']      # mr_gan.py:237
@@ -69,6 +69,12 @@ def argument_parser(description, group, nets=True):
     parser.add_argument('--data-dir', default='data_processed')
     parser.add_argument('--synthetic', action='store_true', help='synthetic data of the MREO shape instead of the processed pickles')
     results.add_arguments(parser, saliency=nets)
+    if nets:
+        parser.add_argument('--checkpoint', metavar='DIR', default=None,
+                            help='write each fold-training\'s final state to DIR/<tool>_job<id>.npz; on a rerun, take finished '
+                                 'jobs from their files and resume unfinished ones (a file of another run is an error)')
+        parser.add_argument('--checkpoint-every', metavar='E', type=int, default=0,
+                            help='with --checkpoint, also write the state every E epochs')
     return parser
 
 
@@ -76,10 +82,12 @@ def _chunks(seq, n):
     return [seq[a:a + n] for a in range(0, len(seq), n)]
 
 
-def run(args, tool, train, key, cost, tables):
+def run(args, tool, train, key, cost, tables, checkpoint_fields=None):
     """Run and print the CLI's ``tables`` that ``args.tables`` asks for.  train(jobs, device, seed, report) trains one
     group of jobs; key and cost group and deal the jobs (sweep.run_sharded).  Job ids count up in printed order over the
-    whole invocation, so a job's streams depend only on the tables asked for and the seed."""
+    whole invocation, so a job's streams depend only on the tables asked for and the seed.  With ``--checkpoint``
+    (checkpoint.Sweep), train also takes ``start_states`` and ``on_epoch``, and checkpoint_fields are the fingerprint fields
+    the CLI fixes (model, shared_t, batch, perm)."""
     from .mr_gan import dataset      # the reference's dataset() lives in mr_gan.py, which imports this module
     rank = sweep.dist_env()[0]
     seed = sweep.shared_seed(args.seed)          # one seed for every rank: same dataset, same splits, same job streams
@@ -90,6 +98,12 @@ def run(args, tool, train, key, cost, tables):
     rep = results.Report(args, tool, rank, say, seed=seed, **nets)
     want = [t for t in tables if t in args.tables]
     next_id = [0]
+    ck = None
+    if getattr(args, 'checkpoint_every', 0) and not args.checkpoint:
+        raise SystemExit('--checkpoint-every needs --checkpoint DIR')
+    if getattr(args, 'checkpoint', None):
+        ck = checkpoint.Sweep(args.checkpoint, tool, seed, args.epochs, args.checkpoint_every,
+                              dict(checkpoint_fields, precision=args.precision))
 
     def data(modality, **kw):
         return dataset(modalities=modality, seed=seed, data_dir=args.data_dir, synthetic_data=args.synthetic, **kw)
@@ -98,7 +112,11 @@ def run(args, tool, train, key, cost, tables):
         for j in jobs:
             j['job_id'] = next_id[0]
             next_id[0] += 1
-        return sweep.run_sharded(jobs, lambda js, dev: train(js, dev, seed, rep), group_size=args.group, key=key, cost=cost)
+        if ck is None:
+            return sweep.run_sharded(jobs, lambda js, dev: train(js, dev, seed, rep), group_size=args.group, key=key, cost=cost)
+        start = {j['job_id']: ck.start(j) for j in jobs}        # folds of a group train in lockstep: group by start epoch too
+        return sweep.run_sharded(jobs, lambda js, dev: ck.train(js, dev, rep, train), group_size=args.group,
+                                 key=lambda j: (key(j), start[j['job_id']]), cost=cost)
 
     def title(text):
         say('\n', '-' * 25, text, '-' * 25)
