@@ -283,9 +283,6 @@ int  mrgan_debug_buffer(mrgan_handle* h, int fold, int which, float* dst, int ro
  * mode 0: C[M,N] = A[M,K] B[K,N]   mode 1: C[M,N] = A[M,K] B[N,K]^T   mode 2: C[M,N] = A[K,M]^T B[K,N]
  * Dense row-major host arrays. */
 int  mrgan_debug_gemm(mrgan_handle* h, int mode, int M, int N, int K, const float* A, const float* B, float* C, int use_tc);
-/* Test hook: average device ms of `reps` launches of the stand-alone GEMM above on zero-filled operands,
- * replicated over `groups` independent problems (grid.z), tcgen05 path. */
-int  mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int groups, int reps, float* ms);
 int64_t mrgan_kernel_launches(const mrgan_handle* h); /* kernels launched so far (graph nodes count per replay) */
 double  mrgan_last_device_ms(const mrgan_handle* h);  /* CUDA-event time of the last train_epoch */
 const char* mrgan_version(void);

@@ -85,7 +85,6 @@ SYMBOLS = {
     "mrgan_time_op": (C.c_int, [_H, C.c_int, C.c_int, _fp]),
     "mrgan_debug_buffer": (C.c_int, [_H, C.c_int, C.c_int, _fp, C.c_int, C.c_int]),
     "mrgan_debug_gemm": (C.c_int, [_H, C.c_int, C.c_int, C.c_int, C.c_int, _fp, _fp, _fp, C.c_int]),
-    "mrgan_debug_gemm_time": (C.c_int, [_H, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _fp]),
     "mrgan_kernel_launches": (C.c_int64, [_H]),
     "mrgan_last_device_ms": (C.c_double, [_H]),
     "mrgan_version": (C.c_char_p, []),

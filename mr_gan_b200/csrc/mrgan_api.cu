@@ -45,6 +45,19 @@ constexpr int NUM_EX = NUM_OPS_ALL - NUM_OPS;
 
 struct OpInfo { bool at = false, bt = false, used = false; int maxM = 0, maxN = 0; };
 
+// How a tcgen05 op is launched: decided once per handle by tc_plan_op, read by tc_launch_gemm.
+struct TcKernel;
+struct TcPlan {
+  const TcKernel* k = nullptr;   // the k_gemm_tc instantiation (tc_kernel); null for an unused op or a fused one
+  bool fused = false;            // dW runs fused with Adam in k_dw_adam_tc (tc_launch_dw_adam)
+  int gx = 0;                    // grid.x: feature tiles
+  int bn = 0;                    // batch rows per tile, the most of any fold (grid.y)
+  int bn_big = 256;              // batch rows per tile of a fold with more than 256 rows (forward / dX)
+  int maxME = 0, maxNE = 0;      // extents over the folds: MMA-M (features), MMA-N (batch rows)
+  size_t smem = 0;               // dynamic shared memory of a launch
+  int ks = 1;                    // contraction slices per tile (deterministic split-K of a large-batch dW)
+};
+
 struct Arena {
   char* base = nullptr; size_t off = 0;
   template <typename T> T* take(size_t count) {
@@ -82,9 +95,8 @@ namespace {
 int tc_setup(mrgan_handle* h);
 int tc_ex_setup(mrgan_handle* h, TcOp* dst);
 void tc_teardown(mrgan_handle* h);
-bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st);
+void tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st, const OperandMode& om);
 void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cudaStream_t st);
-bool tc_dw_merge(const mrgan_handle* h);
 int tc_debug_gemm(mrgan_handle* h, int mode, const GemmDesc& g, int esz);
 }
 
@@ -149,11 +161,9 @@ struct mrgan_handle {
   float *dp_bnf = nullptr, *dp_bnb = nullptr, *dp_fm = nullptr;   // [nf][2*500], [nf][2*500], [nf][2*250]
   float* dp_losspart = nullptr; unsigned* dp_lossctr = nullptr;    // k_loss_disc block partials [nf][4*64] and arrival counters [nf]
   TcOp* d_tcops = nullptr;            // [NUM_OPS][nf] tensor maps + epilogue descriptors
-  int tc_bn[NUM_OPS_ALL] = {0}, tc_maxME[NUM_OPS_ALL] = {0}, tc_maxNE[NUM_OPS_ALL] = {0};
-  int tc_ksplit[NUM_OPS] = {0};       // large-batch dW: contraction slices per tile (deterministic split-K), 0/1 = off
-  bool tc_mt1[NUM_OPS_ALL] = {false}; // large-batch forward / dX whose 256 x 256 tiling would leave SMs idle: 128-feature CTAs (tc_pick_tile)
-  float* d_tcws = nullptr;            // ... and their partial-product workspace
-  bool tc_fused_adam = true;          // dW and Adam in one kernel, k_dw_adam_tc (no gradient round trip)
+  TcPlan tc_plan[NUM_OPS_ALL];
+  float* d_tcws = nullptr;            // partial products of the split-K dW ops
+  bool tc_fused_adam = false;         // dW and Adam in one kernel, k_dw_adam_tc (no gradient round trip); tcgen05 handles only
   int tc_heads = 0;                   // losses / feature matching / BatchNorm fused into GEMM epilogues (set by tc_setup), bit mask:
                                       // 1 = HEAD_DISC (no k_loss_disc, no k_adam of D), 2 = HEAD_FM (no k_fm), 4 = HEAD_BN (no k_bn_fwd)
   TcAdamOp* d_tcadam = nullptr;       // [NUM_OPS][nf]
@@ -680,11 +690,11 @@ int split_chunks(int rows) {
 // ------------------------------------------------------------------ launch sequences
 void launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st = nullptr) {
   if (!st) st = h->stream;
+  if (h->cfg.precision != MRGAN_PREC_FP32) { tc_launch_gemm(h, op, f0, nfl, rows_override, st, h->om); return; }
   const OpInfo& oi = h->ops[op];
   int M = oi.maxM;
   if (rows_override > 0 && !oi.at) M = rows_override;
   const GemmDesc* d = (op < NUM_OPS ? h->d_descs + (size_t)op * h->nf : h->sal.descs + (size_t)(op - NUM_OPS) * h->nf) + f0;
-  if (h->cfg.precision != MRGAN_PREC_FP32 && tc_launch_gemm(h, op, f0, nfl, rows_override, st)) return;
   dim3 grid((oi.maxN + 63) / 64, (M + 63) / 64, nfl);
   if (!oi.at && !oi.bt) launch_k(h, k_gemm_simt<false, false>, grid, dim3(256), 0, st, d, (const FoldState*)h->d_folds, rows_override, h->hp);
   else if (!oi.at && oi.bt) launch_k(h, k_gemm_simt<false, true>, grid, dim3(256), 0, st, d, (const FoldState*)h->d_folds, rows_override, h->hp);
@@ -734,7 +744,7 @@ void launch_adam(mrgan_handle* h, int f0, int nfl, int net) {
   if (blocks > 2048) blocks = 2048;
   if (blocks < 1) blocks = 1;
   const AdamRange* ranges = h->d_ranges[net];
-  if (h->cfg.precision != MRGAN_PREC_FP32 && h->tc_fused_adam) { ranges = h->d_ranges_tc[net]; blocks = 1; }
+  if (h->tc_fused_adam) { ranges = h->d_ranges_tc[net]; blocks = 1; }
   // f16 mode: the gradient buffer carries the loss scale, and every parameter update refreshes the fp16 operand copy
   const float ginv = h->om.mode == 2 ? 1.0f / h->om.gscale : 1.0f;
   __half* Ph = h->om.mode == 2 ? h->harena + (h->P - reinterpret_cast<float*>(h->arena)) : nullptr;
@@ -742,11 +752,9 @@ void launch_adam(mrgan_handle* h, int f0, int nfl, int net) {
            ginv, Ph);
 }
 
-int heads_on(const mrgan_handle* h) { return h->cfg.precision != MRGAN_PREC_FP32 ? h->tc_heads : 0; }
-
 void enqueue_gen_fwd(mrgan_handle* h, int f0, int nfl, int op_g3) {
   launch_gemm(h, OP_G1, f0, nfl, 0);
-  if (heads_on(h) & 4) {                       // BatchNorm ran in G1's epilogue
+  if (h->tc_heads & 4) {                     // BatchNorm ran in G1's epilogue
     launch_gemm(h, OP_G2, f0, nfl, 0);
     launch_gemm(h, op_g3, f0, nfl, 0);
     return;
@@ -769,7 +777,7 @@ void enqueue_gen_fwd(mrgan_handle* h, int f0, int nfl, int op_g3) {
 void enqueue_disc_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
   const mrgan_config& c = h->cfg;
   const int B = c.batch;
-  const bool heads = (heads_on(h) & 1) != 0;
+  const bool heads = (h->tc_heads & 1) != 0;
   h->hp.t = t;
   launch_prep(h, f0, nfl, 0, from_stage, t, 2 * B);
   enqueue_gen_fwd(h, f0, nfl, OP_G3D);
@@ -781,7 +789,7 @@ void enqueue_disc_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) 
     launch_k(h, k_loss_disc, dim3(lb, 1, nfl), dim3(256), 0, h->stream, (const LossDesc*)(h->d_loss + f0), h->d_step_stats, f0, h->nf, t, B,
              c.n_classes, c.unlabeled_weight, h->om, h->hp.dp_bg, h->dp_losspart, h->dp_lossctr);
   }
-  const bool merge = tc_dw_merge(h);
+  const bool merge = h->tc_plan[OP_DW3].fused;    // fused dW+Adam: narrow layers may share launches
   for (int l = 6; l >= 1; --l) {      // dX first: it reads W_l, which the fused-Adam dW epilogue overwrites
     if (l >= 2) launch_gemm(h, OP_DX2 + l - 2, f0, nfl, 0);
     if (merge && l > 3) continue;     // the narrow layers 3..6 share ONE dW+Adam launch, after the last dX that reads their weights
@@ -803,7 +811,7 @@ void enqueue_disc_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) 
 void enqueue_gen_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
   const mrgan_config& c = h->cfg;
   const int B = c.batch;
-  const int hm = heads_on(h);
+  const int hm = h->tc_heads;
   h->hp.t = t;
   launch_prep(h, f0, nfl, 1, from_stage, t, 2 * B);
   enqueue_gen_fwd(h, f0, nfl, OP_G3G);
@@ -824,7 +832,7 @@ void enqueue_gen_step(mrgan_handle* h, int f0, int nfl, int t, int from_stage) {
   fork_side(h);
   launch_gemm(h, OP_GW3, f0, nfl, 0, h->side);
   launch_gemm(h, OP_GX2, f0, nfl, 0);
-  const bool merge = tc_dw_merge(h);
+  const bool merge = h->tc_plan[OP_GW1].fused;
   if (!merge) {
     fork_side(h);
     launch_gemm(h, OP_GW2, f0, nfl, 0, h->side);
@@ -1189,38 +1197,44 @@ int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 // forward / dX: 4-stage ring, up to 256 accumulator columns, 1 CTA per SM
 // dW (+ fused Adam): 2-stage ring (the contraction is only ~150 rows = 5 blocks), 128 columns, 2 CTAs per SM
+// large-batch regime (more than 256 batch rows: data-parallel config 5): 256 x 256 tiles, 3-stage ring of 64 KB stages
 #define TC_FWD_STAGES 4
 #define TC_DW_STAGES 2
+#define TC_BIG_STAGES 3
 #define TC_FWD_THREADS (64 + 32 * 8)
 #define TC_DW_THREADS (64 + 32 * 4)
-// kernel instantiations, indexed by the operand format F (false: fp32 operands as tf32, true: fp16 operand copies)
-#define K_TC_FWD(F, V) k_gemm_tc<true, false, TC_FWD_STAGES, 256, 1, 8, 1, F, V>
-#define K_TC_FWD_N(F, V) k_gemm_tc<true, false, TC_FWD_STAGES, 512, 1, 8, 1, F, V>   // all 512 TMEM columns: room to park the epilogue's noise
-#define K_TC_DX(F, V) k_gemm_tc<false, false, TC_FWD_STAGES, 256, 1, 8, 1, F, V>
-#define K_TC_FWD2(F, V) k_gemm_tc<true, false, TC_FWD_STAGES, 512, 1, 8, 2, F, V>     // 256 features per CTA (layers >= 500 wide)
-#define K_TC_DX_N(F, V) k_gemm_tc<false, false, TC_FWD_STAGES, 512, 1, 8, 1, F, V>
-#define K_TC_DX2(F, V) k_gemm_tc<false, false, TC_FWD_STAGES, 512, 1, 8, 2, F, V>
-#define K_TC_DW(F, V) k_gemm_tc<true, true, TC_DW_STAGES, 128, 2, 4, 1, F, V>
-// large-batch regime (more than 256 batch rows: data-parallel config 5): 256 x 256 tiles, 3-stage ring of 64 KB stages
-#define TC_BIG_STAGES 3
-#define K_TC_FWD_BIG(F, V) k_gemm_tc<true, false, TC_BIG_STAGES, 512, 1, 8, 2, F, V>
-#define K_TC_DX_BIG(F, V) k_gemm_tc<false, false, TC_BIG_STAGES, 512, 1, 8, 2, F, V>
-#define K_TC_DW_BIG(F, V) k_gemm_tc<true, true, TC_BIG_STAGES, 512, 1, 8, 2, F, V>
-// launches K(operand format, variant) with identical arguments: f16 = fp16 operand copies, var = the handle uses the
-// LeakyReLU / Dropout discriminator variants (their epilogue code lives in separate instantiations)
-#define TC_LAUNCH(h, f16, K, grid, block, smem, st, ...)                          \
-  do {                                                                            \
-    const bool var_ = (h)->cfg.hidden_act != MRGAN_ACT_RELU || (h)->cfg.dropout > 0.0f;                \
-    if (f16 && var_) launch_k(h, K(true, true), grid, block, smem, st, __VA_ARGS__);                   \
-    else if (f16) launch_k(h, K(true, false), grid, block, smem, st, __VA_ARGS__);                     \
-    else if (var_) launch_k(h, K(false, true), grid, block, smem, st, __VA_ARGS__);                    \
-    else launch_k(h, K(false, false), grid, block, smem, st, __VA_ARGS__);                             \
-  } while (0)
-size_t tc_smem_bytes(int bn, int stages, int mt = 1) { return 1024 + (size_t)stages * ((size_t)mt * 128 * 128 + (size_t)bn * 128) + 256; }
-// two feature sub-tiles per CTA when the layer is wide enough and the 4-stage ring still fits in 227 KB
-bool tc_use_mt2(int maxME, int bn) { return maxME >= 500 && tc_smem_bytes(bn, TC_FWD_STAGES, 2) <= 227 * 1024; }
+constexpr int kTcSmemMax = 227 * 1024;     // the most dynamic shared memory a block may have
+constexpr size_t tc_smem_bytes(int bn, int stages, int mt = 1) { return 1024 + (size_t)stages * ((size_t)mt * 128 * 128 + (size_t)bn * 128) + 256; }
 
-int tc_setup(mrgan_handle* h);
+// The k_gemm_tc instantiations the library launches, by role, operand format F (false: fp32 operands as tf32, true: fp16
+// operand copies) and variant V (the handle uses the LeakyReLU / Dropout discriminator variants, whose epilogue code lives
+// in separate instantiations; dW does not read V, so both variants share its kernels).  smem_attr is the max dynamic shared
+// memory the kernel is cleared for (tc_plan_op).  The attribute is process-wide: a constant per instantiation, the largest
+// tile any handle launches it with, never one op's own size.
+enum TcRole { TC_FWD, TC_FWD_N, TC_FWD2, TC_DX, TC_DX_N, TC_DX2, TC_DW, TC_FWD_BIG, TC_DX_BIG, TC_DW_BIG, TC_ROLES };
+struct TcKernel {
+  void (*fn)(const TcOp*, FoldState*, int, AdamHyper, OperandMode);
+  int threads, smem_attr;
+};
+constexpr int kTcSmemFwd = (int)tc_smem_bytes(256, TC_FWD_STAGES), kTcSmemDw = (int)tc_smem_bytes(128, TC_DW_STAGES);
+template <bool F, bool V> const TcKernel kTcKernels[TC_ROLES] = {
+    {k_gemm_tc<true, false, TC_FWD_STAGES, 256, 1, 8, 1, F, V>, TC_FWD_THREADS, kTcSmemFwd},
+    {k_gemm_tc<true, false, TC_FWD_STAGES, 512, 1, 8, 1, F, V>, TC_FWD_THREADS, kTcSmemFwd},   // all 512 TMEM columns: room to park the epilogue's noise
+    {k_gemm_tc<true, false, TC_FWD_STAGES, 512, 1, 8, 2, F, V>, TC_FWD_THREADS, kTcSmemMax},   // 256 features per CTA (layers >= 500 wide)
+    {k_gemm_tc<false, false, TC_FWD_STAGES, 256, 1, 8, 1, F, V>, TC_FWD_THREADS, kTcSmemFwd},
+    {k_gemm_tc<false, false, TC_FWD_STAGES, 512, 1, 8, 1, F, V>, TC_FWD_THREADS, kTcSmemFwd},
+    {k_gemm_tc<false, false, TC_FWD_STAGES, 512, 1, 8, 2, F, V>, TC_FWD_THREADS, kTcSmemMax},
+    {k_gemm_tc<true, true, TC_DW_STAGES, 128, 2, 4, 1, F, false>, TC_DW_THREADS, kTcSmemDw},
+    {k_gemm_tc<true, false, TC_BIG_STAGES, 512, 1, 8, 2, F, V>, TC_FWD_THREADS, kTcSmemMax},
+    {k_gemm_tc<false, false, TC_BIG_STAGES, 512, 1, 8, 2, F, V>, TC_FWD_THREADS, kTcSmemMax},
+    {k_gemm_tc<true, true, TC_BIG_STAGES, 512, 1, 8, 2, F, false>, TC_FWD_THREADS, kTcSmemMax},
+};
+const TcKernel& tc_kernel(int role, bool f16, bool var) {
+  static const TcKernel* const by_format[2][2] = {{kTcKernels<false, false>, kTcKernels<false, true>},
+                                                  {kTcKernels<true, false>, kTcKernels<true, true>}};
+  return by_format[f16][var][role];
+}
+bool tc_variant(const mrgan_handle* h) { return h->cfg.hidden_act != MRGAN_ACT_RELU || h->cfg.dropout > 0.0f; }
 
 EncodeTiledFn tc_encoder() {
   EncodeTiledFn fn = nullptr;
@@ -1230,26 +1244,6 @@ EncodeTiledFn tc_encoder() {
   return fn;
 }
 
-template <bool F, bool V> void tc_set_smem_attr_fmt() {
-  cudaFuncSetAttribute(K_TC_FWD(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(256, TC_FWD_STAGES));
-  cudaFuncSetAttribute(K_TC_FWD_N(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(256, TC_FWD_STAGES));
-  cudaFuncSetAttribute(K_TC_DX(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(256, TC_FWD_STAGES));
-  cudaFuncSetAttribute(K_TC_DX_N(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(256, TC_FWD_STAGES));
-  cudaFuncSetAttribute(K_TC_FWD_BIG(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  cudaFuncSetAttribute(K_TC_DX_BIG(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  cudaFuncSetAttribute(K_TC_DW_BIG(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  cudaFuncSetAttribute(K_TC_FWD2(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  cudaFuncSetAttribute(K_TC_DX2(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  cudaFuncSetAttribute(K_TC_DW(F, V), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(128, TC_DW_STAGES));
-  if (!V) cudaFuncSetAttribute(k_dw_adam_tc<F, (F ? 32 : 16)>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcAdamCfg<F, (F ? 32 : 16)>::SMEM);
-}
-void tc_set_smem_attr() {
-  tc_set_smem_attr_fmt<false, false>(); tc_set_smem_attr_fmt<true, false>();
-  tc_set_smem_attr_fmt<false, true>(); tc_set_smem_attr_fmt<true, true>();
-}
-
-// fills the tcgen05 view of one GEMM (shapes in the fp32 path's convention); mode 0 fwd, 1 dX, 2 dW
-// esz = 2: g.A / g.B point at fp16 operand copies (pitches in elements); the epilogue side of g is unchanged.
 // Large-batch forward / dX (more than 256 stacked rows): batch rows per tile and feature sub-tiles per CTA.  256 x 256
 // tiles are the efficient shape, but a narrow layer or a rank's slice of the batch leaves most of the 148 SMs without a
 // tile (D layer 1 at 3072 local rows: 4 x 12 = 48 CTAs; the generator's dX over K = 12032: 2 x 4 = 8 CTAs, each alone on
@@ -1262,21 +1256,27 @@ void tc_pick_tile(int rows, int feats, int nf, int* bn, bool* mt1) {
   for (int b : {256, 128, 64}) { *bn = b; if (tiles(b, true) >= 120) return; }
 }
 
+int tc_mode(const OpInfo& oi) { return oi.at ? 2 : (oi.bt ? 1 : 0); }   // 0 fwd, 1 dX, 2 dW
+
+// Batch rows per tile (MMA-N) of one fold's GEMM; bn_big: those of a forward / dX with more than 256 rows (tc_pick_tile).
+int tc_fold_bn(const GemmDesc& g, int mode, int bn_big) {
+  if (mode == 2) return g.K > 512 ? 256 : 128;   // dW: a long contraction (large batch) is a regular big GEMM: 256 x 256 tiles
+  return g.M <= 256 ? round_up(g.M, 16) : bn_big;
+}
+
+// fills the tcgen05 view of one GEMM (shapes in the fp32 path's convention)
+// esz = 2: g.A / g.B point at fp16 operand copies (pitches in elements); the epilogue side of g is unchanged.
 bool tc_fill_op(EncodeTiledFn fn, TcOp& t, const GemmDesc& g, int mode, int esz = 4, int bn_big = 256) {
   t.g = g;
   t.esz = esz;
   t.ME = g.N; t.NE = g.M; t.KE = g.K;
+  t.bn = tc_fold_bn(g, mode, bn_big);
   const int kb = 128 / esz;   // contraction rows of an MN-major box = elements of one 128-byte row
-  if (mode == 0) {            // forward: C[M rows, N feats] = act[M, K] @ W[K, N]
-    t.bn = g.M <= 256 ? round_up(g.M, 16) : bn_big;
+  if (mode == 0)              // forward: C[M rows, N feats] = act[M, K] @ W[K, N]
     return make_map(fn, &t.mapA, g.B, g.N, g.K, g.ldb, kb, true, 0, esz) && make_map(fn, &t.mapB, g.A, g.K, g.M, g.lda, t.bn, false, 0, esz);
-  }
-  if (mode == 1) {            // dX: C[M rows, N in-feats] = dZ[M, K] @ W[N, K]^T
-    t.bn = g.M <= 256 ? round_up(g.M, 16) : bn_big;
+  if (mode == 1)              // dX: C[M rows, N in-feats] = dZ[M, K] @ W[N, K]^T
     return make_map(fn, &t.mapA, g.B, g.K, g.N, g.ldb, 128, false, 0, esz) && make_map(fn, &t.mapB, g.A, g.K, g.M, g.lda, t.bn, false, 0, esz);
-  }
   // dW: C[M in-feats(+1), N out-feats] = act[K rows, M]^T @ dZ[K rows, N]
-  t.bn = g.K > 512 ? 256 : 128;   // a long contraction (large batch) is a regular big GEMM: 256 x 256 tiles
   return make_map(fn, &t.mapA, g.B, g.N, g.K, g.ldb, kb, true, 0, esz) && make_map(fn, &t.mapB, g.A, g.M, g.K, g.lda, kb, true, 0, esz);
 }
 
@@ -1289,28 +1289,88 @@ int tc_debug_gemm(mrgan_handle* h, int mode, const GemmDesc& g, int esz) {
   TcOp* d = nullptr;
   CK(tmp.alloc(&d, sizeof(TcOp)));
   CK(cudaMemcpyAsync(d, &t, sizeof(t), cudaMemcpyHostToDevice, h->stream));
-  tc_set_smem_attr();
-  dim3 grid((t.ME + 127) / 128, (t.NE + t.bn - 1) / t.bn, 1);
+  const TcKernel& k = tc_kernel(mode == 0 ? TC_FWD : (mode == 1 ? TC_DX : TC_DW), esz == 2, tc_variant(h));
+  CK(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, k.smem_attr));
+  const dim3 grid((t.ME + 127) / 128, (t.NE + t.bn - 1) / t.bn, 1);
   const OperandMode om0{0, 1.0f, nullptr, nullptr};
-  const bool f16 = esz == 2;
-  if (mode == 0) TC_LAUNCH(h, f16, K_TC_FWD, grid, dim3(TC_FWD_THREADS), tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream, (const TcOp*)d, h->d_folds, 0, h->hp, om0);
-  else if (mode == 1) TC_LAUNCH(h, f16, K_TC_DX, grid, dim3(TC_FWD_THREADS), tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream, (const TcOp*)d, h->d_folds, 0, h->hp, om0);
-  else TC_LAUNCH(h, f16, K_TC_DW, grid, dim3(TC_DW_THREADS), tc_smem_bytes(t.bn, TC_DW_STAGES), h->stream, (const TcOp*)d, h->d_folds, 0, h->hp, om0);
+  launch_k(h, k.fn, grid, k.threads, tc_smem_bytes(t.bn, mode == 2 ? TC_DW_STAGES : TC_FWD_STAGES), h->stream, (const TcOp*)d,
+           h->d_folds, 0, h->hp, om0);
   CK(cudaStreamSynchronize(h->stream));
   return MRGAN_OK;
 }
 
-// the tcgen05 views of op's descriptors, one per fold (t[0 .. nf)), and the op's tile geometry; no-op for an unused op
+// The launch plan of one op: which k_gemm_tc instantiation runs it (or the fused dW+Adam kernel), on what grid and with
+// how much shared memory, from the op's shapes over the folds, the precision and variant, the fused heads and the
+// fused-Adam flag.  Clears the chosen kernel for its shared memory.  No-op for an unused op.
+int tc_plan_op(mrgan_handle* h, int op) {
+  const OpInfo& oi = h->ops[op];
+  TcPlan& p = h->tc_plan[op];
+  p = TcPlan();
+  if (!oi.used) return MRGAN_OK;
+  const int nf = h->nf, mode = tc_mode(oi);
+  const bool f16 = h->om.mode == 2;
+  bool mt1 = false;   // large-batch forward / dX whose 256 x 256 tiling would leave SMs idle: 128-feature CTAs
+  if (mode != 2 && oi.maxM > 256) tc_pick_tile(oi.maxM, oi.maxN, nf, &p.bn_big, &mt1);
+  for (int f = 0; f < nf; ++f) {
+    const GemmDesc& g = h->h_descs[(size_t)op * nf + f];
+    p.bn = std::max(p.bn, tc_fold_bn(g, mode, p.bn_big));
+    p.maxME = std::max(p.maxME, g.N);
+    p.maxNE = std::max(p.maxNE, g.M);
+  }
+  p.gx = (p.maxME + 127) / 128;
+  // two feature sub-tiles per CTA when the layer is wide enough and the 4-stage ring still fits in 227 KB
+  const bool mt2 = p.maxME >= 500 && tc_smem_bytes(p.bn, TC_FWD_STAGES, 2) <= kTcSmemMax;
+  const bool head_mt2 = (h->tc_heads & 2) && op == OP_D5G;      // feature matching: one CTA sums the loss over all 250 features
+  int role;
+  if (p.bn == 256 && (oi.at || p.maxME >= 500) && !mt1) {     // large-batch regime
+    role = mode == 0 ? TC_FWD_BIG : (mode == 1 ? TC_DX_BIG : TC_DW_BIG);
+    p.gx = (p.maxME + 255) / 256;
+    p.smem = tc_smem_bytes(256, TC_BIG_STAGES, 2);
+    // Large-batch dW without the fused Adam: the narrow layers' gradients are a handful of 256x256 tiles with a contraction
+    // of thousands of rows -> split the contraction over ~2 CTAs per SM, partial products to a workspace (tc_setup), summed
+    // in slice order.
+    if (oi.at && !h->tc_fused_adam) {
+      const int kblk = f16 ? 64 : TC_KBLK;      // contraction rows per stage (one 128-byte row of operand elements)
+      const int nkb = (h->h_descs[(size_t)op * nf].K + kblk - 1) / kblk;
+      const int tiles = ((p.maxME + 255) / 256) * ((p.maxNE + 255) / 256) * nf;
+      const int ks = std::min(std::min(2 * 148 / tiles, nkb / 8), 32);
+      if (ks >= 2) {
+        const int per = (nkb + ks - 1) / ks;
+        p.ks = (nkb + per - 1) / per;           // no empty slice
+      }
+    }
+  } else if (!oi.at && !mt1 && (mt2 || head_mt2)) {
+    role = mode == 0 ? TC_FWD2 : TC_DX2;
+    p.gx = (p.maxME + 255) / 256;
+    p.smem = tc_smem_bytes(p.bn, TC_FWD_STAGES, 2);
+  } else if (!oi.at) {
+    // one CTA per SM anyway once the stages exceed half the shared memory: take the whole TMEM then (noise parking)
+    p.smem = tc_smem_bytes(p.bn, TC_FWD_STAGES);
+    const bool whole = 2 * p.smem > kTcSmemMax;
+    role = mode == 0 ? (whole ? TC_FWD_N : TC_FWD) : (whole ? TC_DX_N : TC_DX);
+  } else if (h->tc_fused_adam) {
+    p.fused = true;
+    if (f16) CK(cudaFuncSetAttribute(k_dw_adam_tc<true, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcAdamCfg<true, 32>::SMEM));
+    else CK(cudaFuncSetAttribute(k_dw_adam_tc<false, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcAdamCfg<false, 16>::SMEM));
+    return MRGAN_OK;
+  } else {
+    role = TC_DW;
+    p.smem = tc_smem_bytes(p.bn, TC_DW_STAGES);
+  }
+  p.k = &tc_kernel(role, f16, tc_variant(h));
+  CK(cudaFuncSetAttribute(p.k->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, p.k->smem_attr));
+  return MRGAN_OK;
+}
+
+// the launch plan of op and the tcgen05 views of its descriptors, one per fold (ts[0 .. nf)); no-op for an unused op
 int tc_make_op(mrgan_handle* h, EncodeTiledFn fn, int op, TcOp* ts) {
+  TRY(tc_plan_op(h, op));
   const OpInfo& oi = h->ops[op];
   if (!oi.used) return MRGAN_OK;
-  const int nf = h->nf;
+  const int nf = h->nf, mode = tc_mode(oi), bn_big = h->tc_plan[op].bn_big;
   for (int f = 0; f < nf; ++f) {
     const GemmDesc& g = h->h_descs[(size_t)op * nf + f];
     TcOp& t = ts[f];
-    const int mode = (!oi.at && !oi.bt) ? 0 : ((!oi.at && oi.bt) ? 1 : 2);
-    int bn_big = 256;
-    if (mode != 2 && oi.maxM > 256) { bool m1; tc_pick_tile(oi.maxM, oi.maxN, nf, &bn_big, &m1); h->tc_mt1[op] = m1; }
     if (h->om.mode == 2) {    // operands come from the fp16 copies (same element offsets and pitches as the fp32 buffers)
       GemmDesc gh = g;
       gh.A = reinterpret_cast<const float*>(h->harena + (g.A - h->om.fbase));
@@ -1326,9 +1386,6 @@ int tc_make_op(mrgan_handle* h, EncodeTiledFn fn, int op, TcOp* ts) {
       else if (op == OP_D5G && (h->tc_heads & 2)) { t.head = HEAD_FM; t.hd = h->d_loss + f; }
       else if (op == OP_G1 && (h->tc_heads & 4)) { t.head = HEAD_BN; t.hd = h->d_bn + f; }
     }
-    if (t.bn > h->tc_bn[op]) h->tc_bn[op] = t.bn;
-    if (t.ME > h->tc_maxME[op]) h->tc_maxME[op] = t.ME;
-    if (t.NE > h->tc_maxNE[op]) h->tc_maxNE[op] = t.NE;
   }
   return MRGAN_OK;
 }
@@ -1348,38 +1405,23 @@ int tc_setup(mrgan_handle* h) {
     const int rc = tc_make_op(h, fn, op, &ops[(size_t)op * nf]);
     if (rc != MRGAN_OK) return rc;
   }
-  // Large-batch dW without the fused Adam: the narrow layers' gradients are a handful of 256x256 tiles with a contraction of
-  // thousands of rows -> split the contraction over ~2 CTAs per SM, partial products to a workspace, summed in slice order.
-  if (!h->tc_fused_adam) {
-    size_t ws_floats = 0;
-    for (int op = 0; op < NUM_OPS; ++op) {
-      const OpInfo& oi = h->ops[op];
-      if (!oi.used || !oi.at || h->tc_bn[op] != 256) continue;
-      const int kblk = h->om.mode == 2 ? 64 : TC_KBLK;      // contraction rows per stage (one 128-byte row of operand elements)
-      const int nkb = (ops[(size_t)op * nf].KE + kblk - 1) / kblk;
-      const int tiles = ((h->tc_maxME[op] + 255) / 256) * ((h->tc_maxNE[op] + 255) / 256) * nf;
-      int ks = std::min(std::min(2 * 148 / tiles, nkb / 8), 32);
-      if (ks < 2) continue;
-      const int per = (nkb + ks - 1) / ks;
-      ks = (nkb + per - 1) / per;                       // no empty slice
-      h->tc_ksplit[op] = ks;
-      for (int f = 0; f < nf; ++f) {
+  // the split-K dW ops (tc_plan_op): the partial products of each contraction slice, laid out like C
+  size_t ws_floats = 0;
+  for (int op = 0; op < NUM_OPS; ++op)
+    for (int f = 0; f < nf && h->tc_plan[op].ks > 1; ++f) {
+      TcOp& t = ops[(size_t)op * nf + f];
+      t.ws_stride = t.NE * t.g.ldc;
+      t.ws = reinterpret_cast<float*>(ws_floats);     // offset now, pointer once the workspace exists
+      ws_floats += (size_t)h->tc_plan[op].ks * t.ws_stride;
+    }
+  if (ws_floats) {
+    if (cudaMalloc(&h->d_tcws, ws_floats * sizeof(float)) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMalloc split-K workspace");
+    cudaMemset(h->d_tcws, 0, ws_floats * sizeof(float));      // pad columns are never written and must read as zero
+    for (int op = 0; op < NUM_OPS; ++op)
+      for (int f = 0; f < nf && h->tc_plan[op].ks > 1; ++f) {
         TcOp& t = ops[(size_t)op * nf + f];
-        t.ws_stride = t.NE * t.g.ldc;
-        t.ws = reinterpret_cast<float*>(ws_floats);     // offset now, pointer once the workspace exists
-        ws_floats += (size_t)ks * t.ws_stride;
+        t.ws = h->d_tcws + reinterpret_cast<size_t>(t.ws);
       }
-    }
-    if (ws_floats) {
-      if (cudaMalloc(&h->d_tcws, ws_floats * sizeof(float)) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMalloc split-K workspace");
-      cudaMemset(h->d_tcws, 0, ws_floats * sizeof(float));      // pad columns are never written and must read as zero
-      for (int op = 0; op < NUM_OPS; ++op)
-        if (h->tc_ksplit[op] > 1)
-          for (int f = 0; f < nf; ++f) {
-            TcOp& t = ops[(size_t)op * nf + f];
-            t.ws = h->d_tcws + reinterpret_cast<size_t>(t.ws);
-          }
-    }
   }
   if (cudaMalloc(&h->d_tcops, ops.size() * sizeof(TcOp)) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMalloc tc ops");
   if (cudaMemcpy(h->d_tcops, ops.data(), ops.size() * sizeof(TcOp), cudaMemcpyHostToDevice) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMemcpy tc ops");
@@ -1434,7 +1476,6 @@ int tc_setup(mrgan_handle* h) {
     if (cudaMalloc(&h->d_ranges_tc[n], nf * sizeof(AdamRange)) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMalloc");
     if (cudaMemcpy(h->d_ranges_tc[n], (n == 0 ? r0 : r1).data(), nf * sizeof(AdamRange), cudaMemcpyHostToDevice) != cudaSuccess) return fail(nullptr, MRGAN_ERR_CUDA, "cudaMemcpy adam ranges");
   }
-  tc_set_smem_attr();
   return MRGAN_OK;
 }
 
@@ -1457,9 +1498,8 @@ void tc_teardown(mrgan_handle* h) {
   if (h->d_tcadam) cudaFree(h->d_tcadam);
   if (h->d_tcws) cudaFree(h->d_tcws);
   h->d_tcws = nullptr;
-  for (int i = 0; i < NUM_OPS; ++i) h->tc_ksplit[i] = 0;
   for (int n = 0; n < 2; ++n) { if (h->d_ranges_tc[n]) cudaFree(h->d_ranges_tc[n]); h->d_ranges_tc[n] = nullptr; }
-  for (int i = 0; i < NUM_OPS; ++i) { h->tc_bn[i] = 0; h->tc_maxME[i] = 0; h->tc_maxNE[i] = 0; h->tc_mt1[i] = false; }
+  for (int i = 0; i < NUM_OPS; ++i) h->tc_plan[i] = TcPlan();
   h->d_tcadam = nullptr;
   h->d_tcops = nullptr;
 }
@@ -1470,8 +1510,8 @@ void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cu
   const bool f16 = h->om.mode == 2;
   int gx = 0, gy = 0;
   for (int l = 0; l < nlayers; ++l) {
-    gx = std::max(gx, (h->tc_maxME[op + l] + 127) / 128);
-    gy = std::max(gy, (h->tc_maxNE[op + l] + 127) / 128);
+    gx = std::max(gx, (h->tc_plan[op + l].maxME + 127) / 128);
+    gy = std::max(gy, (h->tc_plan[op + l].maxNE + 127) / 128);
   }
   const dim3 grid(gx, gy, nlayers * nfl);
   const TcAdamOp* ad = h->d_tcadam + (size_t)op * h->nf + f0;
@@ -1479,56 +1519,20 @@ void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cu
   else launch_k(h, k_dw_adam_tc<false, 16>, grid, dim3(192), TcAdamCfg<false, 16>::SMEM, st, ad, h->d_folds, h->hp, nfl, h->nf);
 }
 
-// the fused-Adam dW path is active (tcgen05 precision, reference batch regime): narrow layers may share launches
-bool tc_dw_merge(const mrgan_handle* h) { return h->cfg.precision != MRGAN_PREC_FP32 && h->d_tcadam != nullptr; }
-
-bool tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st) {
-  const OpInfo& oi = h->ops[op];
-  const bool f16 = h->om.mode == 2;
-  const int bn = h->tc_bn[op];
-  int NE = h->tc_maxNE[op];
-  if (rows_override > 0 && !oi.at) NE = rows_override;
-  dim3 grid((h->tc_maxME[op] + 127) / 128, (NE + bn - 1) / bn, nfl);
+// one launch of op's plan over folds [f0, f0 + nfl); rows_override > 0: fewer batch rows (forward / dX)
+void tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st, const OperandMode& om) {
+  const TcPlan& p = h->tc_plan[op];
+  if (p.fused) { tc_launch_dw_adam(h, op, 1, f0, nfl, st); return; }
+  const bool at = h->ops[op].at;
+  const int NE = rows_override > 0 && !at ? rows_override : p.maxNE;
+  const dim3 grid(p.gx, (NE + p.bn - 1) / p.bn, nfl * p.ks);
   const TcOp* d = (op < NUM_OPS ? h->d_tcops + (size_t)op * h->nf : h->sal.tcops + (size_t)(op - NUM_OPS) * h->nf) + f0;
-  if (bn == 256 && (oi.at || h->tc_maxME[op] >= 500) && !h->tc_mt1[op]) {     // large-batch regime
-    grid.x = (h->tc_maxME[op] + 255) / 256;
-    const size_t smem = tc_smem_bytes(256, TC_BIG_STAGES, 2);
-    if (oi.at) {
-      const int ks = h->tc_ksplit[op] > 1 ? h->tc_ksplit[op] : 1;
-      grid.z = nfl * ks;
-      TC_LAUNCH(h, f16, K_TC_DW_BIG, grid, dim3(TC_FWD_THREADS), smem, st, d, h->d_folds, ks, h->hp, h->om);
-      if (ks > 1) {
-        const int n4 = h->tc_maxNE[op] * pitch8(h->tc_maxME[op]) / 4;
-        launch_k(h, k_splitk_reduce, dim3(std::min((n4 + 255) / 256, 1184), nfl, 1), dim3(256), 0, st, d, ks);
-      }
-    } else if (!oi.bt) TC_LAUNCH(h, f16, K_TC_FWD_BIG, grid, dim3(TC_FWD_THREADS), smem, st, d, h->d_folds, rows_override, h->hp, h->om);
-    else TC_LAUNCH(h, f16, K_TC_DX_BIG, grid, dim3(TC_FWD_THREADS), smem, st, d, h->d_folds, rows_override, h->hp, h->om);
-    return true;
+  // dW kernels take the number of contraction slices in place of rows_override
+  launch_k(h, p.k->fn, grid, p.k->threads, p.smem, st, d, h->d_folds, at ? p.ks : rows_override, h->hp, om);
+  if (p.ks > 1) {
+    const int n4 = p.maxNE * pitch8(p.maxME) / 4;
+    launch_k(h, k_splitk_reduce, dim3(std::min((n4 + 255) / 256, 1184), nfl, 1), dim3(256), 0, st, d, p.ks);
   }
-  const bool head_mt2 = (h->tc_heads & 2) && op == OP_D5G;      // feature matching: one CTA sums the loss over all 250 features
-  if (!oi.at && !h->tc_mt1[op] && (tc_use_mt2(h->tc_maxME[op], bn) || head_mt2)) {
-    grid.x = (h->tc_maxME[op] + 255) / 256;
-    const size_t smem = tc_smem_bytes(bn, TC_FWD_STAGES, 2);
-    if (!oi.bt) TC_LAUNCH(h, f16, K_TC_FWD2, grid, dim3(TC_FWD_THREADS), smem, st, d, h->d_folds, rows_override, h->hp, h->om);
-    else TC_LAUNCH(h, f16, K_TC_DX2, grid, dim3(TC_FWD_THREADS), smem, st, d, h->d_folds, rows_override, h->hp, h->om);
-    return true;
-  }
-  if (!oi.at && !oi.bt) {
-    // one CTA per SM anyway once the stages exceed half the shared memory: take the whole TMEM then (noise parking)
-    if (2 * tc_smem_bytes(bn, TC_FWD_STAGES) > 227 * 1024)
-      TC_LAUNCH(h, f16, K_TC_FWD_N, grid, dim3(TC_FWD_THREADS), tc_smem_bytes(bn, TC_FWD_STAGES), st, d, h->d_folds, rows_override, h->hp, h->om);
-    else
-      TC_LAUNCH(h, f16, K_TC_FWD, grid, dim3(TC_FWD_THREADS), tc_smem_bytes(bn, TC_FWD_STAGES), st, d, h->d_folds, rows_override, h->hp, h->om);
-  }
-  else if (!oi.at && oi.bt) {
-    if (2 * tc_smem_bytes(bn, TC_FWD_STAGES) > 227 * 1024)
-      TC_LAUNCH(h, f16, K_TC_DX_N, grid, dim3(TC_FWD_THREADS), tc_smem_bytes(bn, TC_FWD_STAGES), st, d, h->d_folds, rows_override, h->hp, h->om);
-    else
-      TC_LAUNCH(h, f16, K_TC_DX, grid, dim3(TC_FWD_THREADS), tc_smem_bytes(bn, TC_FWD_STAGES), st, d, h->d_folds, rows_override, h->hp, h->om);
-  }
-  else if (h->d_tcadam) { tc_launch_dw_adam(h, op, 1, f0, nfl, st); return true; }
-  else TC_LAUNCH(h, f16, K_TC_DW, grid, dim3(TC_DW_THREADS), tc_smem_bytes(bn, TC_DW_STAGES), st, d, h->d_folds, 0, h->hp, h->om);
-  return true;
 }
 
 }  // namespace
@@ -1676,6 +1680,7 @@ int mrgan_create(const mrgan_config* cfg, const mrgan_fold_shape* folds, mrgan_h
     if (rc != MRGAN_OK) return cleanup(rc);
   }
   if (cfg->precision != MRGAN_PREC_FP32) {
+    h->tc_fused_adam = true;
     int rc = tc_setup(h);
     if (rc != MRGAN_OK) return cleanup(rc);
   }
@@ -2345,42 +2350,6 @@ int mrgan_debug_gemm(mrgan_handle* h, int mode, int M, int N, int K, const float
   CK(cudaMemcpy2DAsync(C, (size_t)N * 4, dC, (size_t)ldc * 4, (size_t)N * 4, M, cudaMemcpyDeviceToHost, h->stream));
   return complete(h);
 }
-
-int mrgan_debug_gemm_time(mrgan_handle* h, int mode, int M, int N, int K, int groups, int reps, float* ms) {
-  TRY(enter(h, "debug_gemm_time", NETS));
-  if (mode < 0 || mode > 2 || M < 1 || N < 1 || K < 1 || groups < 1 || reps < 1 || !ms) return fail(h, MRGAN_ERR_ARG, "debug_gemm_time: bad argument");
-  TRY(ready(h, "debug_gemm_time", NETS));
-  EncodeTiledFn fn = tc_encoder();
-  if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available");
-  const int ar = mode == 2 ? K : M, ac = mode == 2 ? M : K;
-  const int br = mode == 1 ? N : K, bc = mode == 1 ? K : N;
-  const int lda = pitch8(ac), ldb = pitch8(bc), ldc = pitch8(N);
-  const size_t sa = (size_t)ar * lda, sb = (size_t)br * ldb, sc = (size_t)M * ldc;
-  Temps tmp;
-  float* buf = nullptr;
-  CK(tmp.alloc(&buf, (sa + sb + sc) * groups * 4));
-  CK(cudaMemsetAsync(buf, 0, (sa + sb + sc) * groups * 4, h->stream));
-  std::vector<TcOp> ops(groups);
-  memset(ops.data(), 0, sizeof(TcOp) * groups);
-  for (int g = 0; g < groups; ++g) {
-    float* A = buf + (sa + sb + sc) * g; float* B = A + sa; float* C = B + sb;
-    GemmDesc d = make_desc(A, lda, B, ldb, C, ldc, M, N, K, mode == 0 ? EPI_FWD : (mode == 1 ? EPI_DX : EPI_STORE), ACT_NONE, 0);
-    if (!tc_fill_op(fn, ops[g], d, mode)) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-  }
-  TcOp* dops = nullptr;
-  CK(tmp.alloc(&dops, sizeof(TcOp) * groups));
-  CK(cudaMemcpyAsync(dops, ops.data(), sizeof(TcOp) * groups, cudaMemcpyHostToDevice, h->stream));
-  tc_set_smem_attr();
-  const TcOp& t = ops[0];
-  const dim3 grid((t.ME + 127) / 128, (t.NE + t.bn - 1) / t.bn, groups);
-  const OperandMode om0{0, 1.0f, nullptr, nullptr};
-  return time_reps(h, reps, [&]() {
-    if (mode == 0) launch_k(h, K_TC_FWD(false, false), grid, TC_FWD_THREADS, tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream, dops, h->d_folds, 0, h->hp, om0);
-    else if (mode == 1) launch_k(h, K_TC_DX(false, false), grid, TC_FWD_THREADS, tc_smem_bytes(t.bn, TC_FWD_STAGES), h->stream, dops, h->d_folds, 0, h->hp, om0);
-    else launch_k(h, K_TC_DW(false, false), grid, TC_DW_THREADS, tc_smem_bytes(t.bn, TC_DW_STAGES), h->stream, dops, h->d_folds, 0, h->hp, om0);
-  }, ms);
-}
-
 
 // ------------------------------------------------------------------ RBF C-SVC (MRGAN_MODEL_SVM, csrc/kernels_svm.cuh)
 static void svm_launch(mrgan_handle* h, int phase) {

@@ -513,11 +513,6 @@ class FoldGroup:
         self._chk(self.lib.mrgan_debug_gemm(self._h, mode, M, N, K, _lib.fptr(A), _lib.fptr(B), _lib.fptr(out), int(use_tc)))
         return out
 
-    def debug_gemm_time(self, mode, M, N, K, groups=1, reps=20):
-        out = np.zeros(1, dtype=np.float32)
-        self._chk(self.lib.mrgan_debug_gemm_time(self._h, mode, M, N, K, groups, reps, _lib.fptr(out)))
-        return float(out[0])
-
     TIME_OPS = {"adam_d": 0, "adam_g": 1, "dw1": 2, "fwd1": 3, "disc_step": 4, "gen_step": 5, "dx1": 6,
                 "svm_kmat": 7, "svm_smo": 8, "svm_predict": 9, "saliency": 10}
 

@@ -180,9 +180,6 @@ def _cases():
     add("debug_gemm/model-S", "S", lambda l, h, b: l.mrgan_debug_gemm(h, 0, 2, 2, 2, b.F, b.F, b.F, 0), STATE, nets)
     add("debug_gemm/mode", "G", lambda l, h, b: l.mrgan_debug_gemm(h, 3, 2, 2, 2, b.F, b.F, b.F, 0), ARG, "bad argument")
     add("debug_gemm/out", "G", lambda l, h, b: l.mrgan_debug_gemm(h, 0, 2, 2, 2, b.F, b.F, None, 0), ARG, "bad argument")
-    add("debug_gemm_time/null", None, lambda l, h, b: l.mrgan_debug_gemm_time(h, 0, 2, 2, 2, 1, 1, b.F), ARG, "null")
-    add("debug_gemm_time/model-S", "S", lambda l, h, b: l.mrgan_debug_gemm_time(h, 0, 2, 2, 2, 1, 1, b.F), STATE, nets)
-    add("debug_gemm_time/groups", "G", lambda l, h, b: l.mrgan_debug_gemm_time(h, 0, 2, 2, 2, 0, 1, b.F), ARG, "bad argument")
 
     # data-parallel set-up
     add("dp_init/null", None, lambda l, h, b: l.mrgan_dp_init(h, 0, 2, b.id), ARG, "null")
