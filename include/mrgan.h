@@ -255,6 +255,31 @@ int  mrgan_input_grad(mrgan_handle* h, int fold, const float* x, int n, const in
  * a pending asynchronous epoch, whose statistics it leaves unchanged, and changes no later result of the handle. */
 int  mrgan_saliency(mrgan_handle* h, float* profile);
 
+/* Samples of a trained GAN fold's generator and D's view of them (GAN handles only).
+ *   A sample is G's linear output G(z) (mr_gan.py:110-114) in the fold's SCALED input space, without the sigma = 0.3
+ *   GaussianNoise, which is D's input layer (mr_gan.py:118).  The reference never runs G in test phase and never trains
+ *   BatchNorm's moving averages, so rows are made the only way G ever ran: in consecutive batches of cfg.batch rows, each
+ *   normalised with its own biased batch statistics.  n must be a positive multiple of cfg.batch.
+ *   z: the caller's rows [n][noise_dim], or NULL = N(0,1) drawn on the device from the fold key with the Philox counter
+ *   (row >> 2, col, step = seed, tensor id 6), rows numbered 0 .. n-1 over the request (independent of how the library chunks
+ *   them).  Tensor id 6 is used by no training stream.
+ * mrgan_generate: x [n][D_fold], fp32.  Needs the fold's parameters only.
+ * mrgan_sample_stats: for every fold, n generated rows (z drawn from seed) and the fold's resident test rows ("real"), seen by D
+ *   exactly as mrgan_predict_rows sees rows: the phase-0 forward, the generated rows in the operand format predict_rows gives
+ *   them (tf32-rounded or fp16), so predict_rows(fold, mrgan_generate(fold, n, seed, NULL)) reproduces the logits used here.
+ *     counts [n_folds][K]: classes of D's predictions of the generated rows (first maximal logit);
+ *     score  [n_folds][2]: mean of sigma(logsumexp(l)), the K-logit discriminator's "real" probability (mr_gan.py:147-149);
+ *     mean   [n_folds][2][250], cov [n_folds][2][250][250]: mean and unbiased covariance (n - 1, np.cov) of D's layer-5
+ *            phase-0 features, the mid features feature matching compares (mr_gan.py:127,152-154); a side with one row has NaN cov.
+ *   [.][0] = generated rows, [.][1] = real rows.  Sums in double, every element in row order: bitwise reproducible and
+ *   independent of the fold grouping and of the chunking.  Needs loaded folds.
+ * Memory: a workspace on the first call (a handle that never calls them allocates nothing more).
+ * MRGAN_ERR_ARG: null pointer, fold out of range, n < 1 or n % batch != 0.  MRGAN_ERR_STATE: an NN or SVM handle, a
+ * data-parallel or virtual-rank handle, unloaded folds (mrgan_sample_stats).  Each call first completes a pending asynchronous
+ * epoch and changes no later result of the handle. */
+int  mrgan_generate(mrgan_handle* h, int fold, int n, uint32_t seed, const float* z, float* x);
+int  mrgan_sample_stats(mrgan_handle* h, int n, uint32_t seed, int32_t* counts, double* score, double* mean, double* cov);
+
 /* Utilities used by tests and bench */
 int  mrgan_fill_normal(mrgan_handle* h, int fold, int step, int tensor_id, int rows, int cols,
                        int row0, float* dst /* host [rows, cols] */);
@@ -271,7 +296,9 @@ enum { MRGAN_TIME_ADAM_D = 0, MRGAN_TIME_ADAM_G = 1, MRGAN_TIME_DW1 = 2, MRGAN_T
        MRGAN_TIME_SVM_SMO = 8,      /* the SMO solver of every (fold, class pair) */
        MRGAN_TIME_SVM_PREDICT = 9, /* decision values, vote and error count of every test row */
        /* GAN / NN handles, read-only (the training state is unchanged): */
-       MRGAN_TIME_SALIENCY = 10 }; /* mrgan_saliency's pass: eval forward, seed, dX chain and profile of every fold */
+       MRGAN_TIME_SALIENCY = 10,   /* mrgan_saliency's pass: eval forward, seed, dX chain and profile of every fold */
+       MRGAN_TIME_SAMPLE_STATS = 11 }; /* GAN: mrgan_sample_stats's pass with n = batch * floor(NE / batch) rows (one chunk),
+                                          NE = max(3 batch, n_test of every fold), seed 0 */
 int  mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg);
 /* Debug/test hook: copy an intermediate buffer of the last step of one fold to the host
  * (dst is [rows, cols] dense).  which: 0..5 = noisy layer inputs a[l], 10+l = post-ReLU h[l],

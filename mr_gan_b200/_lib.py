@@ -33,6 +33,7 @@ class EpochStats(C.Structure):
 
 _fp = C.POINTER(C.c_float)
 _ip = C.POINTER(C.c_int32)
+_dp = C.POINTER(C.c_double)
 _H = C.c_void_p
 
 # every symbol include/mrgan.h declares: name -> (restype, argtypes)
@@ -80,6 +81,8 @@ SYMBOLS = {
     "mrgan_confusion": (C.c_int, [_H, _ip]),
     "mrgan_input_grad": (C.c_int, [_H, C.c_int, _fp, C.c_int, _ip, _fp]),
     "mrgan_saliency": (C.c_int, [_H, _fp]),
+    "mrgan_generate": (C.c_int, [_H, C.c_int, C.c_int, C.c_uint32, _fp, _fp]),
+    "mrgan_sample_stats": (C.c_int, [_H, C.c_int, C.c_uint32, _ip, _dp, _dp, _dp]),
     "mrgan_fill_normal": (C.c_int, [_H, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _fp]),
     "mrgan_adam_flat": (C.c_int, [_H, _fp, _fp, _fp, _fp, C.c_int64, C.c_int]),
     "mrgan_time_op": (C.c_int, [_H, C.c_int, C.c_int, _fp]),
@@ -132,3 +135,7 @@ def fptr(a):
 
 def iptr(a):
     return a.ctypes.data_as(_ip)
+
+
+def dptr(a):
+    return a.ctypes.data_as(_dp)

@@ -75,7 +75,8 @@ def check(meta, expected, path):
                                      % (path, k, meta.get(k), want))
 
 
-def _scaler(job):
+def job_scaler(job):
+    """The float64 StandardScaler (mean, scale) of a job's training rows (mr_gan.py:96-98)."""
     if 'train_idx' in job:
         x = np.asarray(job['X'])[np.asarray(job['train_idx'])]
     else:
@@ -102,7 +103,7 @@ def save(path, fg, fold, job, *, seed, epochs, epochs_done, perm, rng_state=None
             arrays['%s%d' % (k[0], net)] = np.concatenate([np.asarray(a, np.float32).ravel() for a in st[k][i]])
     y_test = np.asarray(job['y'])[np.asarray(job['test_idx'])] if 'train_idx' in job else job['trainTestSets'][3]
     arrays['y_test'] = np.asarray(y_test, np.int32)
-    arrays['scaler_mean'], arrays['scaler_scale'] = _scaler(job)
+    arrays['scaler_mean'], arrays['scaler_scale'] = job_scaler(job)
     d = os.path.dirname(os.path.abspath(path))
     fd, tmp = tempfile.mkstemp(prefix='.ckpt.', suffix='.tmp', dir=d)
     try:
@@ -182,7 +183,8 @@ def rng_states(rngs):
 
 class LoadedModel(FoldGroup):
     """A one-fold inference group of a saved fold-training: ``predict``, ``predict_rows``, ``confusion``, ``eval``,
-    ``test_error``, ``input_grad`` and ``saliency`` work as on the live group; ``transform`` scales raw rows."""
+    ``test_error``, ``input_grad``, ``saliency``, ``generate`` and ``sample_stats`` work as on the live group; ``transform``
+    scales raw rows and ``inverse_transform`` returns scaled rows (a generated sample) to raw feature units."""
 
     def transform(self, X_raw):
         """Raw feature rows [n, D] -> the fold's scaled input space (the saved scaler, float64, then float32)."""
@@ -190,6 +192,13 @@ class LoadedModel(FoldGroup):
         if x.ndim != 2 or x.shape[1] != self.scaler_mean.size:
             raise ValueError("transform: X_raw must be [n, %d]" % self.scaler_mean.size)
         return ((x - self.scaler_mean) / self.scaler_scale).astype(np.float32)
+
+    def inverse_transform(self, x):
+        """Scaled rows [n, D] (e.g. generate()'s) -> raw feature units, float64 (the saved scaler)."""
+        x = np.asarray(x, dtype=np.float64)
+        if x.ndim != 2 or x.shape[1] != self.scaler_mean.size:
+            raise ValueError("inverse_transform: x must be [n, %d]" % self.scaler_mean.size)
+        return x * self.scaler_scale + self.scaler_mean
 
 
 def load_model(path, device=0):
@@ -248,7 +257,8 @@ class Sweep:
             out = []
             for j in jobs:
                 with load_model(self.path(j), device) as fg:
-                    out += results.collect(fg, [fg.test_error(0)], rep.details, rep.saliency)
+                    out += results.collect(fg, [fg.test_error(0)], rep.details, rep.saliency, samples=getattr(rep, 'samples', False),
+                                           scalers=[(fg.scaler_mean, fg.scaler_scale)])
             return out
         states = [load_state(self.path(j)) for j in jobs] if done else None
 

@@ -14,6 +14,7 @@
 #include <stdint.h>
 
 #define MRGAN_TID_Z 5   // noise stream ids 0..4 = GaussianNoise layers of D, 5 = z
+#define MRGAN_TID_GEN 6 // z of mrgan_generate / mrgan_sample_stats (step word = the caller's seed); no training stream uses it
 
 enum { ACT_NONE = 0, ACT_RELU = 1, ACT_SOFTPLUS = 2, ACT_LEAKY = 3 };   // ACT_LEAKY: LeakyReLU(alpha), others/wganlpctsemi.py:169
 enum { EPI_FWD = 0, EPI_DX = 1, EPI_STORE = 2 };

@@ -807,6 +807,101 @@ k_saliency(const GemmDesc* __restrict__ gx, const EvalDesc* __restrict__ ev, int
   }
 }
 
+// ------------------------------------------------------------------ samples of the generator (mrgan_generate / mrgan_sample_stats)
+// Generator input of rows [row0, row0 + rows) of a request, in the operand format of the handle, with the ones column at nd:
+// the caller's rows zs [rows][nd], or N(0,1) from the fold's key with counter (row >> 2, col, seed, MRGAN_TID_GEN), rows
+// numbered over the whole request (so the draw does not depend on the chunking).  grid (column blocks over nd + 1, 4-row
+// groups of the range, folds); z of fold f0 + blockIdx.z at z + blockIdx.z * zstride.
+__global__ void __launch_bounds__(128)
+k_gen_z(const FoldState* __restrict__ folds, int f0, float* __restrict__ z, size_t zstride, int ldz, const float* __restrict__ zs,
+        int row0, int rows, int nd, uint32_t seed, OperandMode om) {
+  const int c = blockIdx.x * 128 + threadIdx.x;
+  if (c > nd) return;
+  const uint32_t g = ((uint32_t)row0 >> 2) + blockIdx.y;      // global 4-row group
+  float nz[4] = {1.f, 1.f, 1.f, 1.f};
+  if (c < nd && !zs) { const FoldState& fs = folds[f0 + blockIdx.z]; normal4(fs.key0, fs.key1, g, (uint32_t)c, seed, MRGAN_TID_GEN, nz); }
+  float* const zf = z + (size_t)blockIdx.z * zstride;
+  for (int i = 0; i < 4; ++i) {
+    const int r = (int)(4 * g) + i - row0;                      // row inside this chunk
+    if (r < 0 || r >= rows) continue;
+    put_operand(zf + (size_t)r * ldz + c, (c < nd && zs) ? zs[(size_t)r * nd + c] : nz[i], om);
+  }
+}
+
+// Statistics of D's phase-0 view of n rows of one fold (generated rows, or its resident test rows): the layer-5 features
+// feat [n][ldf] (W = 250 columns) and logits [n][ldl].  Raw sums in double, ADDED TO the fold's accumulators, which persist
+// across the chunks of a request: s1[j] += x_j, s2[i][j] += x_i x_j (i <= j, [W][W]), score += sigma(logsumexp(l)), and with
+// counts != null counts[first maximal logit] += 1.  Every accumulator element adds the rows strictly in row order (one
+// thread per element, no atomics), so the sums are bitwise independent of the chunking and of the fold grouping.
+struct StatsDesc { const float* feat; const float* logits; int ldf, ldl, n; double* s1; double* s2; double* score; int* counts; };
+#define SS_W 250                          // D's layer-5 width (mr_gan.py:127)
+#define SS_T 32                           // 32 x 32 tiles of s2
+#define SS_NT ((SS_W + SS_T - 1) / SS_T)
+#define SS_TILES (SS_NT * (SS_NT + 1) / 2)  // upper-triangular tiles; block SS_TILES: s1, score, counts
+#define SS_THREADS 512                    // a tile thread owns elements (ty, tx) and (ty + 16, tx)
+// grid (SS_TILES + 1, folds), SS_THREADS threads; rows > 0: n of every fold (a chunk of generated rows), else d.n
+__global__ void __launch_bounds__(SS_THREADS) k_sample_stats(const StatsDesc* __restrict__ descs, int rows, int K) {
+  const StatsDesc d = descs[blockIdx.y];
+  const int n = rows > 0 ? rows : d.n;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  if (blockIdx.x < SS_TILES) {
+    int I = 0, t = blockIdx.x;
+    while (t >= SS_NT - I) { t -= SS_NT - I; ++I; }
+    const int J = I + t;
+    __shared__ float xi[SS_T][SS_T + 1], xj[SS_T][SS_T + 1];
+    const int i0 = I * SS_T + ty, i1 = i0 + 16, j = J * SS_T + tx;
+    const bool ok0 = i0 < SS_W && j < SS_W && i0 <= j, ok1 = i1 < SS_W && j < SS_W && i1 <= j;
+    double a0 = ok0 ? d.s2[(size_t)i0 * SS_W + j] : 0.0, a1 = ok1 ? d.s2[(size_t)i1 * SS_W + j] : 0.0;
+    for (int r0 = 0; r0 < n; r0 += SS_T) {      // thread (ty, tx) stages rows r0 + ty and r0 + ty + 16, column tx, of both tiles
+      for (int h = 0; h < 2; ++h) {
+        const int rr = ty + 16 * h, r = r0 + rr;
+        xi[rr][tx] = (r < n && I * SS_T + tx < SS_W) ? d.feat[(size_t)r * d.ldf + I * SS_T + tx] : 0.f;
+        xj[rr][tx] = (r < n && J * SS_T + tx < SS_W) ? d.feat[(size_t)r * d.ldf + J * SS_T + tx] : 0.f;
+      }
+      __syncthreads();
+      const int m = min(SS_T, n - r0);
+      for (int k = 0; k < m; ++k) {
+        const double y = xj[k][tx];
+        a0 = fma((double)xi[k][ty], y, a0);
+        a1 = fma((double)xi[k][ty + 16], y, a1);
+      }
+      __syncthreads();
+    }
+    if (ok0) d.s2[(size_t)i0 * SS_W + j] = a0;
+    if (ok1) d.s2[(size_t)i1 * SS_W + j] = a1;
+    return;
+  }
+  // column sums (threads < W), and the per-row score and class in parallel, added in row order by thread W
+  __shared__ double p[SS_THREADS];
+  __shared__ int am[SS_THREADS];
+  const int tid = threadIdx.x;
+  double s = tid < SS_W ? d.s1[tid] : 0.0, sc = tid == SS_W ? *d.score : 0.0;
+  for (int r0 = 0; r0 < n; r0 += SS_THREADS) {
+    const int r = r0 + tid;
+    if (r < n) {
+      const float* l = d.logits + (size_t)r * d.ldl;
+      double mx = l[0];
+      for (int k = 1; k < K; ++k) mx = fmax(mx, (double)l[k]);
+      double se = 0.0;
+      for (int k = 0; k < K; ++k) se += exp((double)l[k] - mx);
+      p[tid] = 1.0 / (1.0 + exp(-(mx + log(se))));
+      am[tid] = row_argmax(l, K);
+    }
+    __syncthreads();
+    const int m = min(SS_THREADS, n - r0);
+    if (tid < SS_W)
+      for (int k = 0; k < m; ++k) s += d.feat[(size_t)(r0 + k) * d.ldf + tid];
+    else if (tid == SS_W)
+      for (int k = 0; k < m; ++k) {
+        sc += p[k];
+        if (d.counts) d.counts[am[k]] += 1;
+      }
+    __syncthreads();
+  }
+  if (tid < SS_W) d.s1[tid] = s;
+  else if (tid == SS_W) *d.score = sc;
+}
+
 // Means over the epoch's batches (mr_gan.py:215-217) -> epoch_stats[f][0..3]; [4] = batch-wise test error.
 __global__ void k_epoch_reduce(const float* __restrict__ step_stats, const EvalDesc* __restrict__ evals,
                                float* __restrict__ epoch_stats, int nf, int nb, int with_eval) {

@@ -39,9 +39,15 @@ enum Op {
   // device descriptors live in a workspace made on first use (SalWork), outside the arena's [NUM_OPS][nf] table.
   OP_EX2 = NUM_OPS, OP_EX3, OP_EX4, OP_EX5, OP_EX6,   // OP_EXl: dZ[l] -> dZ[l-1], written over eh[l-1]
   OP_EX1,                                            // dZ[1] -> d/dx, fp32 into ex_stage
+  // samples of the generator (mrgan_generate / mrgan_sample_stats), over up to NG = batch * floor(NE / batch) rows per fold;
+  // device descriptors in the workspace GenWork.  OP_GGl: twins of OP_G1, OP_G2, OP_G3G (no noise: OP_GG3 writes the clean rows
+  // and their operand copy into ex_stage); OP_Sl: D's eval forward over those staged rows (twins of OP_E1S, OP_E2 .. OP_E6)
+  OP_GG1, OP_GG2, OP_GG3,
+  OP_S1, OP_S2, OP_S3, OP_S4, OP_S5, OP_S6,
   NUM_OPS_ALL
 };
-constexpr int NUM_EX = NUM_OPS_ALL - NUM_OPS;
+constexpr int NUM_EX = OP_GG1 - NUM_OPS;
+constexpr int NUM_GEN = NUM_OPS_ALL - OP_GG1;
 
 struct OpInfo { bool at = false, bt = false, used = false; int maxM = 0, maxN = 0; };
 
@@ -93,7 +99,7 @@ struct FoldBuffers {
 struct mrgan_handle;
 namespace {
 int tc_setup(mrgan_handle* h);
-int tc_ex_setup(mrgan_handle* h, TcOp* dst);
+int tc_views(mrgan_handle* h, int op0, int op1, TcOp* dst);
 void tc_teardown(mrgan_handle* h);
 void tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st, const OperandMode& om);
 void tc_launch_dw_adam(mrgan_handle* h, int op, int nlayers, int f0, int nfl, cudaStream_t st);
@@ -131,6 +137,23 @@ struct mrgan_handle {
     float* profile = nullptr;         // [nf][K][D_max]
     TcOp* tcops = nullptr;            // [NUM_EX][nf] their tcgen05 views (tf32 / f16 handles)
   } sal;
+  // mrgan_generate / mrgan_sample_stats: the same pattern.  The generator's activations live here, the operand buffers (z, u,
+  // h2) first, covered by the workspace's own fp16 shadow (f16 handles) and OperandMode; the eval buffers stay untouched
+  // except ex_stage / eh / elg, whose contents are dead between calls.
+  struct GenWork {
+    char* mem = nullptr; __half* hmem = nullptr;
+    OperandMode om = {0, 1.0f, nullptr, nullptr};   // fbase = mem, hbase = hmem
+    size_t hfloats = 0;               // floats of mem with an fp16 copy
+    int NG = 0, nseg = 0, ldz = 0;    // rows per chunk (whole batches), batch segments per chunk, pitch of z
+    size_t zstride = 0;               // floats between the z buffers of consecutive folds
+    float* z = nullptr;               // [nf][NG][ldz]
+    float* zs = nullptr;              // [NG][noise_dim]: a chunk of the caller's z (mrgan_generate)
+    GemmDesc* descs = nullptr;        // [NUM_GEN][nf]
+    TcOp* tcops = nullptr;            // [NUM_GEN][nf] (tf32 / f16 handles)
+    BnDesc* bn = nullptr;             // [nf][nseg]: BatchNorm of each batch segment
+    StatsDesc* st = nullptr;          // [2][nf]: generated rows, resident test rows
+    double *s1 = nullptr, *s2 = nullptr, *score = nullptr; int* counts = nullptr;   // [nf][2][SS_W], [nf][2][SS_W^2], [nf][2], [nf][64]
+  } gen;
   AdamRange* d_ranges[2] = {nullptr, nullptr};
   OpInfo ops[NUM_OPS_ALL];
   float *d_step_stats = nullptr, *d_epoch_stats = nullptr, *h_epoch_stats = nullptr;
@@ -364,6 +387,16 @@ GemmDesc make_desc(const float* A, int lda, const float* Bm, int ldb, float* C, 
   return d;
 }
 
+// the host descriptor of op for fold f; rnd: which outputs feed a tensor-core GEMM as operands (tf32 / f16 handles)
+void set_op(mrgan_handle* h, int op, int f, GemmDesc d, bool at, bool bt, int rnd) {
+  d.rnd = h->cfg.precision != MRGAN_PREC_FP32 ? rnd : 0;
+  h->h_descs[(size_t)op * h->nf + f] = d;
+  OpInfo& oi = h->ops[op];
+  oi.at = at; oi.bt = bt; oi.used = true;
+  if (d.M > oi.maxM) oi.maxM = d.M;
+  if (d.N > oi.maxN) oi.maxN = d.N;
+}
+
 int build_descs(mrgan_handle* h) {
   const mrgan_config& c = h->cfg;
   const int B = c.batch, R = h->R, K = c.n_classes, nd = c.noise_dim, nf = h->nf;
@@ -372,15 +405,7 @@ int build_descs(mrgan_handle* h) {
   h->h_folds.assign(nf, FoldState{});
   std::vector<BnDesc> bn(nf); std::vector<LossDesc> ls(nf); std::vector<EvalDesc> ev(nf), evs(nf);
   std::vector<AdamRange> rg0(nf), rg1(nf);
-  const bool tensor = c.precision != MRGAN_PREC_FP32;      // tf32 / f16: which outputs feed a tensor-core GEMM as operands
-  auto setop = [&](int op, int f, GemmDesc d, bool at, bool bt, int rnd = 0) {
-    d.rnd = tensor ? rnd : 0;
-    h->h_descs[(size_t)op * nf + f] = d;
-    OpInfo& oi = h->ops[op];
-    oi.at = at; oi.bt = bt; oi.used = true;
-    if (d.M > oi.maxM) oi.maxM = d.M;
-    if (d.N > oi.maxN) oi.maxN = d.N;
-  };
+  auto setop = [&](int op, int f, GemmDesc d, bool at, bool bt, int rnd = 0) { set_op(h, op, f, d, at, bt, rnd); };
   for (int f = 0; f < nf; ++f) {
     FoldBuffers& b = h->fb[f];
     const int D = h->shapes[f].D;
@@ -408,6 +433,7 @@ int build_descs(mrgan_handle* h) {
                              win[l - 1] + 1, EPI_FWD, l <= 5 ? hact : ACT_NONE, f);
       setop(l == 1 ? OP_E1 : OP_E2 + l - 2, f, e, false, false, l <= 5 ? 1 : 0);
       if (l == 1) { e.A = b.ex_stage; setop(OP_E1S, f, e, false, false, 1); }
+      if (gan) { e.M = B * (h->NE / B); setop(OP_S1 + l - 1, f, e, false, false, l <= 5 ? 1 : 0); }   // generated rows (GenWork)
       // dW (+db): grad(Waug_l) = a[l-1]^T @ dZ[l]
       const float* dZ = (l <= 5) ? b.dz[l] : b.dlg;
       const int lddz = (l <= 5) ? b.ldz[l] : pitch8(K);
@@ -688,13 +714,21 @@ int split_chunks(int rows) {
 }
 
 // ------------------------------------------------------------------ launch sequences
-void launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st = nullptr) {
+// the device descriptors [nf] of op: in the arena's table, or in the workspace of its entry points
+const GemmDesc* op_descs(const mrgan_handle* h, int op) {
+  if (op < NUM_OPS) return h->d_descs + (size_t)op * h->nf;
+  if (op < OP_GG1) return h->sal.descs + (size_t)(op - NUM_OPS) * h->nf;
+  return h->gen.descs + (size_t)(op - OP_GG1) * h->nf;
+}
+
+// om: where the epilogue's operand copies go (null: the arena's, h->om)
+void launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override, cudaStream_t st = nullptr, const OperandMode* om = nullptr) {
   if (!st) st = h->stream;
-  if (h->cfg.precision != MRGAN_PREC_FP32) { tc_launch_gemm(h, op, f0, nfl, rows_override, st, h->om); return; }
+  if (h->cfg.precision != MRGAN_PREC_FP32) { tc_launch_gemm(h, op, f0, nfl, rows_override, st, om ? *om : h->om); return; }
   const OpInfo& oi = h->ops[op];
   int M = oi.maxM;
   if (rows_override > 0 && !oi.at) M = rows_override;
-  const GemmDesc* d = (op < NUM_OPS ? h->d_descs + (size_t)op * h->nf : h->sal.descs + (size_t)(op - NUM_OPS) * h->nf) + f0;
+  const GemmDesc* d = op_descs(h, op) + f0;
   dim3 grid((oi.maxN + 63) / 64, (M + 63) / 64, nfl);
   if (!oi.at && !oi.bt) launch_k(h, k_gemm_simt<false, false>, grid, dim3(256), 0, st, d, (const FoldState*)h->d_folds, rows_override, h->hp);
   else if (!oi.at && oi.bt) launch_k(h, k_gemm_simt<false, true>, grid, dim3(256), 0, st, d, (const FoldState*)h->d_folds, rows_override, h->hp);
@@ -936,10 +970,135 @@ int saliency_setup(mrgan_handle* h) {
   int rc = MRGAN_OK;
   if (cudaMemcpy(S.descs, h->h_descs.data() + (size_t)NUM_OPS * nf, (size_t)NUM_EX * nf * sizeof(GemmDesc), cudaMemcpyHostToDevice) != cudaSuccess)
     rc = fail(h, MRGAN_ERR_CUDA, "saliency workspace: descriptor upload failed");
-  if (rc == MRGAN_OK && tc) rc = tc_ex_setup(h, S.tcops);
+  if (rc == MRGAN_OK && tc) rc = tc_views(h, NUM_OPS, OP_GG1, S.tcops);
   if (rc != MRGAN_OK) { cudaFree(mem); return rc; }
   S.mem = mem;
   return MRGAN_OK;
+}
+
+void gen_free(mrgan_handle* h) {
+  mrgan_handle::GenWork& G = h->gen;
+  if (G.mem) cudaFree(G.mem);
+  if (G.hmem) cudaFree(G.hmem);
+  G = mrgan_handle::GenWork();
+}
+
+// The workspace of the sample entry points, on first use: the generator's activations of NG rows per fold, the descriptors of
+// OP_GG* (built here: they point into the workspace) and OP_S* (built with the handle), the BatchNorm segments, the statistics
+// descriptors and accumulators.  Ones columns: z's is written with every draw (k_gen_z), u's and h2's once here.
+int gen_setup(mrgan_handle* h) {
+  mrgan_handle::GenWork& G = h->gen;
+  if (G.mem) return MRGAN_OK;
+  const mrgan_config& c = h->cfg;
+  const int nf = h->nf, B = c.batch, nd = c.noise_dim, NG = B * (h->NE / B), NS = NG / B;
+  const int ldz = pitch8(nd + 1), ldg = pitch8(kGH), ldu = pitch8(kGH + 1);
+  const bool tc = c.precision != MRGAN_PREC_FP32;
+  std::vector<float*> u(nf), h2(nf), h1(nf), xh(nf), is(nf), xo(nf);
+  size_t hfloats = 0;
+  auto layout = [&](Arena& ar) {
+    G.z = ar.take<float>((size_t)nf * NG * ldz);          // operands first: the fp16 shadow covers [0, hfloats)
+    for (int f = 0; f < nf; ++f) { u[f] = ar.take<float>((size_t)NG * ldu); h2[f] = ar.take<float>((size_t)NG * ldu); }
+    hfloats = (ar.off + 255) / 256 * 256 / sizeof(float);
+    G.zs = ar.take<float>((size_t)NG * nd);
+    for (int f = 0; f < nf; ++f) {
+      h1[f] = ar.take<float>((size_t)NG * ldg); xh[f] = ar.take<float>((size_t)NG * ldg);
+      is[f] = ar.take<float>((size_t)NS * ldg); xo[f] = ar.take<float>((size_t)NG * pitch8(h->shapes[f].D));
+    }
+    G.descs = ar.take<GemmDesc>((size_t)NUM_GEN * nf);
+    G.tcops = tc ? ar.take<TcOp>((size_t)NUM_GEN * nf) : nullptr;
+    G.bn = ar.take<BnDesc>((size_t)nf * NS);
+    G.st = ar.take<StatsDesc>((size_t)2 * nf);
+    G.s1 = ar.take<double>((size_t)nf * 2 * SS_W);
+    G.s2 = ar.take<double>((size_t)nf * 2 * SS_W * SS_W);
+    G.score = ar.take<double>((size_t)nf * 2);
+    G.counts = ar.take<int>((size_t)nf * 64);
+  };
+  Arena sizing;
+  layout(sizing);
+  char* mem = nullptr;
+  CK(cudaMalloc(&mem, sizing.off + 256));
+  G.mem = mem;                  // from here on gen_free releases everything on a failed return
+  Arena real; real.base = mem;
+  layout(real);
+  G.om = h->om; G.om.fbase = reinterpret_cast<const float*>(mem); G.om.hbase = nullptr;
+  G.hfloats = hfloats; G.NG = NG; G.nseg = NS; G.ldz = ldz; G.zstride = (size_t)NG * ldz;
+  auto bail = [&](int rc) { gen_free(h); return rc; };
+  if (cudaMemset(mem, 0, sizing.off + 256) != cudaSuccess) return bail(fail(h, MRGAN_ERR_CUDA, "sample workspace: cudaMemset failed"));
+  if (h->om.mode == 2) {        // pad columns of the copies are zero like those of the fp32 buffers
+    if (cudaMalloc(&G.hmem, hfloats * sizeof(__half)) != cudaSuccess || cudaMemset(G.hmem, 0, hfloats * sizeof(__half)) != cudaSuccess)
+      return bail(fail(h, MRGAN_ERR_CUDA, "sample workspace: fp16 shadow allocation failed"));
+    G.om.hbase = G.hmem;
+  }
+  std::vector<BnDesc> bn((size_t)nf * NS);
+  std::vector<StatsDesc> st((size_t)2 * nf);
+  for (int f = 0; f < nf; ++f) {
+    const FoldBuffers& b = h->fb[f];
+    const NetLayout& LG = h->net[1][f];
+    const float* PG = h->P + LG.off;
+    const TensorLayout &W1 = LG.t[0], &Tg = LG.t[1], &Tb = LG.t[2], &W2 = LG.t[3], &W3 = LG.t[4];
+    const int D = h->shapes[f].D;
+    float* z = G.z + (size_t)f * G.zstride;
+    set_op(h, OP_GG1, f, make_desc(z, ldz, PG + W1.off, W1.pitch, h1[f], ldg, NG, kGH, nd + 1, EPI_FWD, ACT_SOFTPLUS, f), false, false, 0);
+    set_op(h, OP_GG2, f, make_desc(u[f], ldu, PG + W2.off, W2.pitch, h2[f], ldu, NG, kGH, kGH + 1, EPI_FWD, ACT_SOFTPLUS, f), false, false, 1);
+    GemmDesc g3 = make_desc(h2[f], ldu, PG + W3.off, W3.pitch, xo[f], pitch8(D), NG, D, kGH + 1, EPI_FWD, ACT_NONE, f);
+    g3.C2 = b.ex_stage; g3.ldc2 = b.lda[0];          // sigma = 0: the clean rows again, as D's first operand
+    set_op(h, OP_GG3, f, g3, false, false, 2);
+    for (int s = 0; s < NS; ++s) {
+      const size_t r = (size_t)s * B;
+      bn[(size_t)f * NS + s] = BnDesc{h1[f] + r * ldg, xh[f] + r * ldg, u[f] + r * ldu, is[f] + (size_t)s * ldg, PG + Tg.off, PG + Tb.off,
+                                      nullptr, nullptr, nullptr, nullptr, ldg, ldu, B, kGH};
+    }
+    for (int side = 0; side < 2; ++side)
+      st[(size_t)side * nf + f] = StatsDesc{b.eh[5], b.elg, b.lda[5], pitch8(c.n_classes), side ? h->shapes[f].n_test : NG,
+                                            G.s1 + ((size_t)f * 2 + side) * SS_W, G.s2 + ((size_t)f * 2 + side) * SS_W * SS_W,
+                                            G.score + (size_t)f * 2 + side, side ? nullptr : G.counts + (size_t)f * 64};
+    launch_k(h, k_set_col, (NG + 127) / 128, 128, 0, h->stream, u[f], ldu, NG, kGH, 1.0f, G.om);
+    launch_k(h, k_set_col, (NG + 127) / 128, 128, 0, h->stream, h2[f], ldu, NG, kGH, 1.0f, G.om);
+  }
+  if (cudaMemcpy(G.descs, h->h_descs.data() + (size_t)OP_GG1 * nf, (size_t)NUM_GEN * nf * sizeof(GemmDesc), cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(G.bn, bn.data(), bn.size() * sizeof(BnDesc), cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(G.st, st.data(), st.size() * sizeof(StatsDesc), cudaMemcpyHostToDevice) != cudaSuccess)
+    return bail(fail(h, MRGAN_ERR_CUDA, "sample workspace: descriptor upload failed"));
+  if (tc) { const int rc = tc_views(h, OP_GG1, NUM_OPS_ALL, G.tcops); if (rc != MRGAN_OK) return bail(rc); }
+  if (cudaStreamSynchronize(h->stream) != cudaSuccess) return bail(fail(h, MRGAN_ERR_CUDA, "sample workspace: ones columns failed"));
+  const int sk = take_sticky(h);
+  return sk != MRGAN_OK ? bail(sk) : MRGAN_OK;
+}
+
+// G's forward over rows [r0, r0 + c) of a request (c: whole batches, at most NG) for folds [f0, f0 + nfl): z (drawn, or with
+// staged the caller's rows in zs, one fold), OP_GG1, BatchNorm with the statistics of each batch of the chunk (mr_gan.py:112
+// in training phase: the only way G ever ran), OP_GG2, OP_GG3 -> the clean rows and their operand copy in ex_stage.
+void enqueue_generate(mrgan_handle* h, int f0, int nfl, int r0, int c, uint32_t seed, bool staged) {
+  const mrgan_handle::GenWork& G = h->gen;
+  const int nd = h->cfg.noise_dim, B = h->cfg.batch, ns = c / B;
+  launch_k(h, k_gen_z, dim3((nd + 128) / 128, ((r0 + c - 1) >> 2) - (r0 >> 2) + 1, nfl), 128, 0, h->stream, (const FoldState*)h->d_folds, f0,
+           G.z + (size_t)f0 * G.zstride, G.zstride, G.ldz, staged ? (const float*)G.zs : nullptr, r0, c, nd, seed, G.om);
+  launch_gemm(h, OP_GG1, f0, nfl, c, nullptr, &G.om);
+  // one BnDesc per (fold, segment): a chunk of whole segments is one launch; a short chunk of several folds one per fold
+  const dim3 bgx((kGH + BN_COLS - 1) / BN_COLS), bnt(B > 256 ? 1024 : 256);
+  if (ns == G.nseg || nfl == 1)
+    launch_k(h, k_bn_fwd, dim3(bgx.x, 1, nfl * ns), bnt, 0, h->stream, (const BnDesc*)(G.bn + (size_t)f0 * G.nseg), h->cfg.bn_eps, G.om);
+  else
+    for (int f = f0; f < f0 + nfl; ++f)
+      launch_k(h, k_bn_fwd, dim3(bgx.x, 1, ns), bnt, 0, h->stream, (const BnDesc*)(G.bn + (size_t)f * G.nseg), h->cfg.bn_eps, G.om);
+  launch_gemm(h, OP_GG2, f0, nfl, c, nullptr, &G.om);
+  launch_gemm(h, OP_GG3, f0, nfl, c);
+}
+
+// mrgan_sample_stats's pass over every fold: n generated rows in chunks of NG (z from seed), each through D's eval forward
+// (OP_S*) and into the accumulators, then the resident test rows (OP_E*).  Needs gen_setup.
+void enqueue_sample_stats(mrgan_handle* h, int n, uint32_t seed) {
+  const mrgan_handle::GenWork& G = h->gen;
+  const int nf = h->nf, K = h->cfg.n_classes;
+  cudaMemsetAsync(G.s1, 0, (size_t)(reinterpret_cast<char*>(G.counts + (size_t)nf * 64) - reinterpret_cast<char*>(G.s1)), h->stream);
+  for (int r0 = 0; r0 < n; r0 += G.NG) {
+    const int c = std::min(G.NG, n - r0);
+    enqueue_generate(h, 0, nf, r0, c, seed, false);
+    for (int l = 0; l < 6; ++l) launch_gemm(h, OP_S1 + l, 0, nf, c);
+    launch_k(h, k_sample_stats, dim3(SS_TILES + 1, nf), SS_THREADS, 0, h->stream, (const StatsDesc*)G.st, c, K);
+  }
+  for (int l = 0; l < 6; ++l) launch_gemm(h, l == 0 ? OP_E1 : OP_E2 + l - 1, 0, nf, 0);
+  launch_k(h, k_sample_stats, dim3(SS_TILES + 1, nf), SS_THREADS, 0, h->stream, (const StatsDesc*)(G.st + nf), 0, K);
 }
 
 int finish_pending(mrgan_handle* h) {
@@ -1362,6 +1521,13 @@ int tc_plan_op(mrgan_handle* h, int op) {
   return MRGAN_OK;
 }
 
+// f16 handles: the fp16 copy of an operand buffer, in the arena's shadow or in the generator workspace's own
+const __half* half_copy(const mrgan_handle* h, const float* p) {
+  const mrgan_handle::GenWork& G = h->gen;
+  if (G.mem && p >= G.om.fbase && p < G.om.fbase + G.hfloats) return G.hmem + (p - G.om.fbase);
+  return h->harena + (p - h->om.fbase);
+}
+
 // the launch plan of op and the tcgen05 views of its descriptors, one per fold (ts[0 .. nf)); no-op for an unused op
 int tc_make_op(mrgan_handle* h, EncodeTiledFn fn, int op, TcOp* ts) {
   TRY(tc_plan_op(h, op));
@@ -1373,8 +1539,8 @@ int tc_make_op(mrgan_handle* h, EncodeTiledFn fn, int op, TcOp* ts) {
     TcOp& t = ts[f];
     if (h->om.mode == 2) {    // operands come from the fp16 copies (same element offsets and pitches as the fp32 buffers)
       GemmDesc gh = g;
-      gh.A = reinterpret_cast<const float*>(h->harena + (g.A - h->om.fbase));
-      gh.B = reinterpret_cast<const float*>(h->harena + (g.B - h->om.fbase));
+      gh.A = reinterpret_cast<const float*>(half_copy(h, g.A));
+      gh.B = reinterpret_cast<const float*>(half_copy(h, g.B));
       if (!tc_fill_op(fn, t, gh, mode, 2, bn_big)) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled (fp16 operands) failed");
       t.g = g;                // the epilogue keeps addressing the fp32 buffers (and derives the copies' addresses itself)
     } else if (!tc_fill_op(fn, t, g, mode, 4, bn_big)) return fail(nullptr, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled failed");
@@ -1479,14 +1645,15 @@ int tc_setup(mrgan_handle* h) {
   return MRGAN_OK;
 }
 
-// the tcgen05 views of the eval-backward ops (OP_EX*), made on the first mrgan_input_grad / mrgan_saliency -> dst [NUM_EX][nf]
-int tc_ex_setup(mrgan_handle* h, TcOp* dst) {
+// the tcgen05 views of the ops [op0, op1) of a workspace, made on its first use -> dst [op1 - op0][nf]: the eval-backward ops
+// (OP_EX*: mrgan_input_grad / mrgan_saliency) or the sample ops (OP_GG*, OP_S*: mrgan_generate / mrgan_sample_stats)
+int tc_views(mrgan_handle* h, int op0, int op1, TcOp* dst) {
   EncodeTiledFn fn = tc_encoder();
   if (!fn) return fail(h, MRGAN_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
-  std::vector<TcOp> ops((size_t)NUM_EX * h->nf);
+  std::vector<TcOp> ops((size_t)(op1 - op0) * h->nf);
   memset(ops.data(), 0, ops.size() * sizeof(TcOp));
-  for (int op = NUM_OPS; op < NUM_OPS_ALL; ++op) {
-    const int rc = tc_make_op(h, fn, op, &ops[(size_t)(op - NUM_OPS) * h->nf]);
+  for (int op = op0; op < op1; ++op) {
+    const int rc = tc_make_op(h, fn, op, &ops[(size_t)(op - op0) * h->nf]);
     if (rc != MRGAN_OK) return rc;
   }
   CK(cudaMemcpy(dst, ops.data(), ops.size() * sizeof(TcOp), cudaMemcpyHostToDevice));
@@ -1526,7 +1693,8 @@ void tc_launch_gemm(mrgan_handle* h, int op, int f0, int nfl, int rows_override,
   const bool at = h->ops[op].at;
   const int NE = rows_override > 0 && !at ? rows_override : p.maxNE;
   const dim3 grid(p.gx, (NE + p.bn - 1) / p.bn, nfl * p.ks);
-  const TcOp* d = (op < NUM_OPS ? h->d_tcops + (size_t)op * h->nf : h->sal.tcops + (size_t)(op - NUM_OPS) * h->nf) + f0;
+  const TcOp* d = (op < NUM_OPS ? h->d_tcops + (size_t)op * h->nf
+                   : op < OP_GG1 ? h->sal.tcops + (size_t)(op - NUM_OPS) * h->nf : h->gen.tcops + (size_t)(op - OP_GG1) * h->nf) + f0;
   // dW kernels take the number of contraction slices in place of rows_override
   launch_k(h, p.k->fn, grid, p.k->threads, p.smem, st, d, h->d_folds, at ? p.ks : rows_override, h->hp, om);
   if (p.ks > 1) {
@@ -1712,6 +1880,7 @@ int mrgan_destroy(mrgan_handle* h) {
   if (h->d_dpmem) cudaFree(h->d_dpmem);
   if (h->d_dpbufs) cudaFree(h->d_dpbufs);
   if (h->sal.mem) cudaFree(h->sal.mem);
+  gen_free(h);
   tc_teardown(h);
   if (h->svm.mem) cudaFree(h->svm.mem);
   if (h->svm.cv_mem) cudaFree(h->svm.cv_mem);
@@ -2152,12 +2321,15 @@ int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
   if (!ms_avg || reps < 1) return fail(h, MRGAN_ERR_ARG, "time_op: bad argument");
   const bool svm = h->cfg.model == MRGAN_MODEL_SVM, gan = h->cfg.model == MRGAN_MODEL_GAN;
   if (svm != (which >= MRGAN_TIME_SVM_KMAT && which <= MRGAN_TIME_SVM_PREDICT))
-    return fail(h, which < 0 || which > MRGAN_TIME_SALIENCY ? MRGAN_ERR_ARG : MRGAN_ERR_STATE, "time_op: op does not exist for this model");
-  if (which < 0 || which > MRGAN_TIME_SALIENCY) return fail(h, MRGAN_ERR_ARG, "time_op: unknown op");
-  if (!gan && (which == MRGAN_TIME_ADAM_G || which == MRGAN_TIME_GEN_STEP || which == MRGAN_TIME_DX1)) return fail(h, MRGAN_ERR_STATE, "time_op: no generator in this model");
-  TRY(ready(h, "time_op", svm ? FITTED : (LOADED | (which == MRGAN_TIME_SALIENCY ? LOCAL : 0u))));
+    return fail(h, which < 0 || which > MRGAN_TIME_SAMPLE_STATS ? MRGAN_ERR_ARG : MRGAN_ERR_STATE, "time_op: op does not exist for this model");
+  if (which < 0 || which > MRGAN_TIME_SAMPLE_STATS) return fail(h, MRGAN_ERR_ARG, "time_op: unknown op");
+  if (!gan && (which == MRGAN_TIME_ADAM_G || which == MRGAN_TIME_GEN_STEP || which == MRGAN_TIME_DX1 || which == MRGAN_TIME_SAMPLE_STATS))
+    return fail(h, MRGAN_ERR_STATE, "time_op: no generator in this model");
+  const bool ro = which == MRGAN_TIME_SALIENCY || which == MRGAN_TIME_SAMPLE_STATS;
+  TRY(ready(h, "time_op", svm ? FITTED : (LOADED | (ro ? LOCAL : 0u))));
   if (svm) return time_reps(h, reps, [&]() { svm_launch(h, which); }, ms_avg);
   if (which == MRGAN_TIME_SALIENCY) TRY(saliency_setup(h));
+  if (which == MRGAN_TIME_SAMPLE_STATS) TRY(gen_setup(h));
   return time_reps(h, reps, [&]() {
     switch (which) {
       case MRGAN_TIME_ADAM_D: launch_adam(h, 0, h->nf, 0); break;
@@ -2168,6 +2340,7 @@ int mrgan_time_op(mrgan_handle* h, int which, int reps, float* ms_avg) {
       case MRGAN_TIME_GEN_STEP: enqueue_gen_step(h, 0, h->nf, 0, 0); break;
       case MRGAN_TIME_DX1: launch_gemm(h, OP_DX1G, 0, h->nf, 0); break;
       case MRGAN_TIME_SALIENCY: enqueue_saliency(h); break;
+      case MRGAN_TIME_SAMPLE_STATS: enqueue_sample_stats(h, h->gen.NG, 0); break;
       default: break;
     }
   }, ms_avg);
@@ -2829,6 +3002,61 @@ int mrgan_saliency(mrgan_handle* h, float* profile) {
   CK(cudaMemcpyAsync(profile, h->sal.profile, (size_t)h->nf * h->cfg.n_classes * max_D(h, 0, h->nf) * sizeof(float), cudaMemcpyDeviceToHost,
                      h->stream));
   return complete(h);
+}
+
+// ------------------------------------------------------------------ samples of the generator (include/mrgan.h)
+int mrgan_generate(mrgan_handle* h, int fold, int n, uint32_t seed, const float* z, float* x) {
+  TRY(enter(h, "generate", FOLD | GAN, fold));
+  if (!x) return fail(h, MRGAN_ERR_ARG, "generate: null pointer");
+  if (n < 1 || n % h->cfg.batch) return fail(h, MRGAN_ERR_ARG, "generate: n must be a positive multiple of batch");
+  TRY(ready(h, "generate", FOLD | GAN | LOCAL, fold));
+  TRY(gen_setup(h));
+  const mrgan_handle::GenWork& G = h->gen;
+  const int D = h->shapes[fold].D, nd = h->cfg.noise_dim;
+  const GemmDesc& g3 = h->h_descs[(size_t)OP_GG3 * h->nf + fold];     // C: the clean rows
+  for (int r0 = 0; r0 < n; r0 += G.NG) {
+    const int c = std::min(G.NG, n - r0);
+    if (z) CK(cudaMemcpyAsync(G.zs, z + (size_t)r0 * nd, (size_t)c * nd * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    enqueue_generate(h, fold, 1, r0, c, seed, z != nullptr);
+    CK(cudaMemcpy2DAsync(x + (size_t)r0 * D, (size_t)D * sizeof(float), g3.C, (size_t)g3.ldc * sizeof(float), (size_t)D * sizeof(float), c,
+                         cudaMemcpyDeviceToHost, h->stream));
+  }
+  return complete(h);
+}
+
+int mrgan_sample_stats(mrgan_handle* h, int n, uint32_t seed, int32_t* counts, double* score, double* mean, double* cov) {
+  TRY(enter(h, "sample_stats", GAN));
+  if (!counts || !score || !mean || !cov) return fail(h, MRGAN_ERR_ARG, "sample_stats: null pointer");
+  if (n < 1 || n % h->cfg.batch) return fail(h, MRGAN_ERR_ARG, "sample_stats: n must be a positive multiple of batch");
+  TRY(ready(h, "sample_stats", GAN | LOCAL | LOADED));
+  TRY(gen_setup(h));
+  const mrgan_handle::GenWork& G = h->gen;
+  const int nf = h->nf, K = h->cfg.n_classes, W = SS_W;
+  enqueue_sample_stats(h, n, seed);
+  std::vector<double> s1((size_t)nf * 2 * W), s2((size_t)nf * 2 * W * W), sc((size_t)nf * 2);
+  std::vector<int> cnt((size_t)nf * 64);
+  CK(cudaMemcpyAsync(s1.data(), G.s1, s1.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(s2.data(), G.s2, s2.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(sc.data(), G.score, sc.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(cnt.data(), G.counts, cnt.size() * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  TRY(complete(h));
+  // raw sums -> moments: mean = s1 / m, cov = (s2 - m mean mean^T) / (m - 1) (np.cov), s2 mirrored from its upper triangle
+  for (int f = 0; f < nf; ++f) {
+    for (int k = 0; k < K; ++k) counts[(size_t)f * K + k] = cnt[(size_t)f * 64 + k];
+    for (int side = 0; side < 2; ++side) {
+      const double m = side ? h->shapes[f].n_test : n;
+      const size_t fs = (size_t)f * 2 + side;
+      const double* a = s1.data() + fs * W;
+      const double* q = s2.data() + fs * W * W;
+      double* mu = mean + fs * W;
+      double* cv = cov + fs * W * W;
+      score[fs] = sc[fs] / m;
+      for (int i = 0; i < W; ++i) mu[i] = a[i] / m;
+      for (int i = 0; i < W; ++i)
+        for (int j = i; j < W; ++j) cv[(size_t)i * W + j] = cv[(size_t)j * W + i] = (q[(size_t)i * W + j] - m * mu[i] * mu[j]) / (m - 1.0);
+    }
+  }
+  return MRGAN_OK;
 }
 
 int64_t mrgan_kernel_launches(const mrgan_handle* h) { return h ? h->launches : -1; }

@@ -16,6 +16,8 @@ from .model import disc_shapes, gen_shapes
 
 MODEL = {"gan": 0, "nn": 1, "svm": 2}
 PRECISION = {"fp32": 0, "tf32": 1, "f16": 2}      # f16 (the trainers' and CLIs' default): fp16 operand copies, fp32 master weights / accumulation
+TID_GEN = 6          # Philox tensor id of the z that generate / sample_stats draw (csrc/common.cuh MRGAN_TID_GEN)
+MID_WIDTH = 250      # D's layer-5 width: the features sample_stats describes (mr_gan.py:127)
 
 
 class MrganError(RuntimeError):
@@ -483,6 +485,55 @@ class FoldGroup:
         self._chk(self.lib.mrgan_saliency(self._h, _lib.fptr(out)))
         return [out[f, :, :D].copy() for f, (D, _, _, _) in enumerate(self.shapes)]
 
+    # ------------------------------------------------------------------ samples of the generator (GAN)
+    def generate(self, fold, n, seed=0, z=None):
+        """n rows of the fold's generator G(z), float32 [n, D], in the fold's SCALED input space (without D's input noise).
+        G runs as it ran in training: BatchNorm with the statistics of each batch of ``batch`` rows, so n must be a multiple
+        of ``batch``.  z: [n, noise_dim], or None = N(0,1) drawn on the device from (fold key, seed, stream TID_GEN); the
+        library works through the rows in chunks of whole batches, and the draw does not depend on them."""
+        D = self.shapes[fold][0]
+        n = int(n)
+        if n < 1 or n % self.batch:
+            raise ValueError("generate: n must be a positive multiple of batch (%d)" % self.batch)
+        if z is not None:
+            z = _f32(z)
+            if z.shape != (n, self.noise_dim):
+                raise ValueError("generate: z must be [%d, %d]" % (n, self.noise_dim))
+        x = np.empty((n, D), dtype=np.float32)
+        self._chk(self.lib.mrgan_generate(self._h, int(fold), n, int(seed) & 0xFFFFFFFF, None if z is None else _lib.fptr(z),
+                                          _lib.fptr(x)))
+        return x
+
+    def sample_stats(self, n=None, seed=0):
+        """D's view of n generated rows (z drawn from seed) and of the resident test rows of every fold: a list of dicts
+        ``{'n', 'counts': int32 [K] (D's predicted classes of the generated rows), 'score': float64 [2] (mean sigma(logsumexp of
+        the logits)), 'mean': float64 [2, 250], 'cov': float64 [2, 250, 250]}`` ([0] generated, [1] real) of D's layer-5
+        phase-0 features; cov is unbiased (np.cov).  n: a multiple of batch, or None = each fold's n_test rounded up to a
+        multiple of batch (one library pass per distinct value), so that a fold's result does not depend on its group.
+        Bitwise reproducible, independent of the fold grouping; leaves every later result of the group unchanged."""
+        if n is not None:
+            n = int(n)
+            if n < 1 or n % self.batch:
+                raise ValueError("sample_stats: n must be a positive multiple of batch (%d)" % self.batch)
+            return self._sample_stats(n, seed)
+        per = [-(-nte // self.batch) * self.batch for _, _, nte, _ in self.shapes]
+        out = [None] * self.n_folds
+        for m in sorted(set(per)):
+            for f, r in enumerate(self._sample_stats(m, seed)):
+                if per[f] == m:
+                    out[f] = r
+        return out
+
+    def _sample_stats(self, n, seed):
+        K, F, W = self.cfg.n_classes, self.n_folds, MID_WIDTH
+        counts = np.zeros((F, K), dtype=np.int32)
+        score = np.zeros((F, 2))
+        mean = np.zeros((F, 2, W))
+        cov = np.zeros((F, 2, W, W))
+        self._chk(self.lib.mrgan_sample_stats(self._h, n, int(seed) & 0xFFFFFFFF, _lib.iptr(counts), _lib.dptr(score),
+                                              _lib.dptr(mean), _lib.dptr(cov)))
+        return [dict(n=n, counts=counts[f], score=score[f], mean=mean[f], cov=cov[f]) for f in range(F)]
+
     # ------------------------------------------------------------------ utilities
     def fill_normal(self, fold, step, tensor_id, rows, cols, row0=0):
         out = np.empty((rows, cols), dtype=np.float32)
@@ -514,10 +565,11 @@ class FoldGroup:
         return out
 
     TIME_OPS = {"adam_d": 0, "adam_g": 1, "dw1": 2, "fwd1": 3, "disc_step": 4, "gen_step": 5, "dx1": 6,
-                "svm_kmat": 7, "svm_smo": 8, "svm_predict": 9, "saliency": 10}
+                "svm_kmat": 7, "svm_smo": 8, "svm_predict": 9, "saliency": 10, "sample_stats": 11}
 
     def time_op(self, which, reps=20):
-        """Average device ms of one kernel (or one whole step) over all folds; mutates training state (but 'saliency')."""
+        """Average device ms of one kernel (or one whole step) over all folds; mutates training state (but 'saliency' and
+        'sample_stats')."""
         out = np.zeros(1, dtype=np.float32)
         self._chk(self.lib.mrgan_time_op(self._h, self.TIME_OPS[which], reps, _lib.fptr(out)))
         return float(out[0])

@@ -38,7 +38,7 @@ def dataset(modalities=0, forcetempTime=4, contactmicTime=0.2, leaveObjectOut=Fa
 
 def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16', device=0, batch=50,
                     eval_each_epoch=True, shared_t=True, return_group=False, device_perm=False, details=False, saliency=False,
-                    start_states=None, on_epoch=None):
+                    samples=False, start_states=None, on_epoch=None):
     """Train a GROUP of independent folds side by side on one GPU.
 
     jobs: list of dicts with keys ``trainTestSets`` (or ``X``, ``y``), ``percentlabeled``,
@@ -47,8 +47,9 @@ def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16',
     epoch instead of 3 x int32[n_train] per fold); same distribution, different draws than the host's numpy generator.
     Returns the list of test errors (mr_gan.py:230,234), one per job; details=True: one dict per job instead,
     ``{'error': <the same float>, 'confusion': int32 [K, K]}`` (rows = true class, columns = predicted), from one extra
-    forward pass over every fold's test set; saliency=True: those dicts with ``'saliency'``, float32 [K, D] (FoldGroup.saliency).
-    start_states / on_epoch: resume and snapshots (checkpoint.py)."""
+    forward pass over every fold's test set; saliency=True: those dicts with ``'saliency'``, float32 [K, D] (FoldGroup.saliency);
+    samples=True: those dicts with ``'samples'`` (results.sample_report of FoldGroup.sample_stats) and ``'sample_rows'``, one
+    batch of generated rows in raw feature units.  start_states / on_epoch: resume and snapshots (checkpoint.py)."""
     start = checkpoint.start_epoch(start_states, len(jobs))
 
     def init(fg, i, D, rng):
@@ -103,7 +104,8 @@ def train_gan_folds(jobs, epochs=100, verbose=False, *, seed=0, precision='f16',
         for e in errors:
             print('Test error:', e)
         sys.stdout.flush()
-    errors = results.collect(fg, errors, details, saliency)
+    errors = results.collect(fg, errors, details, saliency, samples=samples,
+                             scalers=[checkpoint.job_scaler(j) for j in jobs] if samples else None)
     if return_group:
         return errors, fg
     fg.close()
@@ -130,11 +132,16 @@ def main(argv=None):
     # --group 84 = two modalities of table 1; the GPU saturates at ~74 folds of D=1200
     parser = tables.argument_parser('Semi-supervised learning with GANs for material recognition on haptic data.', group=84)
     parser.add_argument('--host-perm', action='store_true', help='draw the epoch permutations on the host (numpy) instead of on the device')
+    parser.add_argument('--samples', metavar='FILE', default=None,
+                        help="write one batch of every fold-training's generated rows (raw feature units) to one .npz file (rank "
+                             "0) and print the setting's sample statistics (Frechet distance and feature-matching gap of D's "
+                             "layer-5 features, D's real-vs-fake score, predicted class shares) after its average")
     args = parser.parse_args(argv)
 
     def train(jobs, device, seed, rep, **resume):
         return train_gan_folds(jobs, epochs=args.epochs, verbose=args.verbose, seed=seed, precision=args.precision, device=device,
-                               device_perm=not args.host_perm, details=rep.details, saliency=rep.saliency, **resume)
+                               device_perm=not args.host_perm, details=rep.details, saliency=rep.saliency, samples=rep.samples,
+                               **resume)
 
     return tables.run(args, 'mr_gan', train, job_rows, job_cost, ['1', '3', '5', '6'],
                       checkpoint_fields=dict(model='gan', shared_t=True, batch=50, perm='host' if args.host_perm else 'device'))
